@@ -8,7 +8,7 @@ assembly.  `value` is measured with the reads already resident in HBM; `e2e` goe
 public API (gavisunk_b200.engine.Engine) with HOST buffers, host->device copy of the reads and
 device->host read of the results inside the timed region.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload s150|h3100|tiny] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload s150|h3100|tiny] [--impl reference] [--dump-outputs DIR]
 
 N > 1: launched by torchrun, one rank per GPU; every rank owns its own shard of reads of the same
 size (weak scaling), the SUNK table is replicated; NCCL all-reduces the group-hit histogram and
@@ -18,6 +18,9 @@ all-gathers the union-find forests (the only two exchanges on the path, SURVEY.m
 diag_filter_step2, unmodified prebuilt binaries) on the host cores, one process per chunk with all
 cores busy, followed by the CPU port of the Python stages (oracle/gavisunk_oracle.py; the
 reference's scripts need graph_tool / pyranges which are not installed) -- on a bounded sample.
+
+--dump-outputs DIR: after the timed steps of the GPU path (--impl b200), what its last step computed is written to
+DIR as .npy files (dump_outputs), so that two builds of the project can be compared output for output.
 """
 from __future__ import annotations
 
@@ -67,7 +70,15 @@ def parse_args():
     ap.add_argument("--cpu-sample-mbp", type=float, default=None, help="read Mbp per CPU process of the baseline sample")
     ap.add_argument("--ref-asm-mbp", type=float, default=40.0, help="--impl reference: haploid size of the sample assembly (numpy + oracle set-up)")
     ap.add_argument("--e2e-files-gbp", type=float, default=None, help="read Gbp of the files -> files run (default: 4 at N = 1, skipped at N > 1; 0 = skip)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="--impl b200: write what the last timed step computed to DIR/<name>.npy (float64, at most 64 MB; "
+                         "see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the GPU path's results (--impl b200)")
+    return args
 
 
 WORKLOADS = {
@@ -201,6 +212,39 @@ def result_digest(iv, gaps, eng):
     return h.hexdigest()
 
 
+# --dump-outputs: rows kept per array (a fixed, seeded sample of larger results); together at most DUMP_LIMIT bytes
+DUMP_ROWS = dict(intervals=1 << 18, gaps=1 << 18, bad_groups=1 << 18, pairs=1 << 20)
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, sizes, iv, gaps, eng, seed=0):
+    """What the last timed step handed its caller, as DIR/<name>.npy in float64 (every value is an integer below
+    2**53, so the conversion is exact):
+      size_<name>  one result size of the step as run_step reports it (rows, best, kept, bad_groups,
+                   validated_pairs, intervals, gaps, nodata), as an array of one element
+      intervals    validated intervals (contig, start, end)         gaps        gaps between them (contig, start, end)
+      bad_groups   bad SUNK groups (group index), sorted            pairs       this rank's validated pairs (read,
+                                                                                contig, group, gidx) in engine order
+    An array longer than DUMP_ROWS[name] rows is replaced by the rows at a sorted random sample of its indices
+    (numpy default_rng(seed)), written beside it as <name>_index.npy.  The inputs of a run are fixed by its
+    arguments, so two builds can be compared file by file."""
+    os.makedirs(out_dir, exist_ok=True)
+    pairs = eng.pairs()
+    tables = dict(intervals=[iv[c] for c in ("contig", "start", "end")], gaps=[gaps[c] for c in ("contig", "start", "end")],
+                  bad_groups=[np.sort(eng.bad_list())], pairs=[pairs[c] for c in ("read", "contig", "group", "gidx")])
+    out = {f"size_{k}": np.array([v], np.float64) for k, v in sizes.items()}
+    for name, cols in tables.items():
+        n, cap = len(cols[0]), DUMP_ROWS[name]
+        if n > cap:
+            idx = np.sort(np.random.default_rng(seed).choice(n, cap, replace=False))
+            out[name + "_index"] = idx.astype(np.float64)
+            cols = [c[idx] for c in cols]
+        out[name] = np.stack([np.asarray(c, np.float64) for c in cols], axis=1)
+    assert sum(a.nbytes for a in out.values()) <= DUMP_LIMIT
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main_b200(args):
     import torch
     import torch.distributed as dist
@@ -265,6 +309,8 @@ def main_b200(args):
     total_bases = allsum(my_bases)
     value = total_bases * args.steps / (ms_max * 1e-3) / 1e9
     digest = result_digest(iv, gaps, eng)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res, iv, gaps, eng)
 
     # ---- per-stage device times (CUDA events of the library around each stage, on its stream): one extra pass with
     #      the stage times read after every batch / phase-2 stage (reading them waits for the stage, so it is kept out
@@ -1026,13 +1072,10 @@ def main_reference(args):
     _SAMPLE_CACHE["ref"] = prep
     t_setup = time.perf_counter() - t_setup
     vals, last = [], None
-    t_begin = time.perf_counter()
-    for i in range(min(args.warmup, 1) + max(1, args.steps)):
+    for i in range(min(args.warmup, 1) + args.steps):
         last = run_reference_pipeline(prep, cores)
         if i >= min(args.warmup, 1):
             vals.append(last["value"])
-        if time.perf_counter() - t_begin > 150.0 and vals:  # K steps unless that takes more than ~2.5 minutes in total
-            break
     steps = len(vals)
     v = float(np.mean(vals))
     spec = WORKLOADS[args.workload]

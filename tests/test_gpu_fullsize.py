@@ -1,10 +1,9 @@
 """BASELINE.json config 3 at FULL size (150 Mbp x2 diploid assembly, 30x ONT-like reads, k=20: 5.9 M SUNKs,
 124 k reads / 4.45 Gbp, 2.9 M sunkpos rows) -- too large for the pure-Python oracle, so parity is checked
-through (i) the reference's own executables on a sample of the reads against the FULL database,
-(ii) size-independent properties the reference's algorithm guarantees, (iii) invariance under the
-engine's own batching choices (chunk split, host copy pipeline), (iv) idempotence."""
-import os
-import subprocess
+through (i) the reference's match / diag lines for a sample of the reads against the FULL database (stored in
+tests/golden/fullsize_sample.json.gz), (ii) size-independent properties the reference's algorithm guarantees,
+(iii) invariance under the engine's own batching choices (chunk split, host copy pipeline), (iv) idempotence."""
+import hashlib
 
 import numpy as np
 import pytest
@@ -12,11 +11,13 @@ import pytest
 pytestmark = pytest.mark.gpu
 
 K = 20
+# the sample of the reference comparison: the first SAMPLE_READS reads of one chunk file per haplotype
+SAMPLE_CHUNKS = ((0, 3), (1, 14))  # (haplotype, chunk)
+SAMPLE_READS = 40
 
 
-@pytest.fixture(scope="module")
-def full():
-    import torch
+def build_full():
+    """config 3 on cuda:0, run once through the fused path; returns (engine, workload, results)"""
     from gavisunk_b200 import workload as W
     from gavisunk_b200.engine import Engine
     eng = Engine(K)
@@ -28,6 +29,58 @@ def full():
     gaps, nodata = eng.gaps(wl.contig_len.astype(np.uint32))
     res = dict(rows=eng.rows(0), kept=eng.rows(1), best=eng.best(), pairs=eng.pairs(), bad=eng.bad_list(), iv=iv, gaps=gaps,
                nodata=nodata, off=wl.read_off.cpu().numpy().astype(np.int64))
+    return eng, wl, res
+
+
+def sample_texts(wl, res, r0, r1):
+    """{hap}.sunkpos, {hap}_diag.sunkpos and {hap}_diag2.sunkpos lines of reads [r0, r1) as the reference's
+    kmerpos_annot3 / diag_filter_v3 / diag_filter_step2 write them (reads named r%09d by their index)"""
+    names = wl.contig_names
+    fmt = lambda rows: "".join(
+        f"r{rd:09d}\t{p}\t{names[c]}\t{s}\t{g}\n"
+        for rd, p, c, s, g in zip(rows["read"].tolist(), rows["pos"].tolist(), rows["contig"].tolist(), rows["start"].tolist(),
+                                  rows["group"].tolist()) if r0 <= rd < r1)
+    b = res["best"]
+    sel = (b["read"] >= r0) & (b["read"] < r1)
+    diag = "".join(f"r{rd:09d}\t{names[c]}\t{g}\t{'+' if d else '-'}\t{g}\n"
+                   for rd, c, g, d in zip(b["read"][sel].tolist(), b["contig"][sel].tolist(), b["ngood"][sel].tolist(), b["dir"][sel].tolist()))
+    return dict(sunkpos=fmt(res["rows"]), diag=diag, diag2=fmt(res["kept"]))
+
+
+def sample_reads(wl, res, r0, r1):
+    """[(name, bases)] of reads [r0, r1), named r%09d by their index"""
+    off = res["off"]
+    seq = wl.reads[int(off[r0]):int(off[r1])].cpu().numpy()
+    return [("r%09d" % i, seq[off[i] - off[r0]:off[i + 1] - off[r0]].tobytes()) for i in range(r0, r1)]
+
+
+def bases_sha256(reads):
+    return hashlib.sha256(b"".join(s for _, s in reads)).hexdigest()
+
+
+def sample_loc(wl, db, reads):
+    """indices of the exported database rows that a window of the reads hits, and their kmer.loc lines"""
+    import gavisunk_oracle as O
+    from gavisunk_b200 import cli
+    order = np.argsort(db["kmer"], kind="stable")
+    keys = db["kmer"][order]
+    assert np.all(keys[1:] != keys[:-1]), "a SUNK is one row of the database"
+    hits = []
+    for _, s in reads:
+        canon = O.canonical_windows(O.codes_of(s), K)
+        idx = np.minimum(np.searchsorted(keys, canon), len(keys) - 1)
+        hits.append(order[idx[keys[idx] == canon]])
+    sub = np.unique(np.concatenate(hits))
+    kmers = cli.decode_kmers(db["kmer"][sub], K)
+    text = "".join(f"{wl.contig_names[c]}\t{s}\t{km}\t{g}\n"
+                   for c, s, km, g in zip(db["contig"][sub].tolist(), db["start"][sub].tolist(), kmers, db["group"][sub].tolist()))
+    return sub, text
+
+
+@pytest.fixture(scope="module")
+def full():
+    import torch
+    eng, wl, res = build_full()
     yield eng, wl, res
     eng.close()
     del wl
@@ -168,46 +221,29 @@ def test_host_copy_pipeline_equals_resident(full):
     del h
 
 
-def test_sample_of_reads_against_reference_executables(full, tmp_path):
-    """the reference's own kmerpos_annot3 / diag_filter_v3 / diag_filter_step2 (oracle/_ref, unmodified prebuilt
-    binaries) with the FULL 5.9 M-SUNK database on the first reads of one chunk per haplotype"""
-    import ref_runner as RR
-    if not RR.available():
-        pytest.skip("oracle/_ref executables not present")
-    import pandas as pd
-    from gavisunk_b200 import cli
+def test_sample_of_reads_against_reference_executables(full, golden):
+    """the lines of kmerpos_annot3 / diag_filter_v3 / diag_filter_step2 for the first reads of one chunk per haplotype,
+    matched against the FULL 5.9 M-SUNK database (exported): tests/golden/fullsize_sample.json.gz, made by
+    tests/golden/make_golden_fullsize.py.  Its "source" field names what wrote them: the reference's executables run
+    on the whole exported database, or -- where they are not at hand, as for the stored file -- the oracle's
+    restatement of them (pinned to their own output by test_oracle_golden)"""
     eng, wl, res = full
-    db = eng.db_export()
-    kmers = np.asarray(cli.decode_kmers(db["kmer"], K))
-    names = np.asarray(wl.contig_names)
-    dbp, locp = str(tmp_path / "jellyfish.db"), str(tmp_path / "kmer.loc")
-    pd.DataFrame({"k": kmers}).to_csv(dbp, header=False, index=False)
-    pd.DataFrame({"c": names[db["contig"]], "s": db["start"], "k": kmers, "g": db["group"]}).to_csv(locp, sep="\t", header=False, index=False)
+    case = golden("fullsize_sample")
+    assert case["k"] == K and [(s["hap"], s["chunk"]) for s in case["sample"]] == list(SAMPLE_CHUNKS)
     off = res["off"]
-    cf = wl.chunk_first.astype(np.int64)
-    nc = len(wl.contig_names) // 2
-    for hap, chunk in ((0, 3), (1, 14)):
-        assert wl.chunk_hap[chunk] == hap
-        r0 = int(cf[chunk])
-        r1 = r0 + 40
-        seq = wl.reads[int(off[r0]):int(off[r1])].cpu().numpy()
-        fa = tmp_path / f"hap{hap + 1}.fa"
-        with open(fa, "wb") as f:
-            for i in range(r0, r1):
-                f.write(b">r%09d\n" % i + seq[off[i] - off[r0]:off[i + 1] - off[r0]].tobytes() + b"\n")
-        fai = tmp_path / f"hap{hap + 1}.fai"
-        fai.write_text("".join(f"{wl.contig_names[c]}\t{int(wl.contig_len[c])}\t0\t60\t61\n" for c in range(hap * nc, (hap + 1) * nc)))
-        r = RR.run_chunk(str(tmp_path), f"hap{hap + 1}", str(fa), dbp, locp, str(fai))
-        fmt = lambda rows, lo, hi: "".join(
-            f"r{rd:09d}\t{p}\t{wl.contig_names[c]}\t{s}\t{g}\n"
-            for rd, p, c, s, g in zip(rows["read"].tolist(), rows["pos"].tolist(), rows["contig"].tolist(), rows["start"].tolist(), rows["group"].tolist())
-            if lo <= rd < hi)
+    db = eng.db_export()
+    for s in case["sample"]:
+        r0 = int(wl.chunk_first[s["chunk"]])
+        r1 = r0 + SAMPLE_READS
+        assert wl.chunk_hap[s["chunk"]] == s["hap"] and r0 == s["first_read"]
+        reads = sample_reads(wl, res, r0, r1)
+        assert np.diff(off[r0:r1 + 1]).tolist() == s["read_len"] and bases_sha256(reads) == s["bases_sha256"], \
+            "the workload generator no longer draws the stored sample"
+        # the database rows these reads can hit, as the reference reads them from kmer.loc
+        loc = sample_loc(wl, db, reads)[1]
+        assert hashlib.sha256(loc.encode()).hexdigest() == s["loc_sha256"], s["hap"]
         # the chunk starts at r0, so the prevLoc carry of the full batch restarts exactly there
-        assert open(r["sunkpos"]).read() == fmt(res["rows"], r0, r1)
-        assert open(r["diag2"]).read() == fmt(res["kept"], r0, r1)
-        b = res["best"]
-        sel = (b["read"] >= r0) & (b["read"] < r1)
-        want = "".join(f"r{rd:09d}\t{wl.contig_names[c]}\t{g}\t{'+' if d else '-'}\t{g}\n"
-                       for rd, c, g, d in zip(b["read"][sel].tolist(), b["contig"][sel].tolist(), b["ngood"][sel].tolist(), b["dir"][sel].tolist()))
-        assert open(r["diag"]).read() == want
-        assert len(open(r["sunkpos"]).read().splitlines()) > 500
+        got = sample_texts(wl, res, r0, r1)
+        for f in ("sunkpos", "diag", "diag2"):
+            assert got[f] == s[f], (s["hap"], f)
+        assert len(s["sunkpos"].splitlines()) > 500
