@@ -13,7 +13,8 @@
   python -m gavisunk_b200.cli split_ont --reads R.. --out temp/S/reads/hapN_1-of-10.fq.gz ..   (seqtk seq -F '#' | rustybam fastq-split)
   python -m gavisunk_b200.cli combine_ont_nofilt <chunk.sunkpos>.. <hapN_detailed.sunkpos>
   python -m gavisunk_b200.cli fused --sample S --k K --hap1-asm .. --hap2-asm .. --hap1-reads f.. --hap2-reads f.. --outdir D
-                                    [--devices 0,1,..] [--batch-files N] [--detailed]
+                                    [--devices 0,1,..] [--batch-files N] [--detailed] [--support-tracks]
+  python -m gavisunk_b200.cli support_tracks <sunkpos> <rlen> <bad_sunks.txt> <fai> <valid.bed> <out.reads.bed> <out.bedgraph> <out.tsv>
 
 The first four replace workflow/scripts/{kmerpos_annot3,rlen,diag_filter_v3,diag_filter_step2}
 (workflow/rules/tagONT.smk:36,73,92,110) one to one; the next six replace badsunks_AR.py,
@@ -21,7 +22,9 @@ process-by-contig_lowmem_AR.py, get_gaps.py, `bedtools slop`, covprob.py and spl
 argv of their rules (tagONT.smk:150,189,230,249; the two `script:` rules take their snakemake.input /
 .output / .config values as options, and `covprob_script(snakemake)` / `split_locs_script(snakemake)`
 accept the snakemake object itself); `fused` replaces the rules from jellyfish_count
-to get_gaps and writes the same files under results/{sample}/.  Text parsing / formatting is host
+to get_gaps and writes the same files under results/{sample}/.  `fused --support-tracks` and `support_tracks`
+add per-read placements, support depth and a per-contig summary of the validated reads (no reference
+counterpart: the reference only plots them, viz.py).  Text parsing / formatting is host
 plumbing; all per-base and per-row work runs in libgavisunk_b200.so.  Errors exit non-zero with a
 message on stderr and never leave a partial output file behind.
 """
@@ -192,14 +195,32 @@ def cmd_badsunks(argv):
     _atomic_write(out_p, "".join(b + "\n" for b in sorted(bad)))  # the reference writes set order (SURVEY Q18)
 
 
-def process_by_contig(locs_p, sunkpos_p, rlen_p, badsunks_p, out_tsv, out_bed):
-    """process-by-contig_lowmem_AR.py:30-260 for one breaks/{contig}_{hap}.sunkpos"""
+def _read_rlen(path) -> Dict[str, int]:
+    """{hap}.rlen: read name -> length (the first row of a name wins)"""
     rlen = {}
-    with gio.open_maybe_gz(rlen_p) as f:
+    with gio.open_maybe_gz(path) as f:
         for l in f.read().decode().splitlines():
             p = l.split("\t")
             if len(p) >= 2:
                 rlen.setdefault(p[0], int(p[1]))
+    return rlen
+
+
+def _set_bad(eng, badset, cnames):
+    """bad groups of a bad_sunks.txt ('contig:ID' lines) on the engine's contigs"""
+    bc, bg = [], []
+    cidx = {n: i for i, n in enumerate(cnames)}
+    for b in badset:
+        c, _, g = b.partition(":")  # ID2 = chrom + ":" + ID (process-by-contig_lowmem_AR.py:68)
+        if c in cidx and g.isdigit() and int(g) <= 0xFFFFFFFF:
+            bc.append(cidx[c])
+            bg.append(int(g))
+    eng.bad_set(bc, bg)
+
+
+def process_by_contig(locs_p, sunkpos_p, rlen_p, badsunks_p, out_tsv, out_bed):
+    """process-by-contig_lowmem_AR.py:30-260 for one breaks/{contig}_{hap}.sunkpos"""
+    rlen = _read_rlen(rlen_p)
     open(locs_p).close()  # the reference reads it (:54-57) but none of its outputs depend on it
     rows = gio.read_sunkpos(sunkpos_p)
     if not rows:
@@ -212,14 +233,7 @@ def process_by_contig(locs_p, sunkpos_p, rlen_p, badsunks_p, out_tsv, out_bed):
     eng.set_reads_meta(np.asarray([min(rlen.get(n, 0), 0xFFFFFFFF) for n in rnames], np.uint32))
     eng.set_rows(1, *cols)
     eng.set_contigs([0] * len(cnames))
-    bc, bg = [], []
-    cidx = {n: i for i, n in enumerate(cnames)}
-    for b in badset:
-        c, _, g = b.partition(":")  # ID2 = chrom + ":" + ID (:68)
-        if c in cidx and g.isdigit() and int(g) <= 0xFFFFFFFF:
-            bc.append(cidx[c])
-            bg.append(int(g))
-    eng.bad_set(bc, bg)
+    _set_bad(eng, badset, cnames)
     eng.validate(10000)  # the reference overwrites --minlen with 10000 (:106, SURVEY Q13)
     if eng.n_pairs == 0:  # :92-94, :202-204: contig name only, no bed (the rule touches it)
         _atomic_write(out_tsv, contig + "\n")
@@ -240,6 +254,107 @@ def cmd_process_by_contig(argv):
     ap.add_argument("--opt_filt", action="store_true")
     a = ap.parse_args(argv)
     process_by_contig(a.SUNKs, a.sunkpos, a.rlen, a.badsunks, a.outputfile, a.outputbed)
+
+
+# ------------------------------------------------------------------------------------------------
+# support tracks of the validated reads (no reference counterpart; DESIGN.md section 5)
+# ------------------------------------------------------------------------------------------------
+SUPPORT_TSV_HEADER = "contig\tlength\treads\tvalidated_bases\tcovered_bases\tdepth_bases\tmax_depth\tmin_valid_depth\n"
+_STRAND = gio.NameTable(["+", "-"])
+
+
+def support_texts(hap_contigs, contig_len, names, pl, runs, iv, rtab, read_len, name_rank):
+    """The three support files of one haplotype: hap_contigs = its contig ids in .fai order; pl = Engine.placements()
+    with run-wide read indices, runs = Engine.support(), iv = validated intervals (rows of valid.bed); rtab / read_len /
+    name_rank = name table, length and bytewise name rank of every run-wide read.  -> (reads.bed, bedGraph, tsv) bytes"""
+    ctab = gio.NameTable(names)
+    inhap = np.zeros(len(names), bool)
+    inhap[np.asarray(hap_contigs, np.int64)] = True
+    p = np.flatnonzero(inhap[pl["contig"]])
+    p = p[np.lexsort((name_rank[pl["read"][p]], pl["end"][p], pl["start"][p], pl["contig"][p]))]
+    reads_bed = gio.format_rows([("name", pl["contig"], ctab), ("u32", pl["start"]), ("u32", pl["end"]), ("name", pl["read"], rtab),
+                                 ("u32", pl["n_ids"]), ("name", pl["strand"], _STRAND), ("u32", read_len[pl["read"]])], sel=p)
+    r = np.flatnonzero(inhap[runs["contig"]])
+    bedgraph = gio.format_rows([("name", runs["contig"], ctab), ("u32", runs["start"]), ("u32", runs["end"]), ("u32", runs["depth"])], sel=r)
+    rc = runs["contig"][r].astype(np.int64)
+    rs, re_, rd = (runs[c][r].astype(np.int64) for c in ("start", "end", "depth"))
+    ln = re_ - rs
+    cs, first = np.unique(rc, return_index=True)  # runs come in contig order and tile every contig
+    hi = np.append(first[1:], len(rc))
+    at = {int(c): i for i, c in enumerate(cs)}
+    covered = np.add.reduceat(np.where(rd > 0, ln, 0), first) if len(first) else []
+    depth_b = np.add.reduceat(rd * ln, first) if len(first) else []
+    max_d = np.maximum.reduceat(rd, first) if len(first) else []
+    n_reads = np.bincount(pl["contig"][p], minlength=len(names))
+    ivs = defaultdict(list)
+    for c, a, b in zip(iv["contig"].tolist(), iv["start"].tolist(), iv["end"].tolist()):
+        ivs[c].append((a, b))
+    out = [SUPPORT_TSV_HEADER]
+    for c in hap_contigs:
+        i = at[int(c)]
+        lo, up = int(first[i]), int(hi[i])
+        valid, mvd, cur_s, cur_e = 0, None, -1, -1
+        for a, b in sorted(ivs.get(int(c), [])):
+            if a >= b:
+                continue
+            if a > cur_e:  # union of the intervals: a new block starts
+                valid += cur_e - cur_s
+                cur_s, cur_e = a, b
+            else:
+                cur_e = max(cur_e, b)
+            j0 = lo + int(np.searchsorted(re_[lo:up], a, side="right"))
+            j1 = lo + int(np.searchsorted(rs[lo:up], b, side="left"))
+            m = int(rd[j0:j1].min())
+            mvd = m if mvd is None else min(mvd, m)
+        valid += cur_e - cur_s
+        out.append(f"{names[c]}\t{int(contig_len[c])}\t{int(n_reads[c])}\t{valid}\t{int(covered[i])}\t{int(depth_b[i])}\t{int(max_d[i])}\t"
+                   f"{'.' if mvd is None else mvd}\n")
+    return reads_bed, bedgraph, "".join(out).encode("latin-1")
+
+
+def support_tracks(sunkpos_p, rlen_p, badsunks_p, fai_p, valid_p, out_reads_bed, out_bedgraph, out_tsv):
+    """Support tracks of one haplotype from the files of the per-rule path ({hap}.sunkpos, {hap}.rlen, bad_sunks.txt,
+    the .fai, {hap}.valid.bed): the whole haplotype is validated in one pass, reads grouped by (contig, read name) as
+    process_by_contig groups them per contig."""
+    fai = gio.read_fai(fai_p)
+    names = [n for n, _ in fai]
+    rlen = _read_rlen(rlen_p)
+    with open(badsunks_p) as f:
+        badset = set(f.read().splitlines())
+    valid = _read_bed3(valid_p)
+    rows = list(dict.fromkeys(gio.read_sunkpos(sunkpos_p)))  # drop_duplicates (process-by-contig_lowmem_AR.py:104)
+    known = set(names)
+    for r in rows:
+        if r[2] not in known:
+            raise KeyError(f"contig {r[2]} of {sunkpos_p} is not in {fai_p}")
+    for c, _, _ in valid:
+        if c not in known:
+            raise KeyError(f"contig {c} of {valid_p} is not in {fai_p}")
+    # one engine read per (contig, read name): key the rows by both, the name stays the read's
+    keyed = [(f"{r[2]}\t{r[0]}",) + tuple(r[1:]) for r in rows]
+    eng, keyed, keys, cnames, cols = _engine_with_rows(keyed, names)
+    rnames = [k.split("\t", 1)[1] for k in keys]
+    lens = np.asarray([min(rlen.get(n, 0), 0xFFFFFFFF) for n in rnames], np.uint32)
+    eng.set_reads_meta(lens)
+    eng.set_rows(1, *cols)
+    _set_bad(eng, badset, cnames)
+    eng.validate(10000)  # the reference's fixed minimum read length (process-by-contig_lowmem_AR.py:106, SURVEY Q13)
+    pl = eng.placements()
+    runs = eng.support([l for _, l in fai])
+    cidx = {n: i for i, n in enumerate(cnames)}
+    iv = dict(contig=np.asarray([cidx[c] for c, _, _ in valid], np.uint32), start=np.asarray([s for _, s, _ in valid], np.uint32),
+              end=np.asarray([e for _, _, e in valid], np.uint32))
+    rtab = gio.NameTable(rnames)
+    name_rank = np.empty(len(rnames), np.int64)
+    if rnames:
+        name_rank[np.argsort(rtab.as_bytes_array(), kind="stable")] = np.arange(len(rnames))
+    texts = support_texts(list(range(len(names))), [l for _, l in fai], cnames, pl, runs, iv, rtab, lens, name_rank)
+    for path, data in zip((out_reads_bed, out_bedgraph, out_tsv), texts):
+        _write_bytes(path, data)
+
+
+def cmd_support_tracks(argv):
+    support_tracks(*argv)
 
 
 def cmd_get_gaps(argv):
@@ -568,14 +683,15 @@ class ThreadExchange:
 
 
 def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int], batch_files: int = 0, batch_gbp: float = 12.0,
-              detailed: bool = False, threads: int = 0, min_read_len: int = 10000, coll=None):
+              detailed: bool = False, threads: int = 0, min_read_len: int = 10000, coll=None, support_len=None):
     """The read side of the fused rule on engines whose SUNK database is loaded: the chunk files (scatter order, with
     the haplotype each belongs to) are grouped into batches (plan_batches); engine i owns a contiguous block of the
     batches and runs Engine.run_batches on it (one host thread per GPU, two exchanges per run).  Reads are parsed
     and 2-bit packed in one pass (gio.NativeReads(packed=True)) while the previous batch is on the GPU.
     coll: exchange object of a multi-PROCESS run (gavisunk_b200.parallel.EngineExchange) when `engines` is this rank's
-    single engine.  -> one result dict per engine (read names / lengths / chunk tables, kept rows, validated pairs,
-    intervals)."""
+    single engine.  support_len (contig lengths): also the support placements of every engine and the support runs,
+    with the difference arrays summed across engines by the histogram's exchange.  -> one result dict per engine
+    (read names / lengths / chunk tables, kept rows, validated pairs, intervals[, placements, support runs])."""
     import threading
     from concurrent.futures import ThreadPoolExecutor
     from .parallel import shard_chunks
@@ -631,6 +747,8 @@ def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int]
                 for old in held:
                     old.close()
             info.update(kept=eng.rows(1, pinned=True), pairs=eng.pairs(pinned=True), iv=iv)
+            if support_len is not None:
+                info.update(placements=eng.placements(pinned=True), support=eng.support(support_len, allreduce=cx.allreduce_hist))
             results[di] = info
         except BaseException as ex:  # noqa: BLE001 -- reported by the caller; peers must not wait for this rank
             errors.append(ex)
@@ -652,7 +770,7 @@ def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int]
 
 def run_fused(k: int, hap_asm: Sequence[str], hap_reads: Sequence[Sequence[str]], outdir: str, device: int = 0,
               devices: Sequence[int] = None, batch_files: int = 0, batch_gbp: float = 12.0, detailed: bool = False,
-              threads: int = 0, mrsfast_palindromes: bool = False):
+              threads: int = 0, mrsfast_palindromes: bool = False, support_tracks: bool = False):
     """hap_asm: two FASTA paths; hap_reads: two lists of chunk files in scatter order.  Builds the SUNK database on
     every GPU of `devices`, runs the reads (run_reads) and writes every file of the rules between jellyfish_count and
     slop_gaps under `outdir`.  Returns the first device's engine."""
@@ -679,21 +797,24 @@ def run_fused(k: int, hap_asm: Sequence[str], hap_reads: Sequence[Sequence[str]]
     else:
         with ThreadPoolExecutor(max_workers=len(devices)) as ex:
             engines = list(ex.map(make, devices))
-    results = run_reads(engines, contig_hap, files, file_hap, batch_files, batch_gbp, detailed, threads)
+    clen = [len(s) for _, s in contigs]
+    results = run_reads(engines, contig_hap, files, file_hap, batch_files, batch_gbp, detailed, threads,
+                        support_len=clen if support_tracks else None)
     eng = engines[0]
-    gaps, nodata = eng.gaps(np.asarray([len(s) for _, s in contigs], dtype=np.uint32))
-    write_outputs(k, eng, results, [len(s) for _, s in contigs], contig_hap, eng.contig_names, results[0]["iv"], gaps, nodata, outdir,
-                  detailed=detailed, palindromes=mrsfast_palindromes)
+    gaps, nodata = eng.gaps(np.asarray(clen, dtype=np.uint32))
+    write_outputs(k, eng, results, clen, contig_hap, eng.contig_names, results[0]["iv"], gaps, nodata, outdir,
+                  detailed=detailed, palindromes=mrsfast_palindromes, support_tracks=support_tracks)
     for e in engines[1:]:
         e.close()
     return eng
 
 
 def write_outputs(k, eng, results, contig_len, contig_hap, names, iv, gaps, nodata, outdir, detailed=False, palindromes=False,
-                  db_files=True):
+                  db_files=True, support_tracks=False):
     """every file of SURVEY Appendix C that the rules between jellyfish_count and slop_gaps produce (db_files=False:
     without the exports of the database itself -- db/jellyfish.db|.fa, mrsfast/kmer.loc and its per-contig copies
-    breaks/*.loc -- which belong to the database build, not to a run over reads)"""
+    breaks/*.loc -- which belong to the database build, not to a run over reads); support_tracks: also
+    final_out/hap{N}.reads.bed / .support.bedgraph / .support.tsv (run_reads(support_len=...) results)"""
     d = lambda *p: os.path.join(outdir, *p)
     for sub in ("db", "mrsfast", "sunkpos", "breaks", "inter_outs", "bed_files", "final_out"):
         os.makedirs(d(sub), exist_ok=True)
@@ -786,6 +907,8 @@ def write_outputs(k, eng, results, contig_len, contig_hap, names, iv, gaps, noda
     if nreads:
         name_rank[np.argsort(rtab.as_bytes_array(), kind="stable")] = np.arange(nreads)
     kept_c = by_contig(kept["contig"], kept["read"])
+    if support_tracks:
+        placements = cat_rows("placements", ("read", "contig", "start", "end", "n_ids", "strand"))
     pair_c = by_contig(pairs["contig"], pairs["read"], name_rank)
     if db_files:
         loc_c = by_contig(db["contig"])
@@ -819,6 +942,11 @@ def write_outputs(k, eng, results, contig_len, contig_hap, names, iv, gaps, noda
         emit(d("final_out", f"hap{hn}.nodata.bed"), [("name", nd, ctab), ("u32", np.zeros(len(nd), np.uint32)), ("u32", clen[nd])])
         s2, e2 = eng.slop(gaps["contig"][gsel], gaps["start"][gsel], gaps["end"][gsel], clen, 200000)  # bedtools slop -b 200000 (tagONT.smk:249)
         emit(d("final_out", f"hap{hn}.gaps.slop.bed"), [("name", gaps["contig"][gsel], ctab), ("i64", s2), ("i64", e2)])
+        if support_tracks:
+            texts = support_texts(np.flatnonzero(chap == hap).tolist(), clen, names, placements, results[0]["support"], iv, rtab, lens,
+                                  name_rank)
+            for ext, data in zip(("reads.bed", "support.bedgraph", "support.tsv"), texts):
+                _write_bytes(d("final_out", f"hap{hn}.{ext}"), data)
     from concurrent.futures import ThreadPoolExecutor
     n_cpu = len(os.sched_getaffinity(0)) if hasattr(os, "sched_getaffinity") else (os.cpu_count() or 1)
     workers = max(1, min(8, n_cpu // 2))
@@ -845,17 +973,21 @@ def cmd_fused(argv):
     ap.add_argument("--threads", type=int, default=0, help="ingest threads per GPU")
     ap.add_argument("--mrsfast-palindromes", action="store_true",
                     help="write a palindromic SUNK twice into kmer.loc, as mrsfast reports it on both strands (SURVEY A.2; unpinned)")
+    ap.add_argument("--support-tracks", action="store_true",
+                    help="also write final_out/hap{N}.reads.bed, .support.bedgraph and .support.tsv (support of the validated reads)")
     a = ap.parse_args(argv)
     devs = [int(x) for x in a.devices.split(",")] if a.devices else [a.device]
     run_fused(a.k, [a.hap1_asm, a.hap2_asm], [a.hap1_reads, a.hap2_reads], a.outdir, devices=devs, batch_files=a.batch_files,
-              batch_gbp=a.batch_gbp, detailed=a.detailed, threads=a.threads, mrsfast_palindromes=a.mrsfast_palindromes)
+              batch_gbp=a.batch_gbp, detailed=a.detailed, threads=a.threads, mrsfast_palindromes=a.mrsfast_palindromes,
+              support_tracks=a.support_tracks)
 
 
 COMMANDS = {"kmerpos_annot3": (cmd_kmerpos_annot3, 4), "rlen": (cmd_rlen, 2), "diag_filter_v3": (cmd_diag_filter_v3, 2),
             "diag_filter_step2": (cmd_diag_filter_step2, 2), "badsunks_AR": (cmd_badsunks, 5),
             "process_by_contig": (cmd_process_by_contig, None), "get_gaps": (cmd_get_gaps, 5), "slop_gaps": (cmd_slop_gaps, 3),
             "covprob": (cmd_covprob, None), "split_locs": (cmd_split_locs, None), "fused": (cmd_fused, None),
-            "split_ont": (cmd_split_ont, None), "combine_ont_nofilt": (cmd_combine_ont_nofilt, None)}
+            "split_ont": (cmd_split_ont, None), "combine_ont_nofilt": (cmd_combine_ont_nofilt, None),
+            "support_tracks": (cmd_support_tracks, 8)}
 
 
 def main(argv=None):

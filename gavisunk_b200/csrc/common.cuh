@@ -65,6 +65,7 @@ struct gvs_ctx {
   DevBuf loc_kmer, loc_contig, loc_start, loc_group, loc_gidx;  // per .loc row
   DevBuf loc_pack;                                               // per .loc row: (contig, start, group, 0) in one 16-byte word for the emit pass
   DevBuf grp_contig, grp_start;                                  // per group (index = gidx)
+  u64 grp_gen = 0;                                               // bumped whenever the group table is rebuilt
   DevBuf tab_keys, tab_rows, tab_kv;                             // open-addressed probe table: (build only) keys and rows; buckets of 4 keys + 4 (group index << 32 | row) words
   u64 tab_slots = 0;                                             // power of two, buckets of 4
   DevBuf filt;                                                   // 32-bit-word blocked Bloom filter
@@ -150,8 +151,21 @@ struct gvs_ctx {
   u64 n_kseg = 0;
   DevBuf val_scratch, val_cnt, val_off;
   DevBuf pair_read, pair_contig, pair_group, pair_gidx;
+  DevBuf seg_orient;  // per segment: orientation majority of the read (0: positions rise with starts)
   u64 n_pairs = 0;
   bool val_ready = false;
+
+  // ---- support tracks (support.cu) ----
+  u64 rank_gen = ~0ull;             // grp_gen the rank below was computed for
+  bool rank_identity = false;       // group index order is already (contig, start) order
+  DevBuf rank_of, rank_grp;         // group index -> rank in (contig, start) order, and back (unless identity)
+  DevBuf sup_diff;                  // int32[n_groups] by rank: +1 at a placement's first group, -1 at its last
+  DevBuf pl_read, pl_contig, pl_start, pl_end, pl_nids, pl_strand, pl_tmp;
+  u64 n_pl = 0;
+  bool pl_ready = false;
+  DevBuf sup_depth, sup_gx, sup_cstat, run_contig, run_start, run_end, run_depth;
+  u64 n_runs = 0;
+  bool sup_ready = false;
 
   // ---- components / intervals / gaps ----
   DevBuf parent, present, comp_min, comp_max, comp_cnt;
@@ -469,6 +483,14 @@ static int device_scan(gvs_ctx* ctx, u64 n, F f, G g, Op op, T* total_dev) {
   LAUNCH((k_scan_sums<T, Op>), 1, 1024, 0, sums, n_tiles, total_dev, op);
   LAUNCH((k_scan_apply<T, Op, F, G>), (unsigned)n_tiles, SCAN_THREADS, 0, f, g, n, sums, op);
   return 0;
+}
+
+// *err |= 4 unless groups 0..ng-1 are in strictly ascending (contig, start) order (covprob's lookup, support tracks)
+static __global__ void __launch_bounds__(256) k_groups_sorted(const u32* __restrict__ g_contig, const u32* __restrict__ g_id, u64 ng, u32* err) {
+  u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i + 1 >= ng) return;
+  u32 a = g_contig[i], b = g_contig[i + 1];
+  if (a > b || (a == b && g_id[i] >= g_id[i + 1])) atomicOr(err, 4u);
 }
 
 // small helpers to read device scalars (synchronises the stream)

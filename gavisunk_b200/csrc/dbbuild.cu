@@ -340,6 +340,7 @@ static int db_build_device(gvs_ctx* ctx, const u8* seq, const u64* contig_off, u
   CKR(gvs_reserve(ctx, hrow, n_sunks * 4));
   CKR(gvs_reserve(ctx, gex, n_sunks * 4));
   ctx->n_groups = 0;
+  ctx->grp_gen++;
   if (n_sunks) {
     LAUNCH(k_db_rows, (unsigned)cdiv(n_words, 256), 256, 0, bm, wr, n_words, seq, total, contig_off, n_contigs, k,
            ctx->loc_kmer.as<u64>(), ctx->loc_contig.as<u32>(), ctx->loc_start.as<u32>(), head.as<u8>());

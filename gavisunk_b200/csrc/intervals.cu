@@ -420,12 +420,6 @@ __global__ void __launch_bounds__(128) k_covprob_gaps(const u32* __restrict__ g_
   }
   prob[t] = table[kb];
 }
-__global__ void __launch_bounds__(256) k_groups_sorted(const u32* __restrict__ g_contig, const u32* __restrict__ g_id, u64 ng, u32* err) {
-  u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i + 1 >= ng) return;
-  u32 a = g_contig[i], b = g_contig[i + 1];
-  if (a > b || (a == b && g_id[i] >= g_id[i + 1])) atomicOr(err, 4u);
-}
 
 extern "C" int gvs_covprob_gaps(gvs_ctx* ctx, const uint32_t* grp_contig, const uint32_t* grp_id, uint64_t n_groups,
                                 const uint32_t* gap_contig, const int64_t* gap_start, const int64_t* gap_end, uint64_t n_gaps,

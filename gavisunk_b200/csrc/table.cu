@@ -207,6 +207,7 @@ static int build_group_index_body(gvs_ctx* ctx, const u32* contig, const u32* gr
 // fills gidx_out[n], ctx->n_groups, ctx->grp_contig / grp_start
 int gvs_group_index_rows(gvs_ctx* ctx, const u32* contig, const u32* group, u64 n, u32* gidx_out) {
   CKR(gvs_reserve(ctx, ctx->counters, 64 * sizeof(u64)));
+  ctx->grp_gen++;
   if (n == 0) {
     ctx->n_groups = 0;
     return 0;

@@ -61,6 +61,7 @@ struct ValParams {
   u32* out_id;               // per kept row slot: validated IDs of the read, from its first row on
   u32* out_gidx;
   u32* seg_cnt;              // validated IDs per segment
+  u8* orient;                // orientation majority per segment with validated IDs (0: read positions rise with starts)
   u32 m_lo, m_hi;            // this launch handles reads with m_lo < rows <= m_hi
   u8* gscratch;              // global-scratch variant: per block VROW_BYTES * big_cap
   u32 big_cap;
@@ -528,7 +529,10 @@ __global__ void __launch_bounds__(NT* GROUPS) k_validate(const ValParams V) {
         V.out_gidx[a + rank] = w.G[r];
       }
     }
-    if (tid == 0) V.seg_cnt[s] = w.csize[broot];
+    if (tid == 0) {
+      V.seg_cnt[s] = w.csize[broot];
+      V.orient[s] = (u8)orient;
+    }
   }
 }
 
@@ -559,6 +563,7 @@ extern "C" int gvs_validate(gvs_ctx* ctx, uint32_t min_read_len, uint64_t* n_pai
   CK(cudaSetDevice(ctx->device));
   StageTimer tm(ctx, GVS_ST_VALIDATE);
   ctx->val_ready = false;
+  ctx->pl_ready = ctx->sup_ready = false;
   ctx->n_pairs = 0;
   if (n_pairs_out) *n_pairs_out = 0;
   Rows& R = ctx->kept;
@@ -577,6 +582,7 @@ extern "C" int gvs_validate(gvs_ctx* ctx, uint32_t min_read_len, uint64_t* n_pai
   u32* out_gidx = out_id + n;
   u32* seg_cnt = out_gidx + n;
   u32* seg_off = seg_cnt + n_seg;
+  CKR(gvs_reserve(ctx, ctx->seg_orient, n_seg));
   // largest read (rows) decides which launches are needed
   u32* mx_dev = (u32*)(ctx->counters.as<u64>() + 22);
   {
@@ -595,7 +601,7 @@ extern "C" int gvs_validate(gvs_ctx* ctx, uint32_t min_read_len, uint64_t* n_pai
   V.bad = ctx->bad_ready ? ctx->bad_flag.as<u8>() : nullptr;
   V.read_off = ctx->read_off; V.read_len = ctx->have_read_len ? ctx->read_len.as<u32>() : nullptr;
   V.min_len = min_read_len;
-  V.out_id = out_id; V.out_gidx = out_gidx; V.seg_cnt = seg_cnt;
+  V.out_id = out_id; V.out_gidx = out_gidx; V.seg_cnt = seg_cnt; V.orient = ctx->seg_orient.as<u8>();
   V.gscratch = nullptr; V.big_cap = 0; V.stats = stats;
   const size_t sm_warp = (size_t)VROW_BYTES * VCAP_WARP * 8, sm_blk = (size_t)VROW_BYTES * VCAP;
   if (!ctx->val_attr_set) {

@@ -527,6 +527,33 @@ class Engine:
                                         _ptr(out["gidx"])))
         return out
 
+    def placements(self, pinned: bool = False) -> Dict[str, np.ndarray]:
+        """Support placements of the validated reads (no reference counterpart): one per read with >= 2 validated
+        IDs -- read (run-wide index), contig, start / end (smallest / largest validated ID), n_ids, strand (0 '+',
+        1 '-').  Also leaves the per-rank difference array on the device for support()."""
+        n, p = C.c_uint64(), C.c_void_p()
+        self._ck(self.lib.gvs_placements(self.ctx, C.byref(n), C.byref(p)))
+        self._diff_ptr = int(p.value or 0)
+        n = int(n.value)
+        out = {c: self._out(f"placements.{c}", n, np.uint32, pinned) for c in ("read", "contig", "start", "end", "n_ids")}
+        out["strand"] = self._out("placements.strand", n, np.uint8, pinned)
+        self._ck(self.lib.gvs_placements_get(self.ctx, _ptr(out["read"]), _ptr(out["contig"]), _ptr(out["start"]), _ptr(out["end"]),
+                                             _ptr(out["n_ids"]), _ptr(out["strand"])))
+        return out
+
+    def support(self, contig_len: Sequence[int], allreduce=None) -> Dict[str, np.ndarray]:
+        """Support depth after placements(): runs (contig, start, end, depth) tiling every contig.  With several GPUs
+        `allreduce(ptr, n_groups)` sums the int32 difference array across ranks in place first (the callable that
+        sums the bad-SUNK histogram)."""
+        if allreduce is not None:
+            allreduce(self._diff_ptr, self.db_groups())
+        cl = _c(contig_len, np.uint32)
+        n = C.c_uint64()
+        self._ck(self.lib.gvs_support(self.ctx, _ptr(cl), C.byref(n)))
+        out = {c: np.zeros(int(n.value), np.uint32) for c in ("contig", "start", "end", "depth")}
+        self._ck(self.lib.gvs_support_get(self.ctx, _ptr(out["contig"]), _ptr(out["start"]), _ptr(out["end"]), _ptr(out["depth"])))
+        return out
+
     def components_local(self, accumulate: bool = False) -> int:
         p = C.c_void_p()
         self._ck(self.lib.gvs_components_local(self.ctx, 1 if accumulate else 0, C.byref(p)))

@@ -56,6 +56,7 @@ enum {
   GVS_ST_MODE = 8,      /* badsunks_AR.py mode per haplotype (gvs_hist_mode)                      */
   GVS_ST_BAD = 9,       /* bad SUNK groups (gvs_bad_groups)                                       */
   GVS_ST_MERGE = 10,    /* union with the peers' forests (gvs_components_merge / _merge_all)      */
+  GVS_ST_SUPPORT = 11,  /* support tracks (gvs_placements, gvs_support): no reference counterpart  */
   GVS_ST_COUNT = 12
 };
 
@@ -334,6 +335,25 @@ int gvs_components_merge_all(gvs_ctx* ctx, const uint32_t* gathered_dev, uint32_
  * (contig, start) = rows of bed_files/{contig}_{hap}.bed */
 int gvs_intervals(gvs_ctx* ctx, uint64_t* n_intervals);
 int gvs_intervals_get(gvs_ctx* ctx, uint32_t* contig, uint32_t* start, uint32_t* end);
+
+/* Support tracks of the validated reads.  No reference counterpart: the reference only draws pile-up plots
+ * (viz.py, viz_detailed.py); these are text tracks for genome browsers and assembly QC.
+ * A placement is a read with >= 2 validated IDs (the reads that join groups in gvs_components_local):
+ * start / end = its smallest / largest validated ID (group starts, the convention of the intervals), n_ids = its
+ * validated IDs, strand = 0 when its orientation majority is 0 (read positions rise with assembly starts), else 1.
+ * gvs_placements runs after gvs_validate.  *diff_dev receives an int32 array of n_groups entries indexed by the
+ * group's rank in (contig, start) order (+1 at a placement's first group, -1 at its last), zero without
+ * placements: several GPUs sum it (like the histogram of gvs_group_hist) before gvs_support.
+ * gvs_placements_get: host buffers of *n entries, any pointer may be NULL; read_idx is run-wide as in
+ * gvs_pairs_get; placements come in segment (read) order. */
+int gvs_placements(gvs_ctx* ctx, uint64_t* n, int32_t** diff_dev);
+int gvs_placements_get(gvs_ctx* ctx, uint32_t* read_idx, uint32_t* contig, uint32_t* start, uint32_t* end, uint32_t* n_ids,
+                       uint8_t* strand);
+/* Support depth from the (summed) difference array: the number of placements with start <= x < end at every
+ * base x, as runs (contig, start, end, depth) that tile [0, contig_len[c]) of every contig c (n_contigs
+ * entries, host memory) in (contig, start) order, maximal (adjacent runs of a contig differ in depth). */
+int gvs_support(gvs_ctx* ctx, const uint32_t* contig_len, uint64_t* n_runs);
+int gvs_support_get(gvs_ctx* ctx, uint32_t* contig, uint32_t* start, uint32_t* end, uint32_t* depth);
 
 /* Intervals parsed from bed_files/{contig}_{hap}.bed instead of produced by gvs_intervals (the input
  * of get_gaps.py:30); any order, host memory. */
