@@ -40,6 +40,7 @@ import numpy as np
 
 from . import io as gio
 from .engine import Engine, encode_kmers
+from .parallel import ThreadExchange, shard_chunks
 
 
 def _atomic_write(path: str, text: str):
@@ -623,65 +624,6 @@ def plan_batches(files: Sequence[str], n_devices: int, batch_files: int = 0, bat
     return out
 
 
-class ThreadExchange:
-    """The two exchanges of the path between the engines of one process (one host thread per GPU): the histogram
-    sum and the forest gather of gavisunk_b200.parallel, done with torch copies between the devices (plumbing)."""
-
-    def __init__(self, engines):
-        import threading
-        self.engines = engines
-        self.n = len(engines)
-        self.bar = threading.Barrier(self.n)
-        self.slots = [None] * self.n
-        self.keep = [None] * self.n
-        self.failed = False
-
-    def abort(self):
-        self.failed = True
-        self.bar.abort()
-
-    def for_rank(self, r):
-        x = self
-
-        class _R:
-            @staticmethod
-            def allreduce_hist(ptr, n_groups):
-                if x.n == 1 or not n_groups:
-                    return
-                import torch
-                from .parallel import alias_device_array
-                dev = torch.device("cuda", x.engines[r].device)
-                x.engines[r].sync()
-                x.slots[r] = alias_device_array(ptr, n_groups, "<i4", dev)
-                x.bar.wait()
-                if r == 0:
-                    tot = x.slots[0].clone()
-                    for p in range(1, x.n):
-                        tot += x.slots[p].to(tot.device)
-                    for p in range(x.n):
-                        x.slots[p].copy_(tot.to(x.slots[p].device))
-                    for p in range(x.n):
-                        torch.cuda.synchronize(x.slots[p].device)
-                x.bar.wait()
-
-            @staticmethod
-            def gather_forests(ptr, n_groups):
-                if x.n == 1 or not n_groups:
-                    return []
-                import torch
-                from .parallel import alias_device_array
-                dev = torch.device("cuda", x.engines[r].device)
-                x.engines[r].sync()
-                x.slots[r] = alias_device_array(ptr, n_groups, "<i4", dev)
-                x.bar.wait()
-                peers = [x.slots[p].to(dev) for p in range(x.n) if p != r]
-                torch.cuda.synchronize(dev)
-                x.keep[r] = peers
-                x.bar.wait()  # nobody unions into its own forest while a peer still copies it
-                return [int(t.data_ptr()) for t in peers]
-        return _R
-
-
 def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int], batch_files: int = 0, batch_gbp: float = 12.0,
               detailed: bool = False, threads: int = 0, min_read_len: int = 10000, coll=None, support_len=None):
     """The read side of the fused rule on engines whose SUNK database is loaded: the chunk files (scatter order, with
@@ -694,7 +636,6 @@ def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int]
     (read names / lengths / chunk tables, kept rows, validated pairs, intervals[, placements, support runs])."""
     import threading
     from concurrent.futures import ThreadPoolExecutor
-    from .parallel import shard_chunks
     for p in files:
         if not os.path.exists(p):
             raise FileNotFoundError(p)

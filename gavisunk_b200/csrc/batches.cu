@@ -9,7 +9,7 @@
 //                        -> gvs_batch_stash   (the kept rows, 24 B each, stay resident; the reads may go)
 //   [multi-GPU: ONE all-reduce of the histogram]   gvs_hist_mode / gvs_bad_groups
 //   phase 2, once:       gvs_batches_bind -> gvs_validate -> gvs_components_local
-//   [multi-GPU: ONE all-gather of the forests + gvs_components_merge]   gvs_intervals -> gvs_gaps
+//   [multi-GPU: ONE all-gather of the forests + gvs_components_merge_all]   gvs_intervals -> gvs_gaps
 // Read indices of the bound rows count through the batches in stash order (batch b's reads start at the
 // *read_base gvs_batch_stash returned for it).
 #include "common.cuh"
@@ -58,7 +58,7 @@ extern "C" int gvs_batches_begin(gvs_ctx* ctx) {
   ctx->stash_reads = 0;
   ctx->hist_ready = false;  // the next gvs_group_hist(accumulate = 1) starts from zero
   ctx->bad_ready = false;
-  ctx->comp_ready = false;  // ... and the next gvs_components_local from singletons
+  ctx->comp_ready = false;  // ... and gvs_intervals waits for the run's gvs_components_local
   ctx->val_ready = false;
   return 0;
 }

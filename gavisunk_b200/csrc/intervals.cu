@@ -7,7 +7,8 @@
 // components (:237); connectivity only needs a chain through the read's IDs, so each validated
 // pair is unioned with its predecessor of the same read in a lock-free union-find over the dense
 // group index (hook larger root under smaller: the root is the component's first group).
-// Multi-GPU: every rank builds its forest; forests are merged by unioning g with peer_parent[g].
+// Multi-GPU: every rank builds its forest; the gathered forests are merged in one pass by unioning g with
+// each peer's parent[g].
 #include "common.cuh"
 #include <algorithm>
 
@@ -45,15 +46,6 @@ __global__ void __launch_bounds__(256) k_comp_pairs(const u32* __restrict__ read
   present[a] = 1;
   present[b] = 1;
   if (a != b) guf_union(par, a, b);
-}
-__global__ void __launch_bounds__(256) k_comp_merge(const u32* __restrict__ peer, u64 ng, u32* par, u8* present) {
-  u64 g = (u64)blockIdx.x * blockDim.x + threadIdx.x;
-  if (g >= ng) return;
-  u32 p = peer[g];
-  if (p == (u32)g || p >= ng) return;
-  present[g] = 1;
-  present[p] = 1;
-  guf_union(par, (u32)g, p);
 }
 // forest -> every entry points at its root (depth 1): what the peers receive, and what makes their merge cheap
 __global__ void __launch_bounds__(256) k_comp_flatten(u32* par, u64 ng) {
@@ -113,31 +105,29 @@ __global__ void __launch_bounds__(256) k_iv_write(const u32* __restrict__ excl, 
   iv_end[o] = mx[g];  // end = largest group ID, not +k (Q15)
 }
 
-static int ensure_forest(gvs_ctx* ctx, bool reset) {
+// singleton forest over the group index, no group present
+static int ensure_forest(gvs_ctx* ctx) {
   u64 ng = ctx->n_groups ? ctx->n_groups : 1;
-  bool fresh = ctx->parent.cap < ng * 4 || ctx->present.cap < ng;
   CKR(gvs_reserve(ctx, ctx->parent, ng * 4));
   CKR(gvs_reserve(ctx, ctx->present, ng));
-  if (reset || fresh || !ctx->comp_ready) {
-    LAUNCH(k_iota, (unsigned)cdiv(ng, 256), 256, 0, ctx->parent.as<u32>(), ng);
-    CK(cudaMemsetAsync(ctx->present.p, 0, ng, ctx->stream));
-  }
+  LAUNCH(k_iota, (unsigned)cdiv(ng, 256), 256, 0, ctx->parent.as<u32>(), ng);
+  CK(cudaMemsetAsync(ctx->present.p, 0, ng, ctx->stream));
   return 0;
 }
 
-extern "C" int gvs_components_local(gvs_ctx* ctx, int accumulate, uint32_t** parent_dev) {
+extern "C" int gvs_components_local(gvs_ctx* ctx, uint32_t** parent_dev) {
   if (!ctx) return GVS_E_ARG;
   if (!ctx->val_ready) return gvs_fail(ctx, GVS_E_STATE, "gvs_components_local before gvs_validate");
   if (!ctx->groups_ready) return gvs_fail(ctx, GVS_E_STATE, "gvs_components_local: no group index");
   CK(cudaSetDevice(ctx->device));
   StageTimer tm(ctx, GVS_ST_COMPONENTS);
-  CKR(ensure_forest(ctx, !accumulate));
+  CKR(ensure_forest(ctx));
   u64 n = ctx->n_pairs;
   if (n > 1)
     LAUNCH(k_comp_pairs, (unsigned)cdiv(n, 256), 256, 0, ctx->pair_read.as<u32>(), ctx->pair_gidx.as<u32>(), n,
            ctx->parent.as<u32>(), ctx->present.as<u8>());
   // entries point straight at their roots: the array that crosses GPUs is a depth-1 forest
-  if (n > 1 || accumulate) LAUNCH(k_comp_flatten, (unsigned)cdiv(ctx->n_groups ? ctx->n_groups : 1, 256), 256, 0, ctx->parent.as<u32>(), ctx->n_groups);
+  if (n > 1) LAUNCH(k_comp_flatten, (unsigned)cdiv(ctx->n_groups ? ctx->n_groups : 1, 256), 256, 0, ctx->parent.as<u32>(), ctx->n_groups);
   ctx->comp_ready = true;
   ctx->iv_ready = false;
   if (parent_dev) *parent_dev = ctx->parent.as<u32>();
@@ -152,17 +142,6 @@ extern "C" int gvs_components_merge_all(gvs_ctx* ctx, const uint32_t* gathered_d
   u64 ng = ctx->n_groups;
   if (ng && n_ranks > 1)
     LAUNCH(k_comp_merge_all, (unsigned)cdiv(ng, 256), 256, 0, gathered_dev, n_ranks, own_rank, ng, ctx->parent.as<u32>(), ctx->present.as<u8>());
-  ctx->iv_ready = false;
-  return 0;
-}
-
-extern "C" int gvs_components_merge(gvs_ctx* ctx, const uint32_t* peer_parent_dev) {
-  if (!ctx || !peer_parent_dev) return GVS_E_ARG;
-  if (!ctx->comp_ready) return gvs_fail(ctx, GVS_E_STATE, "gvs_components_merge before gvs_components_local");
-  CK(cudaSetDevice(ctx->device));
-  StageTimer tm(ctx, GVS_ST_MERGE);
-  u64 ng = ctx->n_groups;
-  if (ng) LAUNCH(k_comp_merge, (unsigned)cdiv(ng, 256), 256, 0, peer_parent_dev, ng, ctx->parent.as<u32>(), ctx->present.as<u8>());
   ctx->iv_ready = false;
   return 0;
 }

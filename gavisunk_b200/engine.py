@@ -392,17 +392,23 @@ class Engine:
         """The fused hot path on the reads bound to this engine: match -> diag filter -> bad-SUNK
         histogram -> validation -> contig-wide components -> intervals.  With several GPUs
         `allreduce_hist(ptr, n_groups)` sums the int32 histogram across ranks in place and
-        `gather_forests(ptr, n_groups)` returns device pointers of the peers' parent arrays."""
+        `gather_forests(ptr, n_groups)` gathers the parent arrays: None with a single rank, else
+        (pointer of the [n_ranks][n_groups] array on this device, n_ranks, own rank)."""
         self.match()
         self.diag_filter(contig_hap)
-        hp = self.group_hist()
+        return self._global_stages(self.group_hist(), min_read_len, allreduce_hist, gather_forests)
+
+    def _global_stages(self, hist_ptr: int, min_read_len: int, allreduce_hist, gather_forests):
+        """everything after the histogram: its all-reduce, bad groups, validation, local forest, forest
+        merge, intervals"""
         if allreduce_hist is not None:
-            allreduce_hist(hp, self.db_groups())
+            allreduce_hist(hist_ptr, self.db_groups())
         self.bad_groups()
         self.validate(min_read_len)
         pp = self.components_local()
-        if gather_forests is not None:
-            self._merge_forests(gather_forests, pp)
+        gathered = gather_forests(pp, self.db_groups()) if gather_forests is not None else None
+        if gathered is not None:
+            self.components_merge_all(*gathered)
         return self.intervals()
 
     # ------------------------------------------------------------------------------------
@@ -453,14 +459,7 @@ class Engine:
         if not bases:  # a rank without a batch still takes part in both exchanges
             self.set_contigs(contig_hap)
             hp = self.group_hist(accumulate=True)
-        if allreduce_hist is not None:
-            allreduce_hist(hp, self.db_groups())
-        self.bad_groups()
-        self.validate(min_read_len)
-        pp = self.components_local()
-        if gather_forests is not None:
-            self._merge_forests(gather_forests, pp)
-        return self.intervals(), bases
+        return self._global_stages(hp, min_read_len, allreduce_hist, gather_forests), bases
 
     def db_groups(self) -> int:
         a, b = C.c_uint64(), C.c_uint64()
@@ -554,26 +553,15 @@ class Engine:
         self._ck(self.lib.gvs_support_get(self.ctx, _ptr(out["contig"]), _ptr(out["start"]), _ptr(out["end"]), _ptr(out["depth"])))
         return out
 
-    def components_local(self, accumulate: bool = False) -> int:
+    def components_local(self) -> int:
+        """this GPU's forest of the validated pairs; returns the device pointer of its uint32[n_groups] parent array"""
         p = C.c_void_p()
-        self._ck(self.lib.gvs_components_local(self.ctx, 1 if accumulate else 0, C.byref(p)))
+        self._ck(self.lib.gvs_components_local(self.ctx, C.byref(p)))
         return int(p.value or 0)
-
-    def components_merge(self, peer_parent_ptr: int):
-        self._ck(self.lib.gvs_components_merge(self.ctx, C.c_void_p(peer_parent_ptr)))
 
     def components_merge_all(self, gathered_ptr: int, n_ranks: int, own_rank: int):
         """unions in every peer's forest in one pass (gathered = [n_ranks][n_groups] parent arrays on this device)"""
         self._ck(self.lib.gvs_components_merge_all(self.ctx, C.c_void_p(gathered_ptr), int(n_ranks), int(own_rank)))
-
-    def _merge_forests(self, gather_forests, pp):
-        peers = gather_forests(pp, self.db_groups())
-        if isinstance(peers, tuple):  # (pointer of the gathered [n_ranks][n_groups] array, n_ranks, own rank)
-            if peers[1] > 1:
-                self.components_merge_all(*peers)
-        else:
-            for peer in peers:
-                self.components_merge(peer)
 
     def intervals(self) -> Dict[str, np.ndarray]:
         """process-by-contig_lowmem_AR.py:215-260 -> rows of bed_files/*.bed."""

@@ -5,7 +5,14 @@ replicated, and exactly two exchanges cross GPUs:
      haplotype) -- all-reduce of int32[n_groups];
   2. the contig-wide component merge (process-by-contig_lowmem_AR.py:219-237 sees the reads of ALL
      chunks) -- all-gather of the union-find parent arrays uint32[n_groups]; every rank then unions
-     its forest with each peer's (gvs_components_merge), so the result is replicated.
+     all peers' forests into its own in one pass (gvs_components_merge_all), so the result is replicated.
+
+Two adapters give Engine.run_all / run_batches these exchanges: EngineExchange (one process per GPU,
+torch.distributed) and ThreadExchange (one process, one host thread per GPU, torch copies between
+the devices).  Both follow one convention: allreduce_hist(ptr, n_groups) sums in place, and
+gather_forests(ptr, n_groups) returns None with a single rank or no groups, else (pointer of an
+int32 [n_ranks][n_groups] array on the engine's device whose row r is rank r's forest -- the own row
+may be left unwritten --, n_ranks, own rank), kept alive until the adapter's next gather.
 
 torch.distributed is plumbing only (NCCL on GPUs; gloo in the CPU tests).  The tensors alias the
 library's device buffers, so the collectives run in place on them.
@@ -108,11 +115,11 @@ class Exchange:
         return hist
 
     def gather_forests(self, parent):
-        """parent: int32-typed view of uint32[n_groups]; returns the list of the peers' arrays
-        (views into one gathered tensor), own rank excluded"""
+        """parent: int32-typed view of uint32[n_groups]; returns the gathered [world, n_groups] tensor
+        (row r = rank r's array), None with a single rank or no groups"""
         import torch
         if self.world == 1 or parent.numel() == 0:
-            return []
+            return None
         n = parent.numel()
         buf = getattr(self, "_keep", None)  # one gather buffer per run shape, reused (a rank pays this once per run)
         if buf is None or buf.numel() != self.world * n or buf.dtype != parent.dtype or buf.device != parent.device:
@@ -120,7 +127,7 @@ class Exchange:
         self.dist.all_gather_into_tensor(buf, parent, group=self.group) if parent.is_cuda else \
             self.dist.all_gather(list(buf.view(self.world, n).unbind(0)), parent, group=self.group)
         self._keep = buf
-        return [buf[r * n:(r + 1) * n] for r in range(self.world) if r != self.rank]
+        return buf.view(self.world, n)
 
 
 _ALIASES: dict = {}
@@ -182,9 +189,75 @@ class EngineExchange:
 
     def gather_forests(self, ptr: int, n_groups: int):
         if self.x.world == 1 or not n_groups:
-            return []
+            return None
         self._before()
-        self.x.gather_forests(alias_device_array(ptr, n_groups, "<i4", self.device))
+        gathered = self.x.gather_forests(alias_device_array(ptr, n_groups, "<i4", self.device))
         self._after()
-        # the gathered [world][n_groups] array itself: Engine unions all peers in one pass (gvs_components_merge_all)
-        return int(self.x._keep.data_ptr()), self.x.world, self.x.rank
+        return int(gathered.data_ptr()), self.x.world, self.x.rank
+
+
+class ThreadExchange:
+    """The two exchanges between the engines of one process (one host thread per GPU): the histogram is summed by
+    rank 0 and the forests are gathered with torch copies between the devices (plumbing).  for_rank(r) gives the
+    adapter of engine r; abort() releases the peers of a thread that failed."""
+
+    def __init__(self, engines):
+        import threading
+        self.engines = engines
+        self.n = len(engines)
+        self.bar = threading.Barrier(self.n)
+        self.slots = [None] * self.n  # rank r's aliased device array of the current exchange
+        self.keep = [None] * self.n   # rank r's gather buffer, reused while the shape holds
+
+    def abort(self):
+        self.bar.abort()
+
+    def for_rank(self, r: int) -> "_ThreadRank":
+        return _ThreadRank(self, r)
+
+
+class _ThreadRank:
+    def __init__(self, x: ThreadExchange, r: int):
+        self.x, self.r = x, r
+
+    def _publish(self, ptr: int, n_groups: int):
+        """waits for the engine's work on the array, then for every rank to have published its own"""
+        import torch
+        x, r = self.x, self.r
+        dev = torch.device("cuda", x.engines[r].device)
+        x.engines[r].sync()
+        x.slots[r] = alias_device_array(ptr, n_groups, "<i4", dev)
+        x.bar.wait()
+        return dev
+
+    def allreduce_hist(self, ptr: int, n_groups: int):
+        x, r = self.x, self.r
+        if x.n == 1 or not n_groups:
+            return
+        import torch
+        self._publish(ptr, n_groups)
+        if r == 0:
+            tot = x.slots[0].clone()
+            for p in range(1, x.n):
+                tot += x.slots[p].to(tot.device)
+            for p in range(x.n):
+                x.slots[p].copy_(tot.to(x.slots[p].device))
+            for p in range(x.n):
+                torch.cuda.synchronize(x.slots[p].device)
+        x.bar.wait()
+
+    def gather_forests(self, ptr: int, n_groups: int):
+        x, r = self.x, self.r
+        if x.n == 1 or not n_groups:
+            return None
+        import torch
+        dev = self._publish(ptr, n_groups)
+        buf = x.keep[r]
+        if buf is None or buf.shape != (x.n, n_groups):
+            buf = x.keep[r] = torch.empty(x.n, n_groups, dtype=torch.int32, device=dev)
+        for p in range(x.n):
+            if p != r:
+                buf[p].copy_(x.slots[p])
+        torch.cuda.synchronize(dev)
+        x.bar.wait()  # nobody unions into its own forest while a peer still copies it
+        return int(buf.data_ptr()), x.n, r

@@ -55,7 +55,7 @@ enum {
   GVS_ST_COMPONENTS = 7, /* local forest of the validated pairs (gvs_components_local)             */
   GVS_ST_MODE = 8,      /* badsunks_AR.py mode per haplotype (gvs_hist_mode)                      */
   GVS_ST_BAD = 9,       /* bad SUNK groups (gvs_bad_groups)                                       */
-  GVS_ST_MERGE = 10,    /* union with the peers' forests (gvs_components_merge / _merge_all)      */
+  GVS_ST_MERGE = 10,    /* union with the peers' forests (gvs_components_merge_all)               */
   GVS_ST_SUPPORT = 11,  /* support tracks (gvs_placements, gvs_support): no reference counterpart  */
   GVS_ST_COUNT = 12
 };
@@ -307,7 +307,7 @@ int gvs_groups_get(gvs_ctx* ctx, uint32_t* contig, uint32_t* group, int32_t* his
  *   per batch:  gvs_reads_set* -> gvs_match -> gvs_diag_filter -> gvs_group_hist(accumulate = 1) -> gvs_batch_stash
  *   (several GPUs: ONE all-reduce of the histogram)  gvs_hist_mode -> gvs_bad_groups
  *   gvs_batches_bind -> gvs_validate -> gvs_components_local
- *   (several GPUs: ONE all-gather of the forests, gvs_components_merge)  gvs_intervals -> gvs_gaps
+ *   (several GPUs: ONE all-gather of the forests, gvs_components_merge_all)  gvs_intervals -> gvs_gaps
  * gvs_batch_stash keeps the batch's kept rows (24 B each) and read lengths resident and returns the index its
  * first read has in the run (*read_base); gvs_batches_bind makes the stashed rows of all batches the input of
  * gvs_validate (as if one gvs_diag_filter had kept them; gvs_rows_get(1) / gvs_pairs_get then report run-wide
@@ -324,12 +324,11 @@ int gvs_pairs_get(gvs_ctx* ctx, uint32_t* read_idx, uint32_t* contig, uint32_t* 
 
 /* process-by-contig_lowmem_AR.py:215-260 contig-wide components.  The union-find parent array
  * (n_groups uint32, index = group_index) is exposed so that several GPUs can merge their
- * forests: gvs_components_local builds this GPU's forest, gvs_components_merge unions in a
- * peer's forest (device pointer, e.g. an all-gathered copy), gvs_intervals finalises. */
-int gvs_components_local(gvs_ctx* ctx, int accumulate, uint32_t** parent_dev);
-int gvs_components_merge(gvs_ctx* ctx, const uint32_t* peer_parent_dev);
-/* All peers at once: gathered_dev = the all-gathered parent arrays, rank r's at gathered_dev + r * n_groups (own_rank's
- * slice is skipped).  One pass over the groups instead of one launch per peer. */
+ * forests: gvs_components_local builds this GPU's forest from singletons, gvs_components_merge_all
+ * unions in every peer's forest in one pass, gvs_intervals finalises.  gathered_dev = the all-gathered
+ * parent arrays on this GPU, rank r's at gathered_dev + r * n_groups (own_rank's slice is skipped and
+ * may be left unwritten). */
+int gvs_components_local(gvs_ctx* ctx, uint32_t** parent_dev);
 int gvs_components_merge_all(gvs_ctx* ctx, const uint32_t* gathered_dev, uint32_t n_ranks, uint32_t own_rank);
 /* validated intervals (contig, min group, max group) of components with >= 3 groups, sorted by
  * (contig, start) = rows of bed_files/{contig}_{hap}.bed */

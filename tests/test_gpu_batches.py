@@ -102,11 +102,11 @@ def test_two_engines_exchange_like_two_ranks():
         e.validate(3000)
         forests.append(e.components_local())
         e.sync()
-    copies = [alias_device_array(f, ng, "<i4", dev).clone() for f in forests]
+    gathered = torch.stack([alias_device_array(f, ng, "<i4", dev) for f in forests])
     torch.cuda.synchronize()
     res = []
     for i, e in enumerate(engines):
-        e.components_merge(int(copies[1 - i].data_ptr()))
+        e.components_merge_all(int(gathered.data_ptr()), 2, i)
         iv = e.intervals()
         gaps, nodata = e.gaps(wl.contig_len.astype(np.uint32))
         res.append((dict(iv={c: v.tolist() for c, v in iv.items()}, gaps={c: v.tolist() for c, v in gaps.items()}, nodata=nodata.tolist(),

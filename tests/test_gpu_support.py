@@ -107,10 +107,10 @@ def test_support_equals_oracle(split):
 
 
 def test_two_contexts_equal_one():
-    """two contexts on one GPU, half of the batches each, exchanging through cli.ThreadExchange: the difference arrays
-    are summed by the callable that sums the bad-SUNK histogram"""
-    from gavisunk_b200 import cli
+    """two contexts on one GPU, half of the batches each, exchanging through parallel.ThreadExchange: the difference
+    arrays are summed by the callable that sums the bad-SUNK histogram"""
     from gavisunk_b200.engine import Engine
+    from gavisunk_b200.parallel import ThreadExchange
     from gavisunk_b200 import workload as W
     eng, wl = _setup(seed=43, nchunks=4)
     hb = _host_batches(wl, [[0, 1, 2], [3], [4, 5], [6, 7]])
@@ -119,7 +119,7 @@ def test_two_contexts_equal_one():
     eng2 = Engine(20)
     W.build_db(eng2, wl)
     engines = [eng, eng2]
-    xch = cli.ThreadExchange(engines)
+    xch = ThreadExchange(engines)
     out, errs = [None, None], []
 
     def work(i):

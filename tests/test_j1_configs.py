@@ -217,8 +217,8 @@ def test_simulated_reads_are_reproducible():
 @pytest.mark.gpu
 def test_fused_on_two_contexts_equals_reference_outputs(j1):
     """`--devices 0,0`: two contexts (one host thread each) share the chunk files of the sample and exchange the
-    histogram and the forests inside the process (cli.ThreadExchange) -- the multi-GPU path of the fused rule; the files
-    are the reference's, byte for byte"""
+    histogram and the forests inside the process (parallel.ThreadExchange) -- the multi-GPU path of the fused rule; the
+    files are the reference's, byte for byte"""
     case, tmp = j1["case"], j1["tmp"]
     outdir = tmp / "results_2ctx"
     argv = ["fused", "--k", str(case["k"]), "--hap1-asm", j1["asm"][0], "--hap2-asm", j1["asm"][1], "--hap1-reads", *j1["chunks"][0],

@@ -63,7 +63,9 @@ def _worker(rank, world, port, q):
         x = P.Exchange()
         h = torch.from_numpy(hist.copy())
         x.allreduce_hist(h)
-        peers = x.gather_forests(torch.from_numpy(par.astype(np.int32)))
+        gathered = x.gather_forests(torch.from_numpy(par.astype(np.int32)))
+        assert gathered.shape == (world, n) and gathered[rank].tolist() == par.tolist()
+        peers = [gathered[r] for r in range(world) if r != rank]
         merged = par.copy()
         for p in peers:
             pp = p.numpy()
