@@ -13,8 +13,9 @@
   python -m gavisunk_b200.cli split_ont --reads R.. --out temp/S/reads/hapN_1-of-10.fq.gz ..   (seqtk seq -F '#' | rustybam fastq-split)
   python -m gavisunk_b200.cli combine_ont_nofilt <chunk.sunkpos>.. <hapN_detailed.sunkpos>
   python -m gavisunk_b200.cli fused --sample S --k K --hap1-asm .. --hap2-asm .. --hap1-reads f.. --hap2-reads f.. --outdir D
-                                    [--devices 0,1,..] [--batch-files N] [--detailed] [--support-tracks]
+                                    [--devices 0,1,..] [--batch-files N] [--detailed] [--support-tracks] [--gap-evidence]
   python -m gavisunk_b200.cli support_tracks <sunkpos> <rlen> <bad_sunks.txt> <fai> <valid.bed> <out.reads.bed> <out.bedgraph> <out.tsv>
+  python -m gavisunk_b200.cli gap_evidence <sunkpos> <rlen> <bad_sunks.txt> <fai> <valid.bed> <out.gaps.reads.tsv> <out.gaps.evidence.tsv>
 
 The first four replace workflow/scripts/{kmerpos_annot3,rlen,diag_filter_v3,diag_filter_step2}
 (workflow/rules/tagONT.smk:36,73,92,110) one to one; the next six replace badsunks_AR.py,
@@ -24,7 +25,9 @@ argv of their rules (tagONT.smk:150,189,230,249; the two `script:` rules take th
 accept the snakemake object itself); `fused` replaces the rules from jellyfish_count
 to get_gaps and writes the same files under results/{sample}/.  `fused --support-tracks` and `support_tracks`
 add per-read placements, support depth and a per-contig summary of the validated reads (no reference
-counterpart: the reference only plots them, viz.py).  Text parsing / formatting is host
+counterpart: the reference only plots them, viz.py).  `fused --gap-evidence` and `gap_evidence` report, per gap, the
+reads that reach both of its sides and the size change their SUNK distances imply (no reference counterpart either).
+Text parsing / formatting is host
 plumbing; all per-base and per-row work runs in libgavisunk_b200.so.  Errors exit non-zero with a
 message on stderr and never leave a partial output file behind.
 """
@@ -358,6 +361,93 @@ def cmd_support_tracks(argv):
     support_tracks(*argv)
 
 
+# ------------------------------------------------------------------------------------------------
+# gap evidence: the reads that bridge each gap (no reference counterpart; DESIGN.md section 5.5b)
+# ------------------------------------------------------------------------------------------------
+GAP_EVIDENCE_HEADER = "contig\tstart\tend\tbridging_reads\tconsistent_reads\tmin_delta\tmedian_delta\tmax_delta\n"
+GAP_READS_HEADER = ("contig\tgap_start\tgap_end\tread\tread_len\tleft_id\tleft_start\tleft_pos\tright_id\tright_start\tright_pos\t"
+                    "delta\tconsistent\n")
+_BIT = gio.NameTable(["0", "1"])
+
+
+def gap_evidence_texts(gsel, gaps, names, ev, rtab, read_len, name_rank):
+    """The two gap-evidence files of one haplotype: gsel = indices into the gap arrays of its rows of hap{N}.gaps.bed, in
+    that file's order; ev = Engine.gap_evidence() with run-wide read indices; rtab / read_len / name_rank = name table,
+    length and bytewise name rank of every run-wide read.  delta = |right_pos - left_pos| - (right_start - left_start);
+    consistent = 9*ds < 10*dp < 11*ds.  -> (gaps.reads.tsv, gaps.evidence.tsv) bytes"""
+    ctab = gio.NameTable(names)
+    gsel = np.asarray(gsel, np.int64)
+    slot_of = np.full(len(gaps["contig"]), -1, np.int64)
+    slot_of[gsel] = np.arange(len(gsel))
+    slot = slot_of[ev["gap"].astype(np.int64)]
+    r = np.flatnonzero(slot >= 0)
+    r = r[np.lexsort((name_rank[ev["read"][r]], slot[r]))]
+    ds = ev["right_start"].astype(np.int64) - ev["left_start"].astype(np.int64)
+    dp = np.abs(ev["right_pos"].astype(np.int64) - ev["left_pos"].astype(np.int64))
+    delta = dp - ds
+    cons = ((9 * ds < 10 * dp) & (10 * dp < 11 * ds)).astype(np.uint32)
+    g = ev["gap"]
+    reads_tsv = GAP_READS_HEADER.encode() + gio.format_rows(
+        [("name", gaps["contig"][g], ctab), ("u32", gaps["start"][g]), ("u32", gaps["end"][g]), ("name", ev["read"], rtab),
+         ("u32", read_len[ev["read"]])] + [("u32", ev[c]) for c in ("left_id", "left_start", "left_pos", "right_id", "right_start", "right_pos")]
+        + [("i64", delta), ("name", cons, _BIT)], sel=r)
+    n = np.bincount(slot[r], minlength=len(gsel))
+    n_cons = np.bincount(slot[r], weights=cons[r], minlength=len(gsel)).astype(np.int64)
+    lo = np.concatenate([[0], np.cumsum(n)])
+    d_r = delta[r]
+    out = [GAP_EVIDENCE_HEADER]
+    for i, gi in enumerate(gsel.tolist()):
+        head = f"{names[gaps['contig'][gi]]}\t{int(gaps['start'][gi])}\t{int(gaps['end'][gi])}\t{int(n[i])}\t{int(n_cons[i])}"
+        if n[i] == 0:
+            out.append(head + "\t.\t.\t.\n")
+            continue
+        d = np.sort(d_r[lo[i]:lo[i + 1]])
+        out.append(head + f"\t{int(d[0])}\t{int(d[(len(d) - 1) // 2])}\t{int(d[-1])}\n")
+    return reads_tsv, "".join(out).encode("latin-1")
+
+
+def gap_evidence(sunkpos_p, rlen_p, badsunks_p, fai_p, valid_p, out_reads_tsv, out_evidence_tsv):
+    """Gap evidence of one haplotype from the files of the per-rule path ({hap}.sunkpos, {hap}.rlen, bad_sunks.txt, the
+    .fai, {hap}.valid.bed): gaps from the validated intervals as get_gaps finds them, reads grouped by (contig, read name)
+    as process_by_contig groups them per contig, the reference's fixed minimum read length."""
+    fai = gio.read_fai(fai_p)
+    names = [n for n, _ in fai]
+    rlen = _read_rlen(rlen_p)
+    with open(badsunks_p) as f:
+        badset = set(f.read().splitlines())
+    valid = _read_bed3(valid_p)
+    rows = list(dict.fromkeys(gio.read_sunkpos(sunkpos_p)))
+    known = set(names)
+    for r in rows:
+        if r[2] not in known:
+            raise KeyError(f"contig {r[2]} of {sunkpos_p} is not in {fai_p}")
+    for c, _, _ in valid:
+        if c not in known:
+            raise KeyError(f"contig {c} of {valid_p} is not in {fai_p}")
+    keyed = [(f"{r[2]}\t{r[0]}",) + tuple(r[1:]) for r in rows]
+    eng, keyed, keys, cnames, cols = _engine_with_rows(keyed, names)
+    rnames = [k.split("\t", 1)[1] for k in keys]
+    lens = np.asarray([min(rlen.get(n, 0), 0xFFFFFFFF) for n in rnames], np.uint32)
+    eng.set_reads_meta(lens)
+    eng.set_rows(1, *cols)
+    _set_bad(eng, badset, cnames)
+    cidx = {n: i for i, n in enumerate(cnames)}
+    eng.set_intervals([cidx[c] for c, _, _ in valid], [s for _, s, _ in valid], [e for _, _, e in valid], len(cnames))
+    gaps, _ = eng.gaps(np.asarray([l for _, l in fai], np.uint32))
+    ev = eng.gap_evidence(10000)  # the reference's fixed minimum read length (process-by-contig_lowmem_AR.py:106, SURVEY Q13)
+    rtab = gio.NameTable(rnames)
+    name_rank = np.empty(len(rnames), np.int64)
+    if rnames:
+        name_rank[np.argsort(rtab.as_bytes_array(), kind="stable")] = np.arange(len(rnames))
+    texts = gap_evidence_texts(np.arange(len(gaps["contig"])), gaps, cnames, ev, rtab, lens, name_rank)
+    for path, data in zip((out_reads_tsv, out_evidence_tsv), texts):
+        _write_bytes(path, data)
+
+
+def cmd_gap_evidence(argv):
+    gap_evidence(*argv)
+
+
 def cmd_get_gaps(argv):
     """get_gaps.py: paths are string-concatenated, so indir / outdir need their trailing slash (:30,70)"""
     fai1, fai2, sample, indir, outdir = argv
@@ -625,15 +715,17 @@ def plan_batches(files: Sequence[str], n_devices: int, batch_files: int = 0, bat
 
 
 def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int], batch_files: int = 0, batch_gbp: float = 12.0,
-              detailed: bool = False, threads: int = 0, min_read_len: int = 10000, coll=None, support_len=None):
+              detailed: bool = False, threads: int = 0, min_read_len: int = 10000, coll=None, support_len=None, gap_len=None):
     """The read side of the fused rule on engines whose SUNK database is loaded: the chunk files (scatter order, with
     the haplotype each belongs to) are grouped into batches (plan_batches); engine i owns a contiguous block of the
     batches and runs Engine.run_batches on it (one host thread per GPU, two exchanges per run).  Reads are parsed
     and 2-bit packed in one pass (gio.NativeReads(packed=True)) while the previous batch is on the GPU.
     coll: exchange object of a multi-PROCESS run (gavisunk_b200.parallel.EngineExchange) when `engines` is this rank's
     single engine.  support_len (contig lengths): also the support placements of every engine and the support runs,
-    with the difference arrays summed across engines by the histogram's exchange.  -> one result dict per engine
-    (read names / lengths / chunk tables, kept rows, validated pairs, intervals[, placements, support runs])."""
+    with the difference arrays summed across engines by the histogram's exchange.  gap_len (contig lengths): also the
+    gaps of every engine (the same on all: intervals are merged across engines) and the gap-evidence records of its own
+    reads.  -> one result dict per engine (read names / lengths / chunk tables, kept rows, validated pairs, intervals[,
+    placements, support runs][, gap evidence])."""
     import threading
     from concurrent.futures import ThreadPoolExecutor
     for p in files:
@@ -690,6 +782,9 @@ def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int]
             info.update(kept=eng.rows(1, pinned=True), pairs=eng.pairs(pinned=True), iv=iv)
             if support_len is not None:
                 info.update(placements=eng.placements(pinned=True), support=eng.support(support_len, allreduce=cx.allreduce_hist))
+            if gap_len is not None:
+                eng.gaps(gap_len)
+                info.update(gap_evidence=eng.gap_evidence(min_read_len))
             results[di] = info
         except BaseException as ex:  # noqa: BLE001 -- reported by the caller; peers must not wait for this rank
             errors.append(ex)
@@ -711,7 +806,7 @@ def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int]
 
 def run_fused(k: int, hap_asm: Sequence[str], hap_reads: Sequence[Sequence[str]], outdir: str, device: int = 0,
               devices: Sequence[int] = None, batch_files: int = 0, batch_gbp: float = 12.0, detailed: bool = False,
-              threads: int = 0, mrsfast_palindromes: bool = False, support_tracks: bool = False):
+              threads: int = 0, mrsfast_palindromes: bool = False, support_tracks: bool = False, gap_evidence: bool = False):
     """hap_asm: two FASTA paths; hap_reads: two lists of chunk files in scatter order.  Builds the SUNK database on
     every GPU of `devices`, runs the reads (run_reads) and writes every file of the rules between jellyfish_count and
     slop_gaps under `outdir`.  Returns the first device's engine."""
@@ -740,22 +835,23 @@ def run_fused(k: int, hap_asm: Sequence[str], hap_reads: Sequence[Sequence[str]]
             engines = list(ex.map(make, devices))
     clen = [len(s) for _, s in contigs]
     results = run_reads(engines, contig_hap, files, file_hap, batch_files, batch_gbp, detailed, threads,
-                        support_len=clen if support_tracks else None)
+                        support_len=clen if support_tracks else None, gap_len=np.asarray(clen, np.uint32) if gap_evidence else None)
     eng = engines[0]
     gaps, nodata = eng.gaps(np.asarray(clen, dtype=np.uint32))
     write_outputs(k, eng, results, clen, contig_hap, eng.contig_names, results[0]["iv"], gaps, nodata, outdir,
-                  detailed=detailed, palindromes=mrsfast_palindromes, support_tracks=support_tracks)
+                  detailed=detailed, palindromes=mrsfast_palindromes, support_tracks=support_tracks, gap_evidence=gap_evidence)
     for e in engines[1:]:
         e.close()
     return eng
 
 
 def write_outputs(k, eng, results, contig_len, contig_hap, names, iv, gaps, nodata, outdir, detailed=False, palindromes=False,
-                  db_files=True, support_tracks=False):
+                  db_files=True, support_tracks=False, gap_evidence=False):
     """every file of SURVEY Appendix C that the rules between jellyfish_count and slop_gaps produce (db_files=False:
     without the exports of the database itself -- db/jellyfish.db|.fa, mrsfast/kmer.loc and its per-contig copies
     breaks/*.loc -- which belong to the database build, not to a run over reads); support_tracks: also
-    final_out/hap{N}.reads.bed / .support.bedgraph / .support.tsv (run_reads(support_len=...) results)"""
+    final_out/hap{N}.reads.bed / .support.bedgraph / .support.tsv (run_reads(support_len=...) results); gap_evidence: also
+    final_out/hap{N}.gaps.reads.tsv / .gaps.evidence.tsv (run_reads(gap_len=...) results)"""
     d = lambda *p: os.path.join(outdir, *p)
     for sub in ("db", "mrsfast", "sunkpos", "breaks", "inter_outs", "bed_files", "final_out"):
         os.makedirs(d(sub), exist_ok=True)
@@ -850,6 +946,8 @@ def write_outputs(k, eng, results, contig_len, contig_hap, names, iv, gaps, noda
     kept_c = by_contig(kept["contig"], kept["read"])
     if support_tracks:
         placements = cat_rows("placements", ("read", "contig", "start", "end", "n_ids", "strand"))
+    if gap_evidence:  # a read lives on one engine: the records of all engines, read indices made run-wide
+        evidence = cat_rows("gap_evidence", Engine.GAP_EVIDENCE_COLUMNS)
     pair_c = by_contig(pairs["contig"], pairs["read"], name_rank)
     if db_files:
         loc_c = by_contig(db["contig"])
@@ -888,6 +986,10 @@ def write_outputs(k, eng, results, contig_len, contig_hap, names, iv, gaps, noda
                                   name_rank)
             for ext, data in zip(("reads.bed", "support.bedgraph", "support.tsv"), texts):
                 _write_bytes(d("final_out", f"hap{hn}.{ext}"), data)
+        if gap_evidence:
+            texts = gap_evidence_texts(gsel, gaps, names, evidence, rtab, lens, name_rank)
+            for ext, data in zip(("gaps.reads.tsv", "gaps.evidence.tsv"), texts):
+                _write_bytes(d("final_out", f"hap{hn}.{ext}"), data)
     from concurrent.futures import ThreadPoolExecutor
     n_cpu = len(os.sched_getaffinity(0)) if hasattr(os, "sched_getaffinity") else (os.cpu_count() or 1)
     workers = max(1, min(8, n_cpu // 2))
@@ -916,11 +1018,13 @@ def cmd_fused(argv):
                     help="write a palindromic SUNK twice into kmer.loc, as mrsfast reports it on both strands (SURVEY A.2; unpinned)")
     ap.add_argument("--support-tracks", action="store_true",
                     help="also write final_out/hap{N}.reads.bed, .support.bedgraph and .support.tsv (support of the validated reads)")
+    ap.add_argument("--gap-evidence", action="store_true",
+                    help="also write final_out/hap{N}.gaps.evidence.tsv and .gaps.reads.tsv (the reads that bridge each gap)")
     a = ap.parse_args(argv)
     devs = [int(x) for x in a.devices.split(",")] if a.devices else [a.device]
     run_fused(a.k, [a.hap1_asm, a.hap2_asm], [a.hap1_reads, a.hap2_reads], a.outdir, devices=devs, batch_files=a.batch_files,
               batch_gbp=a.batch_gbp, detailed=a.detailed, threads=a.threads, mrsfast_palindromes=a.mrsfast_palindromes,
-              support_tracks=a.support_tracks)
+              support_tracks=a.support_tracks, gap_evidence=a.gap_evidence)
 
 
 COMMANDS = {"kmerpos_annot3": (cmd_kmerpos_annot3, 4), "rlen": (cmd_rlen, 2), "diag_filter_v3": (cmd_diag_filter_v3, 2),
@@ -928,7 +1032,7 @@ COMMANDS = {"kmerpos_annot3": (cmd_kmerpos_annot3, 4), "rlen": (cmd_rlen, 2), "d
             "process_by_contig": (cmd_process_by_contig, None), "get_gaps": (cmd_get_gaps, 5), "slop_gaps": (cmd_slop_gaps, 3),
             "covprob": (cmd_covprob, None), "split_locs": (cmd_split_locs, None), "fused": (cmd_fused, None),
             "split_ont": (cmd_split_ont, None), "combine_ont_nofilt": (cmd_combine_ont_nofilt, None),
-            "support_tracks": (cmd_support_tracks, 8)}
+            "support_tracks": (cmd_support_tracks, 8), "gap_evidence": (cmd_gap_evidence, 7)}
 
 
 def main(argv=None):

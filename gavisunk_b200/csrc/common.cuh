@@ -167,6 +167,13 @@ struct gvs_ctx {
   u64 n_runs = 0;
   bool sup_ready = false;
 
+  // ---- gap evidence (gap_evidence.cu) ----
+  DevBuf ge_seg_start;              // segments of the kept rows when gvs_validate's are not current
+  DevBuf ge_cgap, ge_seg, ge_cand, ge_res;  // per contig gap range, per segment (first gap, count), candidates, their results
+  DevBuf ge_rec;                    // records: 8 columns of n_ge_cand entries, the first n_ge of each filled
+  u64 n_ge = 0, n_ge_cand = 0;
+  bool ge_ready = false;
+
   // ---- components / intervals / gaps ----
   DevBuf parent, present, comp_min, comp_max, comp_cnt;
   DevBuf iv_contig, iv_start, iv_end;

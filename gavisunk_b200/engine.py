@@ -587,6 +587,19 @@ class Engine:
         self._ck(self.lib.gvs_gaps_get(self.ctx, _ptr(g["contig"]), _ptr(g["start"]), _ptr(g["end"]), _ptr(nd)))
         return g, nd
 
+    GAP_EVIDENCE_COLUMNS = ("read", "gap", "left_id", "left_start", "left_pos", "right_id", "right_start", "right_pos")
+
+    def gap_evidence(self, min_read_len: int = 10000) -> Dict[str, np.ndarray]:
+        """The reads that bridge each gap of gaps() (no reference counterpart; include/gavisunk_b200.h gvs_gap_evidence):
+        one record per bridging (read, gap) of the kept rows minus the bad groups, reads of length >= min_read_len --
+        read (run-wide index), gap (index into the gaps() arrays), and the (ID, start, pos) of its left and right flank
+        rows.  Call gaps() on this engine first."""
+        n = C.c_uint64()
+        self._ck(self.lib.gvs_gap_evidence(self.ctx, int(min_read_len), C.byref(n)))
+        out = {c: np.zeros(int(n.value), np.uint32) for c in self.GAP_EVIDENCE_COLUMNS}
+        self._ck(self.lib.gvs_gap_evidence_get(self.ctx, *[_ptr(out[c]) for c in self.GAP_EVIDENCE_COLUMNS]))
+        return out
+
     def covprob_table(self, kbp, cnt, genome_kbp: float, pn: float) -> np.ndarray:
         """covprob.py:56-100."""
         kbp = _c(kbp, np.int64)

@@ -57,7 +57,8 @@ enum {
   GVS_ST_BAD = 9,       /* bad SUNK groups (gvs_bad_groups)                                       */
   GVS_ST_MERGE = 10,    /* union with the peers' forests (gvs_components_merge_all)               */
   GVS_ST_SUPPORT = 11,  /* support tracks (gvs_placements, gvs_support): no reference counterpart  */
-  GVS_ST_COUNT = 12
+  GVS_ST_EVIDENCE = 12, /* gap evidence (gvs_gap_evidence): no reference counterpart                */
+  GVS_ST_COUNT = 13
 };
 
 /* ------------------------------------------------------------------------------------------ */
@@ -364,6 +365,25 @@ int gvs_intervals_set(gvs_ctx* ctx, const uint32_t* contig, const uint32_t* star
 int gvs_gaps(gvs_ctx* ctx, const uint32_t* contig_len, uint64_t* n_gaps, uint64_t* n_nodata);
 int gvs_gaps_get(gvs_ctx* ctx, uint32_t* contig, uint32_t* start, uint32_t* end,
                  uint32_t* nodata_contig);
+
+/* Gap evidence: the reads that cross each gap without validating it.  No reference counterpart: the reference only
+ * draws pile-up plots (viz.py); this tells a gap without data from a gap the reads disagree with.
+ * Inputs: the kept rows (read, pos, contig, start, ID = group) of gvs_diag_filter / gvs_batches_bind / gvs_rows_set(1)
+ * minus the bad groups (when set), reads of length >= min_read_len, and the gaps of gvs_gaps (which must have run;
+ * gvs_validate need not).  A read's rows are those of its segment on the contig of its first row (gvs_diag_filter
+ * keeps one contig per read; callers of gvs_rows_set key reads by (contig, name)).  Per gap (contig, gs, ge) and read:
+ *   left row  ID <= gs, right row ID >= ge + 1 (sides by ID, as intervals are built from IDs);
+ *   anchored  another row of the same side with a different ID passes 9*|dstart| < 10*|dpos| < 11*|dstart| with it
+ *             (the validation's ratio test, process-by-contig_lowmem_AR.py:145-147, Q12);
+ *   bridging  at least one anchored left row and one anchored right row;
+ *   flanks    the anchored left row with the largest start (ties: smallest pos, then smallest ID) and the anchored
+ *             right row with the smallest start (ties: smallest pos, then smallest ID).
+ * One record per bridging (read, gap), in (read segment, gap) order.  gvs_gap_evidence_get: host buffers of
+ * *n_records entries, any pointer may be NULL; read is run-wide as in gvs_pairs_get, gap indexes the arrays of
+ * gvs_gaps_get.  The size change is the caller's: delta = |right_pos - left_pos| - (right_start - left_start). */
+int gvs_gap_evidence(gvs_ctx* ctx, uint32_t min_read_len, uint64_t* n_records);
+int gvs_gap_evidence_get(gvs_ctx* ctx, uint32_t* read, uint32_t* gap, uint32_t* left_id, uint32_t* left_start,
+                         uint32_t* left_pos, uint32_t* right_id, uint32_t* right_start, uint32_t* right_pos);
 
 /* covprob.py:56-100: table[0..3499] of gap-spanning probabilities from the read-length
  * histogram.  kbp[n_bins], cnt[n_bins] = distinct int(len/1000) values and their multiplicities
