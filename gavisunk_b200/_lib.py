@@ -71,6 +71,9 @@ PROTOTYPES = {
     "gvs_gaps_get": (C.c_int, [vp, vp, vp, vp, vp]),
     "gvs_gap_evidence": (C.c_int, [vp, C.c_uint32, u64p]),
     "gvs_gap_evidence_get": (C.c_int, [vp, vp, vp, vp, vp, vp, vp, vp, vp]),
+    "gvs_junction_screen": (C.c_int, [vp, C.c_uint32, u64p, u64p]),
+    "gvs_junctions": (C.c_int, [vp, u64p]),
+    "gvs_junctions_get": (C.c_int, [vp] * 14),
     "gvs_covprob_table": (C.c_int, [vp, vp, vp, C.c_uint32, C.c_double, C.c_double, vp]),
     "gvs_covprob_gaps": (C.c_int, [vp, vp, vp, C.c_uint64, vp, vp, vp, C.c_uint64, vp, vp, vp]),
     "gvs_slop": (C.c_int, [vp, vp, vp, vp, C.c_uint64, vp, C.c_uint32, C.c_int64]),
@@ -108,7 +111,8 @@ PROTOTYPES["gvs_format_rows"] = (C.c_int64, [C.POINTER(ColStruct), C.c_uint32, C
 
 GVS_E_KEYERROR = -3
 STAGES = {"probe": 0, "emit": 1, "diag": 2, "hist": 3, "validate": 4, "intervals": 5, "dbbuild": 6, "components": 7, "mode": 8,
-          "bad": 9, "merge": 10, "support": 11, "evidence": 12}
+          "bad": 9, "merge": 10, "support": 11, "evidence": 12, "screen": 13,
+          "junctions": 14}
 
 _lib = None
 

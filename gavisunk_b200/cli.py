@@ -14,8 +14,10 @@
   python -m gavisunk_b200.cli combine_ont_nofilt <chunk.sunkpos>.. <hapN_detailed.sunkpos>
   python -m gavisunk_b200.cli fused --sample S --k K --hap1-asm .. --hap2-asm .. --hap1-reads f.. --hap2-reads f.. --outdir D
                                     [--devices 0,1,..] [--batch-files N] [--detailed] [--support-tracks] [--gap-evidence]
+                                    [--junctions]
   python -m gavisunk_b200.cli support_tracks <sunkpos> <rlen> <bad_sunks.txt> <fai> <valid.bed> <out.reads.bed> <out.bedgraph> <out.tsv>
   python -m gavisunk_b200.cli gap_evidence <sunkpos> <rlen> <bad_sunks.txt> <fai> <valid.bed> <out.gaps.reads.tsv> <out.gaps.evidence.tsv>
+  python -m gavisunk_b200.cli junctions <hapN_detailed.sunkpos> <hapN.rlen> <bad_sunks.txt> <fai1> <fai2> <out.junctions.reads.tsv> <out.junctions.tsv>
 
 The first four replace workflow/scripts/{kmerpos_annot3,rlen,diag_filter_v3,diag_filter_step2}
 (workflow/rules/tagONT.smk:36,73,92,110) one to one; the next six replace badsunks_AR.py,
@@ -27,6 +29,8 @@ to get_gaps and writes the same files under results/{sample}/.  `fused --support
 add per-read placements, support depth and a per-contig summary of the validated reads (no reference
 counterpart: the reference only plots them, viz.py).  `fused --gap-evidence` and `gap_evidence` report, per gap, the
 reads that reach both of its sides and the size change their SUNK distances imply (no reference counterpart either).
+`fused --junctions` and `junctions` report the reads whose SUNKs jump from one contig to another, and cluster them into
+contig links and breakpoints (no reference counterpart: the diag filter keeps one contig per read).
 Text parsing / formatting is host
 plumbing; all per-base and per-row work runs in libgavisunk_b200.so.  Errors exit non-zero with a
 message on stderr and never leave a partial output file behind.
@@ -448,6 +452,127 @@ def cmd_gap_evidence(argv):
     gap_evidence(*argv)
 
 
+# ------------------------------------------------------------------------------------------------
+# junctions: reads whose SUNKs jump from one contig to another (no reference counterpart; DESIGN.md section 5.5c)
+# ------------------------------------------------------------------------------------------------
+JUNCTION_READS_HEADER = ("read\tread_len\tcontig1\tstrand1\tids1\tid1\tstart1\tpos1\tcontig2\tstrand2\tids2\tid2\tstart2\tpos2\t"
+                         "read_gap\tleave1\tenter2\timplied_gap\tclass\n")
+JUNCTION_CLUSTERS_HEADER = ("contig1\tstrand1\thap1\tstart1\tcontig2\tstrand2\thap2\tstart2\trecords\tlinks\tmedian_implied_gap\t"
+                            "class\n")
+_CLASS = gio.NameTable(["link", "breakpoint"])
+JUNCTION_CHAIN = 10000  # start distance that still chains two records into one cluster
+
+
+def junction_columns(jn, contig_len):
+    """Host columns of junction records (Engine.junctions()): read_gap = pos2 - pos1; leave1 = distance from flank 1 to
+    the end of contig1 the read leaves through (len1 - start1 on '+', start1 on '-'); enter2 = distance from the end of
+    contig2 the read enters through to flank 2 (start2 on '+', len2 - start2 on '-'); implied_gap = read_gap - leave1 -
+    enter2; link (class 0) when leave1 + enter2 <= read_gap + read_gap // 10 + 1000, else breakpoint (1).  The class is
+    a heuristic: a link is a read that leaves one contig near an end and enters the other near an end, within the
+    read gap plus 10 % and 1 kb of slack."""
+    clen = np.asarray(contig_len, np.int64)
+    s1, s2 = jn["start1"].astype(np.int64), jn["start2"].astype(np.int64)
+    read_gap = jn["pos2"].astype(np.int64) - jn["pos1"].astype(np.int64)
+    leave1 = np.where(jn["strand1"] == 0, clen[jn["contig1"]] - s1, s1)
+    enter2 = np.where(jn["strand2"] == 0, s2, clen[jn["contig2"]] - s2)
+    cls = (leave1 + enter2 > read_gap + read_gap // 10 + 1000).astype(np.uint32)
+    return read_gap, leave1, enter2, read_gap - leave1 - enter2, cls
+
+
+def junction_texts(jn, sel, names, contig_len, contig_hap, rtab, read_len, name_rank):
+    """The two junction files of one haplotype: jn = Engine.junctions() with run-wide read indices, sel = its records of
+    this haplotype's reads; contig_hap[c] = 0 / 1 (hap1 / hap2 .fai), anything else: neither; rtab / read_len /
+    name_rank = name table, length and bytewise name rank of every run-wide read.  -> (junctions.reads.tsv,
+    junctions.tsv) bytes.  Clusters: each record is canonicalised (sides swapped and both strands flipped when
+    (contig2, start2) < (contig1, start1)), keyed by (contig1, strand1, contig2, strand2), chained by start1 and then by
+    start2 (consecutive starts at most JUNCTION_CHAIN apart); a cluster reports lower medians and is a link when more
+    than half of its records are."""
+    ctab = gio.NameTable(names)
+    sel = np.asarray(sel, np.int64)
+    r = sel[np.lexsort((sel, name_rank[jn["read"][sel]]))]
+    read_gap, leave1, enter2, implied, cls = junction_columns(jn, contig_len)
+    cols = [("name", jn["read"], rtab), ("u32", read_len[jn["read"]])]
+    for side in "12":
+        cols += [("name", jn["contig" + side], ctab), ("name", jn["strand" + side], _STRAND)] + [("u32", jn[c + side]) for c in ("ids", "id", "start", "pos")]
+    cols += [("i64", read_gap), ("i64", leave1), ("i64", enter2), ("i64", implied), ("name", cls, _CLASS)]
+    reads_tsv = JUNCTION_READS_HEADER.encode() + gio.format_rows(cols, sel=r)
+    keyed = defaultdict(list)
+    for i in sel.tolist():
+        a = (int(jn["contig1"][i]), int(jn["strand1"][i]), int(jn["start1"][i]))
+        b = (int(jn["contig2"][i]), int(jn["strand2"][i]), int(jn["start2"][i]))
+        if (b[0], b[2]) < (a[0], a[2]):
+            a, b = (b[0], 1 - b[1], b[2]), (a[0], 1 - a[1], a[2])
+        keyed[(a[0], a[1], b[0], b[1])].append((a[2], b[2], int(implied[i]), int(cls[i]) == 0))
+
+    def chains(items, at):
+        items = sorted(items, key=lambda t: t[at])
+        out = [[items[0]]]
+        for t in items[1:]:
+            if t[at] - out[-1][-1][at] <= JUNCTION_CHAIN:
+                out[-1].append(t)
+            else:
+                out.append([t])
+        return out
+    lower_median = lambda v: sorted(v)[(len(v) - 1) // 2]
+    clusters = []
+    for (c1, d1, c2, d2), items in keyed.items():
+        for ch in chains(items, 0):
+            for cl in chains(ch, 1):
+                links = sum(t[3] for t in cl)
+                clusters.append((c1, lower_median([t[0] for t in cl]), c2, lower_median([t[1] for t in cl]), d1, d2, len(cl), links,
+                                 lower_median([t[2] for t in cl])))
+    clusters.sort()
+    hap = lambda c: str(int(contig_hap[c]) + 1) if int(contig_hap[c]) in (0, 1) else "."
+    sd = "+-"
+    out = [JUNCTION_CLUSTERS_HEADER]
+    for c1, s1, c2, s2, d1, d2, n, links, gap in clusters:
+        out.append(f"{names[c1]}\t{sd[d1]}\t{hap(c1)}\t{s1}\t{names[c2]}\t{sd[d2]}\t{hap(c2)}\t{s2}\t{n}\t{links}\t{gap}\t"
+                   f"{'link' if 2 * links > n else 'breakpoint'}\n")
+    return reads_tsv, "".join(out).encode("latin-1")
+
+
+def junctions(sunkpos_p, rlen_p, badsunks_p, fai1_p, fai2_p, out_reads_tsv, out_clusters_tsv):
+    """Junctions of one haplotype from the files of the per-rule path: {hap}_detailed.sunkpos (combine_ont_nofilt: every
+    match row, before the diag filter), {hap}.rlen, bad_sunks.txt and both .fai files (contigs in fai1-then-fai2 order).
+    A read is a run of consecutive rows with one name (diag_filter_v3.nim:64); the reference's fixed minimum read
+    length."""
+    fai = [gio.read_fai(fai1_p), gio.read_fai(fai2_p)]
+    names = [n for f in fai for n, _ in f]
+    clen = [l for f in fai for _, l in f]
+    chap = [0] * len(fai[0]) + [1] * len(fai[1])
+    rlen = _read_rlen(rlen_p)
+    with open(badsunks_p) as f:
+        badset = set(f.read().splitlines())
+    rows, cnames, rnames, cols = _rows_from_sunkpos(sunkpos_p)
+    cidx = {}
+    for i, n in enumerate(names):
+        cidx.setdefault(n, i)
+    for c in cnames:
+        if c not in cidx:
+            raise KeyError(f"contig {c} of {sunkpos_p} is in neither {fai1_p} nor {fai2_p}")
+    remap = np.asarray([cidx[c] for c in cnames] + [0], np.uint32)
+    cols = (cols[0], cols[1], remap[cols[2]], cols[3], cols[4])
+    eng = Engine(20)
+    eng.contig_names = names
+    lens = np.asarray([min(rlen.get(n, 0), 0xFFFFFFFF) for n in rnames], np.uint32)
+    eng.set_reads_meta(lens)
+    eng.set_rows(0, *cols)
+    _set_bad(eng, badset, names)
+    eng.junction_screen(10000)  # the reference's fixed minimum read length (process-by-contig_lowmem_AR.py:106, SURVEY Q13)
+    jn = eng.junctions()
+    rtab = gio.NameTable(rnames)
+    name_rank = np.empty(len(rnames), np.int64)
+    if rnames:
+        name_rank[np.argsort(rtab.as_bytes_array(), kind="stable")] = np.arange(len(rnames))
+    texts = junction_texts(jn, np.arange(len(jn["read"])), names, clen, chap, rtab, lens, name_rank)
+    for path, data in zip((out_reads_tsv, out_clusters_tsv), texts):
+        _write_bytes(path, data)
+
+
+def cmd_junctions(argv):
+    junctions(*argv)
+
+
 def cmd_get_gaps(argv):
     """get_gaps.py: paths are string-concatenated, so indir / outdir need their trailing slash (:30,70)"""
     fai1, fai2, sample, indir, outdir = argv
@@ -715,7 +840,8 @@ def plan_batches(files: Sequence[str], n_devices: int, batch_files: int = 0, bat
 
 
 def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int], batch_files: int = 0, batch_gbp: float = 12.0,
-              detailed: bool = False, threads: int = 0, min_read_len: int = 10000, coll=None, support_len=None, gap_len=None):
+              detailed: bool = False, threads: int = 0, min_read_len: int = 10000, coll=None, support_len=None, gap_len=None,
+              junctions: bool = False):
     """The read side of the fused rule on engines whose SUNK database is loaded: the chunk files (scatter order, with
     the haplotype each belongs to) are grouped into batches (plan_batches); engine i owns a contiguous block of the
     batches and runs Engine.run_batches on it (one host thread per GPU, two exchanges per run).  Reads are parsed
@@ -724,8 +850,9 @@ def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int]
     single engine.  support_len (contig lengths): also the support placements of every engine and the support runs,
     with the difference arrays summed across engines by the histogram's exchange.  gap_len (contig lengths): also the
     gaps of every engine (the same on all: intervals are merged across engines) and the gap-evidence records of its own
-    reads.  -> one result dict per engine (read names / lengths / chunk tables, kept rows, validated pairs, intervals[,
-    placements, support runs][, gap evidence])."""
+    reads.  junctions: also the junction records of every engine's own reads (each batch screened after its diag
+    filter, resolved with the run's bad groups).  -> one result dict per engine (read names / lengths / chunk tables,
+    kept rows, validated pairs, intervals[, placements, support runs][, gap evidence][, junctions])."""
     import threading
     from concurrent.futures import ThreadPoolExecutor
     for p in files:
@@ -776,7 +903,8 @@ def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int]
                         r0["read"] = r0["read"] + np.uint32(base)
                         info["rows0"].append(r0)
                 iv, bases = eng.run_batches([bind_for(bi) for bi in range(len(mine))], contig_hap, min_read_len=min_read_len,
-                                            allreduce_hist=cx.allreduce_hist, gather_forests=cx.gather_forests, on_batch=on_batch)
+                                            allreduce_hist=cx.allreduce_hist, gather_forests=cx.gather_forests, on_batch=on_batch,
+                                            junctions=junctions)
                 for old in held:
                     old.close()
             info.update(kept=eng.rows(1, pinned=True), pairs=eng.pairs(pinned=True), iv=iv)
@@ -785,6 +913,8 @@ def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int]
             if gap_len is not None:
                 eng.gaps(gap_len)
                 info.update(gap_evidence=eng.gap_evidence(min_read_len))
+            if junctions:
+                info.update(junctions=eng.junctions())
             results[di] = info
         except BaseException as ex:  # noqa: BLE001 -- reported by the caller; peers must not wait for this rank
             errors.append(ex)
@@ -806,7 +936,8 @@ def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int]
 
 def run_fused(k: int, hap_asm: Sequence[str], hap_reads: Sequence[Sequence[str]], outdir: str, device: int = 0,
               devices: Sequence[int] = None, batch_files: int = 0, batch_gbp: float = 12.0, detailed: bool = False,
-              threads: int = 0, mrsfast_palindromes: bool = False, support_tracks: bool = False, gap_evidence: bool = False):
+              threads: int = 0, mrsfast_palindromes: bool = False, support_tracks: bool = False, gap_evidence: bool = False,
+              junctions: bool = False):
     """hap_asm: two FASTA paths; hap_reads: two lists of chunk files in scatter order.  Builds the SUNK database on
     every GPU of `devices`, runs the reads (run_reads) and writes every file of the rules between jellyfish_count and
     slop_gaps under `outdir`.  Returns the first device's engine."""
@@ -835,23 +966,26 @@ def run_fused(k: int, hap_asm: Sequence[str], hap_reads: Sequence[Sequence[str]]
             engines = list(ex.map(make, devices))
     clen = [len(s) for _, s in contigs]
     results = run_reads(engines, contig_hap, files, file_hap, batch_files, batch_gbp, detailed, threads,
-                        support_len=clen if support_tracks else None, gap_len=np.asarray(clen, np.uint32) if gap_evidence else None)
+                        support_len=clen if support_tracks else None, gap_len=np.asarray(clen, np.uint32) if gap_evidence else None,
+                        junctions=junctions)
     eng = engines[0]
     gaps, nodata = eng.gaps(np.asarray(clen, dtype=np.uint32))
     write_outputs(k, eng, results, clen, contig_hap, eng.contig_names, results[0]["iv"], gaps, nodata, outdir,
-                  detailed=detailed, palindromes=mrsfast_palindromes, support_tracks=support_tracks, gap_evidence=gap_evidence)
+                  detailed=detailed, palindromes=mrsfast_palindromes, support_tracks=support_tracks, gap_evidence=gap_evidence,
+                  junctions=junctions)
     for e in engines[1:]:
         e.close()
     return eng
 
 
 def write_outputs(k, eng, results, contig_len, contig_hap, names, iv, gaps, nodata, outdir, detailed=False, palindromes=False,
-                  db_files=True, support_tracks=False, gap_evidence=False):
+                  db_files=True, support_tracks=False, gap_evidence=False, junctions=False):
     """every file of SURVEY Appendix C that the rules between jellyfish_count and slop_gaps produce (db_files=False:
     without the exports of the database itself -- db/jellyfish.db|.fa, mrsfast/kmer.loc and its per-contig copies
     breaks/*.loc -- which belong to the database build, not to a run over reads); support_tracks: also
     final_out/hap{N}.reads.bed / .support.bedgraph / .support.tsv (run_reads(support_len=...) results); gap_evidence: also
-    final_out/hap{N}.gaps.reads.tsv / .gaps.evidence.tsv (run_reads(gap_len=...) results)"""
+    final_out/hap{N}.gaps.reads.tsv / .gaps.evidence.tsv (run_reads(gap_len=...) results); junctions: also
+    final_out/hap{N}.junctions.reads.tsv / .junctions.tsv (run_reads(junctions=True) results)"""
     d = lambda *p: os.path.join(outdir, *p)
     for sub in ("db", "mrsfast", "sunkpos", "breaks", "inter_outs", "bed_files", "final_out"):
         os.makedirs(d(sub), exist_ok=True)
@@ -948,6 +1082,9 @@ def write_outputs(k, eng, results, contig_len, contig_hap, names, iv, gaps, noda
         placements = cat_rows("placements", ("read", "contig", "start", "end", "n_ids", "strand"))
     if gap_evidence:  # a read lives on one engine: the records of all engines, read indices made run-wide
         evidence = cat_rows("gap_evidence", Engine.GAP_EVIDENCE_COLUMNS)
+    if junctions:  # likewise
+        jn = cat_rows("junctions", Engine.JUNCTION_COLUMNS)
+        jn_hap = read_hap[jn["read"]] if len(jn["read"]) else np.zeros(0, np.uint8)
     pair_c = by_contig(pairs["contig"], pairs["read"], name_rank)
     if db_files:
         loc_c = by_contig(db["contig"])
@@ -990,6 +1127,10 @@ def write_outputs(k, eng, results, contig_len, contig_hap, names, iv, gaps, noda
             texts = gap_evidence_texts(gsel, gaps, names, evidence, rtab, lens, name_rank)
             for ext, data in zip(("gaps.reads.tsv", "gaps.evidence.tsv"), texts):
                 _write_bytes(d("final_out", f"hap{hn}.{ext}"), data)
+        if junctions:
+            texts = junction_texts(jn, np.flatnonzero(jn_hap == hap), names, clen, contig_hap, rtab, lens, name_rank)
+            for ext, data in zip(("junctions.reads.tsv", "junctions.tsv"), texts):
+                _write_bytes(d("final_out", f"hap{hn}.{ext}"), data)
     from concurrent.futures import ThreadPoolExecutor
     n_cpu = len(os.sched_getaffinity(0)) if hasattr(os, "sched_getaffinity") else (os.cpu_count() or 1)
     workers = max(1, min(8, n_cpu // 2))
@@ -1020,11 +1161,13 @@ def cmd_fused(argv):
                     help="also write final_out/hap{N}.reads.bed, .support.bedgraph and .support.tsv (support of the validated reads)")
     ap.add_argument("--gap-evidence", action="store_true",
                     help="also write final_out/hap{N}.gaps.evidence.tsv and .gaps.reads.tsv (the reads that bridge each gap)")
+    ap.add_argument("--junctions", action="store_true",
+                    help="also write final_out/hap{N}.junctions.reads.tsv and .junctions.tsv (reads that jump between contigs)")
     a = ap.parse_args(argv)
     devs = [int(x) for x in a.devices.split(",")] if a.devices else [a.device]
     run_fused(a.k, [a.hap1_asm, a.hap2_asm], [a.hap1_reads, a.hap2_reads], a.outdir, devices=devs, batch_files=a.batch_files,
               batch_gbp=a.batch_gbp, detailed=a.detailed, threads=a.threads, mrsfast_palindromes=a.mrsfast_palindromes,
-              support_tracks=a.support_tracks, gap_evidence=a.gap_evidence)
+              support_tracks=a.support_tracks, gap_evidence=a.gap_evidence, junctions=a.junctions)
 
 
 COMMANDS = {"kmerpos_annot3": (cmd_kmerpos_annot3, 4), "rlen": (cmd_rlen, 2), "diag_filter_v3": (cmd_diag_filter_v3, 2),
@@ -1032,7 +1175,8 @@ COMMANDS = {"kmerpos_annot3": (cmd_kmerpos_annot3, 4), "rlen": (cmd_rlen, 2), "d
             "process_by_contig": (cmd_process_by_contig, None), "get_gaps": (cmd_get_gaps, 5), "slop_gaps": (cmd_slop_gaps, 3),
             "covprob": (cmd_covprob, None), "split_locs": (cmd_split_locs, None), "fused": (cmd_fused, None),
             "split_ont": (cmd_split_ont, None), "combine_ont_nofilt": (cmd_combine_ont_nofilt, None),
-            "support_tracks": (cmd_support_tracks, 8), "gap_evidence": (cmd_gap_evidence, 7)}
+            "support_tracks": (cmd_support_tracks, 8), "gap_evidence": (cmd_gap_evidence, 7),
+            "junctions": (cmd_junctions, 7)}
 
 
 def main(argv=None):

@@ -15,7 +15,7 @@
 #include "common.cuh"
 
 // grow a device buffer to `need` bytes keeping its first `keep` bytes
-static int grow_keep(gvs_ctx* ctx, DevBuf& b, size_t need, size_t keep) {
+int grow_keep(gvs_ctx* ctx, DevBuf& b, size_t need, size_t keep) {
   if (b.cap >= need) return 0;
   size_t want = need + need / 2 + 256;
   void* p = nullptr;
@@ -60,6 +60,9 @@ extern "C" int gvs_batches_begin(gvs_ctx* ctx) {
   ctx->bad_ready = false;
   ctx->comp_ready = false;  // ... and gvs_intervals waits for the run's gvs_components_local
   ctx->val_ready = false;
+  ctx->jn_stash.n = 0;  // the junction screens of the run append from here (junctions.cu)
+  ctx->jn_reads = 0;
+  ctx->jn_in_run = true;
   return 0;
 }
 
@@ -112,6 +115,7 @@ extern "C" int gvs_batches_bind(gvs_ctx* ctx, uint64_t* n_rows, uint64_t* n_read
   ctx->match_ready = false;
   ctx->diag_ready = true;
   ctx->val_ready = false;
+  ctx->jn_in_run = false;
   if (n_rows) *n_rows = ctx->kept.n;
   if (n_reads) *n_reads = ctx->n_reads;
   return 0;

@@ -174,6 +174,16 @@ struct gvs_ctx {
   u64 n_ge = 0, n_ge_cand = 0;
   bool ge_ready = false;
 
+  // ---- junctions (junctions.cu) ----
+  Rows jn_stash;                    // rows gvs_junction_screen kept (run-wide read indices), input of gvs_junctions
+  u64 jn_reads = 0;                 // reads in jn_stash
+  bool jn_in_run = false;           // between gvs_batches_begin and gvs_batches_bind: a screen appends to jn_stash
+  DevBuf jn_seg_start, jn_row_seg, jn_seg_cnt;  // segments of the screened / stashed rows, per segment count or offset
+  DevBuf jn_flags, jn_scr;          // per-row flags (2 bytes) and per-row u32 scratch of gvs_junctions
+  DevBuf jn_rec;                    // records: 13 columns of jn_stride entries, the first n_jn of each filled
+  u64 n_jn = 0, jn_stride = 0;
+  bool jn_ready = false;
+
   // ---- components / intervals / gaps ----
   DevBuf parent, present, comp_min, comp_max, comp_cnt;
   DevBuf iv_contig, iv_start, iv_end;
@@ -500,6 +510,14 @@ static __global__ void __launch_bounds__(256) k_groups_sorted(const u32* __restr
   if (a > b || (a == b && g_id[i] >= g_id[i + 1])) atomicOr(err, 4u);
 }
 
+// the validation's ratio test on two rows (pos, start): 9*|dstart| < 10*|dpos| < 11*|dstart|
+// (process-by-contig_lowmem_AR.py:145-147, Q12); gap evidence and junctions anchor rows with it
+__device__ __forceinline__ bool gvs_ratio_ok(u32 pi, u32 si, u32 pj, u32 sj) {
+  const u64 ds = si > sj ? si - sj : sj - si;
+  const u64 dp = pi > pj ? pi - pj : pj - pi;
+  return 9 * ds < 10 * dp && 10 * dp < 11 * ds;
+}
+
 // small helpers to read device scalars (synchronises the stream)
 template <typename T>
 static int read_dev(gvs_ctx* ctx, const T* d, T* h, size_t n = 1) {
@@ -526,3 +544,4 @@ int gvs_tab_attach_gidx(gvs_ctx* ctx);                                 // table.
 int gvs_group_index_rows(gvs_ctx* ctx, const u32* contig, const u32* group, u64 n, u32* gidx_out);  // table.cu
 int gvs_build_segments(gvs_ctx* ctx, const u32* read, u64 n, DevBuf& seg_start, DevBuf& row_seg, u64* n_seg_out);  // diag.cu
 int gvs_reserve_rows(gvs_ctx* ctx, Rows& r, u64 n);
+int grow_keep(gvs_ctx* ctx, DevBuf& b, size_t need, size_t keep);  // batches.cu: grow to `need` bytes keeping the first `keep`

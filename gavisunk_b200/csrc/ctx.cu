@@ -179,10 +179,12 @@ extern "C" void gvs_destroy(gvs_ctx* c) {
                    &c->gap_contig, &c->gap_start, &c->gap_end, &c->nodata_contig, &c->read_len, &c->gt_keys, &c->gt_val,
                    &c->seg_orient, &c->rank_of, &c->rank_grp, &c->sup_diff, &c->pl_read, &c->pl_contig, &c->pl_start, &c->pl_end,
                    &c->pl_nids, &c->pl_strand, &c->pl_tmp, &c->sup_depth, &c->sup_gx, &c->sup_cstat, &c->run_contig, &c->run_start,
-                   &c->run_end, &c->run_depth, &c->ge_seg_start, &c->ge_cgap, &c->ge_seg, &c->ge_cand, &c->ge_res, &c->ge_rec};
+                   &c->run_end, &c->run_depth, &c->ge_seg_start, &c->ge_cgap, &c->ge_seg, &c->ge_cand, &c->ge_res, &c->ge_rec,
+                   &c->jn_seg_start, &c->jn_row_seg, &c->jn_seg_cnt, &c->jn_flags, &c->jn_scr, &c->jn_rec};
   for (DevBuf* b : all) gvs_release(*b);
   release_rows(c->rows);
   release_rows(c->kept);
+  release_rows(c->jn_stash);
   release_rows(c->stash);
   gvs_release(c->stash_len);
   for (int i = 0; i < GVS_ST_COUNT; i++) {

@@ -97,7 +97,7 @@ static inline char* put_cell(char* p, const gvs_col& c, uint64_t r) {
 
 extern "C" int64_t gvs_format_rows(const gvs_col* cols, uint32_t n_cols, uint64_t n_rows, const uint64_t* sel, uint64_t n_sel,
                                    char* out, uint64_t cap, int threads) {
-  if ((n_cols && !cols) || n_cols > 16) return GVS_E_ARG;
+  if ((n_cols && !cols) || n_cols > 32) return GVS_E_ARG;  // junctions.reads.tsv has 19 columns
   const uint64_t n = sel ? n_sel : n_rows;
   for (uint32_t c = 0; c < n_cols; c++) {
     if (cols[c].kind < GVS_COL_U32 || cols[c].kind > GVS_COL_KMER) return GVS_E_ARG;

@@ -14,12 +14,6 @@
 // picks the flanks with warp reductions; a second scan compacts the bridging candidates in candidate order.
 #include "common.cuh"
 
-__device__ __forceinline__ bool ge_pair_ok(u32 pi, u32 si, u32 pj, u32 sj) {
-  const u64 ds = si > sj ? si - sj : sj - si;
-  const u64 dp = pi > pj ? pi - pj : pj - pi;
-  return 9 * ds < 10 * dp && 10 * dp < 11 * ds;
-}
-
 // per contig [lo, hi) of its gaps (gaps are sorted by (contig, start)); contigs without gaps keep lo = hi = 0
 __global__ void __launch_bounds__(256) k_ge_contig_gaps(const u32* __restrict__ gc, u64 n, u32* lo, u32* hi) {
   const u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
@@ -108,7 +102,7 @@ __global__ void __launch_bounds__(256) k_ge_resolve(const GeRows R, const u32* _
     for (u32 j = a; j < b && !anchored; j++) {
       u32 idj = 0;
       if (side(j, idj) != si || idj == idi) continue;
-      anchored = ge_pair_ok(pi, sti, R.pos[j], R.start[j]);
+      anchored = gvs_ratio_ok(pi, sti, R.pos[j], R.start[j]);
     }
     if (!anchored) continue;
     if (si == 1) {

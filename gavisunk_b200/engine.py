@@ -430,7 +430,7 @@ class Engine:
         return self.n_kept, self.n_reads
 
     def run_batches(self, binds, contig_hap: Sequence[int], min_read_len: int = 10000, allreduce_hist=None,
-                    gather_forests=None, on_batch=None):
+                    gather_forests=None, on_batch=None, junctions: bool = False):
         """The hot path over a run whose reads come in several batches (a sample's chunk files, or the shard of
         them this GPU owns).  The reference gathers all chunks of a haplotype before the global stages
         (workflow/Snakefile:23-24, workflow/rules/tagONT.smk:112-131; badsunks_AR.py:20-27 counts over every
@@ -441,7 +441,8 @@ class Engine:
           2. ONE histogram all-reduce (`allreduce_hist`), bad groups, validation of all stashed rows, local
              forest, ONE forest all-gather (`gather_forests`), intervals.
         Results equal run_all() on the concatenation of the batches; read indices of rows(1) / pairs() count
-        through the batches in order.  Returns (intervals, [read_base of every batch])."""
+        through the batches in order.  junctions: also screen every batch after its diag filter (junction_screen),
+        so that junctions() reports the run's records afterwards.  Returns (intervals, [read_base of every batch])."""
         self.batches_begin()
         bases, hp = [], 0
         rows = best = 0
@@ -449,6 +450,8 @@ class Engine:
             bind(self)
             rows += self.match()
             best += self.diag_filter(contig_hap)[0]
+            if junctions:
+                self.junction_screen(min_read_len)
             hp = self.group_hist(accumulate=True)
             base = self.batch_stash()
             if on_batch is not None:
@@ -598,6 +601,28 @@ class Engine:
         self._ck(self.lib.gvs_gap_evidence(self.ctx, int(min_read_len), C.byref(n)))
         out = {c: np.zeros(int(n.value), np.uint32) for c in self.GAP_EVIDENCE_COLUMNS}
         self._ck(self.lib.gvs_gap_evidence_get(self.ctx, *[_ptr(out[c]) for c in self.GAP_EVIDENCE_COLUMNS]))
+        return out
+
+    JUNCTION_COLUMNS = ("read", "contig1", "strand1", "ids1", "id1", "start1", "pos1", "contig2", "strand2", "ids2", "id2",
+                        "start2", "pos2")
+
+    def junction_screen(self, min_read_len: int = 10000) -> Tuple[int, int]:
+        """Junction screen of the current match rows (after match() or set_rows(0); in run_batches before the batch's
+        stash): the anchored rows of qualifying contigs of reads with >= 2 of them join the run's junction stash
+        (include/gavisunk_b200.h gvs_junction_screen).  -> (rows, reads) in the stash"""
+        a, b = C.c_uint64(), C.c_uint64()
+        self._ck(self.lib.gvs_junction_screen(self.ctx, int(min_read_len), C.byref(a), C.byref(b)))
+        return int(a.value), int(b.value)
+
+    def junctions(self) -> Dict[str, np.ndarray]:
+        """Reads whose SUNKs jump from one contig to another (no reference counterpart; include/gavisunk_b200.h
+        gvs_junctions): one record per pair of consecutive blocks of a screened read, with the bad groups of this engine
+        (or none) -- read (run-wide index), then per side contig, strand (0 '+', 1 '-'), distinct IDs of the block and
+        the (ID, start, pos) of its row next to the junction."""
+        n = C.c_uint64()
+        self._ck(self.lib.gvs_junctions(self.ctx, C.byref(n)))
+        out = {c: np.zeros(int(n.value), np.uint32) for c in self.JUNCTION_COLUMNS}
+        self._ck(self.lib.gvs_junctions_get(self.ctx, *[_ptr(out[c]) for c in self.JUNCTION_COLUMNS]))
         return out
 
     def covprob_table(self, kbp, cnt, genome_kbp: float, pn: float) -> np.ndarray:

@@ -58,7 +58,9 @@ enum {
   GVS_ST_MERGE = 10,    /* union with the peers' forests (gvs_components_merge_all)               */
   GVS_ST_SUPPORT = 11,  /* support tracks (gvs_placements, gvs_support): no reference counterpart  */
   GVS_ST_EVIDENCE = 12, /* gap evidence (gvs_gap_evidence): no reference counterpart                */
-  GVS_ST_COUNT = 13
+  GVS_ST_SCREEN = 13,   /* junction screen of one batch (gvs_junction_screen)                     */
+  GVS_ST_JUNCTIONS = 14, /* junction records (gvs_junctions): no reference counterpart            */
+  GVS_ST_COUNT = 15
 };
 
 /* ------------------------------------------------------------------------------------------ */
@@ -384,6 +386,36 @@ int gvs_gaps_get(gvs_ctx* ctx, uint32_t* contig, uint32_t* start, uint32_t* end,
 int gvs_gap_evidence(gvs_ctx* ctx, uint32_t min_read_len, uint64_t* n_records);
 int gvs_gap_evidence_get(gvs_ctx* ctx, uint32_t* read, uint32_t* gap, uint32_t* left_id, uint32_t* left_start,
                          uint32_t* left_pos, uint32_t* right_id, uint32_t* right_start, uint32_t* right_pos);
+
+/* Junctions: reads whose SUNKs jump from one contig to another (contig-end links, misjoins, haplotype switches).  No
+ * reference counterpart: the diag filter keeps each read's rows on one best contig, and every later stage sees only those.
+ * Inputs: the rows (read, pos, contig, start, ID = group) of gvs_match / gvs_rows_set(0), in row order (gvs_match: pos
+ * ascending within a read), minus the rows of bad groups when bad groups are set, reads of length >= min_read_len.
+ * Every contig counts, both haplotypes included; the diag filter's choice plays no part.  Per read:
+ *   anchored     a row is anchored when another row of the read on the same contig with a different ID passes
+ *                9*|dstart| < 10*|dpos| < 11*|dstart| with it (the validation's ratio test, process-by-contig_lowmem_AR.py:145-147, Q12);
+ *   qualifying   a contig on which the read has >= 3 distinct anchored IDs;
+ *   blocks       the anchored rows of qualifying contigs, in row order, cut into maximal runs on one contig; runs of fewer
+ *                than 3 distinct IDs are dropped, then runs left adjacent on the same contig are merged (one pass);
+ *   strand       of a block: over the pairs of its rows with different IDs that pass the ratio test, 0 ('+') when at least
+ *                half have positions rising with starts, else 1 ('-');
+ *   records      one per consecutive block pair (B_i, B_i+1): read (run-wide, as in gvs_pairs_get), contig1, strand1,
+ *                ids1 (distinct IDs of B_i), (id1, start1, pos1) of B_i's last row, contig2, strand2, ids2,
+ *                (id2, start2, pos2) of B_i+1's first row; in (read, block) order.  Consecutive blocks lie on different
+ *                contigs: two clusters on one contig with no other contig between them give no record.
+ * gvs_junction_screen runs per batch between gvs_match (or gvs_rows_set(0)) and gvs_batch_stash: without bad groups
+ * it keeps the anchored rows of qualifying contigs of the reads with >= 2 qualifying contigs, with the read indices
+ * gvs_batch_stash gives the batch (exact: removing bad rows only removes anchors, and an anchor's partner is itself
+ * anchored).  gvs_batches_begin empties that stash and the screens of the run append to it; outside a batches run a
+ * screen replaces it.  *stash_rows / *stash_reads (may be NULL) = its size afterwards.  The screen writes no buffer of
+ * the other stages (rows(0), rows(1), gvs_best_get and the diag filter's segments stay as they were).
+ * gvs_junctions resolves the stash with the bad groups of gvs_bad_groups / gvs_bad_set (or none).
+ * gvs_junctions_get: host buffers of *n_records entries, any pointer may be NULL. */
+int gvs_junction_screen(gvs_ctx* ctx, uint32_t min_read_len, uint64_t* stash_rows, uint64_t* stash_reads);
+int gvs_junctions(gvs_ctx* ctx, uint64_t* n_records);
+int gvs_junctions_get(gvs_ctx* ctx, uint32_t* read, uint32_t* contig1, uint32_t* strand1, uint32_t* ids1, uint32_t* id1,
+                      uint32_t* start1, uint32_t* pos1, uint32_t* contig2, uint32_t* strand2, uint32_t* ids2, uint32_t* id2,
+                      uint32_t* start2, uint32_t* pos2);
 
 /* covprob.py:56-100: table[0..3499] of gap-spanning probabilities from the read-length
  * histogram.  kbp[n_bins], cnt[n_bins] = distinct int(len/1000) values and their multiplicities
