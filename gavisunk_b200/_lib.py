@@ -64,6 +64,10 @@ PROTOTYPES = {
     "gvs_placements_get": (C.c_int, [vp, vp, vp, vp, vp, vp, vp]),
     "gvs_support": (C.c_int, [vp, vp, u64p]),
     "gvs_support_get": (C.c_int, [vp, vp, vp, vp, vp]),
+    "gvs_spans": (C.c_int, [vp, C.c_uint32, C.c_uint32, u64p, C.POINTER(vp)]),
+    "gvs_spans_get": (C.c_int, [vp] * 9),
+    "gvs_discordance": (C.c_int, [vp, vp, u64p]),
+    "gvs_discordance_get": (C.c_int, [vp] * 7),
     "gvs_intervals": (C.c_int, [vp, u64p]),
     "gvs_intervals_get": (C.c_int, [vp, vp, vp, vp]),
     "gvs_intervals_set": (C.c_int, [vp, vp, vp, vp, C.c_uint64, C.c_uint32]),
@@ -112,7 +116,7 @@ PROTOTYPES["gvs_format_rows"] = (C.c_int64, [C.POINTER(ColStruct), C.c_uint32, C
 GVS_E_KEYERROR = -3
 STAGES = {"probe": 0, "emit": 1, "diag": 2, "hist": 3, "validate": 4, "intervals": 5, "dbbuild": 6, "components": 7, "mode": 8,
           "bad": 9, "merge": 10, "support": 11, "evidence": 12, "screen": 13,
-          "junctions": 14}
+          "junctions": 14, "discordance": 15}
 
 _lib = None
 

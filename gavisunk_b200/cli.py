@@ -14,10 +14,11 @@
   python -m gavisunk_b200.cli combine_ont_nofilt <chunk.sunkpos>.. <hapN_detailed.sunkpos>
   python -m gavisunk_b200.cli fused --sample S --k K --hap1-asm .. --hap2-asm .. --hap1-reads f.. --hap2-reads f.. --outdir D
                                     [--devices 0,1,..] [--batch-files N] [--detailed] [--support-tracks] [--gap-evidence]
-                                    [--junctions]
+                                    [--junctions] [--discordance]
   python -m gavisunk_b200.cli support_tracks <sunkpos> <rlen> <bad_sunks.txt> <fai> <valid.bed> <out.reads.bed> <out.bedgraph> <out.tsv>
   python -m gavisunk_b200.cli gap_evidence <sunkpos> <rlen> <bad_sunks.txt> <fai> <valid.bed> <out.gaps.reads.tsv> <out.gaps.evidence.tsv>
   python -m gavisunk_b200.cli junctions <hapN_detailed.sunkpos> <hapN.rlen> <bad_sunks.txt> <fai1> <fai2> <out.junctions.reads.tsv> <out.junctions.tsv>
+  python -m gavisunk_b200.cli discordance <sunkpos> <rlen> <bad_sunks.txt> <fai> <out.discordance.reads.tsv> <out.discordance.tsv> <out.discordance.bed>
 
 The first four replace workflow/scripts/{kmerpos_annot3,rlen,diag_filter_v3,diag_filter_step2}
 (workflow/rules/tagONT.smk:36,73,92,110) one to one; the next six replace badsunks_AR.py,
@@ -31,6 +32,8 @@ counterpart: the reference only plots them, viz.py).  `fused --gap-evidence` and
 reads that reach both of its sides and the size change their SUNK distances imply (no reference counterpart either).
 `fused --junctions` and `junctions` report the reads whose SUNKs jump from one contig to another, and cluster them into
 contig links and breakpoints (no reference counterpart: the diag filter keeps one contig per read).
+`fused --discordance` and `discordance` report collapses and expansions inside validated intervals, from the SUNK spacing
+of the validated reads across them (no reference counterpart).
 Text parsing / formatting is host
 plumbing; all per-base and per-row work runs in libgavisunk_b200.so.  Errors exit non-zero with a
 message on stderr and never leave a partial output file behind.
@@ -573,6 +576,108 @@ def cmd_junctions(argv):
     junctions(*argv)
 
 
+# ------------------------------------------------------------------------------------------------
+# distance discordance: collapses and expansions inside validated intervals (no reference counterpart; DESIGN.md 5.5d)
+# ------------------------------------------------------------------------------------------------
+DISCORDANCE_READS_HEADER = "contig\tread\tread_len\tid1\tstart1\tpos1\tid2\tstart2\tpos2\tdelta\tkind\n"
+DISCORDANCE_RUNS_HEADER = "contig\tstart\tend\tspans\tlonger\tshorter\n"
+DISCORDANCE_MIN_READS = 3  # supporting spans of a called segment (with a majority of all spans covering it)
+_SPAN_KIND = gio.NameTable(["longer", "shorter"])
+
+
+def discordance_calls(rec, runs, sel_runs, min_reads=DISCORDANCE_MIN_READS):
+    """Calls from the runs of Engine.discordance() (indices sel_runs, in run order) and the records of Engine.spans(): a run
+    is `collapse` when longer >= min_reads and 2*longer > spans, `expansion` likewise with shorter; adjacent runs of a
+    contig with the same call merge.  Peak = the run with the most supporting spans (ties: larger fraction, then the first);
+    size = lower median delta of the call's kind among the records that cover the peak's first base x (id1 <= x < id2: runs
+    start at group IDs, so these are the spans that cover the peak's segments).
+    -> list of (contig, start, end, kind, peak_start, peak_end, spans, supporting, size or None)"""
+    delta = np.abs(rec["pos2"].astype(np.int64) - rec["pos1"].astype(np.int64)) - (rec["start2"].astype(np.int64) - rec["start1"].astype(np.int64))
+    calls, cur = [], None
+    for i in np.asarray(sel_runs, np.int64).tolist():
+        c, sp, lo, sh = (int(runs[k][i]) for k in ("contig", "spans", "longer", "shorter"))
+        kind = "collapse" if lo >= min_reads and 2 * lo > sp else ("expansion" if sh >= min_reads and 2 * sh > sp else None)
+        if cur is not None and (kind is None or cur[0] != c or cur[1] != kind):
+            calls.append(cur)
+            cur = None
+        if kind is None:
+            continue
+        sup = lo if kind == "collapse" else sh
+        if cur is None:
+            cur = [c, kind, int(runs["start"][i]), 0, i, sp, sup]
+        elif sup > cur[6] or (sup == cur[6] and sup * cur[5] > cur[6] * sp):
+            cur[4:7] = [i, sp, sup]
+        cur[3] = int(runs["end"][i])
+    if cur is not None:
+        calls.append(cur)
+    out = []
+    for c, kind, a, b, pk, sp, sup in calls:
+        x = int(runs["start"][pk])
+        m = (rec["contig"] == c) & (rec["id1"] <= x) & (rec["id2"] > x) & ((delta >= 0) if kind == "collapse" else (delta < 0))
+        d = np.sort(delta[m])
+        out.append((c, a, b, kind, x, int(runs["end"][pk]), sp, sup, int(d[(len(d) - 1) // 2]) if len(d) else None))
+    return out
+
+
+def discordance_texts(hap_contigs, names, rec, runs, rtab, read_len, name_rank):
+    """The three discordance files of one haplotype: hap_contigs = its contig ids; rec = Engine.spans() with run-wide read
+    indices, runs = Engine.discordance(); rtab / read_len / name_rank = name table, length and bytewise name rank of every
+    run-wide read.  -> (discordance.reads.tsv, discordance.tsv, discordance.bed) bytes"""
+    ctab = gio.NameTable(names)
+    inhap = np.zeros(len(names), bool)
+    inhap[np.asarray(hap_contigs, np.int64)] = True
+    r = np.flatnonzero(inhap[rec["contig"]])
+    r = r[np.lexsort((name_rank[rec["read"][r]], rec["start2"][r], rec["start1"][r], rec["contig"][r]))]
+    delta = np.abs(rec["pos2"].astype(np.int64) - rec["pos1"].astype(np.int64)) - (rec["start2"].astype(np.int64) - rec["start1"].astype(np.int64))
+    reads_tsv = DISCORDANCE_READS_HEADER.encode() + gio.format_rows(
+        [("name", rec["contig"], ctab), ("name", rec["read"], rtab), ("u32", read_len[rec["read"]])]
+        + [("u32", rec[c]) for c in ("id1", "start1", "pos1", "id2", "start2", "pos2")]
+        + [("i64", delta), ("name", (delta < 0).astype(np.uint32), _SPAN_KIND)], sel=r)
+    q = np.flatnonzero(inhap[runs["contig"]])
+    runs_tsv = DISCORDANCE_RUNS_HEADER.encode() + gio.format_rows(
+        [("name", runs["contig"], ctab)] + [("u32", runs[c]) for c in ("start", "end", "spans", "longer", "shorter")], sel=q)
+    bed = "".join(f"{names[c]}\t{a}\t{b}\t{kind}\t{ps}\t{pe}\t{sp}\t{sup}\t{'.' if size is None else size}\n"
+                  for c, a, b, kind, ps, pe, sp, sup, size in discordance_calls(rec, runs, q))
+    return reads_tsv, runs_tsv, bed.encode("latin-1")
+
+
+def discordance(sunkpos_p, rlen_p, badsunks_p, fai_p, out_reads_tsv, out_runs_tsv, out_bed):
+    """Distance discordance of one haplotype from the files of the per-rule path ({hap}.sunkpos, {hap}.rlen,
+    bad_sunks.txt, the .fai): the whole haplotype is validated in one pass, reads grouped by (contig, read name) as
+    process_by_contig groups them per contig, the reference's fixed minimum read length."""
+    fai = gio.read_fai(fai_p)
+    names = [n for n, _ in fai]
+    rlen = _read_rlen(rlen_p)
+    with open(badsunks_p) as f:
+        badset = set(f.read().splitlines())
+    rows = list(dict.fromkeys(gio.read_sunkpos(sunkpos_p)))  # drop_duplicates (process-by-contig_lowmem_AR.py:104)
+    known = set(names)
+    for r in rows:
+        if r[2] not in known:
+            raise KeyError(f"contig {r[2]} of {sunkpos_p} is not in {fai_p}")
+    keyed = [(f"{r[2]}\t{r[0]}",) + tuple(r[1:]) for r in rows]
+    eng, keyed, keys, cnames, cols = _engine_with_rows(keyed, names)
+    rnames = [k.split("\t", 1)[1] for k in keys]
+    lens = np.asarray([min(rlen.get(n, 0), 0xFFFFFFFF) for n in rnames], np.uint32)
+    eng.set_reads_meta(lens)
+    eng.set_rows(1, *cols)
+    _set_bad(eng, badset, cnames)
+    eng.validate(10000)  # the reference's fixed minimum read length (process-by-contig_lowmem_AR.py:106, SURVEY Q13)
+    rec = eng.spans()
+    runs = eng.discordance([l for _, l in fai])
+    rtab = gio.NameTable(rnames)
+    name_rank = np.empty(len(rnames), np.int64)
+    if rnames:
+        name_rank[np.argsort(rtab.as_bytes_array(), kind="stable")] = np.arange(len(rnames))
+    texts = discordance_texts(list(range(len(names))), cnames, rec, runs, rtab, lens, name_rank)
+    for path, data in zip((out_reads_tsv, out_runs_tsv, out_bed), texts):
+        _write_bytes(path, data)
+
+
+def cmd_discordance(argv):
+    discordance(*argv)
+
+
 def cmd_get_gaps(argv):
     """get_gaps.py: paths are string-concatenated, so indir / outdir need their trailing slash (:30,70)"""
     fai1, fai2, sample, indir, outdir = argv
@@ -841,7 +946,7 @@ def plan_batches(files: Sequence[str], n_devices: int, batch_files: int = 0, bat
 
 def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int], batch_files: int = 0, batch_gbp: float = 12.0,
               detailed: bool = False, threads: int = 0, min_read_len: int = 10000, coll=None, support_len=None, gap_len=None,
-              junctions: bool = False):
+              junctions: bool = False, discordance_len=None):
     """The read side of the fused rule on engines whose SUNK database is loaded: the chunk files (scatter order, with
     the haplotype each belongs to) are grouped into batches (plan_batches); engine i owns a contiguous block of the
     batches and runs Engine.run_batches on it (one host thread per GPU, two exchanges per run).  Reads are parsed
@@ -851,8 +956,10 @@ def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int]
     with the difference arrays summed across engines by the histogram's exchange.  gap_len (contig lengths): also the
     gaps of every engine (the same on all: intervals are merged across engines) and the gap-evidence records of its own
     reads.  junctions: also the junction records of every engine's own reads (each batch screened after its diag
-    filter, resolved with the run's bad groups).  -> one result dict per engine (read names / lengths / chunk tables,
-    kept rows, validated pairs, intervals[, placements, support runs][, gap evidence][, junctions])."""
+    filter, resolved with the run's bad groups).  discordance_len (contig lengths): also the discordant spans of every
+    engine's own reads and the discordance runs, with the difference arrays summed like the support's.  -> one result dict
+    per engine (read names / lengths / chunk tables, kept rows, validated pairs, intervals[, placements, support runs][, gap
+    evidence][, junctions][, spans, discordance runs])."""
     import threading
     from concurrent.futures import ThreadPoolExecutor
     for p in files:
@@ -915,6 +1022,8 @@ def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int]
                 info.update(gap_evidence=eng.gap_evidence(min_read_len))
             if junctions:
                 info.update(junctions=eng.junctions())
+            if discordance_len is not None:
+                info.update(spans=eng.spans(), discordance=eng.discordance(discordance_len, allreduce=cx.allreduce_hist))
             results[di] = info
         except BaseException as ex:  # noqa: BLE001 -- reported by the caller; peers must not wait for this rank
             errors.append(ex)
@@ -937,7 +1046,7 @@ def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int]
 def run_fused(k: int, hap_asm: Sequence[str], hap_reads: Sequence[Sequence[str]], outdir: str, device: int = 0,
               devices: Sequence[int] = None, batch_files: int = 0, batch_gbp: float = 12.0, detailed: bool = False,
               threads: int = 0, mrsfast_palindromes: bool = False, support_tracks: bool = False, gap_evidence: bool = False,
-              junctions: bool = False):
+              junctions: bool = False, discordance: bool = False):
     """hap_asm: two FASTA paths; hap_reads: two lists of chunk files in scatter order.  Builds the SUNK database on
     every GPU of `devices`, runs the reads (run_reads) and writes every file of the rules between jellyfish_count and
     slop_gaps under `outdir`.  Returns the first device's engine."""
@@ -967,25 +1076,26 @@ def run_fused(k: int, hap_asm: Sequence[str], hap_reads: Sequence[Sequence[str]]
     clen = [len(s) for _, s in contigs]
     results = run_reads(engines, contig_hap, files, file_hap, batch_files, batch_gbp, detailed, threads,
                         support_len=clen if support_tracks else None, gap_len=np.asarray(clen, np.uint32) if gap_evidence else None,
-                        junctions=junctions)
+                        junctions=junctions, discordance_len=clen if discordance else None)
     eng = engines[0]
     gaps, nodata = eng.gaps(np.asarray(clen, dtype=np.uint32))
     write_outputs(k, eng, results, clen, contig_hap, eng.contig_names, results[0]["iv"], gaps, nodata, outdir,
                   detailed=detailed, palindromes=mrsfast_palindromes, support_tracks=support_tracks, gap_evidence=gap_evidence,
-                  junctions=junctions)
+                  junctions=junctions, discordance=discordance)
     for e in engines[1:]:
         e.close()
     return eng
 
 
 def write_outputs(k, eng, results, contig_len, contig_hap, names, iv, gaps, nodata, outdir, detailed=False, palindromes=False,
-                  db_files=True, support_tracks=False, gap_evidence=False, junctions=False):
+                  db_files=True, support_tracks=False, gap_evidence=False, junctions=False, discordance=False):
     """every file of SURVEY Appendix C that the rules between jellyfish_count and slop_gaps produce (db_files=False:
     without the exports of the database itself -- db/jellyfish.db|.fa, mrsfast/kmer.loc and its per-contig copies
     breaks/*.loc -- which belong to the database build, not to a run over reads); support_tracks: also
     final_out/hap{N}.reads.bed / .support.bedgraph / .support.tsv (run_reads(support_len=...) results); gap_evidence: also
     final_out/hap{N}.gaps.reads.tsv / .gaps.evidence.tsv (run_reads(gap_len=...) results); junctions: also
-    final_out/hap{N}.junctions.reads.tsv / .junctions.tsv (run_reads(junctions=True) results)"""
+    final_out/hap{N}.junctions.reads.tsv / .junctions.tsv (run_reads(junctions=True) results); discordance: also
+    final_out/hap{N}.discordance.reads.tsv / .discordance.tsv / .discordance.bed (run_reads(discordance_len=...) results)"""
     d = lambda *p: os.path.join(outdir, *p)
     for sub in ("db", "mrsfast", "sunkpos", "breaks", "inter_outs", "bed_files", "final_out"):
         os.makedirs(d(sub), exist_ok=True)
@@ -1085,6 +1195,8 @@ def write_outputs(k, eng, results, contig_len, contig_hap, names, iv, gaps, noda
     if junctions:  # likewise
         jn = cat_rows("junctions", Engine.JUNCTION_COLUMNS)
         jn_hap = read_hap[jn["read"]] if len(jn["read"]) else np.zeros(0, np.uint8)
+    if discordance:  # likewise; the runs are the same on every engine
+        spans = cat_rows("spans", Engine.SPAN_COLUMNS)
     pair_c = by_contig(pairs["contig"], pairs["read"], name_rank)
     if db_files:
         loc_c = by_contig(db["contig"])
@@ -1131,6 +1243,10 @@ def write_outputs(k, eng, results, contig_len, contig_hap, names, iv, gaps, noda
             texts = junction_texts(jn, np.flatnonzero(jn_hap == hap), names, clen, contig_hap, rtab, lens, name_rank)
             for ext, data in zip(("junctions.reads.tsv", "junctions.tsv"), texts):
                 _write_bytes(d("final_out", f"hap{hn}.{ext}"), data)
+        if discordance:
+            texts = discordance_texts(np.flatnonzero(chap == hap).tolist(), names, spans, results[0]["discordance"], rtab, lens, name_rank)
+            for ext, data in zip(("discordance.reads.tsv", "discordance.tsv", "discordance.bed"), texts):
+                _write_bytes(d("final_out", f"hap{hn}.{ext}"), data)
     from concurrent.futures import ThreadPoolExecutor
     n_cpu = len(os.sched_getaffinity(0)) if hasattr(os, "sched_getaffinity") else (os.cpu_count() or 1)
     workers = max(1, min(8, n_cpu // 2))
@@ -1163,11 +1279,15 @@ def cmd_fused(argv):
                     help="also write final_out/hap{N}.gaps.evidence.tsv and .gaps.reads.tsv (the reads that bridge each gap)")
     ap.add_argument("--junctions", action="store_true",
                     help="also write final_out/hap{N}.junctions.reads.tsv and .junctions.tsv (reads that jump between contigs)")
+    ap.add_argument("--discordance", action="store_true",
+                    help="also write final_out/hap{N}.discordance.reads.tsv, .discordance.tsv and .discordance.bed (collapses and "
+                         "expansions inside validated intervals)")
     a = ap.parse_args(argv)
     devs = [int(x) for x in a.devices.split(",")] if a.devices else [a.device]
     run_fused(a.k, [a.hap1_asm, a.hap2_asm], [a.hap1_reads, a.hap2_reads], a.outdir, devices=devs, batch_files=a.batch_files,
               batch_gbp=a.batch_gbp, detailed=a.detailed, threads=a.threads, mrsfast_palindromes=a.mrsfast_palindromes,
-              support_tracks=a.support_tracks, gap_evidence=a.gap_evidence, junctions=a.junctions)
+              support_tracks=a.support_tracks, gap_evidence=a.gap_evidence, junctions=a.junctions,
+              discordance=a.discordance)
 
 
 COMMANDS = {"kmerpos_annot3": (cmd_kmerpos_annot3, 4), "rlen": (cmd_rlen, 2), "diag_filter_v3": (cmd_diag_filter_v3, 2),
@@ -1176,7 +1296,7 @@ COMMANDS = {"kmerpos_annot3": (cmd_kmerpos_annot3, 4), "rlen": (cmd_rlen, 2), "d
             "covprob": (cmd_covprob, None), "split_locs": (cmd_split_locs, None), "fused": (cmd_fused, None),
             "split_ont": (cmd_split_ont, None), "combine_ont_nofilt": (cmd_combine_ont_nofilt, None),
             "support_tracks": (cmd_support_tracks, 8), "gap_evidence": (cmd_gap_evidence, 7),
-            "junctions": (cmd_junctions, 7)}
+            "junctions": (cmd_junctions, 7), "discordance": (cmd_discordance, 7)}
 
 
 def main(argv=None):

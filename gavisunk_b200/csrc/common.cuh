@@ -184,6 +184,16 @@ struct gvs_ctx {
   u64 n_jn = 0, jn_stride = 0;
   bool jn_ready = false;
 
+  // ---- discordance (discordance.cu) ----
+  DevBuf dc_diff;                   // int32[3][n_groups] by rank: spans, longer, shorter (+1 at a span's first group, -1 at its last)
+  DevBuf dc_scr, dc_seg;            // per kept row u32 scratch (4 arrays); per segment usable rows, records, record offset
+  DevBuf dc_rec;                    // records: 8 columns of dc_stride entries, the first n_dc of each filled
+  u64 n_dc = 0, dc_stride = 0;
+  bool dc_ready = false;
+  DevBuf dc_run_contig, dc_run_start, dc_run_end, dc_run_val;  // runs of gvs_discordance (val: 3 columns of n_dc_runs)
+  u64 n_dc_runs = 0;
+  bool dc_runs_ready = false;
+
   // ---- components / intervals / gaps ----
   DevBuf parent, present, comp_min, comp_max, comp_cnt;
   DevBuf iv_contig, iv_start, iv_end;
@@ -544,4 +554,12 @@ int gvs_tab_attach_gidx(gvs_ctx* ctx);                                 // table.
 int gvs_group_index_rows(gvs_ctx* ctx, const u32* contig, const u32* group, u64 n, u32* gidx_out);  // table.cu
 int gvs_build_segments(gvs_ctx* ctx, const u32* read, u64 n, DevBuf& seg_start, DevBuf& row_seg, u64* n_seg_out);  // diag.cu
 int gvs_reserve_rows(gvs_ctx* ctx, Rows& r, u64 n);
+// support.cu: group ranks in (contig, start) order (rank_of / rank_grp unless rank_identity), cached per group table
+int gvs_ensure_rank(gvs_ctx* ctx);
+// support.cu: runs of equal values over the groups in rank order that tile [0, contig_len) of every contig: diff = nv
+// difference arrays of n_groups int32 by rank, prefix-summed here; out.val receives nv columns of *n_runs entries
+struct RankRuns {
+  DevBuf *contig, *start, *end, *val;
+};
+int gvs_rank_runs(gvs_ctx* ctx, const i32* diff, u32 nv, const uint32_t* contig_len, RankRuns& out, u64* n_runs, const char* who);
 int grow_keep(gvs_ctx* ctx, DevBuf& b, size_t need, size_t keep);  // batches.cu: grow to `need` bytes keeping the first `keep`

@@ -180,7 +180,8 @@ extern "C" void gvs_destroy(gvs_ctx* c) {
                    &c->seg_orient, &c->rank_of, &c->rank_grp, &c->sup_diff, &c->pl_read, &c->pl_contig, &c->pl_start, &c->pl_end,
                    &c->pl_nids, &c->pl_strand, &c->pl_tmp, &c->sup_depth, &c->sup_gx, &c->sup_cstat, &c->run_contig, &c->run_start,
                    &c->run_end, &c->run_depth, &c->ge_seg_start, &c->ge_cgap, &c->ge_seg, &c->ge_cand, &c->ge_res, &c->ge_rec,
-                   &c->jn_seg_start, &c->jn_row_seg, &c->jn_seg_cnt, &c->jn_flags, &c->jn_scr, &c->jn_rec};
+                   &c->jn_seg_start, &c->jn_row_seg, &c->jn_seg_cnt, &c->jn_flags, &c->jn_scr, &c->jn_rec, &c->dc_diff, &c->dc_scr,
+                   &c->dc_seg, &c->dc_rec, &c->dc_run_contig, &c->dc_run_start, &c->dc_run_end, &c->dc_run_val};
   for (DevBuf* b : all) gvs_release(*b);
   release_rows(c->rows);
   release_rows(c->kept);

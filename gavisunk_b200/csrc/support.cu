@@ -53,7 +53,7 @@ static int rank_sort(gvs_ctx* ctx, DevBuf& key) {
   return 0;
 }
 
-static int ensure_rank(gvs_ctx* ctx) {
+int gvs_ensure_rank(gvs_ctx* ctx) {
   if (ctx->rank_gen == ctx->grp_gen) return 0;
   const u64 ng = ctx->n_groups;
   u32* err = (u32*)(ctx->counters.as<u64>() + 32);
@@ -121,7 +121,7 @@ extern "C" int gvs_placements(gvs_ctx* ctx, uint64_t* n, int32_t** diff_dev) {
   ctx->pl_ready = ctx->sup_ready = false;
   ctx->n_pl = 0;
   if (n) *n = 0;
-  CKR(ensure_rank(ctx));
+  CKR(gvs_ensure_rank(ctx));
   const u64 ng = ctx->n_groups;
   CKR(gvs_reserve(ctx, ctx->sup_diff, (ng ? ng : 1) * 4));
   CK(cudaMemsetAsync(ctx->sup_diff.p, 0, (ng ? ng : 1) * 4, ctx->stream));
@@ -193,13 +193,15 @@ extern "C" int gvs_placements_get(gvs_ctx* ctx, uint32_t* read_idx, uint32_t* co
 }
 
 // ---------------------------------------------------------------------------------------------
-// depth runs.  Per contig: a head run from 0 (depth 0) unless the first group starts at 0, then one run per group
-// whose depth differs from the previous group's; a run ends where the next run of its contig starts, the last at
-// the contig's length.  Contigs without groups are one head run.
+// runs of equal per-group values: support depth (one value), discordance counts (three, discordance.cu).  Per contig:
+// a head run from 0 (all values 0) unless the first group starts at 0, then one run per group whose values differ from
+// the previous group's; a run ends where the next run of its contig starts, the last at the contig's length.
+// Contigs without groups are one head run.
 // ---------------------------------------------------------------------------------------------
 struct RankView {
   const u32 *rg, *gc, *gs;  // rg null: rank = group index
-  const i32* depth;         // per rank
+  const i32* val;           // per rank, nv columns of ng
+  u32 nv;
   u64 ng;
   __device__ __forceinline__ u32 grp(u64 r) const { return rg ? rg[r] : (u32)r; }
   __device__ __forceinline__ u32 contig(u64 r) const { return gc[grp(r)]; }
@@ -207,15 +209,17 @@ struct RankView {
   __device__ __forceinline__ bool last(u64 r, u32 c) const { return r + 1 == ng || contig(r + 1) != c; }
   __device__ __forceinline__ u32 starts_run(u64 r) const {
     const u32 g = grp(r), c = gc[g];
-    const i32 d = depth[r];
-    return first(r, c) ? (gs[g] == 0 || d != 0) : (d != depth[r - 1]);
+    const bool head = first(r, c);
+    bool differs = false;
+    for (u32 t = 0; t < nv; t++) differs |= val[t * ng + r] != (head ? 0 : val[t * ng + r - 1]);
+    return (head && gs[g] == 0) || differs;
   }
 };
 
 // per contig: [0] run starts among its groups before it (exclusive scan), [1] ... after its last group,
 // [2] start of its first group (none: 0xFFFFFFFF), [3] index of its first run
 __global__ void __launch_bounds__(256) k_runs_groups(const RankView V, const u32* __restrict__ gx, const u32* __restrict__ cst, u32 nc,
-                                                     const u32* __restrict__ clen, u32* rc, u32* rs, u32* rd, u32* err) {
+                                                     const u32* __restrict__ clen, u32* rc, u32* rs, u32* rv, u64 nr, u32* err) {
   const u64 r = (u64)blockIdx.x * blockDim.x + threadIdx.x;
   if (r >= V.ng) return;
   const u32 g = V.grp(r), c = V.gc[g], s = V.gs[g];
@@ -225,15 +229,15 @@ __global__ void __launch_bounds__(256) k_runs_groups(const RankView V, const u32
   const u32 o = cst[3 * nc + c] + head + gx[r] - cst[c];
   rc[o] = c;
   rs[o] = s;
-  rd[o] = (u32)V.depth[r];
+  for (u32 t = 0; t < V.nv; t++) rv[t * nr + o] = (u32)V.val[t * V.ng + r];
 }
-__global__ void __launch_bounds__(256) k_runs_heads(const u32* __restrict__ cst, u32 nc, u32* rc, u32* rs, u32* rd) {
+__global__ void __launch_bounds__(256) k_runs_heads(const u32* __restrict__ cst, u32 nc, u32* rc, u32* rs, u32* rv, u32 nv, u64 nr) {
   const u32 c = blockIdx.x * blockDim.x + threadIdx.x;
   if (c >= nc || cst[2 * nc + c] == 0) return;
   const u32 o = cst[3 * nc + c];
   rc[o] = c;
   rs[o] = 0;
-  rd[o] = 0;
+  for (u32 t = 0; t < nv; t++) rv[t * nr + o] = 0;
 }
 __global__ void __launch_bounds__(256) k_runs_end(const u32* __restrict__ rc, const u32* __restrict__ rs, u64 n, const u32* __restrict__ clen,
                                                   u32* re) {
@@ -242,19 +246,13 @@ __global__ void __launch_bounds__(256) k_runs_end(const u32* __restrict__ rc, co
   re[i] = (i + 1 < n && rc[i + 1] == rc[i]) ? rs[i + 1] : clen[rc[i]];
 }
 
-extern "C" int gvs_support(gvs_ctx* ctx, const uint32_t* contig_len, uint64_t* n_runs) {
-  if (!ctx) return GVS_E_ARG;
-  if (!ctx->pl_ready) return gvs_fail(ctx, GVS_E_STATE, "gvs_support before gvs_placements");
+int gvs_rank_runs(gvs_ctx* ctx, const i32* diff, u32 nv, const uint32_t* contig_len, RankRuns& out, u64* n_runs, const char* who) {
   const u32 nc = ctx->n_contigs;
-  if (nc && !contig_len) return gvs_fail(ctx, GVS_E_ARG, "gvs_support: null contig_len");
-  CK(cudaSetDevice(ctx->device));
-  StageTimer tm(ctx, GVS_ST_SUPPORT);
-  ctx->sup_ready = false;
-  ctx->n_runs = 0;
-  if (n_runs) *n_runs = 0;
+  if (nc && !contig_len) return gvs_fail(ctx, GVS_E_ARG, "%s: null contig_len", who);
+  *n_runs = 0;
   const u64 ng = ctx->n_groups;
   CKR(to_dev(ctx, ctx->contig_len, contig_len, nc));
-  CKR(gvs_reserve(ctx, ctx->sup_depth, (ng ? ng : 1) * 4));
+  CKR(gvs_reserve(ctx, ctx->sup_depth, (ng ? ng : 1) * 4 * nv));
   CKR(gvs_reserve(ctx, ctx->sup_gx, (ng ? ng : 1) * 4));
   CKR(gvs_reserve(ctx, ctx->sup_cstat, ((u64)nc ? nc : 1) * 16));
   u32* cst = ctx->sup_cstat.as<u32>();
@@ -264,16 +262,17 @@ extern "C" int gvs_support(gvs_ctx* ctx, const uint32_t* contig_len, uint64_t* n
   V.rg = ctx->rank_identity ? nullptr : ctx->rank_grp.as<u32>();
   V.gc = ctx->grp_contig.as<u32>();
   V.gs = ctx->grp_start.as<u32>();
-  V.depth = ctx->sup_depth.as<i32>();
+  V.val = ctx->sup_depth.as<i32>();
+  V.nv = nv;
   V.ng = ng;
   u32* err = (u32*)(ctx->counters.as<u64>() + 35);
   CK(cudaMemsetAsync(err, 0, 4, ctx->stream));
   if (ng) {
-    const i32* diff = ctx->sup_diff.as<i32>();
-    i32* depth = ctx->sup_depth.as<i32>();
-    {
-      auto f = [diff] __device__(u64 r) -> i32 { return diff[r]; };
-      auto g = [depth] __device__(u64 r, i32 ex, i32 v) { depth[r] = ex + v; };
+    for (u32 t = 0; t < nv; t++) {
+      const i32* d = diff + t * ng;
+      i32* v = ctx->sup_depth.as<i32>() + t * ng;
+      auto f = [d] __device__(u64 r) -> i32 { return d[r]; };
+      auto g = [v] __device__(u64 r, i32 ex, i32 x) { v[r] = ex + x; };
       CKR((device_scan<i32>(ctx, ng, f, g, OpSum(), (i32*)nullptr)));
     }
     u32* gx = ctx->sup_gx.as<u32>();
@@ -297,18 +296,33 @@ extern "C" int gvs_support(gvs_ctx* ctx, const uint32_t* contig_len, uint64_t* n
   }
   u32 nr = 0;
   CKR(read_dev(ctx, tot, &nr));
-  CKR(gvs_reserve(ctx, ctx->run_contig, (u64)nr * 4));
-  CKR(gvs_reserve(ctx, ctx->run_start, (u64)nr * 4));
-  CKR(gvs_reserve(ctx, ctx->run_end, (u64)nr * 4));
-  CKR(gvs_reserve(ctx, ctx->run_depth, (u64)nr * 4));
+  CKR(gvs_reserve(ctx, *out.contig, (u64)nr * 4));
+  CKR(gvs_reserve(ctx, *out.start, (u64)nr * 4));
+  CKR(gvs_reserve(ctx, *out.end, (u64)nr * 4));
+  CKR(gvs_reserve(ctx, *out.val, (u64)nr * 4 * nv));
   const u32* clen = ctx->contig_len.as<u32>();
-  u32 *rc = ctx->run_contig.as<u32>(), *rs = ctx->run_start.as<u32>(), *rd = ctx->run_depth.as<u32>();
-  if (ng) LAUNCH(k_runs_groups, (unsigned)cdiv(ng, 256), 256, 0, V, ctx->sup_gx.as<u32>(), cst, nc, clen, rc, rs, rd, err);
-  if (nc) LAUNCH(k_runs_heads, (unsigned)cdiv(nc, 256), 256, 0, cst, nc, rc, rs, rd);
-  if (nr) LAUNCH(k_runs_end, (unsigned)cdiv(nr, 256), 256, 0, rc, rs, nr, clen, ctx->run_end.as<u32>());
+  u32 *rc = out.contig->as<u32>(), *rs = out.start->as<u32>(), *rv = out.val->as<u32>();
+  if (ng) LAUNCH(k_runs_groups, (unsigned)cdiv(ng, 256), 256, 0, V, ctx->sup_gx.as<u32>(), cst, nc, clen, rc, rs, rv, (u64)nr, err);
+  if (nc) LAUNCH(k_runs_heads, (unsigned)cdiv(nc, 256), 256, 0, cst, nc, rc, rs, rv, nv, (u64)nr);
+  if (nr) LAUNCH(k_runs_end, (unsigned)cdiv(nr, 256), 256, 0, rc, rs, nr, clen, out.end->as<u32>());
   u32 h = 0;
   CKR(read_dev(ctx, err, &h));
-  if (h) return gvs_fail(ctx, GVS_E_ARG, "gvs_support: a SUNK group starts at or beyond its contig's length");
+  if (h) return gvs_fail(ctx, GVS_E_ARG, "%s: a SUNK group starts at or beyond its contig's length", who);
+  *n_runs = nr;
+  return 0;
+}
+
+extern "C" int gvs_support(gvs_ctx* ctx, const uint32_t* contig_len, uint64_t* n_runs) {
+  if (!ctx) return GVS_E_ARG;
+  if (!ctx->pl_ready) return gvs_fail(ctx, GVS_E_STATE, "gvs_support before gvs_placements");
+  CK(cudaSetDevice(ctx->device));
+  StageTimer tm(ctx, GVS_ST_SUPPORT);
+  ctx->sup_ready = false;
+  ctx->n_runs = 0;
+  if (n_runs) *n_runs = 0;
+  RankRuns out{&ctx->run_contig, &ctx->run_start, &ctx->run_end, &ctx->run_depth};
+  u64 nr = 0;
+  CKR(gvs_rank_runs(ctx, ctx->sup_diff.as<i32>(), 1, contig_len, out, &nr, "gvs_support"));
   ctx->n_runs = nr;
   ctx->sup_ready = true;
   if (n_runs) *n_runs = nr;

@@ -564,6 +564,7 @@ extern "C" int gvs_validate(gvs_ctx* ctx, uint32_t min_read_len, uint64_t* n_pai
   StageTimer tm(ctx, GVS_ST_VALIDATE);
   ctx->val_ready = false;
   ctx->pl_ready = ctx->sup_ready = false;
+  ctx->dc_ready = ctx->dc_runs_ready = false;
   ctx->n_pairs = 0;
   if (n_pairs_out) *n_pairs_out = 0;
   Rows& R = ctx->kept;

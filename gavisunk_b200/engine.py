@@ -556,6 +556,34 @@ class Engine:
         self._ck(self.lib.gvs_support_get(self.ctx, _ptr(out["contig"]), _ptr(out["start"]), _ptr(out["end"]), _ptr(out["depth"])))
         return out
 
+    SPAN_COLUMNS = ("read", "contig", "id1", "start1", "pos1", "id2", "start2", "pos2")
+
+    def spans(self, min_delta: int = 300, rel_permille: int = 30) -> Dict[str, np.ndarray]:
+        """Distance discordance of the validated reads (no reference counterpart; include/gavisunk_b200.h gvs_spans), after
+        validate(): one record per non-concordant span between consecutive usable rows of a read -- read (run-wide
+        index), contig, and the (ID, start, pos) of both rows; delta = |pos2 - pos1| - (start2 - start1), longer when
+        delta >= 0.  Also leaves the per-rank difference arrays (spans, longer, shorter) on the device for discordance()."""
+        n, p = C.c_uint64(), C.c_void_p()
+        self._ck(self.lib.gvs_spans(self.ctx, int(min_delta), int(rel_permille), C.byref(n), C.byref(p)))
+        self._dc_diff_ptr = int(p.value or 0)
+        out = {c: np.zeros(int(n.value), np.uint32) for c in self.SPAN_COLUMNS}
+        self._ck(self.lib.gvs_spans_get(self.ctx, *[_ptr(out[c]) for c in self.SPAN_COLUMNS]))
+        return out
+
+    def discordance(self, contig_len: Sequence[int], allreduce=None) -> Dict[str, np.ndarray]:
+        """Discordance runs after spans(): (contig, start, end, spans, longer, shorter) tiling every contig.  With several
+        GPUs `allreduce(ptr, n)` sums the int32 difference arrays (n = 3 * n_groups) across ranks in place first (the
+        callable that sums the bad-SUNK histogram)."""
+        if allreduce is not None:
+            allreduce(self._dc_diff_ptr, 3 * self.db_groups())
+        cl = _c(contig_len, np.uint32)
+        n = C.c_uint64()
+        self._ck(self.lib.gvs_discordance(self.ctx, _ptr(cl), C.byref(n)))
+        cols = ("contig", "start", "end", "spans", "longer", "shorter")
+        out = {c: np.zeros(int(n.value), np.uint32) for c in cols}
+        self._ck(self.lib.gvs_discordance_get(self.ctx, *[_ptr(out[c]) for c in cols]))
+        return out
+
     def components_local(self) -> int:
         """this GPU's forest of the validated pairs; returns the device pointer of its uint32[n_groups] parent array"""
         p = C.c_void_p()

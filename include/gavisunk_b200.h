@@ -60,7 +60,8 @@ enum {
   GVS_ST_EVIDENCE = 12, /* gap evidence (gvs_gap_evidence): no reference counterpart                */
   GVS_ST_SCREEN = 13,   /* junction screen of one batch (gvs_junction_screen)                     */
   GVS_ST_JUNCTIONS = 14, /* junction records (gvs_junctions): no reference counterpart            */
-  GVS_ST_COUNT = 15
+  GVS_ST_DISCORDANCE = 15, /* distance discordance (gvs_spans, gvs_discordance): no reference counterpart */
+  GVS_ST_COUNT = 16
 };
 
 /* ------------------------------------------------------------------------------------------ */
@@ -356,6 +357,36 @@ int gvs_placements_get(gvs_ctx* ctx, uint32_t* read_idx, uint32_t* contig, uint3
  * entries, host memory) in (contig, start) order, maximal (adjacent runs of a contig differ in depth). */
 int gvs_support(gvs_ctx* ctx, const uint32_t* contig_len, uint64_t* n_runs);
 int gvs_support_get(gvs_ctx* ctx, uint32_t* contig, uint32_t* start, uint32_t* end, uint32_t* depth);
+
+/* Distance discordance: collapses and expansions inside validated intervals.  No reference counterpart.  The validation's
+ * ratio test passes a SUNK pair whose distances agree within 10 %, so a read validates across an event smaller than about a
+ * tenth of its reach; the spacing of its SUNKs still shows the event.
+ * Inputs: the kept rows (read, pos, contig, start, ID = group) of gvs_diag_filter / gvs_batches_bind / gvs_rows_set(1) minus
+ * the rows of bad groups (when set), and the validated IDs of each read from gvs_validate (which must have run; its
+ * min_read_len applies).  Per read (validation segment), on its rows of the contig of its first row:
+ *   usable row  a non-bad row whose ID is one of the read's validated IDs and which is the read's only non-bad row with
+ *               that ID (repeated IDs are ambiguous and skipped);
+ *   order       usable rows by (start, ID) -- distinct starts, as different groups cover disjoint start ranges;
+ *   span        each pair (a, b) of consecutive usable rows: dstart = start_b - start_a, dpos = |pos_b - pos_a|,
+ *               delta = dpos - dstart (signed, as gap evidence);
+ *   covers      segment r = [ID_r, ID_r+1) of a contig, r the group's rank in (contig, start) order, for
+ *               rank(ID_a) <= r < rank(ID_b): every span that covers a segment contains all of it;
+ *   class       longer when 1000*delta >= 1000*min_delta + rel_permille*dstart (the read has more sequence: collapse in
+ *               the assembly), else shorter when -1000*delta meets the same bound (expansion), else concordant.
+ * gvs_spans: *diff_dev receives int32[3][n_groups] by rank -- spans, longer, shorter -- with +1 at rank(ID_a) and -1 at
+ * rank(ID_b) of every span of its kind (zero without spans): several GPUs sum its 3*n_groups entries (as the histogram of
+ * gvs_group_hist) before gvs_discordance.  Records: one per non-concordant span, in (segment, span) order: read (run-wide,
+ * as in gvs_pairs_get), contig, (id1, start1, pos1) of a, (id2, start2, pos2) of b; longer iff delta >= 0.
+ * rel_permille <= 1000000.  gvs_spans_get: host buffers of *n_records entries, any pointer may be NULL.
+ * gvs_discordance: per base x, the spans covering x's segment, as runs (contig, start, end, spans, longer, shorter) that
+ * tile [0, contig_len[c]) of every contig in (contig, start) order, maximal (adjacent runs of a contig differ in one of
+ * the three), with a zero head run before a contig's first group as gvs_support tiles the depth. */
+int gvs_spans(gvs_ctx* ctx, uint32_t min_delta, uint32_t rel_permille, uint64_t* n_records, int32_t** diff_dev);
+int gvs_spans_get(gvs_ctx* ctx, uint32_t* read, uint32_t* contig, uint32_t* id1, uint32_t* start1, uint32_t* pos1, uint32_t* id2,
+                  uint32_t* start2, uint32_t* pos2);
+int gvs_discordance(gvs_ctx* ctx, const uint32_t* contig_len, uint64_t* n_runs);
+int gvs_discordance_get(gvs_ctx* ctx, uint32_t* contig, uint32_t* start, uint32_t* end, uint32_t* spans, uint32_t* longer,
+                        uint32_t* shorter);
 
 /* Intervals parsed from bed_files/{contig}_{hap}.bed instead of produced by gvs_intervals (the input
  * of get_gaps.py:30); any order, host memory. */
