@@ -44,7 +44,7 @@ import argparse
 import os
 import sys
 from collections import defaultdict
-from typing import Dict, List, Sequence, Tuple
+from typing import Dict, List, NamedTuple, Sequence, Tuple
 
 import numpy as np
 
@@ -217,6 +217,25 @@ def _read_rlen(path) -> Dict[str, int]:
     return rlen
 
 
+def _read_badsunks(path) -> set:
+    with open(path) as f:
+        return set(f.read().splitlines())
+
+
+def _read_lens(rlen: Dict[str, int], rnames) -> np.ndarray:
+    """u32 length of every read name ({hap}.rlen; 0 when missing, clipped to u32)"""
+    return np.asarray([min(rlen.get(n, 0), 0xFFFFFFFF) for n in rnames], np.uint32)
+
+
+def bytewise_rank(rtab) -> np.ndarray:
+    """Rank of every name of a NameTable in bytewise order, equal names in table order: the order in which
+    `for rname, g in grouped` visits reads (groupby sorts the names, process-by-contig_lowmem_AR.py:135-136) and in which
+    every per-read file lists them"""
+    rank = np.empty(len(rtab), np.int64)
+    rank[np.argsort(rtab.as_bytes_array(), kind="stable")] = np.arange(len(rtab))
+    return rank
+
+
 def _set_bad(eng, badset, cnames):
     """bad groups of a bad_sunks.txt ('contig:ID' lines) on the engine's contigs"""
     bc, bg = [], []
@@ -229,6 +248,40 @@ def _set_bad(eng, badset, cnames):
     eng.bad_set(bc, bg)
 
 
+def _keyed_hap(sunkpos_p, rlen_p, badsunks_p, fai_p, valid_p=None):
+    """One haplotype of the per-rule path ({hap}.sunkpos, {hap}.rlen, bad_sunks.txt, the .fai[, {hap}.valid.bed]) on a
+    kept-row engine with one read per (contig, read name), as process_by_contig groups the reads per contig, and the
+    read lengths and bad groups set.  -> (engine, contig names, contig lengths, validated intervals (None without
+    valid_p), (name table, lengths, bytewise name rank) of the reads)"""
+    fai = gio.read_fai(fai_p)
+    names = [n for n, _ in fai]
+    rlen = _read_rlen(rlen_p)
+    badset = _read_badsunks(badsunks_p)
+    valid = _read_bed3(valid_p) if valid_p is not None else []
+    rows = list(dict.fromkeys(gio.read_sunkpos(sunkpos_p)))  # drop_duplicates (process-by-contig_lowmem_AR.py:104)
+    cidx = {n: i for i, n in enumerate(names)}
+    for r in rows:
+        if r[2] not in cidx:
+            raise KeyError(f"contig {r[2]} of {sunkpos_p} is not in {fai_p}")
+    for c, _, _ in valid:
+        if c not in cidx:
+            raise KeyError(f"contig {c} of {valid_p} is not in {fai_p}")
+    # one engine read per (contig, read name): key the rows by both, the name stays the read's; every contig is in the
+    # .fai, so the engine's contigs are its contigs in its order
+    keyed = [(f"{r[2]}\t{r[0]}",) + tuple(r[1:]) for r in rows]
+    eng, keyed, keys, _, cols = _engine_with_rows(keyed, names)
+    rnames = [k.split("\t", 1)[1] for k in keys]
+    lens = _read_lens(rlen, rnames)
+    eng.set_reads_meta(lens)
+    eng.set_rows(1, *cols)
+    _set_bad(eng, badset, names)
+    iv = None if valid_p is None else dict(contig=np.asarray([cidx[c] for c, _, _ in valid], np.uint32),
+                                           start=np.asarray([s for _, s, _ in valid], np.uint32),
+                                           end=np.asarray([e for _, _, e in valid], np.uint32))
+    rtab = gio.NameTable(rnames)
+    return eng, names, [l for _, l in fai], iv, (rtab, lens, bytewise_rank(rtab))
+
+
 def process_by_contig(locs_p, sunkpos_p, rlen_p, badsunks_p, out_tsv, out_bed):
     """process-by-contig_lowmem_AR.py:30-260 for one breaks/{contig}_{hap}.sunkpos"""
     rlen = _read_rlen(rlen_p)
@@ -237,11 +290,10 @@ def process_by_contig(locs_p, sunkpos_p, rlen_p, badsunks_p, out_tsv, out_bed):
     if not rows:
         raise ValueError("No columns to parse from file (empty sunkpos, process-by-contig_lowmem_AR.py:60)")
     contig = rows[0][2]  # sunkposcat['chrom'].unique()[0] (:62)
-    with open(badsunks_p) as f:
-        badset = set(f.read().splitlines())
+    badset = _read_badsunks(badsunks_p)
     rows = list(dict.fromkeys(rows))  # drop_duplicates (:104) keeps the first of identical rows
     eng, rows, rnames, cnames, cols = _engine_with_rows(rows)
-    eng.set_reads_meta(np.asarray([min(rlen.get(n, 0), 0xFFFFFFFF) for n in rnames], np.uint32))
+    eng.set_reads_meta(_read_lens(rlen, rnames))
     eng.set_rows(1, *cols)
     eng.set_contigs([0] * len(cnames))
     _set_bad(eng, badset, cnames)
@@ -327,41 +379,10 @@ def support_tracks(sunkpos_p, rlen_p, badsunks_p, fai_p, valid_p, out_reads_bed,
     """Support tracks of one haplotype from the files of the per-rule path ({hap}.sunkpos, {hap}.rlen, bad_sunks.txt,
     the .fai, {hap}.valid.bed): the whole haplotype is validated in one pass, reads grouped by (contig, read name) as
     process_by_contig groups them per contig."""
-    fai = gio.read_fai(fai_p)
-    names = [n for n, _ in fai]
-    rlen = _read_rlen(rlen_p)
-    with open(badsunks_p) as f:
-        badset = set(f.read().splitlines())
-    valid = _read_bed3(valid_p)
-    rows = list(dict.fromkeys(gio.read_sunkpos(sunkpos_p)))  # drop_duplicates (process-by-contig_lowmem_AR.py:104)
-    known = set(names)
-    for r in rows:
-        if r[2] not in known:
-            raise KeyError(f"contig {r[2]} of {sunkpos_p} is not in {fai_p}")
-    for c, _, _ in valid:
-        if c not in known:
-            raise KeyError(f"contig {c} of {valid_p} is not in {fai_p}")
-    # one engine read per (contig, read name): key the rows by both, the name stays the read's
-    keyed = [(f"{r[2]}\t{r[0]}",) + tuple(r[1:]) for r in rows]
-    eng, keyed, keys, cnames, cols = _engine_with_rows(keyed, names)
-    rnames = [k.split("\t", 1)[1] for k in keys]
-    lens = np.asarray([min(rlen.get(n, 0), 0xFFFFFFFF) for n in rnames], np.uint32)
-    eng.set_reads_meta(lens)
-    eng.set_rows(1, *cols)
-    _set_bad(eng, badset, cnames)
+    eng, names, clen, iv, reads = _keyed_hap(sunkpos_p, rlen_p, badsunks_p, fai_p, valid_p)
     eng.validate(10000)  # the reference's fixed minimum read length (process-by-contig_lowmem_AR.py:106, SURVEY Q13)
-    pl = eng.placements()
-    runs = eng.support([l for _, l in fai])
-    cidx = {n: i for i, n in enumerate(cnames)}
-    iv = dict(contig=np.asarray([cidx[c] for c, _, _ in valid], np.uint32), start=np.asarray([s for _, s, _ in valid], np.uint32),
-              end=np.asarray([e for _, _, e in valid], np.uint32))
-    rtab = gio.NameTable(rnames)
-    name_rank = np.empty(len(rnames), np.int64)
-    if rnames:
-        name_rank[np.argsort(rtab.as_bytes_array(), kind="stable")] = np.arange(len(rnames))
-    texts = support_texts(list(range(len(names))), [l for _, l in fai], cnames, pl, runs, iv, rtab, lens, name_rank)
-    for path, data in zip((out_reads_bed, out_bedgraph, out_tsv), texts):
-        _write_bytes(path, data)
+    texts = support_texts(list(range(len(names))), clen, names, eng.placements(), eng.support(clen), iv, *reads)
+    _write_all((out_reads_bed, out_bedgraph, out_tsv), texts)
 
 
 def cmd_support_tracks(argv):
@@ -377,6 +398,12 @@ GAP_READS_HEADER = ("contig\tgap_start\tgap_end\tread\tread_len\tleft_id\tleft_s
 _BIT = gio.NameTable(["0", "1"])
 
 
+def span_delta(start1, pos1, start2, pos2) -> np.ndarray:
+    """Size change a read implies between two SUNKs it carries (gap evidence, discordant spans): |pos2 - pos1| -
+    (start2 - start1) in int64, > 0 when the read holds more bases between them than the assembly"""
+    return np.abs(pos2.astype(np.int64) - pos1.astype(np.int64)) - (start2.astype(np.int64) - start1.astype(np.int64))
+
+
 def gap_evidence_texts(gsel, gaps, names, ev, rtab, read_len, name_rank):
     """The two gap-evidence files of one haplotype: gsel = indices into the gap arrays of its rows of hap{N}.gaps.bed, in
     that file's order; ev = Engine.gap_evidence() with run-wide read indices; rtab / read_len / name_rank = name table,
@@ -390,8 +417,8 @@ def gap_evidence_texts(gsel, gaps, names, ev, rtab, read_len, name_rank):
     r = np.flatnonzero(slot >= 0)
     r = r[np.lexsort((name_rank[ev["read"][r]], slot[r]))]
     ds = ev["right_start"].astype(np.int64) - ev["left_start"].astype(np.int64)
-    dp = np.abs(ev["right_pos"].astype(np.int64) - ev["left_pos"].astype(np.int64))
-    delta = dp - ds
+    delta = span_delta(ev["left_start"], ev["left_pos"], ev["right_start"], ev["right_pos"])
+    dp = delta + ds
     cons = ((9 * ds < 10 * dp) & (10 * dp < 11 * ds)).astype(np.uint32)
     g = ev["gap"]
     reads_tsv = GAP_READS_HEADER.encode() + gio.format_rows(
@@ -417,38 +444,12 @@ def gap_evidence(sunkpos_p, rlen_p, badsunks_p, fai_p, valid_p, out_reads_tsv, o
     """Gap evidence of one haplotype from the files of the per-rule path ({hap}.sunkpos, {hap}.rlen, bad_sunks.txt, the
     .fai, {hap}.valid.bed): gaps from the validated intervals as get_gaps finds them, reads grouped by (contig, read name)
     as process_by_contig groups them per contig, the reference's fixed minimum read length."""
-    fai = gio.read_fai(fai_p)
-    names = [n for n, _ in fai]
-    rlen = _read_rlen(rlen_p)
-    with open(badsunks_p) as f:
-        badset = set(f.read().splitlines())
-    valid = _read_bed3(valid_p)
-    rows = list(dict.fromkeys(gio.read_sunkpos(sunkpos_p)))
-    known = set(names)
-    for r in rows:
-        if r[2] not in known:
-            raise KeyError(f"contig {r[2]} of {sunkpos_p} is not in {fai_p}")
-    for c, _, _ in valid:
-        if c not in known:
-            raise KeyError(f"contig {c} of {valid_p} is not in {fai_p}")
-    keyed = [(f"{r[2]}\t{r[0]}",) + tuple(r[1:]) for r in rows]
-    eng, keyed, keys, cnames, cols = _engine_with_rows(keyed, names)
-    rnames = [k.split("\t", 1)[1] for k in keys]
-    lens = np.asarray([min(rlen.get(n, 0), 0xFFFFFFFF) for n in rnames], np.uint32)
-    eng.set_reads_meta(lens)
-    eng.set_rows(1, *cols)
-    _set_bad(eng, badset, cnames)
-    cidx = {n: i for i, n in enumerate(cnames)}
-    eng.set_intervals([cidx[c] for c, _, _ in valid], [s for _, s, _ in valid], [e for _, _, e in valid], len(cnames))
-    gaps, _ = eng.gaps(np.asarray([l for _, l in fai], np.uint32))
+    eng, names, clen, iv, reads = _keyed_hap(sunkpos_p, rlen_p, badsunks_p, fai_p, valid_p)
+    eng.set_intervals(iv["contig"], iv["start"], iv["end"], len(names))
+    gaps, _ = eng.gaps(clen)
     ev = eng.gap_evidence(10000)  # the reference's fixed minimum read length (process-by-contig_lowmem_AR.py:106, SURVEY Q13)
-    rtab = gio.NameTable(rnames)
-    name_rank = np.empty(len(rnames), np.int64)
-    if rnames:
-        name_rank[np.argsort(rtab.as_bytes_array(), kind="stable")] = np.arange(len(rnames))
-    texts = gap_evidence_texts(np.arange(len(gaps["contig"])), gaps, cnames, ev, rtab, lens, name_rank)
-    for path, data in zip((out_reads_tsv, out_evidence_tsv), texts):
-        _write_bytes(path, data)
+    texts = gap_evidence_texts(np.arange(len(gaps["contig"])), gaps, names, ev, *reads)
+    _write_all((out_reads_tsv, out_evidence_tsv), texts)
 
 
 def cmd_gap_evidence(argv):
@@ -544,8 +545,7 @@ def junctions(sunkpos_p, rlen_p, badsunks_p, fai1_p, fai2_p, out_reads_tsv, out_
     clen = [l for f in fai for _, l in f]
     chap = [0] * len(fai[0]) + [1] * len(fai[1])
     rlen = _read_rlen(rlen_p)
-    with open(badsunks_p) as f:
-        badset = set(f.read().splitlines())
+    badset = _read_badsunks(badsunks_p)
     rows, cnames, rnames, cols = _rows_from_sunkpos(sunkpos_p)
     cidx = {}
     for i, n in enumerate(names):
@@ -557,19 +557,15 @@ def junctions(sunkpos_p, rlen_p, badsunks_p, fai1_p, fai2_p, out_reads_tsv, out_
     cols = (cols[0], cols[1], remap[cols[2]], cols[3], cols[4])
     eng = Engine(20)
     eng.contig_names = names
-    lens = np.asarray([min(rlen.get(n, 0), 0xFFFFFFFF) for n in rnames], np.uint32)
+    lens = _read_lens(rlen, rnames)
     eng.set_reads_meta(lens)
     eng.set_rows(0, *cols)
     _set_bad(eng, badset, names)
     eng.junction_screen(10000)  # the reference's fixed minimum read length (process-by-contig_lowmem_AR.py:106, SURVEY Q13)
     jn = eng.junctions()
     rtab = gio.NameTable(rnames)
-    name_rank = np.empty(len(rnames), np.int64)
-    if rnames:
-        name_rank[np.argsort(rtab.as_bytes_array(), kind="stable")] = np.arange(len(rnames))
-    texts = junction_texts(jn, np.arange(len(jn["read"])), names, clen, chap, rtab, lens, name_rank)
-    for path, data in zip((out_reads_tsv, out_clusters_tsv), texts):
-        _write_bytes(path, data)
+    texts = junction_texts(jn, np.arange(len(jn["read"])), names, clen, chap, rtab, lens, bytewise_rank(rtab))
+    _write_all((out_reads_tsv, out_clusters_tsv), texts)
 
 
 def cmd_junctions(argv):
@@ -592,7 +588,7 @@ def discordance_calls(rec, runs, sel_runs, min_reads=DISCORDANCE_MIN_READS):
     size = lower median delta of the call's kind among the records that cover the peak's first base x (id1 <= x < id2: runs
     start at group IDs, so these are the spans that cover the peak's segments).
     -> list of (contig, start, end, kind, peak_start, peak_end, spans, supporting, size or None)"""
-    delta = np.abs(rec["pos2"].astype(np.int64) - rec["pos1"].astype(np.int64)) - (rec["start2"].astype(np.int64) - rec["start1"].astype(np.int64))
+    delta = span_delta(rec["start1"], rec["pos1"], rec["start2"], rec["pos2"])
     calls, cur = [], None
     for i in np.asarray(sel_runs, np.int64).tolist():
         c, sp, lo, sh = (int(runs[k][i]) for k in ("contig", "spans", "longer", "shorter"))
@@ -628,7 +624,7 @@ def discordance_texts(hap_contigs, names, rec, runs, rtab, read_len, name_rank):
     inhap[np.asarray(hap_contigs, np.int64)] = True
     r = np.flatnonzero(inhap[rec["contig"]])
     r = r[np.lexsort((name_rank[rec["read"][r]], rec["start2"][r], rec["start1"][r], rec["contig"][r]))]
-    delta = np.abs(rec["pos2"].astype(np.int64) - rec["pos1"].astype(np.int64)) - (rec["start2"].astype(np.int64) - rec["start1"].astype(np.int64))
+    delta = span_delta(rec["start1"], rec["pos1"], rec["start2"], rec["pos2"])
     reads_tsv = DISCORDANCE_READS_HEADER.encode() + gio.format_rows(
         [("name", rec["contig"], ctab), ("name", rec["read"], rtab), ("u32", read_len[rec["read"]])]
         + [("u32", rec[c]) for c in ("id1", "start1", "pos1", "id2", "start2", "pos2")]
@@ -645,33 +641,10 @@ def discordance(sunkpos_p, rlen_p, badsunks_p, fai_p, out_reads_tsv, out_runs_ts
     """Distance discordance of one haplotype from the files of the per-rule path ({hap}.sunkpos, {hap}.rlen,
     bad_sunks.txt, the .fai): the whole haplotype is validated in one pass, reads grouped by (contig, read name) as
     process_by_contig groups them per contig, the reference's fixed minimum read length."""
-    fai = gio.read_fai(fai_p)
-    names = [n for n, _ in fai]
-    rlen = _read_rlen(rlen_p)
-    with open(badsunks_p) as f:
-        badset = set(f.read().splitlines())
-    rows = list(dict.fromkeys(gio.read_sunkpos(sunkpos_p)))  # drop_duplicates (process-by-contig_lowmem_AR.py:104)
-    known = set(names)
-    for r in rows:
-        if r[2] not in known:
-            raise KeyError(f"contig {r[2]} of {sunkpos_p} is not in {fai_p}")
-    keyed = [(f"{r[2]}\t{r[0]}",) + tuple(r[1:]) for r in rows]
-    eng, keyed, keys, cnames, cols = _engine_with_rows(keyed, names)
-    rnames = [k.split("\t", 1)[1] for k in keys]
-    lens = np.asarray([min(rlen.get(n, 0), 0xFFFFFFFF) for n in rnames], np.uint32)
-    eng.set_reads_meta(lens)
-    eng.set_rows(1, *cols)
-    _set_bad(eng, badset, cnames)
+    eng, names, clen, _, reads = _keyed_hap(sunkpos_p, rlen_p, badsunks_p, fai_p)
     eng.validate(10000)  # the reference's fixed minimum read length (process-by-contig_lowmem_AR.py:106, SURVEY Q13)
-    rec = eng.spans()
-    runs = eng.discordance([l for _, l in fai])
-    rtab = gio.NameTable(rnames)
-    name_rank = np.empty(len(rnames), np.int64)
-    if rnames:
-        name_rank[np.argsort(rtab.as_bytes_array(), kind="stable")] = np.arange(len(rnames))
-    texts = discordance_texts(list(range(len(names))), cnames, rec, runs, rtab, lens, name_rank)
-    for path, data in zip((out_reads_tsv, out_runs_tsv, out_bed), texts):
-        _write_bytes(path, data)
+    texts = discordance_texts(list(range(len(names))), names, eng.spans(), eng.discordance(clen), *reads)
+    _write_all((out_reads_tsv, out_runs_tsv, out_bed), texts)
 
 
 def cmd_discordance(argv):
@@ -910,6 +883,35 @@ def _write_bytes(path: str, data):
     os.replace(tmp, path)
 
 
+def _write_all(paths: Sequence[str], texts: Sequence[bytes]):
+    for path, data in zip(paths, texts):
+        _write_bytes(path, data)
+
+
+class Evidence(NamedTuple):
+    """An optional output of `fused` that the reference does not produce"""
+    flag: str
+    help: str
+    records: str                  # run_reads' result key of its per-engine records, concatenated run-wide
+    columns: Tuple[str, ...]      # their columns
+    suffixes: Tuple[str, ...]     # final_out/hap{N}.{suffix}, in the order its *_texts returns them
+
+
+EVIDENCE_PRODUCTS = {
+    "support_tracks": Evidence("--support-tracks", "also write final_out/hap{N}.reads.bed, .support.bedgraph and .support.tsv "
+                               "(support of the validated reads)", "placements", Engine.PLACEMENT_COLUMNS,
+                               ("reads.bed", "support.bedgraph", "support.tsv")),
+    "gap_evidence": Evidence("--gap-evidence", "also write final_out/hap{N}.gaps.evidence.tsv and .gaps.reads.tsv (the reads "
+                             "that bridge each gap)", "gap_evidence", Engine.GAP_EVIDENCE_COLUMNS,
+                             ("gaps.reads.tsv", "gaps.evidence.tsv")),
+    "junctions": Evidence("--junctions", "also write final_out/hap{N}.junctions.reads.tsv and .junctions.tsv (reads that jump "
+                          "between contigs)", "junctions", Engine.JUNCTION_COLUMNS, ("junctions.reads.tsv", "junctions.tsv")),
+    "discordance": Evidence("--discordance", "also write final_out/hap{N}.discordance.reads.tsv, .discordance.tsv and "
+                            ".discordance.bed (collapses and expansions inside validated intervals)", "spans", Engine.SPAN_COLUMNS,
+                            ("discordance.reads.tsv", "discordance.tsv", "discordance.bed")),
+}
+
+
 def plan_batches(files: Sequence[str], n_devices: int, batch_files: int = 0, batch_gbp: float = 12.0) -> List[List[int]]:
     """groups of consecutive chunk files (scatter order: hap1 chunks, then hap2 chunks).  batch_files > 0 fixes the
     group size; otherwise groups hold about `batch_gbp` Gbp (estimated from the file sizes: FASTQ = 2 bytes per
@@ -945,26 +947,29 @@ def plan_batches(files: Sequence[str], n_devices: int, batch_files: int = 0, bat
 
 
 def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int], batch_files: int = 0, batch_gbp: float = 12.0,
-              detailed: bool = False, threads: int = 0, min_read_len: int = 10000, coll=None, support_len=None, gap_len=None,
-              junctions: bool = False, discordance_len=None):
+              detailed: bool = False, threads: int = 0, min_read_len: int = 10000, coll=None, products: Sequence[str] = (),
+              contig_len=None):
     """The read side of the fused rule on engines whose SUNK database is loaded: the chunk files (scatter order, with
     the haplotype each belongs to) are grouped into batches (plan_batches); engine i owns a contiguous block of the
     batches and runs Engine.run_batches on it (one host thread per GPU, two exchanges per run).  Reads are parsed
     and 2-bit packed in one pass (gio.NativeReads(packed=True)) while the previous batch is on the GPU.
     coll: exchange object of a multi-PROCESS run (gavisunk_b200.parallel.EngineExchange) when `engines` is this rank's
-    single engine.  support_len (contig lengths): also the support placements of every engine and the support runs,
-    with the difference arrays summed across engines by the histogram's exchange.  gap_len (contig lengths): also the
-    gaps of every engine (the same on all: intervals are merged across engines) and the gap-evidence records of its own
-    reads.  junctions: also the junction records of every engine's own reads (each batch screened after its diag
-    filter, resolved with the run's bad groups).  discordance_len (contig lengths): also the discordant spans of every
-    engine's own reads and the discordance runs, with the difference arrays summed like the support's.  -> one result dict
-    per engine (read names / lengths / chunk tables, kept rows, validated pairs, intervals[, placements, support runs][, gap
-    evidence][, junctions][, spans, discordance runs])."""
+    single engine.  products: names of EVIDENCE_PRODUCTS to compute as well (contig_len: the contig lengths) --
+    support_tracks: the support placements of every engine and the support runs, with the difference arrays summed
+    across engines by the histogram's exchange; gap_evidence: the gaps of every engine (the same on all: intervals are
+    merged across engines) and the gap-evidence records of its own reads; junctions: the junction records of every
+    engine's own reads (each batch screened after its diag filter, resolved with the run's bad groups); discordance: the
+    discordant spans of every engine's own reads and the discordance runs, with the difference arrays summed like the
+    support's.  -> one result dict per engine (read names / lengths / chunk tables, kept rows, validated pairs,
+    intervals[, placements, support runs][, gap evidence][, junctions][, spans, discordance runs])."""
     import threading
     from concurrent.futures import ThreadPoolExecutor
     for p in files:
         if not os.path.exists(p):
             raise FileNotFoundError(p)
+    for p in products:
+        if p not in EVIDENCE_PRODUCTS:
+            raise ValueError(f"unknown evidence product {p!r}")
     n_dev = len(engines)
     batches = plan_batches(files, n_dev, batch_files, batch_gbp)
     shards = shard_chunks(len(batches), n_dev)
@@ -1011,19 +1016,19 @@ def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int]
                         info["rows0"].append(r0)
                 iv, bases = eng.run_batches([bind_for(bi) for bi in range(len(mine))], contig_hap, min_read_len=min_read_len,
                                             allreduce_hist=cx.allreduce_hist, gather_forests=cx.gather_forests, on_batch=on_batch,
-                                            junctions=junctions)
+                                            junctions="junctions" in products)
                 for old in held:
                     old.close()
             info.update(kept=eng.rows(1, pinned=True), pairs=eng.pairs(pinned=True), iv=iv)
-            if support_len is not None:
-                info.update(placements=eng.placements(pinned=True), support=eng.support(support_len, allreduce=cx.allreduce_hist))
-            if gap_len is not None:
-                eng.gaps(gap_len)
+            if "support_tracks" in products:
+                info.update(placements=eng.placements(pinned=True), support=eng.support(contig_len, allreduce=cx.allreduce_hist))
+            if "gap_evidence" in products:
+                eng.gaps(contig_len)
                 info.update(gap_evidence=eng.gap_evidence(min_read_len))
-            if junctions:
+            if "junctions" in products:
                 info.update(junctions=eng.junctions())
-            if discordance_len is not None:
-                info.update(spans=eng.spans(), discordance=eng.discordance(discordance_len, allreduce=cx.allreduce_hist))
+            if "discordance" in products:
+                info.update(spans=eng.spans(), discordance=eng.discordance(contig_len, allreduce=cx.allreduce_hist))
             results[di] = info
         except BaseException as ex:  # noqa: BLE001 -- reported by the caller; peers must not wait for this rank
             errors.append(ex)
@@ -1045,11 +1050,11 @@ def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int]
 
 def run_fused(k: int, hap_asm: Sequence[str], hap_reads: Sequence[Sequence[str]], outdir: str, device: int = 0,
               devices: Sequence[int] = None, batch_files: int = 0, batch_gbp: float = 12.0, detailed: bool = False,
-              threads: int = 0, mrsfast_palindromes: bool = False, support_tracks: bool = False, gap_evidence: bool = False,
-              junctions: bool = False, discordance: bool = False):
+              threads: int = 0, mrsfast_palindromes: bool = False, products: Sequence[str] = ()):
     """hap_asm: two FASTA paths; hap_reads: two lists of chunk files in scatter order.  Builds the SUNK database on
     every GPU of `devices`, runs the reads (run_reads) and writes every file of the rules between jellyfish_count and
-    slop_gaps under `outdir`.  Returns the first device's engine."""
+    slop_gaps under `outdir`, and the files of the EVIDENCE_PRODUCTS named in `products`.  Returns the first device's
+    engine."""
     from concurrent.futures import ThreadPoolExecutor
     devices = list(devices) if devices else [device]
     contigs, contig_hap, fai = [], [], [[], []]
@@ -1074,28 +1079,23 @@ def run_fused(k: int, hap_asm: Sequence[str], hap_reads: Sequence[Sequence[str]]
         with ThreadPoolExecutor(max_workers=len(devices)) as ex:
             engines = list(ex.map(make, devices))
     clen = [len(s) for _, s in contigs]
-    results = run_reads(engines, contig_hap, files, file_hap, batch_files, batch_gbp, detailed, threads,
-                        support_len=clen if support_tracks else None, gap_len=np.asarray(clen, np.uint32) if gap_evidence else None,
-                        junctions=junctions, discordance_len=clen if discordance else None)
+    results = run_reads(engines, contig_hap, files, file_hap, batch_files, batch_gbp, detailed, threads, products=products,
+                        contig_len=clen)
     eng = engines[0]
     gaps, nodata = eng.gaps(np.asarray(clen, dtype=np.uint32))
     write_outputs(k, eng, results, clen, contig_hap, eng.contig_names, results[0]["iv"], gaps, nodata, outdir,
-                  detailed=detailed, palindromes=mrsfast_palindromes, support_tracks=support_tracks, gap_evidence=gap_evidence,
-                  junctions=junctions, discordance=discordance)
+                  detailed=detailed, palindromes=mrsfast_palindromes, products=products)
     for e in engines[1:]:
         e.close()
     return eng
 
 
 def write_outputs(k, eng, results, contig_len, contig_hap, names, iv, gaps, nodata, outdir, detailed=False, palindromes=False,
-                  db_files=True, support_tracks=False, gap_evidence=False, junctions=False, discordance=False):
+                  db_files=True, products: Sequence[str] = ()):
     """every file of SURVEY Appendix C that the rules between jellyfish_count and slop_gaps produce (db_files=False:
     without the exports of the database itself -- db/jellyfish.db|.fa, mrsfast/kmer.loc and its per-contig copies
-    breaks/*.loc -- which belong to the database build, not to a run over reads); support_tracks: also
-    final_out/hap{N}.reads.bed / .support.bedgraph / .support.tsv (run_reads(support_len=...) results); gap_evidence: also
-    final_out/hap{N}.gaps.reads.tsv / .gaps.evidence.tsv (run_reads(gap_len=...) results); junctions: also
-    final_out/hap{N}.junctions.reads.tsv / .junctions.tsv (run_reads(junctions=True) results); discordance: also
-    final_out/hap{N}.discordance.reads.tsv / .discordance.tsv / .discordance.bed (run_reads(discordance_len=...) results)"""
+    breaks/*.loc -- which belong to the database build, not to a run over reads), and final_out/hap{N}.{suffix} of every
+    product named in `products` (EVIDENCE_PRODUCTS; results of run_reads with the same products)"""
     d = lambda *p: os.path.join(outdir, *p)
     for sub in ("db", "mrsfast", "sunkpos", "breaks", "inter_outs", "bed_files", "final_out"):
         os.makedirs(d(sub), exist_ok=True)
@@ -1128,8 +1128,8 @@ def write_outputs(k, eng, results, contig_len, contig_hap, names, iv, gaps, noda
                     parts.append(t[c] + np.uint32(read_base[i]) if (c == "read" and read_base[i]) else t[c])
             out[c] = parts[0] if len(parts) == 1 else (np.concatenate(parts) if parts else np.zeros(0, np.uint32))
         return out
-    kept = cat_rows("kept", ("read", "pos", "contig", "start", "group"))
-    pairs = cat_rows("pairs", ("read", "contig", "group"))
+    kept = cat_rows("kept", Engine.ROW_COLUMNS)
+    pairs = cat_rows("pairs", Engine.PAIR_COLUMNS)
     sunk_cols = lambda t: [("name", t["read"], rtab), ("u32", t["pos"]), ("name", t["contig"], ctab), ("u32", t["start"]), ("u32", t["group"])]
     # ---- SUNK database files (defineSUNKs.smk:59-60, 126) ----
     from .engine import revcomp_kmers
@@ -1148,7 +1148,7 @@ def write_outputs(k, eng, results, contig_len, contig_hap, names, iv, gaps, noda
     khap = read_hap[kept["read"]] if len(kept["read"]) else np.zeros(0, np.uint8)
     all_reads = np.arange(nreads, dtype=np.uint32)
     if detailed:
-        rows0 = cat_rows("rows0", ("read", "pos", "contig", "start", "group"))
+        rows0 = cat_rows("rows0", Engine.ROW_COLUMNS)
         r0hap = read_hap[rows0["read"]] if len(rows0["read"]) else np.zeros(0, np.uint8)
     for hap in range(2):
         emit(d("sunkpos", f"hap{hap + 1}.sunkpos"), sunk_cols(kept), sel=np.flatnonzero(khap == hap))
@@ -1182,22 +1182,12 @@ def write_outputs(k, eng, results, contig_len, contig_hap, names, iv, gaps, noda
         lo = (ends - lens)[first]
         hi = np.append(lo[1:], ends[-1])
         return {int(c): rows[a:b] for c, a, b in zip(cs, lo, hi)}
-    # `for rname, g in grouped`: groupby sorts read names (process-by-contig_lowmem_AR.py:135-136); rank of every read
-    # name in that order (stable for equal names), pairs of a read stay in vertex order
-    name_rank = np.empty(nreads, np.int64)
-    if nreads:
-        name_rank[np.argsort(rtab.as_bytes_array(), kind="stable")] = np.arange(nreads)
+    name_rank = bytewise_rank(rtab)
     kept_c = by_contig(kept["contig"], kept["read"])
-    if support_tracks:
-        placements = cat_rows("placements", ("read", "contig", "start", "end", "n_ids", "strand"))
-    if gap_evidence:  # a read lives on one engine: the records of all engines, read indices made run-wide
-        evidence = cat_rows("gap_evidence", Engine.GAP_EVIDENCE_COLUMNS)
-    if junctions:  # likewise
-        jn = cat_rows("junctions", Engine.JUNCTION_COLUMNS)
-        jn_hap = read_hap[jn["read"]] if len(jn["read"]) else np.zeros(0, np.uint8)
-    if discordance:  # likewise; the runs are the same on every engine
-        spans = cat_rows("spans", Engine.SPAN_COLUMNS)
-    pair_c = by_contig(pairs["contig"], pairs["read"], name_rank)
+    # a read lives on one engine: the evidence records of all engines, read indices made run-wide (runs are the same on
+    # every engine)
+    rec = {p: cat_rows(EVIDENCE_PRODUCTS[p].records, EVIDENCE_PRODUCTS[p].columns) for p in products}
+    pair_c = by_contig(pairs["contig"], pairs["read"], name_rank)  # reads in name order, pairs of a read in vertex order
     if db_files:
         loc_c = by_contig(db["contig"])
     iv_c = by_contig(iv["contig"])
@@ -1219,6 +1209,7 @@ def write_outputs(k, eng, results, contig_len, contig_hap, names, iv, gaps, noda
             _write_bytes(d("bed_files", stem + ".bed"), b"")
     clen = np.asarray(contig_len, dtype=np.uint32)
     chap = np.asarray(contig_hap, np.uint8)
+    reads = (rtab, lens, name_rank)
     for hap in range(2):
         hn = hap + 1
         open(d("breaks", f"hap{hn}_splits_pos.done"), "a").close()  # touch() of the checkpoint (tagONT.smk:158)
@@ -1230,23 +1221,14 @@ def write_outputs(k, eng, results, contig_len, contig_hap, names, iv, gaps, noda
         emit(d("final_out", f"hap{hn}.nodata.bed"), [("name", nd, ctab), ("u32", np.zeros(len(nd), np.uint32)), ("u32", clen[nd])])
         s2, e2 = eng.slop(gaps["contig"][gsel], gaps["start"][gsel], gaps["end"][gsel], clen, 200000)  # bedtools slop -b 200000 (tagONT.smk:249)
         emit(d("final_out", f"hap{hn}.gaps.slop.bed"), [("name", gaps["contig"][gsel], ctab), ("i64", s2), ("i64", e2)])
-        if support_tracks:
-            texts = support_texts(np.flatnonzero(chap == hap).tolist(), clen, names, placements, results[0]["support"], iv, rtab, lens,
-                                  name_rank)
-            for ext, data in zip(("reads.bed", "support.bedgraph", "support.tsv"), texts):
-                _write_bytes(d("final_out", f"hap{hn}.{ext}"), data)
-        if gap_evidence:
-            texts = gap_evidence_texts(gsel, gaps, names, evidence, rtab, lens, name_rank)
-            for ext, data in zip(("gaps.reads.tsv", "gaps.evidence.tsv"), texts):
-                _write_bytes(d("final_out", f"hap{hn}.{ext}"), data)
-        if junctions:
-            texts = junction_texts(jn, np.flatnonzero(jn_hap == hap), names, clen, contig_hap, rtab, lens, name_rank)
-            for ext, data in zip(("junctions.reads.tsv", "junctions.tsv"), texts):
-                _write_bytes(d("final_out", f"hap{hn}.{ext}"), data)
-        if discordance:
-            texts = discordance_texts(np.flatnonzero(chap == hap).tolist(), names, spans, results[0]["discordance"], rtab, lens, name_rank)
-            for ext, data in zip(("discordance.reads.tsv", "discordance.tsv", "discordance.bed"), texts):
-                _write_bytes(d("final_out", f"hap{hn}.{ext}"), data)
+        hap_contigs = np.flatnonzero(chap == hap).tolist()
+        texts = dict(
+            support_tracks=lambda r: support_texts(hap_contigs, clen, names, r, results[0]["support"], iv, *reads),
+            gap_evidence=lambda r: gap_evidence_texts(gsel, gaps, names, r, *reads),
+            junctions=lambda r: junction_texts(r, np.flatnonzero(read_hap[r["read"]] == hap), names, clen, contig_hap, *reads),
+            discordance=lambda r: discordance_texts(hap_contigs, names, r, results[0]["discordance"], *reads))
+        for p in products:
+            _write_all([d("final_out", f"hap{hn}.{ext}") for ext in EVIDENCE_PRODUCTS[p].suffixes], texts[p](rec[p]))
     from concurrent.futures import ThreadPoolExecutor
     n_cpu = len(os.sched_getaffinity(0)) if hasattr(os, "sched_getaffinity") else (os.cpu_count() or 1)
     workers = max(1, min(8, n_cpu // 2))
@@ -1273,21 +1255,13 @@ def cmd_fused(argv):
     ap.add_argument("--threads", type=int, default=0, help="ingest threads per GPU")
     ap.add_argument("--mrsfast-palindromes", action="store_true",
                     help="write a palindromic SUNK twice into kmer.loc, as mrsfast reports it on both strands (SURVEY A.2; unpinned)")
-    ap.add_argument("--support-tracks", action="store_true",
-                    help="also write final_out/hap{N}.reads.bed, .support.bedgraph and .support.tsv (support of the validated reads)")
-    ap.add_argument("--gap-evidence", action="store_true",
-                    help="also write final_out/hap{N}.gaps.evidence.tsv and .gaps.reads.tsv (the reads that bridge each gap)")
-    ap.add_argument("--junctions", action="store_true",
-                    help="also write final_out/hap{N}.junctions.reads.tsv and .junctions.tsv (reads that jump between contigs)")
-    ap.add_argument("--discordance", action="store_true",
-                    help="also write final_out/hap{N}.discordance.reads.tsv, .discordance.tsv and .discordance.bed (collapses and "
-                         "expansions inside validated intervals)")
+    for p, e in EVIDENCE_PRODUCTS.items():
+        ap.add_argument(e.flag, dest=p, action="store_true", help=e.help)
     a = ap.parse_args(argv)
     devs = [int(x) for x in a.devices.split(",")] if a.devices else [a.device]
     run_fused(a.k, [a.hap1_asm, a.hap2_asm], [a.hap1_reads, a.hap2_reads], a.outdir, devices=devs, batch_files=a.batch_files,
               batch_gbp=a.batch_gbp, detailed=a.detailed, threads=a.threads, mrsfast_palindromes=a.mrsfast_palindromes,
-              support_tracks=a.support_tracks, gap_evidence=a.gap_evidence, junctions=a.junctions,
-              discordance=a.discordance)
+              products=[p for p in EVIDENCE_PRODUCTS if getattr(a, p)])
 
 
 COMMANDS = {"kmerpos_annot3": (cmd_kmerpos_annot3, 4), "rlen": (cmd_rlen, 2), "diag_filter_v3": (cmd_diag_filter_v3, 2),

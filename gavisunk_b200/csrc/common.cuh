@@ -541,6 +541,15 @@ static int read_dev(gvs_ctx* ctx, const T* d, T* h, size_t n = 1) {
   CK(cudaStreamSynchronize(ctx->stream));
   return 0;
 }
+// the first n entries of N u32 columns stored `stride` entries apart from `src` to host buffers (null ones skipped):
+// the record getters; returns when the copies (and any queued before them) have finished
+template <int N>
+static int columns_to_host(gvs_ctx* ctx, const u32* src, u64 stride, u64 n, uint32_t* const (&dst)[N]) {
+  for (int t = 0; t < N; t++)
+    if (dst[t]) CK(cudaMemcpyAsync(dst[t], src + (u64)t * stride, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  return 0;
+}
 template <typename T>
 static int to_dev(gvs_ctx* ctx, DevBuf& b, const T* h, size_t n) {
   CKR(gvs_reserve(ctx, b, n * sizeof(T)));

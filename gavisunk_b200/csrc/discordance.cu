@@ -226,11 +226,7 @@ extern "C" int gvs_spans_get(gvs_ctx* ctx, uint32_t* read, uint32_t* contig, uin
   const u64 n = ctx->n_dc, stride = ctx->dc_stride;
   if (n == 0) return 0;
   uint32_t* dst[8] = {read, contig, id1, start1, pos1, id2, start2, pos2};
-  const u32* rec = ctx->dc_rec.as<u32>();
-  for (int t = 0; t < 8; t++)
-    if (dst[t]) CK(cudaMemcpyAsync(dst[t], rec + (u64)t * stride, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaStreamSynchronize(ctx->stream));
-  return 0;
+  return columns_to_host(ctx, ctx->dc_rec.as<u32>(), stride, n, dst);
 }
 
 extern "C" int gvs_discordance(gvs_ctx* ctx, const uint32_t* contig_len, uint64_t* n_runs) {
@@ -257,13 +253,9 @@ extern "C" int gvs_discordance_get(gvs_ctx* ctx, uint32_t* contig, uint32_t* sta
   CK(cudaSetDevice(ctx->device));
   const u64 n = ctx->n_dc_runs;
   if (n == 0) return 0;
-  const u32* val = ctx->dc_run_val.as<u32>();
   if (contig) CK(cudaMemcpyAsync(contig, ctx->dc_run_contig.p, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
   if (start) CK(cudaMemcpyAsync(start, ctx->dc_run_start.p, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
   if (end) CK(cudaMemcpyAsync(end, ctx->dc_run_end.p, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
   uint32_t* dst[3] = {spans, longer, shorter};
-  for (int t = 0; t < 3; t++)
-    if (dst[t]) CK(cudaMemcpyAsync(dst[t], val + (u64)t * n, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaStreamSynchronize(ctx->stream));
-  return 0;
+  return columns_to_host(ctx, ctx->dc_run_val.as<u32>(), n, n, dst);
 }

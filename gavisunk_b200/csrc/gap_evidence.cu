@@ -239,9 +239,5 @@ extern "C" int gvs_gap_evidence_get(gvs_ctx* ctx, uint32_t* read, uint32_t* gap,
   const u64 n = ctx->n_ge, stride = ctx->n_ge_cand;
   if (n == 0) return 0;
   uint32_t* dst[8] = {read, gap, left_id, left_start, left_pos, right_id, right_start, right_pos};
-  const u32* rec = ctx->ge_rec.as<u32>();
-  for (int t = 0; t < 8; t++)
-    if (dst[t]) CK(cudaMemcpyAsync(dst[t], rec + (u64)t * stride, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaStreamSynchronize(ctx->stream));
-  return 0;
+  return columns_to_host(ctx, ctx->ge_rec.as<u32>(), stride, n, dst);
 }

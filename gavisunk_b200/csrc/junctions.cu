@@ -374,9 +374,5 @@ extern "C" int gvs_junctions_get(gvs_ctx* ctx, uint32_t* read, uint32_t* contig1
   const u64 n = ctx->n_jn, stride = ctx->jn_stride;
   if (n == 0) return 0;
   uint32_t* dst[13] = {read, contig1, strand1, ids1, id1, start1, pos1, contig2, strand2, ids2, id2, start2, pos2};
-  const u32* rec = ctx->jn_rec.as<u32>();
-  for (int t = 0; t < 13; t++)
-    if (dst[t]) CK(cudaMemcpyAsync(dst[t], rec + (u64)t * stride, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaStreamSynchronize(ctx->stream));
-  return 0;
+  return columns_to_host(ctx, ctx->jn_rec.as<u32>(), stride, n, dst);
 }

@@ -166,6 +166,26 @@ class Engine:
         buf = (C.c_uint8 * need).from_address(ptr)
         return np.frombuffer(buf, dtype=dt, count=n)
 
+    def _table(self, name: str, get, n: int, cols: Sequence[Optional[str]], lead=(), dtypes=None, counts=None,
+               pinned: bool = False) -> Dict[str, np.ndarray]:
+        """Host columns of table `name` from get(ctx, *lead, one pointer per entry of cols): n entries each (counts[c]
+        for a column given there), uint32 unless dtypes[c] says otherwise; a None in cols passes a null pointer.
+        pinned: views of page-locked buffers keyed "name.column" (see _out)."""
+        dtypes, counts = dtypes or {}, counts or {}
+        out = {c: self._out(f"{name}.{c}", counts.get(c, n), dtypes.get(c, np.uint32), pinned) for c in cols if c is not None}
+        self._ck(get(self.ctx, *lead, *[_ptr(out.get(c)) for c in cols]))
+        return out
+
+    def _runs(self, name: str, run, get, cols: Sequence[str], diff: str, contig_len, allreduce):
+        """support() / discordance(): runs (contig, start, end, one column per value) tiling every contig, after the
+        optional in-place all-reduce of the int32 difference arrays (one per value column) at the pointer attribute `diff`"""
+        if allreduce is not None:
+            allreduce(getattr(self, diff), (len(cols) - 3) * self.db_groups())
+        cl = _c(contig_len, np.uint32)
+        n = C.c_uint64()
+        self._ck(run(self.ctx, _ptr(cl), C.byref(n)))
+        return self._table(name, get, int(n.value), cols)
+
     def __del__(self):
         try:
             self.close()
@@ -244,11 +264,8 @@ class Engine:
 
     def db_export(self) -> Dict[str, np.ndarray]:
         n, _ = self.db_size()
-        out = dict(kmer=np.zeros(n, np.uint64), contig=np.zeros(n, np.uint32), start=np.zeros(n, np.uint32),
-                   group=np.zeros(n, np.uint32), gidx=np.zeros(n, np.uint32))
-        self._ck(self.lib.gvs_db_export(self.ctx, _ptr(out["kmer"]), _ptr(out["contig"]), _ptr(out["start"]),
-                                        _ptr(out["group"]), _ptr(out["gidx"])))
-        return out
+        return self._table("db", self.lib.gvs_db_export, n, ("kmer", "contig", "start", "group", "gidx"),
+                           dtypes=dict(kmer=np.uint64))
 
     # ------------------------------------------------------------------------------------
     # reads
@@ -347,13 +364,12 @@ class Engine:
         self.n_rows = int(n.value)
         return self.n_rows
 
+    ROW_COLUMNS = ("read", "pos", "contig", "start", "group")
+
     def rows(self, which: int = 0, n: Optional[int] = None, pinned: bool = False) -> Dict[str, np.ndarray]:
         if n is None:
             n = self.n_rows if which == 0 else self.n_kept
-        out = {c: self._out(f"rows{which}.{c}", n, np.uint32, pinned) for c in ("read", "pos", "contig", "start", "group")}
-        self._ck(self.lib.gvs_rows_get(self.ctx, which, _ptr(out["read"]), _ptr(out["pos"]), _ptr(out["contig"]),
-                                       _ptr(out["start"]), _ptr(out["group"])))
-        return out
+        return self._table(f"rows{which}", self.lib.gvs_rows_get, n, self.ROW_COLUMNS, lead=(which,), pinned=pinned)
 
     def diag_filter(self, contig_hap: Sequence[int]) -> Tuple[int, int]:
         """diag_filter_v3 + diag_filter_step2 (workflow/src/diag_filter_v3.nim:18-229,
@@ -368,12 +384,8 @@ class Engine:
         return self.n_best, self.n_kept
 
     def best(self) -> Dict[str, np.ndarray]:
-        n = self.n_best
-        out = dict(read=np.zeros(n, np.uint32), contig=np.zeros(n, np.uint32), ngood=np.zeros(n, np.uint32),
-                   dir=np.zeros(n, np.uint8))
-        self._ck(self.lib.gvs_best_get(self.ctx, _ptr(out["read"]), _ptr(out["contig"]), _ptr(out["ngood"]),
-                                       _ptr(out["dir"])))
-        return out
+        return self._table("best", self.lib.gvs_best_get, self.n_best, ("read", "contig", "ngood", "dir"),
+                           dtypes=dict(dir=np.uint8))
 
     def filter_best(self, best_contig_of_read) -> int:
         """diag_filter_step2 (workflow/src/diag_filter_step2.nim:13-66) with the best contigs given."""
@@ -508,12 +520,8 @@ class Engine:
         """group table behind every group index: (contig, group start[, row count of group_hist])"""
         n = C.c_uint64()
         self._ck(self.lib.gvs_groups_count(self.ctx, C.byref(n)))
-        n = int(n.value)
-        out = dict(contig=np.zeros(n, np.uint32), group=np.zeros(n, np.uint32))
-        if with_hist:
-            out["count"] = np.zeros(n, np.int32)
-        self._ck(self.lib.gvs_groups_get(self.ctx, _ptr(out["contig"]), _ptr(out["group"]), _ptr(out.get("count"))))
-        return out
+        return self._table("groups", self.lib.gvs_groups_get, int(n.value), ("contig", "group", "count" if with_hist else None),
+                           dtypes=dict(count=np.int32))
 
     def validate(self, min_read_len: int = 10000) -> int:
         """process-by-contig_lowmem_AR.py:50-207 (per-read part)."""
@@ -522,12 +530,12 @@ class Engine:
         self.n_pairs = int(n.value)
         return self.n_pairs
 
+    PAIR_COLUMNS = ("read", "contig", "group", "gidx")
+
     def pairs(self, pinned: bool = False) -> Dict[str, np.ndarray]:
-        n = self.n_pairs
-        out = {c: self._out(f"pairs.{c}", n, np.uint32, pinned) for c in ("read", "contig", "group", "gidx")}
-        self._ck(self.lib.gvs_pairs_get(self.ctx, _ptr(out["read"]), _ptr(out["contig"]), _ptr(out["group"]),
-                                        _ptr(out["gidx"])))
-        return out
+        return self._table("pairs", self.lib.gvs_pairs_get, self.n_pairs, self.PAIR_COLUMNS, pinned=pinned)
+
+    PLACEMENT_COLUMNS = ("read", "contig", "start", "end", "n_ids", "strand")
 
     def placements(self, pinned: bool = False) -> Dict[str, np.ndarray]:
         """Support placements of the validated reads (no reference counterpart): one per read with >= 2 validated
@@ -536,25 +544,17 @@ class Engine:
         n, p = C.c_uint64(), C.c_void_p()
         self._ck(self.lib.gvs_placements(self.ctx, C.byref(n), C.byref(p)))
         self._diff_ptr = int(p.value or 0)
-        n = int(n.value)
-        out = {c: self._out(f"placements.{c}", n, np.uint32, pinned) for c in ("read", "contig", "start", "end", "n_ids")}
-        out["strand"] = self._out("placements.strand", n, np.uint8, pinned)
-        self._ck(self.lib.gvs_placements_get(self.ctx, _ptr(out["read"]), _ptr(out["contig"]), _ptr(out["start"]), _ptr(out["end"]),
-                                             _ptr(out["n_ids"]), _ptr(out["strand"])))
-        return out
+        return self._table("placements", self.lib.gvs_placements_get, int(n.value), self.PLACEMENT_COLUMNS,
+                           dtypes=dict(strand=np.uint8), pinned=pinned)
+
+    SUPPORT_COLUMNS = ("contig", "start", "end", "depth")
 
     def support(self, contig_len: Sequence[int], allreduce=None) -> Dict[str, np.ndarray]:
         """Support depth after placements(): runs (contig, start, end, depth) tiling every contig.  With several GPUs
         `allreduce(ptr, n_groups)` sums the int32 difference array across ranks in place first (the callable that
         sums the bad-SUNK histogram)."""
-        if allreduce is not None:
-            allreduce(self._diff_ptr, self.db_groups())
-        cl = _c(contig_len, np.uint32)
-        n = C.c_uint64()
-        self._ck(self.lib.gvs_support(self.ctx, _ptr(cl), C.byref(n)))
-        out = {c: np.zeros(int(n.value), np.uint32) for c in ("contig", "start", "end", "depth")}
-        self._ck(self.lib.gvs_support_get(self.ctx, _ptr(out["contig"]), _ptr(out["start"]), _ptr(out["end"]), _ptr(out["depth"])))
-        return out
+        return self._runs("support", self.lib.gvs_support, self.lib.gvs_support_get, self.SUPPORT_COLUMNS, "_diff_ptr",
+                          contig_len, allreduce)
 
     SPAN_COLUMNS = ("read", "contig", "id1", "start1", "pos1", "id2", "start2", "pos2")
 
@@ -566,23 +566,16 @@ class Engine:
         n, p = C.c_uint64(), C.c_void_p()
         self._ck(self.lib.gvs_spans(self.ctx, int(min_delta), int(rel_permille), C.byref(n), C.byref(p)))
         self._dc_diff_ptr = int(p.value or 0)
-        out = {c: np.zeros(int(n.value), np.uint32) for c in self.SPAN_COLUMNS}
-        self._ck(self.lib.gvs_spans_get(self.ctx, *[_ptr(out[c]) for c in self.SPAN_COLUMNS]))
-        return out
+        return self._table("spans", self.lib.gvs_spans_get, int(n.value), self.SPAN_COLUMNS)
+
+    DISCORDANCE_COLUMNS = ("contig", "start", "end", "spans", "longer", "shorter")
 
     def discordance(self, contig_len: Sequence[int], allreduce=None) -> Dict[str, np.ndarray]:
         """Discordance runs after spans(): (contig, start, end, spans, longer, shorter) tiling every contig.  With several
         GPUs `allreduce(ptr, n)` sums the int32 difference arrays (n = 3 * n_groups) across ranks in place first (the
         callable that sums the bad-SUNK histogram)."""
-        if allreduce is not None:
-            allreduce(self._dc_diff_ptr, 3 * self.db_groups())
-        cl = _c(contig_len, np.uint32)
-        n = C.c_uint64()
-        self._ck(self.lib.gvs_discordance(self.ctx, _ptr(cl), C.byref(n)))
-        cols = ("contig", "start", "end", "spans", "longer", "shorter")
-        out = {c: np.zeros(int(n.value), np.uint32) for c in cols}
-        self._ck(self.lib.gvs_discordance_get(self.ctx, *[_ptr(out[c]) for c in cols]))
-        return out
+        return self._runs("discordance", self.lib.gvs_discordance, self.lib.gvs_discordance_get, self.DISCORDANCE_COLUMNS,
+                          "_dc_diff_ptr", contig_len, allreduce)
 
     def components_local(self) -> int:
         """this GPU's forest of the validated pairs; returns the device pointer of its uint32[n_groups] parent array"""
@@ -598,10 +591,7 @@ class Engine:
         """process-by-contig_lowmem_AR.py:215-260 -> rows of bed_files/*.bed."""
         n = C.c_uint64()
         self._ck(self.lib.gvs_intervals(self.ctx, C.byref(n)))
-        n = int(n.value)
-        out = {c: np.zeros(n, np.uint32) for c in ("contig", "start", "end")}
-        self._ck(self.lib.gvs_intervals_get(self.ctx, _ptr(out["contig"]), _ptr(out["start"]), _ptr(out["end"])))
-        return out
+        return self._table("intervals", self.lib.gvs_intervals_get, int(n.value), ("contig", "start", "end"))
 
     def set_intervals(self, contig, start, end, n_contigs: int):
         """rows of bed_files/*.bed as the input of gaps() (get_gaps.py:30)."""
@@ -613,9 +603,9 @@ class Engine:
         cl = _c(contig_len, np.uint32)
         a, b = C.c_uint64(), C.c_uint64()
         self._ck(self.lib.gvs_gaps(self.ctx, _ptr(cl), C.byref(a), C.byref(b)))
-        g = {c: np.zeros(int(a.value), np.uint32) for c in ("contig", "start", "end")}
-        nd = np.zeros(int(b.value), np.uint32)
-        self._ck(self.lib.gvs_gaps_get(self.ctx, _ptr(g["contig"]), _ptr(g["start"]), _ptr(g["end"]), _ptr(nd)))
+        g = self._table("gaps", self.lib.gvs_gaps_get, int(a.value), ("contig", "start", "end", "nodata"),
+                        counts=dict(nodata=int(b.value)))
+        nd = g.pop("nodata")
         return g, nd
 
     GAP_EVIDENCE_COLUMNS = ("read", "gap", "left_id", "left_start", "left_pos", "right_id", "right_start", "right_pos")
@@ -627,9 +617,7 @@ class Engine:
         rows.  Call gaps() on this engine first."""
         n = C.c_uint64()
         self._ck(self.lib.gvs_gap_evidence(self.ctx, int(min_read_len), C.byref(n)))
-        out = {c: np.zeros(int(n.value), np.uint32) for c in self.GAP_EVIDENCE_COLUMNS}
-        self._ck(self.lib.gvs_gap_evidence_get(self.ctx, *[_ptr(out[c]) for c in self.GAP_EVIDENCE_COLUMNS]))
-        return out
+        return self._table("gap_evidence", self.lib.gvs_gap_evidence_get, int(n.value), self.GAP_EVIDENCE_COLUMNS)
 
     JUNCTION_COLUMNS = ("read", "contig1", "strand1", "ids1", "id1", "start1", "pos1", "contig2", "strand2", "ids2", "id2",
                         "start2", "pos2")
@@ -649,9 +637,7 @@ class Engine:
         the (ID, start, pos) of its row next to the junction."""
         n = C.c_uint64()
         self._ck(self.lib.gvs_junctions(self.ctx, C.byref(n)))
-        out = {c: np.zeros(int(n.value), np.uint32) for c in self.JUNCTION_COLUMNS}
-        self._ck(self.lib.gvs_junctions_get(self.ctx, *[_ptr(out[c]) for c in self.JUNCTION_COLUMNS]))
-        return out
+        return self._table("junctions", self.lib.gvs_junctions_get, int(n.value), self.JUNCTION_COLUMNS)
 
     def covprob_table(self, kbp, cnt, genome_kbp: float, pn: float) -> np.ndarray:
         """covprob.py:56-100."""

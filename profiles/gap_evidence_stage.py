@@ -83,8 +83,7 @@ def main():
     # host egress: names of every read as the fused rule holds them, then the two files per haplotype
     n_reads = eng.n_reads
     rtab = gio.NameTable([f"read{i}" for i in range(n_reads)])
-    name_rank = np.empty(n_reads, np.int64)
-    name_rank[np.argsort(rtab.as_bytes_array(), kind="stable")] = np.arange(n_reads)
+    name_rank = cli.bytewise_rank(rtab)
     chap = wl.contig_hap
     egress = []
     with tempfile.TemporaryDirectory() as td:
@@ -93,8 +92,8 @@ def main():
             for hap in range(2):
                 gsel = np.flatnonzero(chap[gaps["contig"]] == hap)
                 texts = cli.gap_evidence_texts(gsel, gaps, wl.contig_names, ev, rtab, lens, name_rank)
-                for ext, data in zip(("gaps.reads.tsv", "gaps.evidence.tsv"), texts):
-                    cli._write_bytes(os.path.join(td, f"hap{hap + 1}.{ext}"), data)
+                cli._write_all([os.path.join(td, f"hap{hap + 1}.{ext}") for ext in cli.EVIDENCE_PRODUCTS["gap_evidence"].suffixes],
+                               texts)
             egress.append((time.perf_counter() - t0) * 1e3)
     print(json.dumps(dict(
         metric="gap_evidence_stage_ms", workload="h3100 (bench.py default: 3.1 Gbp x2, 8 batches of 3.75x, k 20), 1 GPU",

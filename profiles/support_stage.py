@@ -64,8 +64,7 @@ def main():
     rnames = [f"read{i}" for i in range(n_reads)]
     rtab = gio.NameTable(rnames)
     lens = np.concatenate([np.diff(b.read_off.cpu().numpy()) for b in batches]).astype(np.uint32)
-    name_rank = np.empty(n_reads, np.int64)
-    name_rank[np.argsort(rtab.as_bytes_array(), kind="stable")] = np.arange(n_reads)
+    name_rank = cli.bytewise_rank(rtab)
     egress = []
     with tempfile.TemporaryDirectory() as td:
         for _ in range(3):
@@ -73,8 +72,8 @@ def main():
             for hap in range(2):
                 texts = cli.support_texts(np.flatnonzero(wl.contig_hap == hap).tolist(), clen, wl.contig_names, pl, runs, iv, rtab,
                                           lens, name_rank)
-                for ext, data in zip(("reads.bed", "support.bedgraph", "support.tsv"), texts):
-                    cli._write_bytes(os.path.join(td, f"hap{hap + 1}.{ext}"), data)
+                cli._write_all([os.path.join(td, f"hap{hap + 1}.{ext}") for ext in cli.EVIDENCE_PRODUCTS["support_tracks"].suffixes],
+                               texts)
             egress.append((time.perf_counter() - t0) * 1e3)
     print(json.dumps(dict(
         metric="support_stage_ms", workload="h3100 (bench.py default: 3.1 Gbp x2, 8 batches of 3.75x, k 20), 1 GPU",
