@@ -157,6 +157,7 @@ struct gvs_ctx {
 
   // ---- support tracks (support.cu) ----
   u64 rank_gen = ~0ull;             // grp_gen the rank below was computed for
+  u64 order_gen = ~0ull;            // grp_gen rank_identity was found for
   bool rank_identity = false;       // group index order is already (contig, start) order
   DevBuf rank_of, rank_grp;         // group index -> rank in (contig, start) order, and back (unless identity)
   DevBuf sup_diff;                  // int32[n_groups] by rank: +1 at a placement's first group, -1 at its last
@@ -196,6 +197,7 @@ struct gvs_ctx {
 
   // ---- components / intervals / gaps ----
   DevBuf parent, present, comp_min, comp_max, comp_cnt;
+  DevBuf comp_rank;  // unsorted group tables only: [smallest member rank per root | root per interval rank]
   DevBuf iv_contig, iv_start, iv_end;
   u64 n_iv = 0;
   DevBuf gap_contig, gap_start, gap_end, nodata_contig;
@@ -565,6 +567,9 @@ int gvs_build_segments(gvs_ctx* ctx, const u32* read, u64 n, DevBuf& seg_start, 
 int gvs_reserve_rows(gvs_ctx* ctx, Rows& r, u64 n);
 // support.cu: group ranks in (contig, start) order (rank_of / rank_grp unless rank_identity), cached per group table
 int gvs_ensure_rank(gvs_ctx* ctx);
+// support.cu: rank_identity of a freshly built group table (one launch; called by every table build, so that the
+// rank of a sorted table costs the later stages nothing)
+int gvs_check_group_order(gvs_ctx* ctx);
 // support.cu: runs of equal values over the groups in rank order that tile [0, contig_len) of every contig: diff = nv
 // difference arrays of n_groups int32 by rank, prefix-summed here; out.val receives nv columns of *n_runs entries
 struct RankRuns {

@@ -175,7 +175,7 @@ extern "C" void gvs_destroy(gvs_ctx* c) {
                    &c->diag_scratch, &c->best_read, &c->best_contig, &c->best_good, &c->best_dir, &c->hist,
                    &c->cnt_hist, &c->bad_flag, &c->bad_list, &c->kseg_start, &c->val_scratch, &c->val_cnt,
                    &c->val_off, &c->pair_read, &c->pair_contig, &c->pair_group, &c->pair_gidx, &c->parent,
-                   &c->present, &c->comp_min, &c->comp_max, &c->comp_cnt, &c->iv_contig, &c->iv_start, &c->iv_end,
+                   &c->present, &c->comp_min, &c->comp_max, &c->comp_cnt, &c->comp_rank, &c->iv_contig, &c->iv_start, &c->iv_end,
                    &c->gap_contig, &c->gap_start, &c->gap_end, &c->nodata_contig, &c->read_len, &c->gt_keys, &c->gt_val,
                    &c->seg_orient, &c->rank_of, &c->rank_grp, &c->sup_diff, &c->pl_read, &c->pl_contig, &c->pl_start, &c->pl_end,
                    &c->pl_nids, &c->pl_strand, &c->pl_tmp, &c->sup_depth, &c->sup_gx, &c->sup_cstat, &c->run_contig, &c->run_start,

@@ -409,6 +409,7 @@ extern "C" int gvs_db_build(gvs_ctx* ctx, const uint8_t* seq, const uint64_t* co
     // contigs must fit 32-bit starts
     rc = db_build_device(ctx, s, o, n_contigs, total, keys, vals, bitmap, wrank, head, hrow, gex);
   }
+  if (!rc) rc = gvs_check_group_order(ctx);
   cudaStreamSynchronize(ctx->stream);
   DevBuf* tmp[] = {&dseq, &doff, &keys, &vals, &bitmap, &wrank, &head, &hrow, &gex};
   for (DevBuf* b : tmp) gvs_release(*b);

@@ -8,7 +8,7 @@
 // pair is unioned with its predecessor of the same read in a lock-free union-find over the dense
 // group index (hook larger root under smaller: the root is the component's first group).
 // Multi-GPU: every rank builds its forest; the gathered forests are merged in one pass by unioning g with
-// each peer's parent[g].
+// each peer's parent[g].  Intervals come out in (contig, start) order whatever the order of the group table.
 #include "common.cuh"
 #include <algorithm>
 
@@ -70,14 +70,20 @@ __global__ void __launch_bounds__(256) k_comp_merge_all(const u32* __restrict__ 
 }
 // count / smallest / largest group start per component root.  Neighbouring groups almost always share their root
 // (a component is a run of groups along a contig; at 30x a contig is a handful of components), so the lanes of a
-// warp are combined per distinct root first: one atomic triple per root and warp instead of per group
+// warp are combined per distinct root first: one atomic triple per root and warp instead of per group.
+// BY_RANK (group index not in (contig, start) order): also the smallest (contig, start) rank of the members, which
+// places the component's interval in the output
+template <bool BY_RANK>
 __global__ void __launch_bounds__(256) k_comp_stats(u32* par, const u8* __restrict__ present, u64 ng,
-                                                    const u32* __restrict__ grp_start, u32* cnt, u32* mn, u32* mx) {
+                                                    const u32* __restrict__ grp_start, u32* cnt, u32* mn, u32* mx,
+                                                    const u32* __restrict__ rank_of, u32* rmn) {
   const u64 g = (u64)blockIdx.x * blockDim.x + threadIdx.x;
   const int lane = threadIdx.x & 31;
   const bool act = g < ng && present[g];
   const u32 r = act ? guf_find(par, (u32)g) : 0xFFFFFFFFu;
   const u32 s = act ? grp_start[g] : 0u;
+  u32 q = 0;
+  if (BY_RANK) q = act ? rank_of[g] : 0xFFFFFFFFu;
   u32 todo = __ballot_sync(0xFFFFFFFFu, act);
   while (todo) {  // warp-uniform
     const int leader = __ffs(todo) - 1;
@@ -86,10 +92,13 @@ __global__ void __launch_bounds__(256) k_comp_stats(u32* par, const u8* __restri
     const u32 m = __ballot_sync(0xFFFFFFFFu, mine);
     const u32 lo = __reduce_min_sync(0xFFFFFFFFu, mine ? s : 0xFFFFFFFFu);
     const u32 hi = __reduce_max_sync(0xFFFFFFFFu, mine ? s : 0u);
+    u32 qlo = 0;
+    if (BY_RANK) qlo = __reduce_min_sync(0xFFFFFFFFu, mine ? q : 0xFFFFFFFFu);
     if (lane == leader) {
       atomicAdd(&cnt[rl], (u32)__popc(m));
       atomicMin(&mn[rl], lo);
       atomicMax(&mx[rl], hi);
+      if (BY_RANK) atomicMin(&rmn[rl], qlo);
     }
     todo &= ~m;
   }
@@ -103,6 +112,25 @@ __global__ void __launch_bounds__(256) k_iv_write(const u32* __restrict__ excl, 
   iv_contig[o] = grp_contig[g];
   iv_start[o] = mn[g];
   iv_end[o] = mx[g];  // end = largest group ID, not +k (Q15)
+}
+// unsorted group table: every kept component's root at its smallest member rank, so that a scan over rank space
+// numbers the intervals in (contig, start) order
+__global__ void __launch_bounds__(256) k_iv_slot(const u32* __restrict__ cnt, const u32* __restrict__ rmn, u64 ng, u32* slot) {
+  u64 g = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+  if (g >= ng || cnt[g] < 3) return;
+  slot[rmn[g]] = (u32)g;
+}
+__global__ void __launch_bounds__(256) k_iv_write_rank(const u32* __restrict__ excl, const u32* __restrict__ slot, u64 ng,
+                                                       const u32* __restrict__ grp_contig, const u32* __restrict__ mn,
+                                                       const u32* __restrict__ mx, u32* iv_contig, u32* iv_start, u32* iv_end) {
+  u64 q = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+  if (q >= ng) return;
+  const u32 g = slot[q];
+  if (g == 0xFFFFFFFFu) return;
+  u32 o = excl[q];
+  iv_contig[o] = grp_contig[g];
+  iv_start[o] = mn[g];
+  iv_end[o] = mx[g];
 }
 
 // singleton forest over the group index, no group present
@@ -162,17 +190,33 @@ extern "C" int gvs_intervals(gvs_ctx* ctx, uint64_t* n_intervals) {
     ctx->iv_ready = true;
     return 0;
   }
+  // intervals come out in (contig, start) order, as the reference's bed rows and gvs_gaps want them.  The root of a
+  // component is its smallest group index, which is its leftmost group when the group table is sorted (a built
+  // database, a sorted kmer.loc): then the roots are written in index order.  Otherwise (groups from rows, an
+  // unsorted kmer.loc) each component is placed by the smallest (contig, start) rank of its members.
+  CKR(gvs_ensure_rank(ctx));
+  const bool by_rank = !ctx->rank_identity;
   CK(cudaMemsetAsync(ctx->comp_cnt.p, 0, ng * 4, ctx->stream));
   CK(cudaMemsetAsync(ctx->comp_min.p, 0xFF, ng * 4, ctx->stream));
   CK(cudaMemsetAsync(ctx->comp_max.p, 0, ng * 4, ctx->stream));
-  LAUNCH(k_comp_stats, (unsigned)cdiv(ng, 256), 256, 0, ctx->parent.as<u32>(), ctx->present.as<u8>(), ng, ctx->grp_start.as<u32>(),
-         ctx->comp_cnt.as<u32>(), ctx->comp_min.as<u32>(), ctx->comp_max.as<u32>());
   const u32* cnt = ctx->comp_cnt.as<u32>();
   u32* ex = ctx->flags_b.as<u32>();
   u32* tot = (u32*)(ctx->counters.as<u64>() + 26);
-  {
+  if (!by_rank) {
+    LAUNCH(k_comp_stats<false>, (unsigned)cdiv(ng, 256), 256, 0, ctx->parent.as<u32>(), ctx->present.as<u8>(), ng, ctx->grp_start.as<u32>(),
+           ctx->comp_cnt.as<u32>(), ctx->comp_min.as<u32>(), ctx->comp_max.as<u32>(), nullptr, nullptr);
     auto f = [cnt] __device__(u64 g) -> u32 { return cnt[g] >= 3 ? 1u : 0u; };
     auto g2 = [ex] __device__(u64 g, u32 e, u32 v) { ex[g] = e; };
+    CKR((device_scan<u32>(ctx, ng, f, g2, OpSum(), tot)));
+  } else {
+    CKR(gvs_reserve(ctx, ctx->comp_rank, ng * 2 * 4));
+    u32 *rmn = ctx->comp_rank.as<u32>(), *slot = rmn + ng;
+    CK(cudaMemsetAsync(rmn, 0xFF, ng * 2 * 4, ctx->stream));
+    LAUNCH(k_comp_stats<true>, (unsigned)cdiv(ng, 256), 256, 0, ctx->parent.as<u32>(), ctx->present.as<u8>(), ng, ctx->grp_start.as<u32>(),
+           ctx->comp_cnt.as<u32>(), ctx->comp_min.as<u32>(), ctx->comp_max.as<u32>(), ctx->rank_of.as<u32>(), rmn);
+    LAUNCH(k_iv_slot, (unsigned)cdiv(ng, 256), 256, 0, cnt, rmn, ng, slot);
+    auto f = [slot] __device__(u64 q) -> u32 { return slot[q] != 0xFFFFFFFFu ? 1u : 0u; };
+    auto g2 = [ex] __device__(u64 q, u32 e, u32 v) { ex[q] = e; };
     CKR((device_scan<u32>(ctx, ng, f, g2, OpSum(), tot)));
   }
   u32 ni = 0;
@@ -180,9 +224,12 @@ extern "C" int gvs_intervals(gvs_ctx* ctx, uint64_t* n_intervals) {
   CKR(gvs_reserve(ctx, ctx->iv_contig, (u64)ni * 4));
   CKR(gvs_reserve(ctx, ctx->iv_start, (u64)ni * 4));
   CKR(gvs_reserve(ctx, ctx->iv_end, (u64)ni * 4));
-  if (ni)
+  if (ni && !by_rank)
     LAUNCH(k_iv_write, (unsigned)cdiv(ng, 256), 256, 0, ex, cnt, ng, ctx->grp_contig.as<u32>(), ctx->comp_min.as<u32>(),
            ctx->comp_max.as<u32>(), ctx->iv_contig.as<u32>(), ctx->iv_start.as<u32>(), ctx->iv_end.as<u32>());
+  if (ni && by_rank)
+    LAUNCH(k_iv_write_rank, (unsigned)cdiv(ng, 256), 256, 0, ex, ctx->comp_rank.as<u32>() + ng, ng, ctx->grp_contig.as<u32>(),
+           ctx->comp_min.as<u32>(), ctx->comp_max.as<u32>(), ctx->iv_contig.as<u32>(), ctx->iv_start.as<u32>(), ctx->iv_end.as<u32>());
   ctx->n_iv = ni;
   ctx->iv_ready = true;
   ctx->gaps_ready = false;

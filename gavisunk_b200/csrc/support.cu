@@ -53,15 +53,23 @@ static int rank_sort(gvs_ctx* ctx, DevBuf& key) {
   return 0;
 }
 
+int gvs_check_group_order(gvs_ctx* ctx) {
+  const u64 ng = ctx->n_groups;
+  u32 h = 0;
+  if (ng > 1) {
+    u32* err = (u32*)(ctx->counters.as<u64>() + 32);
+    CK(cudaMemsetAsync(err, 0, 4, ctx->stream));
+    LAUNCH(k_groups_sorted, (unsigned)cdiv(ng, 256), 256, 0, ctx->grp_contig.as<u32>(), ctx->grp_start.as<u32>(), ng, err);
+    CKR(read_dev(ctx, err, &h));
+  }
+  ctx->rank_identity = (h & 4u) == 0;
+  ctx->order_gen = ctx->grp_gen;
+  return 0;
+}
+
 int gvs_ensure_rank(gvs_ctx* ctx) {
   if (ctx->rank_gen == ctx->grp_gen) return 0;
-  const u64 ng = ctx->n_groups;
-  u32* err = (u32*)(ctx->counters.as<u64>() + 32);
-  CK(cudaMemsetAsync(err, 0, 4, ctx->stream));
-  if (ng > 1) LAUNCH(k_groups_sorted, (unsigned)cdiv(ng, 256), 256, 0, ctx->grp_contig.as<u32>(), ctx->grp_start.as<u32>(), ng, err);
-  u32 h = 0;
-  CKR(read_dev(ctx, err, &h));
-  ctx->rank_identity = (h & 4u) == 0;
+  if (ctx->order_gen != ctx->grp_gen) CKR(gvs_check_group_order(ctx));
   if (!ctx->rank_identity) {
     DevBuf key;
     int rc = rank_sort(ctx, key);

@@ -210,7 +210,7 @@ int gvs_group_index_rows(gvs_ctx* ctx, const u32* contig, const u32* group, u64 
   ctx->grp_gen++;
   if (n == 0) {
     ctx->n_groups = 0;
-    return 0;
+    return gvs_check_group_order(ctx);
   }
   u64 slots = next_pow2(n * 2 < 1024 ? 1024 : n * 2);
   DevBuf gk, gm, rep, dense;
@@ -219,6 +219,7 @@ int gvs_group_index_rows(gvs_ctx* ctx, const u32* contig, const u32* group, u64 
   if (!rc) rc = gvs_reserve(ctx, rep, n * sizeof(u32));
   if (!rc) rc = gvs_reserve(ctx, dense, n * sizeof(u32));
   if (!rc) rc = build_group_index_body(ctx, contig, group, n, gidx_out, gk, gm, rep, dense, slots);
+  if (!rc) rc = gvs_check_group_order(ctx);
   cudaStreamSynchronize(ctx->stream);
   gvs_release(gk); gvs_release(gm); gvs_release(rep); gvs_release(dense);
   return rc;
