@@ -44,11 +44,10 @@ __global__ void __launch_bounds__(256) k_stash_rows(u64 n, u32 base, const u32* 
   d_group[i] = s_group[i];
   d_gidx[i] = s_gidx[i];
 }
-__global__ void __launch_bounds__(256) k_stash_len(u64 n, const u64* __restrict__ read_off, const u32* __restrict__ read_len, u32* dst) {
+__global__ void __launch_bounds__(256) k_stash_len(u64 n, const ReadLens len, u32* dst) {
   u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  u64 l = read_len ? read_len[i] : read_off[i + 1] - read_off[i];
-  dst[i] = l > 0xFFFFFFFFull ? 0xFFFFFFFFu : (u32)l;
+  dst[i] = len((u32)i);
 }
 
 extern "C" int gvs_batches_begin(gvs_ctx* ctx) {
@@ -84,8 +83,7 @@ extern "C" int gvs_batch_stash(gvs_ctx* ctx, uint64_t* read_base) {
            K.start.as<u32>(), K.group.as<u32>(), K.gidx.as<u32>(), S.read.as<u32>() + have, S.pos.as<u32>() + have,
            S.contig.as<u32>() + have, S.start.as<u32>() + have, S.group.as<u32>() + have, S.gidx.as<u32>() + have);
   if (nr)
-    LAUNCH(k_stash_len, (unsigned)cdiv(nr, 256), 256, 0, nr, ctx->have_read_len ? nullptr : ctx->read_off,
-           ctx->have_read_len ? ctx->read_len.as<u32>() : nullptr, ctx->stash_len.as<u32>() + base);
+    LAUNCH(k_stash_len, (unsigned)cdiv(nr, 256), 256, 0, nr, read_lens(ctx), ctx->stash_len.as<u32>() + base);
   S.n = have + n;
   ctx->stash_reads = base + nr;
   if (read_base) *read_base = base;

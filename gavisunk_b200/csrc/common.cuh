@@ -38,6 +38,15 @@ struct Rows {  // sunkpos rows, structure of arrays (24 B per row)
   u64 n = 0;
 };
 
+// a result table: u32 columns `stride` entries apart in one buffer, the first n entries of each filled; `ready` once the
+// stage that writes it has run (rec_reserve / rec_get below)
+struct RecTable {
+  DevBuf buf;
+  u64 n = 0, stride = 0;
+  bool ready = false;
+  u32* col(u32 t) const { return buf.as<u32>() + t * stride; }
+};
+
 struct gvs_ctx {
   int device = 0;
   int k = 20;
@@ -149,7 +158,10 @@ struct gvs_ctx {
   // ---- validation ----
   DevBuf kseg_start;  // segments of kept rows
   u64 n_kseg = 0;
-  DevBuf val_scratch, val_cnt, val_off;
+  DevBuf val_scratch;
+  // gvs_validate's outputs per kept row (the read's validated IDs, from its first row on) and per segment (their count
+  // and their offset in the pairs)
+  const u32 *val_id = nullptr, *val_seg_cnt = nullptr, *val_seg_off = nullptr;
   DevBuf pair_read, pair_contig, pair_group, pair_gidx;
   DevBuf seg_orient;  // per segment: orientation majority of the read (0: positions rise with starts)
   u64 n_pairs = 0;
@@ -161,19 +173,15 @@ struct gvs_ctx {
   bool rank_identity = false;       // group index order is already (contig, start) order
   DevBuf rank_of, rank_grp;         // group index -> rank in (contig, start) order, and back (unless identity)
   DevBuf sup_diff;                  // int32[n_groups] by rank: +1 at a placement's first group, -1 at its last
-  DevBuf pl_read, pl_contig, pl_start, pl_end, pl_nids, pl_strand, pl_tmp;
-  u64 n_pl = 0;
-  bool pl_ready = false;
-  DevBuf sup_depth, sup_gx, sup_cstat, run_contig, run_start, run_end, run_depth;
-  u64 n_runs = 0;
-  bool sup_ready = false;
+  RecTable pl;                      // placements: read, contig, start, end, IDs
+  DevBuf pl_strand, pl_tmp;         // per placement its strand (u8); per segment (start, end, IDs, strand)
+  DevBuf sup_depth, sup_gx, sup_cstat;
+  RecTable sup;                     // runs of gvs_support: contig, start, end, depth
 
   // ---- gap evidence (gap_evidence.cu) ----
   DevBuf ge_seg_start;              // segments of the kept rows when gvs_validate's are not current
   DevBuf ge_cgap, ge_seg, ge_cand, ge_res;  // per contig gap range, per segment (first gap, count), candidates, their results
-  DevBuf ge_rec;                    // records: 8 columns of n_ge_cand entries, the first n_ge of each filled
-  u64 n_ge = 0, n_ge_cand = 0;
-  bool ge_ready = false;
+  RecTable ge;                      // records: 8 columns, one entry per candidate
 
   // ---- junctions (junctions.cu) ----
   Rows jn_stash;                    // rows gvs_junction_screen kept (run-wide read indices), input of gvs_junctions
@@ -181,19 +189,13 @@ struct gvs_ctx {
   bool jn_in_run = false;           // between gvs_batches_begin and gvs_batches_bind: a screen appends to jn_stash
   DevBuf jn_seg_start, jn_row_seg, jn_seg_cnt;  // segments of the screened / stashed rows, per segment count or offset
   DevBuf jn_flags, jn_scr;          // per-row flags (2 bytes) and per-row u32 scratch of gvs_junctions
-  DevBuf jn_rec;                    // records: 13 columns of jn_stride entries, the first n_jn of each filled
-  u64 n_jn = 0, jn_stride = 0;
-  bool jn_ready = false;
+  RecTable jn;                      // records: 13 columns
 
   // ---- discordance (discordance.cu) ----
   DevBuf dc_diff;                   // int32[3][n_groups] by rank: spans, longer, shorter (+1 at a span's first group, -1 at its last)
   DevBuf dc_scr, dc_seg;            // per kept row u32 scratch (4 arrays); per segment usable rows, records, record offset
-  DevBuf dc_rec;                    // records: 8 columns of dc_stride entries, the first n_dc of each filled
-  u64 n_dc = 0, dc_stride = 0;
-  bool dc_ready = false;
-  DevBuf dc_run_contig, dc_run_start, dc_run_end, dc_run_val;  // runs of gvs_discordance (val: 3 columns of n_dc_runs)
-  u64 n_dc_runs = 0;
-  bool dc_runs_ready = false;
+  RecTable dc;                      // span records of gvs_spans: 8 columns
+  RecTable dc_runs;                 // runs of gvs_discordance: contig, start, end, spans, longer, shorter
 
   // ---- components / intervals / gaps ----
   DevBuf parent, present, comp_min, comp_max, comp_cnt;
@@ -543,12 +545,77 @@ static int read_dev(gvs_ctx* ctx, const T* d, T* h, size_t n = 1) {
   CK(cudaStreamSynchronize(ctx->stream));
   return 0;
 }
-// the first n entries of N u32 columns stored `stride` entries apart from `src` to host buffers (null ones skipped):
-// the record getters; returns when the copies (and any queued before them) have finished
+
+// Slots of the 64-word ctx->counters block (reserved in ctx.cu and table.cu): flags a kernel sets for the host, and
+// totals the host reads later or several at once.  A total read back right after its scan goes through scan_total.
+enum CounterSlot : u32 {
+  CNT_HITS,         // match: hits                                   } cleared and read back together (match.cu)
+  CNT_FLAGS,        // match: probe flags (key error, overflow)      }
+  CNT_EMIT,         // match: (rows << 32) + suppressed hits         }
+  CNT_HIT_MAX,      // match: most hits of one probe span            }
+  CNT_SCAN,         // scan_total
+  CNT_VOTE_BIG,     // diag: candidates left to the block-wide vote
+  CNT_KEPT,         // diag: kept rows  } one read-back
+  CNT_BEST,         // diag: best rows  }
+  CNT_MISS,         // gvs_rows_set: rows whose (contig, group) is not in the database
+  CNT_HIST_MAX,     // gvs_hist_mode: largest group count
+  CNT_MODE,         // gvs_hist_mode: int64 mode per haplotype (two words)
+  CNT_VAL_STATS = CNT_MODE + 2,  // gvs_validate: reads whose clean-up removed every edge
+  CNT_COVPROB_ERR,  // gvs_covprob_gaps
+  CNT_ORDER_ERR,    // gvs_check_group_order
+  CNT_RUNS_ERR,     // gvs_rank_runs
+  CNT_COUNT
+};
+static_assert(CNT_COUNT <= 64, "ctx->counters holds 64 words");
+template <typename T = u32>
+static inline T* counter(gvs_ctx* ctx, CounterSlot s) { return (T*)(ctx->counters.as<u64>() + s); }
+
+// device_scan whose grand total the host needs at once: *total receives it (one read-back)
+template <typename T, typename Op, typename F, typename G>
+static int scan_total(gvs_ctx* ctx, u64 n, F f, G g, Op op, T* total) {
+  T* d = counter<T>(ctx, CNT_SCAN);
+  CKR((device_scan<T>(ctx, n, f, g, op, d)));
+  return read_dev(ctx, d, total);
+}
+
+// the kept rows of a Rows cut into segments (one per read), as the per-read kernels see them
+struct SegRows {
+  const u32 *read, *pos, *contig, *start, *group, *gidx;
+  const u32* seg_start;  // n_seg + 1
+  u32 n_seg;
+  const u8* bad;         // per group index (null: nothing is bad)
+  __device__ __forceinline__ bool is_bad(u32 i) const { return bad && bad[gidx[i]]; }
+};
+static inline SegRows seg_rows(const gvs_ctx* ctx, const Rows& r, const DevBuf& seg_start, u64 n_seg) {
+  return {r.read.as<u32>(), r.pos.as<u32>(), r.contig.as<u32>(), r.start.as<u32>(), r.group.as<u32>(), r.gidx.as<u32>(),
+          seg_start.as<u32>(), (u32)n_seg, ctx->bad_ready ? ctx->bad_flag.as<u8>() : nullptr};
+}
+
+// read lengths: explicit (gvs_reads_meta, a batches run) or from the offsets of the batch, clamped to 32 bits
+struct ReadLens {
+  const u64* off;
+  const u32* len;  // null: from off
+  __device__ __forceinline__ u32 operator()(u32 rd) const {
+    return len ? len[rd] : (u32)min(off[rd + 1] - off[rd], (u64)0xFFFFFFFFu);
+  }
+};
+static inline ReadLens read_lens(const gvs_ctx* ctx) {
+  return {ctx->read_off, ctx->have_read_len ? ctx->read_len.as<u32>() : nullptr};
+}
+
+static inline int rec_reserve(gvs_ctx* ctx, RecTable& t, u32 n_cols, u64 stride) {
+  t.stride = stride;
+  return gvs_reserve(ctx, t.buf, stride * n_cols * 4);
+}
+// a record getter: the first n entries of the table's columns to host buffers (null ones skipped); returns when the
+// copies (and any queued before them) have finished
 template <int N>
-static int columns_to_host(gvs_ctx* ctx, const u32* src, u64 stride, u64 n, uint32_t* const (&dst)[N]) {
-  for (int t = 0; t < N; t++)
-    if (dst[t]) CK(cudaMemcpyAsync(dst[t], src + (u64)t * stride, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+static int rec_get(gvs_ctx* ctx, const RecTable& t, const char* before, uint32_t* const (&dst)[N]) {
+  if (!t.ready) return gvs_fail(ctx, GVS_E_STATE, "%s", before);
+  CK(cudaSetDevice(ctx->device));
+  if (t.n == 0) return 0;
+  for (int c = 0; c < N; c++)
+    if (dst[c]) CK(cudaMemcpyAsync(dst[c], t.col(c), t.n * 4, cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   return 0;
 }
@@ -571,9 +638,6 @@ int gvs_ensure_rank(gvs_ctx* ctx);
 // rank of a sorted table costs the later stages nothing)
 int gvs_check_group_order(gvs_ctx* ctx);
 // support.cu: runs of equal values over the groups in rank order that tile [0, contig_len) of every contig: diff = nv
-// difference arrays of n_groups int32 by rank, prefix-summed here; out.val receives nv columns of *n_runs entries
-struct RankRuns {
-  DevBuf *contig, *start, *end, *val;
-};
-int gvs_rank_runs(gvs_ctx* ctx, const i32* diff, u32 nv, const uint32_t* contig_len, RankRuns& out, u64* n_runs, const char* who);
+// difference arrays of n_groups int32 by rank, prefix-summed here; out receives 3 + nv columns: contig, start, end, values
+int gvs_rank_runs(gvs_ctx* ctx, const i32* diff, u32 nv, const uint32_t* contig_len, RecTable& out, const char* who);
 int grow_keep(gvs_ctx* ctx, DevBuf& b, size_t need, size_t keep);  // batches.cu: grow to `need` bytes keeping the first `keep`

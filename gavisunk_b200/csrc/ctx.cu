@@ -173,15 +173,13 @@ extern "C" void gvs_destroy(gvs_ctx* c) {
                    &c->ohit_w, &c->ohit_row, &c->counters, &c->scan_tmp, &c->scan_tmp2, &c->flags_a, &c->flags_b,
                    &c->flags_c, &c->seg_start, &c->seg_ndist, &c->seg_cap, &c->seg_best, &c->seg_good, &c->seg_dir,
                    &c->diag_scratch, &c->best_read, &c->best_contig, &c->best_good, &c->best_dir, &c->hist,
-                   &c->cnt_hist, &c->bad_flag, &c->bad_list, &c->kseg_start, &c->val_scratch, &c->val_cnt,
-                   &c->val_off, &c->pair_read, &c->pair_contig, &c->pair_group, &c->pair_gidx, &c->parent,
-                   &c->present, &c->comp_min, &c->comp_max, &c->comp_cnt, &c->comp_rank, &c->iv_contig, &c->iv_start, &c->iv_end,
+                   &c->cnt_hist, &c->bad_flag, &c->bad_list, &c->kseg_start, &c->val_scratch, &c->pair_read,
+                   &c->pair_contig, &c->pair_group, &c->pair_gidx, &c->parent, &c->present, &c->comp_min, &c->comp_max, &c->comp_cnt, &c->comp_rank, &c->iv_contig, &c->iv_start, &c->iv_end,
                    &c->gap_contig, &c->gap_start, &c->gap_end, &c->nodata_contig, &c->read_len, &c->gt_keys, &c->gt_val,
-                   &c->seg_orient, &c->rank_of, &c->rank_grp, &c->sup_diff, &c->pl_read, &c->pl_contig, &c->pl_start, &c->pl_end,
-                   &c->pl_nids, &c->pl_strand, &c->pl_tmp, &c->sup_depth, &c->sup_gx, &c->sup_cstat, &c->run_contig, &c->run_start,
-                   &c->run_end, &c->run_depth, &c->ge_seg_start, &c->ge_cgap, &c->ge_seg, &c->ge_cand, &c->ge_res, &c->ge_rec,
-                   &c->jn_seg_start, &c->jn_row_seg, &c->jn_seg_cnt, &c->jn_flags, &c->jn_scr, &c->jn_rec, &c->dc_diff, &c->dc_scr,
-                   &c->dc_seg, &c->dc_rec, &c->dc_run_contig, &c->dc_run_start, &c->dc_run_end, &c->dc_run_val};
+                   &c->seg_orient, &c->rank_of, &c->rank_grp, &c->sup_diff, &c->pl_strand, &c->pl_tmp,
+                   &c->sup_depth, &c->sup_gx, &c->sup_cstat, &c->ge_seg_start, &c->ge_cgap, &c->ge_seg, &c->ge_cand, &c->ge_res,
+                   &c->jn_seg_start, &c->jn_row_seg, &c->jn_seg_cnt, &c->jn_flags, &c->jn_scr, &c->dc_diff, &c->dc_scr, &c->dc_seg,
+                   &c->pl.buf, &c->sup.buf, &c->ge.buf, &c->jn.buf, &c->dc.buf, &c->dc_runs.buf};
   for (DevBuf* b : all) gvs_release(*b);
   release_rows(c->rows);
   release_rows(c->kept);

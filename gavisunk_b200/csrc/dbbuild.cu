@@ -320,14 +320,12 @@ static int db_build_device(gvs_ctx* ctx, const u8* seq, const u64* contig_off, u
   CKR(gvs_reserve(ctx, wrank, n_words * 4));
   const u32* bm = bitmap.as<u32>();
   u32* wr = wrank.as<u32>();
-  u64* tot = ctx->counters.as<u64>() + 4;
+  u64 n_sunks = 0;
   {
     auto f = [bm] __device__(u64 i) -> u64 { return (u64)__popc(bm[i]); };
     auto g = [wr] __device__(u64 i, u64 ex, u64 v) { wr[i] = (u32)ex; };
-    CKR((device_scan<u64>(ctx, n_words, f, g, OpSum(), tot)));
+    CKR(scan_total(ctx, n_words, f, g, OpSum(), &n_sunks));
   }
-  u64 n_sunks = 0;
-  CKR(read_dev(ctx, tot, &n_sunks));
   if (n_sunks >= 0x7FFFFFF0ull) return gvs_fail(ctx, GVS_E_OVERFLOW, "more than 2^31 SUNKs");
   ctx->n_loc = n_sunks;
   ctx->n_contigs = n_contigs;
@@ -352,14 +350,12 @@ static int db_build_device(gvs_ctx* ctx, const u8* seq, const u64* contig_off, u
       auto g = [hr] __device__(u64 i, u32 ex, u32 v) { hr[i] = ex > v ? ex : v; };
       CKR((device_scan<u32>(ctx, n_sunks, f, g, OpMax(), (u32*)nullptr)));
     }
-    u32* gt = (u32*)(ctx->counters.as<u64>() + 5);
+    u32 ng = 0;
     {
       auto f = [hd] __device__(u64 i) -> u32 { return hd[i] ? 1u : 0u; };
       auto g = [ge] __device__(u64 i, u32 ex, u32 v) { ge[i] = ex; };
-      CKR((device_scan<u32>(ctx, n_sunks, f, g, OpSum(), gt)));
+      CKR(scan_total(ctx, n_sunks, f, g, OpSum(), &ng));
     }
-    u32 ng = 0;
-    CKR(read_dev(ctx, gt, &ng));
     ctx->n_groups = ng;
     CKR(gvs_reserve(ctx, ctx->grp_contig, (u64)ng * 4));
     CKR(gvs_reserve(ctx, ctx->grp_start, (u64)ng * 4));

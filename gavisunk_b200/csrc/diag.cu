@@ -32,12 +32,10 @@ __global__ void __launch_bounds__(256) k_seg_fill(const u32* __restrict__ read, 
 int gvs_build_segments(gvs_ctx* ctx, const u32* read, u64 n, DevBuf& seg_start, DevBuf& row_seg, u64* n_seg_out) {
   CKR(gvs_reserve(ctx, row_seg, n * 4));
   u32* rs = row_seg.as<u32>();
-  u32* tot = (u32*)(ctx->counters.as<u64>() + 8);
   auto f = [read] __device__(u64 j) -> u32 { return (j == 0 || read[j] != read[j - 1]) ? 1u : 0u; };
   auto g = [rs] __device__(u64 j, u32 ex, u32 v) { rs[j] = ex + v - 1; };
-  CKR((device_scan<u32>(ctx, n, f, g, OpSum(), tot)));
   u32 ns = 0;
-  CKR(read_dev(ctx, tot, &ns));
+  CKR(scan_total(ctx, n, f, g, OpSum(), &ns));
   CKR(gvs_reserve(ctx, seg_start, ((u64)ns + 1) * 4));
   LAUNCH(k_seg_fill, (unsigned)cdiv(n + 1, 256), 256, 0, read, rs, n, seg_start.as<u32>(), ns);
   *n_seg_out = ns;
@@ -589,7 +587,7 @@ static int diag_impl(gvs_ctx* ctx, u64* n_best_out, u64* n_kept_out) {
   LAUNCH(k_row_first, (unsigned)cdiv(n, 256), 256, 0, contig, row_seg, seg_start, n, D.row_cnt, D.seg_ndist);
   // candidates: first rows whose contig is in the read's haplotype and has >= 2 hits (nim:82,147)
   const u8* contig_hap = ctx->contig_hap.as<u8>();
-  u64* tot = ctx->counters.as<u64>() + 9;
+  u64 packed = 0;
   {
     const u32* rc = D.row_cnt;
     const u8* sh = D.seg_hap;
@@ -605,16 +603,14 @@ static int diag_impl(gvs_ctx* ctx, u64* n_best_out, u64* n_kept_out) {
         cvoff[ex >> 32] = (u32)ex;
       }
     };
-    CKR((device_scan<u64>(ctx, n, f, g, OpSum(), tot)));
+    CKR(scan_total(ctx, n, f, g, OpSum(), &packed));
   }
-  u64 packed = 0;
-  CKR(read_dev(ctx, tot, &packed));
   u32 n_cand = (u32)(packed >> 32);
   CK(cudaMemcpyAsync(D.cidx + n, &n_cand, 4, cudaMemcpyHostToDevice, ctx->stream));
   if (n_cand) {
     LAUNCH(k_cand_gather, (unsigned)cdiv((u64)n_cand * 32, 256), 256, 0, D.cand_row, D.cand_voff, n_cand, contig, pos, start,
            group, row_seg, seg_start, D.v_pos, D.v_start, D.v_group);
-    u32* n_big = (u32*)(ctx->counters.as<u64>() + 30);
+    u32* n_big = counter(ctx, CNT_VOTE_BIG);
     CK(cudaMemsetAsync(n_big, 0, 4, ctx->stream));
     u32* big_list = D.keep_excl;  // free until the keep scan below
     LAUNCH(k_cand_vote_warp, (unsigned)cdiv(n_cand, VOTE_WARPS), VOTE_WARPS * 32, 0, D.cand_row, D.cand_voff, n_cand, D.row_cnt,
@@ -625,38 +621,32 @@ static int diag_impl(gvs_ctx* ctx, u64* n_best_out, u64* n_kept_out) {
   LAUNCH(k_seg_best, (unsigned)cdiv(n_seg, 256), 256, 0, (u32)n_seg, seg_start, D.cidx, D.cand_row, D.row_cnt, contig,
          D.cand_good, D.cand_dir, D.seg_best, D.seg_good, D.seg_dir, D.seg_tie);
   // ---- ties: Table capacity at the start of each read (sticky within a chunk) ----
-  u32* tie_tot = (u32*)(ctx->counters.as<u64>() + 10);
+  u32 n_tie = 0;
   {
     const u8* st = D.seg_tie;
     u32* ts = D.tie_seg;
     auto f = [st] __device__(u64 s) -> u32 { return st[s]; };
     auto g = [ts] __device__(u64 s, u32 ex, u32 v) { if (v) ts[ex] = (u32)s; };
-    CKR((device_scan<u32>(ctx, n_seg, f, g, OpSum(), tie_tot)));
+    CKR(scan_total(ctx, n_seg, f, g, OpSum(), &n_tie));
   }
-  u32 n_tie = 0;
-  CKR(read_dev(ctx, tie_tot, &n_tie));
   if (n_tie) {
     const u32 *sc = D.seg_chunk, *nd = D.seg_ndist;
     u32* cap = D.seg_cap;
-    u64* mx = ctx->counters.as<u64>() + 11;
     auto f = [sc, nd] __device__(u64 s) -> u64 { return ((u64)(sc[s] + 1) << 32) | cap_needed(nd[s]); };
     auto g = [sc, cap] __device__(u64 s, u64 ex, u64 v) {
       cap[s] = ((u32)(ex >> 32) == sc[s] + 1) ? (u32)ex : 64u;  // capacity left by earlier reads of the chunk
     };
-    CKR((device_scan<u64>(ctx, n_seg, f, g, OpMax(), mx)));
     u64 mxv = 0;
-    CKR(read_dev(ctx, mx, &mxv));
+    CKR(scan_total(ctx, n_seg, f, g, OpMax(), &mxv));
     // any read may itself grow the table while it is replayed: bound by the largest need overall
     u32 maxcap = 64;
     {
       // the u64 max is dominated by the chunk id; take a safe bound from the largest segment instead
       u32 max_nd = 0;
       const u32* ndp = D.seg_ndist;
-      u32* mnd = (u32*)(ctx->counters.as<u64>() + 12);
       auto f2 = [ndp] __device__(u64 s) -> u32 { return ndp[s]; };
       auto g2 = [] __device__(u64 s, u32 ex, u32 v) {};
-      CKR((device_scan<u32>(ctx, n_seg, f2, g2, OpMax(), mnd)));
-      CKR(read_dev(ctx, mnd, &max_nd));
+      CKR(scan_total(ctx, n_seg, f2, g2, OpMax(), &max_nd));
       maxcap = cap_needed(max_nd) * 2;
     }
     DevBuf& sb = ctx->scan_tmp2;
@@ -665,7 +655,7 @@ static int diag_impl(gvs_ctx* ctx, u64* n_best_out, u64* n_kept_out) {
            contig, ctx->contig_hash.as<u32>(), D.cand_good, D.cand_dir, sb.as<u32>(), maxcap, D.seg_best, D.seg_dir);
   }
   // ---- kept rows + best list ----
-  u32* kt = (u32*)(ctx->counters.as<u64>() + 13);
+  u32* kt = counter(ctx, CNT_KEPT);
   {
     const u32* sbest = D.seg_best;
     u32* ke = D.keep_excl;
@@ -673,7 +663,7 @@ static int diag_impl(gvs_ctx* ctx, u64* n_best_out, u64* n_kept_out) {
     auto g = [ke] __device__(u64 j, u32 ex, u32 v) { ke[j] = ex; };
     CKR((device_scan<u32>(ctx, n, f, g, OpSum(), kt)));
   }
-  u32* bt = (u32*)(ctx->counters.as<u64>() + 14);
+  u32* bt = counter(ctx, CNT_BEST);
   {
     const u32* sbest = D.seg_best;
     u32* be = D.best_excl;
@@ -681,8 +671,8 @@ static int diag_impl(gvs_ctx* ctx, u64* n_best_out, u64* n_kept_out) {
     auto g = [be] __device__(u64 s, u32 ex, u32 v) { be[s] = ex; };
     CKR((device_scan<u32>(ctx, n_seg, f, g, OpSum(), bt)));
   }
-  u64 kb[2] = {0, 0};  // counters 13 and 14: one read-back for both totals
-  CKR(read_dev(ctx, ctx->counters.as<u64>() + 13, kb, 2));
+  u64 kb[2] = {0, 0};  // one read-back for both totals
+  CKR(read_dev(ctx, counter<u64>(ctx, CNT_KEPT), kb, 2));
   const u32 n_kept = (u32)kb[0], n_best = (u32)kb[1];
   CKR(gvs_reserve_rows(ctx, ctx->kept, n_kept));
   CKR(gvs_reserve(ctx, ctx->best_read, (u64)n_best * 4));
@@ -770,11 +760,9 @@ extern "C" int gvs_filter_best(gvs_ctx* ctx, const uint32_t* best_contig_of_read
     const u32* best = ctx->seg_best.as<u32>();
     const u32 *read = R.read.as<u32>(), *contig = R.contig.as<u32>();
     u32* ke = ctx->flags_b.as<u32>();
-    u32* kt = (u32*)(ctx->counters.as<u64>() + 13);
     auto f = [best, read, contig] __device__(u64 j) -> u32 { return best[read[j]] == contig[j] ? 1u : 0u; };
     auto g = [ke] __device__(u64 j, u32 ex, u32 v) { ke[j] = ex; };
-    CKR((device_scan<u32>(ctx, n, f, g, OpSum(), kt)));
-    CKR(read_dev(ctx, kt, &nk));
+    CKR(scan_total(ctx, n, f, g, OpSum(), &nk));
     CKR(gvs_reserve_rows(ctx, ctx->kept, nk));
     LAUNCH(k_keep_by_table, (unsigned)cdiv(n, 256), 256, 0, n, ke, best, read, R.pos.as<u32>(), contig, R.start.as<u32>(),
            R.group.as<u32>(), R.gidx.as<u32>(), ctx->kept.read.as<u32>(), ctx->kept.pos.as<u32>(), ctx->kept.contig.as<u32>(),

@@ -16,12 +16,8 @@
 
 #define DC_NONE 0xFFFFFFFFu
 
-struct DcParams {
-  const u32 *read, *pos, *contig, *start, *group, *gidx;  // kept rows
-  const u32* seg_start;                                    // n_seg + 1 (gvs_validate's segments)
-  u32 n_seg;
+struct DcParams : SegRows {     // kept rows, gvs_validate's segments
   const u32 *val_cnt, *val_id;  // gvs_validate: validated IDs per segment, and the IDs from the segment's first row on
-  const u8* bad;                // per group index (null: nothing is bad)
   const u32* rank_of;           // null: rank = group index
   u64 ng;
   i64 min_delta, rel_permille;
@@ -34,7 +30,7 @@ struct DcParams {
 // index of row i's ID among the c sorted validated IDs of its read, DC_NONE when the row is bad, on another contig than
 // the read's first row, or not validated
 __device__ __forceinline__ u32 dc_find(const DcParams& P, const u32* vid, u32 c, u32 i, u32 c0) {
-  if (P.contig[i] != c0 || (P.bad && P.bad[P.gidx[i]])) return DC_NONE;
+  if (P.contig[i] != c0 || P.is_bad(i)) return DC_NONE;
   const u32 id = P.group[i];
   u32 l = 0, h = c;
   while (l < h) {
@@ -167,8 +163,8 @@ extern "C" int gvs_spans(gvs_ctx* ctx, uint32_t min_delta, uint32_t rel_permille
   if (rel_permille > 1000000u) return gvs_fail(ctx, GVS_E_ARG, "gvs_spans: rel_permille %u > 1000000", rel_permille);
   CK(cudaSetDevice(ctx->device));
   StageTimer tm(ctx, GVS_ST_DISCORDANCE);
-  ctx->dc_ready = ctx->dc_runs_ready = false;
-  ctx->n_dc = 0;
+  ctx->dc.ready = ctx->dc_runs.ready = false;
+  ctx->dc.n = 0;
   if (n_records) *n_records = 0;
   CKR(gvs_ensure_rank(ctx));
   const u64 ng = ctx->n_groups;
@@ -179,14 +175,9 @@ extern "C" int gvs_spans(gvs_ctx* ctx, uint32_t min_delta, uint32_t rel_permille
   if (n && ctx->n_pairs) {
     const Rows& K = ctx->kept;
     DcParams P;
-    P.read = K.read.as<u32>(); P.pos = K.pos.as<u32>(); P.contig = K.contig.as<u32>(); P.start = K.start.as<u32>();
-    P.group = K.group.as<u32>(); P.gidx = K.gidx.as<u32>();
-    P.seg_start = ctx->kseg_start.as<u32>();
-    P.n_seg = (u32)n_seg;
-    // gvs_validate's scratch: out_id[n], out_gidx[n], seg_cnt[n_seg], seg_off[n_seg]
-    P.val_id = ctx->val_scratch.as<u32>();
-    P.val_cnt = P.val_id + 2 * n;
-    P.bad = ctx->bad_ready ? ctx->bad_flag.as<u8>() : nullptr;
+    (SegRows&)P = seg_rows(ctx, K, ctx->kseg_start, n_seg);
+    P.val_id = ctx->val_id;
+    P.val_cnt = ctx->val_seg_cnt;
     P.rank_of = ctx->rank_identity ? nullptr : ctx->rank_of.as<u32>();
     P.ng = ng;
     P.min_delta = min_delta;
@@ -198,21 +189,19 @@ extern "C" int gvs_spans(gvs_ctx* ctx, uint32_t min_delta, uint32_t rel_permille
     u32* seg_off = P.seg_n + n_seg;
     P.diff = ctx->dc_diff.as<i32>();
     LAUNCH(k_dc_spans, (unsigned)cdiv(n_seg * 32, 256), 256, 0, P);
-    u32* tot = (u32*)(ctx->counters.as<u64>() + 40);
     {
       const u32* seg_n = P.seg_n;
       auto f = [seg_n] __device__(u64 s) -> u32 { return seg_n[s]; };
       auto g = [seg_off] __device__(u64 s, u32 ex, u32 v) { seg_off[s] = ex; };
-      CKR((device_scan<u32>(ctx, n_seg, f, g, OpSum(), tot)));
+      CKR(scan_total(ctx, n_seg, f, g, OpSum(), &nr));
     }
-    CKR(read_dev(ctx, tot, &nr));
     if (nr) {
-      CKR(gvs_reserve(ctx, ctx->dc_rec, (u64)nr * 8 * 4));
-      LAUNCH(k_dc_emit, (unsigned)cdiv(n_seg * 32, 256), 256, 0, P, seg_off, ctx->dc_rec.as<u32>(), (u64)nr);
+      CKR(rec_reserve(ctx, ctx->dc, 8, nr));
+      LAUNCH(k_dc_emit, (unsigned)cdiv(n_seg * 32, 256), 256, 0, P, seg_off, ctx->dc.col(0), (u64)nr);
     }
   }
-  ctx->n_dc = ctx->dc_stride = nr;
-  ctx->dc_ready = true;
+  ctx->dc.n = nr;
+  ctx->dc.ready = true;
   if (n_records) *n_records = nr;
   if (diff_dev) *diff_dev = ctx->dc_diff.as<i32>();
   return 0;
@@ -220,42 +209,22 @@ extern "C" int gvs_spans(gvs_ctx* ctx, uint32_t min_delta, uint32_t rel_permille
 
 extern "C" int gvs_spans_get(gvs_ctx* ctx, uint32_t* read, uint32_t* contig, uint32_t* id1, uint32_t* start1, uint32_t* pos1,
                              uint32_t* id2, uint32_t* start2, uint32_t* pos2) {
-  if (!ctx) return GVS_E_ARG;
-  if (!ctx->dc_ready) return gvs_fail(ctx, GVS_E_STATE, "gvs_spans_get before gvs_spans");
-  CK(cudaSetDevice(ctx->device));
-  const u64 n = ctx->n_dc, stride = ctx->dc_stride;
-  if (n == 0) return 0;
-  uint32_t* dst[8] = {read, contig, id1, start1, pos1, id2, start2, pos2};
-  return columns_to_host(ctx, ctx->dc_rec.as<u32>(), stride, n, dst);
+  return ctx ? rec_get(ctx, ctx->dc, "gvs_spans_get before gvs_spans", {read, contig, id1, start1, pos1, id2, start2, pos2}) : GVS_E_ARG;
 }
 
 extern "C" int gvs_discordance(gvs_ctx* ctx, const uint32_t* contig_len, uint64_t* n_runs) {
   if (!ctx) return GVS_E_ARG;
-  if (!ctx->dc_ready) return gvs_fail(ctx, GVS_E_STATE, "gvs_discordance before gvs_spans");
+  if (!ctx->dc.ready) return gvs_fail(ctx, GVS_E_STATE, "gvs_discordance before gvs_spans");
   CK(cudaSetDevice(ctx->device));
   StageTimer tm(ctx, GVS_ST_DISCORDANCE);
-  ctx->dc_runs_ready = false;
-  ctx->n_dc_runs = 0;
   if (n_runs) *n_runs = 0;
-  RankRuns out{&ctx->dc_run_contig, &ctx->dc_run_start, &ctx->dc_run_end, &ctx->dc_run_val};
-  u64 nr = 0;
-  CKR(gvs_rank_runs(ctx, ctx->dc_diff.as<i32>(), 3, contig_len, out, &nr, "gvs_discordance"));
-  ctx->n_dc_runs = nr;
-  ctx->dc_runs_ready = true;
-  if (n_runs) *n_runs = nr;
+  CKR(gvs_rank_runs(ctx, ctx->dc_diff.as<i32>(), 3, contig_len, ctx->dc_runs, "gvs_discordance"));
+  if (n_runs) *n_runs = ctx->dc_runs.n;
   return 0;
 }
 
 extern "C" int gvs_discordance_get(gvs_ctx* ctx, uint32_t* contig, uint32_t* start, uint32_t* end, uint32_t* spans, uint32_t* longer,
                                    uint32_t* shorter) {
-  if (!ctx) return GVS_E_ARG;
-  if (!ctx->dc_runs_ready) return gvs_fail(ctx, GVS_E_STATE, "gvs_discordance_get before gvs_discordance");
-  CK(cudaSetDevice(ctx->device));
-  const u64 n = ctx->n_dc_runs;
-  if (n == 0) return 0;
-  if (contig) CK(cudaMemcpyAsync(contig, ctx->dc_run_contig.p, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  if (start) CK(cudaMemcpyAsync(start, ctx->dc_run_start.p, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  if (end) CK(cudaMemcpyAsync(end, ctx->dc_run_end.p, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  uint32_t* dst[3] = {spans, longer, shorter};
-  return columns_to_host(ctx, ctx->dc_run_val.as<u32>(), n, n, dst);
+  return ctx ? rec_get(ctx, ctx->dc_runs, "gvs_discordance_get before gvs_discordance", {contig, start, end, spans, longer, shorter})
+             : GVS_E_ARG;
 }

@@ -23,13 +23,8 @@ __global__ void __launch_bounds__(256) k_ge_contig_gaps(const u32* __restrict__ 
   if (i + 1 == n || gc[i + 1] != c) hi[c] = (u32)i + 1;
 }
 
-struct GeRows {
-  const u32 *read, *pos, *contig, *start, *group, *gidx;  // kept rows
-  const u32* seg_start;                                    // n_seg + 1
-  u32 n_seg;
-  const u8* bad;        // per group index (null: nothing is bad)
-  const u64* read_off;  // read lengths from offsets ...
-  const u32* read_len;  // ... or explicit
+struct GeRows : SegRows {  // kept rows
+  ReadLens len;
   u32 min_len;
   const u32 *gap_contig, *gap_start, *gap_end;
   const u32 *cg_lo, *cg_hi;  // per contig: its gaps
@@ -43,7 +38,7 @@ __global__ void __launch_bounds__(256) k_ge_cand(const GeRows R, uint2* seg_cand
   if (s >= R.n_seg) return;
   const u32 a = R.seg_start[s], b = R.seg_start[s + 1];
   const u32 rd = R.read[a], c = R.contig[a];
-  const u32 rlen = R.read_len ? R.read_len[rd] : (u32)(R.read_off[rd + 1] - R.read_off[rd]);
+  const u32 rlen = R.len(rd);
   const u32 glo = c < R.n_contigs ? R.cg_lo[c] : 0, ghi = c < R.n_contigs ? R.cg_hi[c] : 0;
   if (rlen < R.min_len || glo == ghi) {
     if (lane == 0) seg_cand[s] = make_uint2(0, 0);
@@ -51,7 +46,7 @@ __global__ void __launch_bounds__(256) k_ge_cand(const GeRows R, uint2* seg_cand
   }
   u32 mn = 0xFFFFFFFFu, mx = 0;
   for (u32 j = a + lane; j < b; j += 32) {
-    if (R.contig[j] != c || (R.bad && R.bad[R.gidx[j]])) continue;
+    if (R.contig[j] != c || R.is_bad(j)) continue;
     const u32 id = R.group[j];
     mn = min(mn, id);
     mx = max(mx, id);
@@ -85,7 +80,7 @@ __global__ void __launch_bounds__(256) k_ge_resolve(const GeRows R, const u32* _
   const u32 c = R.gap_contig[gi], gs = R.gap_start[gi], ge1 = R.gap_end[gi] + 1;
   // side of a row: 1 left, 2 right, 0 neither (other contig, bad group, inside the gap)
   auto side = [&](u32 j, u32& id) -> u32 {
-    if (R.contig[j] != c || (R.bad && R.bad[R.gidx[j]])) return 0;
+    if (R.contig[j] != c || R.is_bad(j)) return 0;
     id = R.group[j];
     return id <= gs ? 1u : (id >= ge1 ? 2u : 0u);
   };
@@ -144,33 +139,31 @@ extern "C" int gvs_gap_evidence(gvs_ctx* ctx, uint32_t min_read_len, uint64_t* n
   if (!ctx->read_off && !ctx->have_read_len) return gvs_fail(ctx, GVS_E_STATE, "gvs_gap_evidence: read lengths unknown");
   CK(cudaSetDevice(ctx->device));
   StageTimer tm(ctx, GVS_ST_EVIDENCE);
-  ctx->ge_ready = false;
-  ctx->n_ge = 0;
+  ctx->ge.ready = false;
+  ctx->ge.n = 0;
   if (n_records) *n_records = 0;
   Rows& K = ctx->kept;
   const u64 n = K.n, ngap = ctx->n_gaps;
   const u32 nc = ctx->n_contigs;
   if (n == 0 || ngap == 0 || nc == 0) {
-    ctx->ge_ready = true;
+    ctx->ge.ready = true;
     return 0;
   }
   // segments of the kept rows: gvs_validate's while they are current, else built here
-  const u32* seg_start = ctx->kseg_start.as<u32>();
+  const DevBuf* segs = &ctx->kseg_start;
   u64 n_seg = ctx->n_kseg;
   if (!ctx->val_ready) {
     CKR(gvs_build_segments(ctx, K.read.as<u32>(), n, ctx->ge_seg_start, ctx->flags_c, &n_seg));
-    seg_start = ctx->ge_seg_start.as<u32>();
+    segs = &ctx->ge_seg_start;
   }
+  const u32* seg_start = segs->as<u32>();
   CKR(gvs_reserve(ctx, ctx->ge_cgap, (u64)nc * 8));
   u32 *cg_lo = ctx->ge_cgap.as<u32>(), *cg_hi = cg_lo + nc;
   CK(cudaMemsetAsync(cg_lo, 0, (u64)nc * 8, ctx->stream));
   LAUNCH(k_ge_contig_gaps, (unsigned)cdiv(ngap, 256), 256, 0, ctx->gap_contig.as<u32>(), ngap, cg_lo, cg_hi);
   GeRows R;
-  R.read = K.read.as<u32>(); R.pos = K.pos.as<u32>(); R.contig = K.contig.as<u32>(); R.start = K.start.as<u32>();
-  R.group = K.group.as<u32>(); R.gidx = K.gidx.as<u32>();
-  R.seg_start = seg_start; R.n_seg = (u32)n_seg;
-  R.bad = ctx->bad_ready ? ctx->bad_flag.as<u8>() : nullptr;
-  R.read_off = ctx->read_off; R.read_len = ctx->have_read_len ? ctx->read_len.as<u32>() : nullptr;
+  (SegRows&)R = seg_rows(ctx, K, *segs, n_seg);
+  R.len = read_lens(ctx);
   R.min_len = min_read_len;
   R.gap_contig = ctx->gap_contig.as<u32>(); R.gap_start = ctx->gap_start.as<u32>(); R.gap_end = ctx->gap_end.as<u32>();
   R.cg_lo = cg_lo; R.cg_hi = cg_hi; R.n_contigs = nc;
@@ -178,17 +171,14 @@ extern "C" int gvs_gap_evidence(gvs_ctx* ctx, uint32_t min_read_len, uint64_t* n
   uint2* seg_cand = ctx->ge_seg.as<uint2>();
   LAUNCH(k_ge_cand, (unsigned)cdiv(n_seg * 32, 256), 256, 0, R, seg_cand);
   // candidates: count per segment, scan, fill
-  u32* tot = (u32*)(ctx->counters.as<u64>() + 36);
+  u32 ncand = 0;
   {
     auto f = [seg_cand] __device__(u64 s) -> u32 { return seg_cand[s].y; };
     auto g = [] __device__(u64 s, u32 ex, u32 v) {};
-    CKR((device_scan<u32>(ctx, n_seg, f, g, OpSum(), tot)));
+    CKR(scan_total(ctx, n_seg, f, g, OpSum(), &ncand));
   }
-  u32 ncand = 0;
-  CKR(read_dev(ctx, tot, &ncand));
-  ctx->n_ge_cand = ncand;
   if (ncand == 0) {
-    ctx->ge_ready = true;
+    ctx->ge.ready = true;
     return 0;
   }
   CKR(gvs_reserve(ctx, ctx->ge_cand, (u64)ncand * 8));
@@ -208,10 +198,10 @@ extern "C" int gvs_gap_evidence(gvs_ctx* ctx, uint32_t min_read_len, uint64_t* n
   u32* res = ctx->ge_res.as<u32>();
   LAUNCH(k_ge_resolve, (unsigned)cdiv((u64)ncand * 32, 256), 256, 0, R, cseg, cgap, ncand, res);
   // records in candidate order (segment, then gap): 8 columns of ncand entries
-  CKR(gvs_reserve(ctx, ctx->ge_rec, (u64)ncand * 32));
-  u32* rec = ctx->ge_rec.as<u32>();
+  CKR(rec_reserve(ctx, ctx->ge, 8, ncand));
+  u32* rec = ctx->ge.col(0);
   const u32* rread = K.read.as<u32>();
-  tot = (u32*)(ctx->counters.as<u64>() + 37);
+  u32 nr = 0;
   {
     auto f = [res] __device__(u64 k) -> u32 { return res[k * 8]; };
     auto g = [res, rec, ncand, cseg, cgap, seg_start, rread] __device__(u64 k, u32 ex, u32 v) {
@@ -221,23 +211,17 @@ extern "C" int gvs_gap_evidence(gvs_ctx* ctx, uint32_t min_read_len, uint64_t* n
       rec[(u64)ncand + ex] = cgap[k];
       for (int t = 1; t < 7; t++) rec[(u64)(t + 1) * ncand + ex] = r[t];
     };
-    CKR((device_scan<u32>(ctx, ncand, f, g, OpSum(), tot)));
+    CKR(scan_total(ctx, ncand, f, g, OpSum(), &nr));
   }
-  u32 nr = 0;
-  CKR(read_dev(ctx, tot, &nr));
-  ctx->n_ge = nr;
-  ctx->ge_ready = true;
+  ctx->ge.n = nr;
+  ctx->ge.ready = true;
   if (n_records) *n_records = nr;
   return 0;
 }
 
 extern "C" int gvs_gap_evidence_get(gvs_ctx* ctx, uint32_t* read, uint32_t* gap, uint32_t* left_id, uint32_t* left_start,
                                     uint32_t* left_pos, uint32_t* right_id, uint32_t* right_start, uint32_t* right_pos) {
-  if (!ctx) return GVS_E_ARG;
-  if (!ctx->ge_ready) return gvs_fail(ctx, GVS_E_STATE, "gvs_gap_evidence_get before gvs_gap_evidence");
-  CK(cudaSetDevice(ctx->device));
-  const u64 n = ctx->n_ge, stride = ctx->n_ge_cand;
-  if (n == 0) return 0;
-  uint32_t* dst[8] = {read, gap, left_id, left_start, left_pos, right_id, right_start, right_pos};
-  return columns_to_host(ctx, ctx->ge_rec.as<u32>(), stride, n, dst);
+  return ctx ? rec_get(ctx, ctx->ge, "gvs_gap_evidence_get before gvs_gap_evidence",
+                       {read, gap, left_id, left_start, left_pos, right_id, right_start, right_pos})
+             : GVS_E_ARG;
 }

@@ -201,13 +201,13 @@ extern "C" int gvs_intervals(gvs_ctx* ctx, uint64_t* n_intervals) {
   CK(cudaMemsetAsync(ctx->comp_max.p, 0, ng * 4, ctx->stream));
   const u32* cnt = ctx->comp_cnt.as<u32>();
   u32* ex = ctx->flags_b.as<u32>();
-  u32* tot = (u32*)(ctx->counters.as<u64>() + 26);
+  u32 ni = 0;
   if (!by_rank) {
     LAUNCH(k_comp_stats<false>, (unsigned)cdiv(ng, 256), 256, 0, ctx->parent.as<u32>(), ctx->present.as<u8>(), ng, ctx->grp_start.as<u32>(),
            ctx->comp_cnt.as<u32>(), ctx->comp_min.as<u32>(), ctx->comp_max.as<u32>(), nullptr, nullptr);
     auto f = [cnt] __device__(u64 g) -> u32 { return cnt[g] >= 3 ? 1u : 0u; };
     auto g2 = [ex] __device__(u64 g, u32 e, u32 v) { ex[g] = e; };
-    CKR((device_scan<u32>(ctx, ng, f, g2, OpSum(), tot)));
+    CKR(scan_total(ctx, ng, f, g2, OpSum(), &ni));
   } else {
     CKR(gvs_reserve(ctx, ctx->comp_rank, ng * 2 * 4));
     u32 *rmn = ctx->comp_rank.as<u32>(), *slot = rmn + ng;
@@ -217,10 +217,8 @@ extern "C" int gvs_intervals(gvs_ctx* ctx, uint64_t* n_intervals) {
     LAUNCH(k_iv_slot, (unsigned)cdiv(ng, 256), 256, 0, cnt, rmn, ng, slot);
     auto f = [slot] __device__(u64 q) -> u32 { return slot[q] != 0xFFFFFFFFu ? 1u : 0u; };
     auto g2 = [ex] __device__(u64 q, u32 e, u32 v) { ex[q] = e; };
-    CKR((device_scan<u32>(ctx, ng, f, g2, OpSum(), tot)));
+    CKR(scan_total(ctx, ng, f, g2, OpSum(), &ni));
   }
-  u32 ni = 0;
-  CKR(read_dev(ctx, tot, &ni));
   CKR(gvs_reserve(ctx, ctx->iv_contig, (u64)ni * 4));
   CKR(gvs_reserve(ctx, ctx->iv_start, (u64)ni * 4));
   CKR(gvs_reserve(ctx, ctx->iv_end, (u64)ni * 4));
@@ -287,7 +285,7 @@ extern "C" int gvs_gaps(gvs_ctx* ctx, const uint32_t* contig_len, uint64_t* n_ga
       CKR((device_scan<u64>(ctx, n, f, g, OpMax(), (u64*)nullptr)));
     }
     u32 *gc = ctx->gap_contig.as<u32>(), *gs = ctx->gap_start.as<u32>(), *ge = ctx->gap_end.as<u32>();
-    u32* tot = (u32*)(ctx->counters.as<u64>() + 27);
+    u32 ngap = 0;
     {
       // pyranges merge joins overlapping and book-ended intervals: a new run starts iff start > max end
       auto f = [ivc, ivs, pm] __device__(u64 i) -> u32 {
@@ -301,20 +299,16 @@ extern "C" int gvs_gaps(gvs_ctx* ctx, const uint32_t* contig_len, uint64_t* n_ga
           ge[ex] = ivs[i] - 1;
         }
       };
-      CKR((device_scan<u32>(ctx, n, f, g, OpSum(), tot)));
+      CKR(scan_total(ctx, n, f, g, OpSum(), &ngap));
     }
-    u32 ngap = 0;
-    CKR(read_dev(ctx, tot, &ngap));
     ctx->n_gaps = ngap;
   }
   {
     u32* nd = ctx->nodata_contig.as<u32>();
-    u32* tot = (u32*)(ctx->counters.as<u64>() + 28);
     auto f = [has] __device__(u64 c) -> u32 { return has[c] ? 0u : 1u; };
     auto g = [nd] __device__(u64 c, u32 ex, u32 v) { if (v) nd[ex] = (u32)c; };
-    CKR((device_scan<u32>(ctx, nc, f, g, OpSum(), tot)));
     u32 nn = 0;
-    CKR(read_dev(ctx, tot, &nn));
+    CKR(scan_total(ctx, nc, f, g, OpSum(), &nn));
     ctx->n_nodata = nn;
   }
   ctx->gaps_ready = true;
@@ -455,7 +449,7 @@ extern "C" int gvs_covprob_gaps(gvs_ctx* ctx, const uint32_t* grp_contig, const 
   if (n_gaps == 0) return 0;
   CK(cudaSetDevice(ctx->device));
   DevBuf gc, gi, pc, ps, pe, tb, mg, pr;
-  u32* err = (u32*)(ctx->counters.as<u64>() + 24);
+  u32* err = counter(ctx, CNT_COVPROB_ERR);
   int rc = to_dev(ctx, gc, grp_contig, n_groups);
   if (!rc) rc = to_dev(ctx, gi, grp_id, n_groups);
   if (!rc) rc = to_dev(ctx, pc, gap_contig, n_gaps);

@@ -24,22 +24,18 @@
 #define JN_QUAL 2u  // anchored, on a qualifying contig
 #define JN_SURV 4u  // QUAL, in a run of >= JN_MIN_IDS distinct IDs (a block row)
 
-struct JnRows {
-  const u32 *read, *pos, *contig, *start, *group, *gidx;
-  const u32* seg_start;  // n_seg + 1
-  u32 n_seg;
-  const u8* bad;  // per group index (null: nothing is bad)
-  u8 *fa, *fb;    // per row: flag bits, scratch bit (first of its ID)
+struct JnRows : SegRows {
+  u8 *fa, *fb;  // per row: flag bits, scratch bit (first of its ID)
 };
 
 // ANCH and QUAL bits of the rows [a, b) of one read (one warp; fb is scratch)
 __device__ void jn_qualify(const JnRows& R, u32 a, u32 b, int lane) {
   for (u32 i = a + lane; i < b; i += 32) {
     u8 f = 0;
-    if (!(R.bad && R.bad[R.gidx[i]])) {
+    if (!R.is_bad(i)) {
       const u32 c = R.contig[i], id = R.group[i], p = R.pos[i], s = R.start[i];
       for (u32 j = a; j < b; j++) {
-        if (R.contig[j] != c || R.group[j] == id || (R.bad && R.bad[R.gidx[j]])) continue;
+        if (R.contig[j] != c || R.group[j] == id || R.is_bad(j)) continue;
         if (gvs_ratio_ok(p, s, R.pos[j], R.start[j])) {
           f = JN_ANCH;
           break;
@@ -75,20 +71,15 @@ __device__ void jn_qualify(const JnRows& R, u32 a, u32 b, int lane) {
   __syncwarp();
 }
 
-__device__ __forceinline__ u32 jn_read_len(const u64* read_off, const u32* read_len, u32 rd) {
-  return read_len ? read_len[rd] : (u32)min(read_off[rd + 1] - read_off[rd], (u64)0xFFFFFFFFu);
-}
-
 // per segment of the match rows: the rows it stashes (0 unless >= 2 contigs qualify)
-__global__ void __launch_bounds__(256) k_jn_screen(const JnRows R, const u64* __restrict__ read_off, const u32* __restrict__ read_len,
-                                                   u32 min_len, u32* seg_cnt) {
+__global__ void __launch_bounds__(256) k_jn_screen(const JnRows R, const ReadLens len, u32 min_len, u32* seg_cnt) {
   const u32 s = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (s >= R.n_seg) return;
   const u32 a = R.seg_start[s], b = R.seg_start[s + 1];
   const u32 c0 = R.contig[a];
   bool other = false;
-  if (jn_read_len(read_off, read_len, R.read[a]) >= min_len)
+  if (len(R.read[a]) >= min_len)
     for (u32 j = a + lane; j < b; j += 32) other |= R.contig[j] != c0;
   if (!__any_sync(0xFFFFFFFFu, other)) {  // too short, or every row on one contig
     if (lane == 0) seg_cnt[s] = 0;
@@ -232,18 +223,13 @@ __global__ void __launch_bounds__(256) k_jn_resolve(const JnRows R, const JnScra
   if (lane == 0) seg_cnt[s] = nblk >= 2 ? nblk - 1 : 0u;
 }
 
-static void jn_rows(JnRows& J, const Rows& S) {
-  J.read = S.read.as<u32>(); J.pos = S.pos.as<u32>(); J.contig = S.contig.as<u32>(); J.start = S.start.as<u32>();
-  J.group = S.group.as<u32>(); J.gidx = S.gidx.as<u32>();
-}
-
 extern "C" int gvs_junction_screen(gvs_ctx* ctx, uint32_t min_read_len, uint64_t* stash_rows, uint64_t* stash_reads) {
   if (!ctx) return GVS_E_ARG;
   if (!ctx->match_ready) return gvs_fail(ctx, GVS_E_STATE, "gvs_junction_screen before gvs_match / gvs_rows_set(0)");
   if (!ctx->read_off && !ctx->have_read_len) return gvs_fail(ctx, GVS_E_STATE, "gvs_junction_screen: read lengths unknown");
   CK(cudaSetDevice(ctx->device));
   StageTimer tm(ctx, GVS_ST_SCREEN);
-  ctx->jn_ready = false;
+  ctx->jn.ready = false;
   if (!ctx->jn_in_run) {  // outside a batches run a screen replaces the stash
     ctx->jn_stash.n = 0;
     ctx->jn_reads = 0;
@@ -254,29 +240,23 @@ extern "C" int gvs_junction_screen(gvs_ctx* ctx, uint32_t min_read_len, uint64_t
   const u64 n = M.n;
   if (n) {
     if (base + ctx->n_reads >= 0xFFFFFFF0ull) return gvs_fail(ctx, GVS_E_OVERFLOW, "more than 2^32 reads in one run");
-    JnRows R;
-    jn_rows(R, M);
     u64 n_seg = 0;
-    CKR(gvs_build_segments(ctx, R.read, n, ctx->jn_seg_start, ctx->jn_row_seg, &n_seg));
-    R.seg_start = ctx->jn_seg_start.as<u32>();
-    R.n_seg = (u32)n_seg;
+    CKR(gvs_build_segments(ctx, M.read.as<u32>(), n, ctx->jn_seg_start, ctx->jn_row_seg, &n_seg));
+    JnRows R;
+    (SegRows&)R = seg_rows(ctx, M, ctx->jn_seg_start, n_seg);
     R.bad = nullptr;  // bad groups are not known before the run's histogram
     CKR(gvs_reserve(ctx, ctx->jn_flags, n * 2));
     R.fa = ctx->jn_flags.as<u8>();
     R.fb = R.fa + n;
     CKR(gvs_reserve(ctx, ctx->jn_seg_cnt, n_seg * 8));
     u32 *seg_cnt = ctx->jn_seg_cnt.as<u32>(), *seg_off = seg_cnt + n_seg;
-    LAUNCH(k_jn_screen, (unsigned)cdiv(n_seg * 32, 256), 256, 0, R, ctx->have_read_len ? nullptr : ctx->read_off,
-           ctx->have_read_len ? ctx->read_len.as<u32>() : nullptr, min_read_len, seg_cnt);
-    // (reads << 32) + rows
-    u64* tot = ctx->counters.as<u64>() + 38;
+    LAUNCH(k_jn_screen, (unsigned)cdiv(n_seg * 32, 256), 256, 0, R, read_lens(ctx), min_read_len, seg_cnt);
+    u64 packed = 0;  // (reads << 32) + rows
     {
       auto f = [seg_cnt] __device__(u64 s) -> u64 { return seg_cnt[s] ? (1ull << 32) | seg_cnt[s] : 0ull; };
       auto g = [seg_off] __device__(u64 s, u64 ex, u64 v) { seg_off[s] = (u32)ex; };
-      CKR((device_scan<u64>(ctx, n_seg, f, g, OpSum(), tot)));
+      CKR(scan_total(ctx, n_seg, f, g, OpSum(), &packed));
     }
-    u64 packed = 0;
-    CKR(read_dev(ctx, tot, &packed));
     const u64 add = packed & 0xFFFFFFFFull;
     if (add) {
       if (have + add >= 0xFFFFFFF0ull) return gvs_fail(ctx, GVS_E_OVERFLOW, "more than 2^32 junction rows in one run");
@@ -299,22 +279,19 @@ extern "C" int gvs_junctions(gvs_ctx* ctx, uint64_t* n_records) {
   if (!ctx) return GVS_E_ARG;
   CK(cudaSetDevice(ctx->device));
   StageTimer tm(ctx, GVS_ST_JUNCTIONS);
-  ctx->jn_ready = false;
-  ctx->n_jn = 0;
+  ctx->jn.ready = false;
+  ctx->jn.n = 0;
   if (n_records) *n_records = 0;
   const Rows& S = ctx->jn_stash;
   const u64 n = S.n;
   if (n == 0) {
-    ctx->jn_ready = true;
+    ctx->jn.ready = true;
     return 0;
   }
-  JnRows R;
-  jn_rows(R, S);
   u64 n_seg = 0;
-  CKR(gvs_build_segments(ctx, R.read, n, ctx->jn_seg_start, ctx->jn_row_seg, &n_seg));
-  R.seg_start = ctx->jn_seg_start.as<u32>();
-  R.n_seg = (u32)n_seg;
-  R.bad = ctx->bad_ready ? ctx->bad_flag.as<u8>() : nullptr;
+  CKR(gvs_build_segments(ctx, S.read.as<u32>(), n, ctx->jn_seg_start, ctx->jn_row_seg, &n_seg));
+  JnRows R;
+  (SegRows&)R = seg_rows(ctx, S, ctx->jn_seg_start, n_seg);
   CKR(gvs_reserve(ctx, ctx->jn_flags, n * 2));
   R.fa = ctx->jn_flags.as<u8>();
   R.fb = R.fa + n;
@@ -327,9 +304,9 @@ extern "C" int gvs_junctions(gvs_ctx* ctx, uint64_t* n_records) {
   LAUNCH(k_jn_resolve, (unsigned)cdiv(n_seg * 32, 256), 256, 0, R, X, seg_cnt);
   // a block holds >= 3 rows, so a read has fewer records than rows / 3
   const u64 stride = n / JN_MIN_IDS + 1;
-  CKR(gvs_reserve(ctx, ctx->jn_rec, stride * 13 * 4));
-  u32* rec = ctx->jn_rec.as<u32>();
-  u32* tot = (u32*)(ctx->counters.as<u64>() + 39);
+  CKR(rec_reserve(ctx, ctx->jn, 13, stride));
+  u32* rec = ctx->jn.col(0);
+  u32 nr = 0;
   {
     const JnRows Rc = R;
     const JnScratch Xc = X;
@@ -354,13 +331,10 @@ extern "C" int gvs_junctions(gvs_ctx* ctx, uint64_t* n_records) {
         o[12 * stride] = Rc.pos[j];
       }
     };
-    CKR((device_scan<u32>(ctx, n_seg, f, g, OpSum(), tot)));
+    CKR(scan_total(ctx, n_seg, f, g, OpSum(), &nr));
   }
-  u32 nr = 0;
-  CKR(read_dev(ctx, tot, &nr));
-  ctx->n_jn = nr;
-  ctx->jn_stride = stride;
-  ctx->jn_ready = true;
+  ctx->jn.n = nr;
+  ctx->jn.ready = true;
   if (n_records) *n_records = nr;
   return 0;
 }
@@ -368,11 +342,7 @@ extern "C" int gvs_junctions(gvs_ctx* ctx, uint64_t* n_records) {
 extern "C" int gvs_junctions_get(gvs_ctx* ctx, uint32_t* read, uint32_t* contig1, uint32_t* strand1, uint32_t* ids1, uint32_t* id1,
                                  uint32_t* start1, uint32_t* pos1, uint32_t* contig2, uint32_t* strand2, uint32_t* ids2,
                                  uint32_t* id2, uint32_t* start2, uint32_t* pos2) {
-  if (!ctx) return GVS_E_ARG;
-  if (!ctx->jn_ready) return gvs_fail(ctx, GVS_E_STATE, "gvs_junctions_get before gvs_junctions");
-  CK(cudaSetDevice(ctx->device));
-  const u64 n = ctx->n_jn, stride = ctx->jn_stride;
-  if (n == 0) return 0;
-  uint32_t* dst[13] = {read, contig1, strand1, ids1, id1, start1, pos1, contig2, strand2, ids2, id2, start2, pos2};
-  return columns_to_host(ctx, ctx->jn_rec.as<u32>(), stride, n, dst);
+  return ctx ? rec_get(ctx, ctx->jn, "gvs_junctions_get before gvs_junctions",
+                       {read, contig1, strand1, ids1, id1, start1, pos1, contig2, strand2, ids2, id2, start2, pos2})
+             : GVS_E_ARG;
 }

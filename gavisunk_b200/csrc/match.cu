@@ -149,7 +149,7 @@ __device__ u32 k32_hit(const K32View& v, u64 g, u32* rd, u32* w, u32* gi) {
 
 static int match_k32(gvs_ctx* ctx, u64* n_hits) {
   StageTimer tm(ctx, GVS_ST_PROBE);
-  u64* counters = ctx->counters.as<u64>();
+  u64* counters = counter<u64>(ctx, CNT_HITS);
   CK(cudaMemsetAsync(counters, 0, 4 * sizeof(u64), ctx->stream));
   if (!ctx->seg_packed.empty()) return gvs_fail(ctx, GVS_E_STATE, "k = 32: host batches are not packed on the way");
   K32View v;
@@ -160,7 +160,7 @@ static int match_k32(gvs_ctx* ctx, u64* n_hits) {
   v.total = ctx->total_bases;
   v.tab.kv = ctx->tab_kv.as<u64>();
   v.tab.slots = ctx->tab_slots;
-  v.flags = (u32*)(counters + 1);
+  v.flags = counter(ctx, CNT_FLAGS);
   // the segments of a pipelined host batch must have landed (gvs_probe_launch waits per segment)
   for (size_t s = 0; s < ctx->seg_tile_end.size() && ctx->seq == ctx->own_seq.as<u8>(); s++)
     CK(cudaStreamWaitEvent(ctx->stream, ctx->seg_ev[s], 0));
@@ -170,7 +170,7 @@ static int match_k32(gvs_ctx* ctx, u64* n_hits) {
   };
   auto g0 = [] __device__(u64 i, u64 ex, u64 val) {};
   CKR((device_scan<u64>(ctx, v.total, f, g0, OpSum(), counters)));
-  u64 h[2];
+  u64 h[2];  // hits, flags
   CKR(read_dev(ctx, counters, h, 2));
   if ((u32)h[1] & FLAG_KEYERROR)
     return gvs_fail(ctx, GVS_E_KEYERROR, "KeyError: a read matched a db k-mer that has no .loc row (kmerpos_annot3.nim:90)");
@@ -201,7 +201,7 @@ static int match_k32(gvs_ctx* ctx, u64* n_hits) {
 }
 
 static int match_once(gvs_ctx* ctx, u64* n_warps, u64* cap_w, bool* overflow, u64* total_hits, u64* max_per_warp) {
-  u64* counters = ctx->counters.as<u64>();
+  u64* counters = counter<u64>(ctx, CNT_HITS);
   CK(cudaMemsetAsync(counters, 0, 4 * sizeof(u64), ctx->stream));
   {
     StageTimer tm(ctx, GVS_ST_PROBE);
@@ -215,13 +215,13 @@ static int match_once(gvs_ctx* ctx, u64* n_warps, u64* cap_w, bool* overflow, u6
     auto g = [wd] __device__(u64 i, u64 ex, u64 v) { wd[i] = ex; };
     CKR((device_scan<u64>(ctx, *n_warps, f, g, OpSum(), counters)));
     auto g2 = [] __device__(u64 i, u64 ex, u64 v) {};
-    CKR((device_scan<u64>(ctx, *n_warps, f, g2, OpMax(), counters + 3)));
+    CKR((device_scan<u64>(ctx, *n_warps, f, g2, OpMax(), counter<u64>(ctx, CNT_HIT_MAX))));
   }
-  u64 h[4];
+  u64 h[4];  // CNT_HITS .. CNT_HIT_MAX
   CKR(read_dev(ctx, counters, h, 4));
-  *total_hits = h[0];
-  *max_per_warp = h[3];
-  u32 fl = (u32)h[1];
+  *total_hits = h[CNT_HITS];
+  *max_per_warp = h[CNT_HIT_MAX];
+  u32 fl = (u32)h[CNT_FLAGS];
   if (fl & FLAG_KEYERROR)
     return gvs_fail(ctx, GVS_E_KEYERROR, "KeyError: a read matched a db k-mer that has no .loc row (kmerpos_annot3.nim:90)");
   *overflow = (fl & FLAG_OVERFLOW) != 0;
@@ -297,7 +297,7 @@ extern "C" int gvs_match(gvs_ctx* ctx, uint64_t* n_rows_out) {
   const u8* nf = ctx->ohit_nf.as<u8>();
   LAUNCH(k_emit_flags, (unsigned)cdiv(nh, 256), 256, 0, ctx->ohit_read.as<u32>(), ctx->ohit_gidx.as<u32>(), nh,
          ctx->chunk_first.as<u64>(), ctx->n_chunks, fl);
-  u64* tot = ctx->counters.as<u64>() + 2;
+  u64* tot = counter<u64>(ctx, CNT_EMIT);
   {
     // high word: rows emitted; low word: suppressed hits = the record's followers (+ the record's own
     // first hit when it continues the previous record's group)

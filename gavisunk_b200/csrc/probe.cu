@@ -725,13 +725,12 @@ static probe_fn probe_table(int k, bool packed, bool small) {
 }
 
 // launches the probe over ctx's reads; span s's hits land at s * cap_w in ctx->hit_*, its count in
-// ctx->tile_cnt[s] (zeroed here); counters[1] = flags
+// ctx->tile_cnt[s] (zeroed here); flags to the CNT_FLAGS counter
 int gvs_probe_launch(gvs_ctx* ctx, u64* n_warps_out, u64* cap_w_out) {
   u64 total = ctx->total_bases;
   u64 n_tiles = cdiv(total, PW_TILE);
   probe_fn fn = probe_table(ctx->k, ctx->seq_packed, !ctx->filt_fp);  // the variant follows the block layout (table.cu)
   if (!fn) return gvs_fail(ctx, GVS_E_ARG, "no probe kernel for k=%d", ctx->k);
-  u64* counters = ctx->counters.as<u64>();
   Probe2Params P;
   P.seq = ctx->seq;
   P.total = total;
@@ -782,7 +781,7 @@ int gvs_probe_launch(gvs_ctx* ctx, u64* n_warps_out, u64* cap_w_out) {
   P.hit_gidx = ctx->hit_gidx.as<u32>();
   P.hit_nf = ctx->hit_nf.as<u8>();
   P.hit_cap = ctx->hit_cap;
-  P.flags = (u32*)(counters + 1);
+  P.flags = counter(ctx, CNT_FLAGS);
   P.warp_cnt = ctx->tile_cnt.as<u32>();
   // L2 persistence: the structure every window group touches (the presence filter) is pinned in the
   // persisting carve-out of L2; everything outside the window (reads, exact table, hit lists) is

@@ -113,7 +113,7 @@ extern "C" int gvs_rows_set(gvs_ctx* ctx, int which, const uint32_t* read_idx, c
   }
   if (ctx->db_ready) {
     CKR(ensure_group_table(ctx));
-    u32* miss = (u32*)(ctx->counters.as<u64>() + 15);
+    u32* miss = counter(ctx, CNT_MISS);
     CK(cudaMemsetAsync(miss, 0, 4, ctx->stream));
     if (n)
       LAUNCH(k_gt_lookup, (unsigned)cdiv(n, 256), 256, 0, R.contig.as<u32>(), R.group.as<u32>(), n, ctx->gt_keys.as<u64>(),

@@ -57,7 +57,7 @@ int gvs_check_group_order(gvs_ctx* ctx) {
   const u64 ng = ctx->n_groups;
   u32 h = 0;
   if (ng > 1) {
-    u32* err = (u32*)(ctx->counters.as<u64>() + 32);
+    u32* err = counter(ctx, CNT_ORDER_ERR);
     CK(cudaMemsetAsync(err, 0, 4, ctx->stream));
     LAUNCH(k_groups_sorted, (unsigned)cdiv(ng, 256), 256, 0, ctx->grp_contig.as<u32>(), ctx->grp_start.as<u32>(), ng, err);
     CKR(read_dev(ctx, err, &h));
@@ -126,8 +126,8 @@ extern "C" int gvs_placements(gvs_ctx* ctx, uint64_t* n, int32_t** diff_dev) {
   if (!ctx->groups_ready) return gvs_fail(ctx, GVS_E_STATE, "gvs_placements: no group index");
   CK(cudaSetDevice(ctx->device));
   StageTimer tm(ctx, GVS_ST_SUPPORT);
-  ctx->pl_ready = ctx->sup_ready = false;
-  ctx->n_pl = 0;
+  ctx->pl.ready = ctx->sup.ready = false;
+  ctx->pl.n = 0;
   if (n) *n = 0;
   CKR(gvs_ensure_rank(ctx));
   const u64 ng = ctx->n_groups;
@@ -135,9 +135,7 @@ extern "C" int gvs_placements(gvs_ctx* ctx, uint64_t* n, int32_t** diff_dev) {
   CK(cudaMemsetAsync(ctx->sup_diff.p, 0, (ng ? ng : 1) * 4, ctx->stream));
   const u64 n_seg = ctx->n_kseg;
   if (ctx->n_pairs) {
-    // gvs_validate's scratch: out_id[n], out_gidx[n], seg_cnt[n_seg], seg_off[n_seg]
-    const u32* seg_cnt = ctx->val_scratch.as<u32>() + 2 * ctx->kept.n;
-    const u32* seg_off = seg_cnt + n_seg;
+    const u32 *seg_cnt = ctx->val_seg_cnt, *seg_off = ctx->val_seg_off;
     CKR(gvs_reserve(ctx, ctx->pl_tmp, n_seg * 16));
     PlaceParams P;
     P.seg_cnt = seg_cnt; P.seg_off = seg_off;
@@ -148,17 +146,11 @@ extern "C" int gvs_placements(gvs_ctx* ctx, uint64_t* n, int32_t** diff_dev) {
     P.diff = ctx->sup_diff.as<i32>();
     P.tmp = ctx->pl_tmp.as<uint4>();
     LAUNCH(k_place, (unsigned)cdiv(n_seg * 32, 256), 256, 0, P);
-    u32* tot = (u32*)(ctx->counters.as<u64>() + 33);
-    CKR(gvs_reserve(ctx, ctx->pl_read, n_seg * 4));
-    CKR(gvs_reserve(ctx, ctx->pl_contig, n_seg * 4));
-    CKR(gvs_reserve(ctx, ctx->pl_start, n_seg * 4));
-    CKR(gvs_reserve(ctx, ctx->pl_end, n_seg * 4));
-    CKR(gvs_reserve(ctx, ctx->pl_nids, n_seg * 4));
+    CKR(rec_reserve(ctx, ctx->pl, 5, n_seg));
     CKR(gvs_reserve(ctx, ctx->pl_strand, n_seg));
     const u32 *prd = ctx->pair_read.as<u32>(), *pct = ctx->pair_contig.as<u32>();
     const uint4* tmp = ctx->pl_tmp.as<uint4>();
-    u32 *o_read = ctx->pl_read.as<u32>(), *o_contig = ctx->pl_contig.as<u32>(), *o_start = ctx->pl_start.as<u32>();
-    u32 *o_end = ctx->pl_end.as<u32>(), *o_nids = ctx->pl_nids.as<u32>();
+    u32 *o_read = ctx->pl.col(0), *o_contig = ctx->pl.col(1), *o_start = ctx->pl.col(2), *o_end = ctx->pl.col(3), *o_nids = ctx->pl.col(4);
     u8* o_strand = ctx->pl_strand.as<u8>();
     auto f = [seg_cnt] __device__(u64 s) -> u32 { return seg_cnt[s] >= 2 ? 1u : 0u; };
     auto g = [=] __device__(u64 s, u32 ex, u32 v) {
@@ -172,13 +164,12 @@ extern "C" int gvs_placements(gvs_ctx* ctx, uint64_t* n, int32_t** diff_dev) {
       o_nids[ex] = t.z;
       o_strand[ex] = (u8)t.w;
     };
-    CKR((device_scan<u32>(ctx, n_seg, f, g, OpSum(), tot)));
     u32 np = 0;
-    CKR(read_dev(ctx, tot, &np));
-    ctx->n_pl = np;
+    CKR(scan_total(ctx, n_seg, f, g, OpSum(), &np));
+    ctx->pl.n = np;
   }
-  ctx->pl_ready = true;
-  if (n) *n = ctx->n_pl;
+  ctx->pl.ready = true;
+  if (n) *n = ctx->pl.n;
   if (diff_dev) *diff_dev = ctx->sup_diff.as<i32>();
   return 0;
 }
@@ -186,18 +177,11 @@ extern "C" int gvs_placements(gvs_ctx* ctx, uint64_t* n, int32_t** diff_dev) {
 extern "C" int gvs_placements_get(gvs_ctx* ctx, uint32_t* read_idx, uint32_t* contig, uint32_t* start, uint32_t* end, uint32_t* n_ids,
                                   uint8_t* strand) {
   if (!ctx) return GVS_E_ARG;
-  if (!ctx->pl_ready) return gvs_fail(ctx, GVS_E_STATE, "gvs_placements_get before gvs_placements");
-  CK(cudaSetDevice(ctx->device));
-  const u64 n = ctx->n_pl;
-  if (n == 0) return 0;
-  if (read_idx) CK(cudaMemcpyAsync(read_idx, ctx->pl_read.p, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  if (contig) CK(cudaMemcpyAsync(contig, ctx->pl_contig.p, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  if (start) CK(cudaMemcpyAsync(start, ctx->pl_start.p, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  if (end) CK(cudaMemcpyAsync(end, ctx->pl_end.p, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  if (n_ids) CK(cudaMemcpyAsync(n_ids, ctx->pl_nids.p, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  if (strand) CK(cudaMemcpyAsync(strand, ctx->pl_strand.p, n, cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaStreamSynchronize(ctx->stream));
-  return 0;
+  if (ctx->pl.ready && ctx->pl.n && strand) {  // (u8: queued before the u32 columns, whose getter waits for both)
+    CK(cudaSetDevice(ctx->device));
+    CK(cudaMemcpyAsync(strand, ctx->pl_strand.p, ctx->pl.n, cudaMemcpyDeviceToHost, ctx->stream));
+  }
+  return rec_get(ctx, ctx->pl, "gvs_placements_get before gvs_placements", {read_idx, contig, start, end, n_ids});
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -254,10 +238,11 @@ __global__ void __launch_bounds__(256) k_runs_end(const u32* __restrict__ rc, co
   re[i] = (i + 1 < n && rc[i + 1] == rc[i]) ? rs[i + 1] : clen[rc[i]];
 }
 
-int gvs_rank_runs(gvs_ctx* ctx, const i32* diff, u32 nv, const uint32_t* contig_len, RankRuns& out, u64* n_runs, const char* who) {
+int gvs_rank_runs(gvs_ctx* ctx, const i32* diff, u32 nv, const uint32_t* contig_len, RecTable& out, const char* who) {
+  out.ready = false;
+  out.n = 0;
   const u32 nc = ctx->n_contigs;
   if (nc && !contig_len) return gvs_fail(ctx, GVS_E_ARG, "%s: null contig_len", who);
-  *n_runs = 0;
   const u64 ng = ctx->n_groups;
   CKR(to_dev(ctx, ctx->contig_len, contig_len, nc));
   CKR(gvs_reserve(ctx, ctx->sup_depth, (ng ? ng : 1) * 4 * nv));
@@ -273,7 +258,7 @@ int gvs_rank_runs(gvs_ctx* ctx, const i32* diff, u32 nv, const uint32_t* contig_
   V.val = ctx->sup_depth.as<i32>();
   V.nv = nv;
   V.ng = ng;
-  u32* err = (u32*)(ctx->counters.as<u64>() + 35);
+  u32* err = counter(ctx, CNT_RUNS_ERR);
   CK(cudaMemsetAsync(err, 0, 4, ctx->stream));
   if (ng) {
     for (u32 t = 0; t < nv; t++) {
@@ -296,57 +281,37 @@ int gvs_rank_runs(gvs_ctx* ctx, const i32* diff, u32 nv, const uint32_t* contig_
     };
     CKR((device_scan<u32>(ctx, ng, f, g, OpSum(), (u32*)nullptr)));
   }
-  u32* tot = (u32*)(ctx->counters.as<u64>() + 34);
+  u32 nr = 0;
   {
     auto f = [cst, nc] __device__(u64 c) -> u32 { return (cst[2 * nc + c] != 0 ? 1u : 0u) + cst[nc + c] - cst[c]; };
     auto g = [cst, nc] __device__(u64 c, u32 ex, u32 v) { cst[3 * nc + c] = ex; };
-    CKR((device_scan<u32>(ctx, nc, f, g, OpSum(), tot)));
+    CKR(scan_total(ctx, nc, f, g, OpSum(), &nr));
   }
-  u32 nr = 0;
-  CKR(read_dev(ctx, tot, &nr));
-  CKR(gvs_reserve(ctx, *out.contig, (u64)nr * 4));
-  CKR(gvs_reserve(ctx, *out.start, (u64)nr * 4));
-  CKR(gvs_reserve(ctx, *out.end, (u64)nr * 4));
-  CKR(gvs_reserve(ctx, *out.val, (u64)nr * 4 * nv));
+  CKR(rec_reserve(ctx, out, 3 + nv, nr));
   const u32* clen = ctx->contig_len.as<u32>();
-  u32 *rc = out.contig->as<u32>(), *rs = out.start->as<u32>(), *rv = out.val->as<u32>();
+  u32 *rc = out.col(0), *rs = out.col(1), *rv = out.col(3);
   if (ng) LAUNCH(k_runs_groups, (unsigned)cdiv(ng, 256), 256, 0, V, ctx->sup_gx.as<u32>(), cst, nc, clen, rc, rs, rv, (u64)nr, err);
   if (nc) LAUNCH(k_runs_heads, (unsigned)cdiv(nc, 256), 256, 0, cst, nc, rc, rs, rv, nv, (u64)nr);
-  if (nr) LAUNCH(k_runs_end, (unsigned)cdiv(nr, 256), 256, 0, rc, rs, nr, clen, out.end->as<u32>());
+  if (nr) LAUNCH(k_runs_end, (unsigned)cdiv(nr, 256), 256, 0, rc, rs, nr, clen, out.col(2));
   u32 h = 0;
   CKR(read_dev(ctx, err, &h));
   if (h) return gvs_fail(ctx, GVS_E_ARG, "%s: a SUNK group starts at or beyond its contig's length", who);
-  *n_runs = nr;
+  out.n = nr;
+  out.ready = true;
   return 0;
 }
 
 extern "C" int gvs_support(gvs_ctx* ctx, const uint32_t* contig_len, uint64_t* n_runs) {
   if (!ctx) return GVS_E_ARG;
-  if (!ctx->pl_ready) return gvs_fail(ctx, GVS_E_STATE, "gvs_support before gvs_placements");
+  if (!ctx->pl.ready) return gvs_fail(ctx, GVS_E_STATE, "gvs_support before gvs_placements");
   CK(cudaSetDevice(ctx->device));
   StageTimer tm(ctx, GVS_ST_SUPPORT);
-  ctx->sup_ready = false;
-  ctx->n_runs = 0;
   if (n_runs) *n_runs = 0;
-  RankRuns out{&ctx->run_contig, &ctx->run_start, &ctx->run_end, &ctx->run_depth};
-  u64 nr = 0;
-  CKR(gvs_rank_runs(ctx, ctx->sup_diff.as<i32>(), 1, contig_len, out, &nr, "gvs_support"));
-  ctx->n_runs = nr;
-  ctx->sup_ready = true;
-  if (n_runs) *n_runs = nr;
+  CKR(gvs_rank_runs(ctx, ctx->sup_diff.as<i32>(), 1, contig_len, ctx->sup, "gvs_support"));
+  if (n_runs) *n_runs = ctx->sup.n;
   return 0;
 }
 
 extern "C" int gvs_support_get(gvs_ctx* ctx, uint32_t* contig, uint32_t* start, uint32_t* end, uint32_t* depth) {
-  if (!ctx) return GVS_E_ARG;
-  if (!ctx->sup_ready) return gvs_fail(ctx, GVS_E_STATE, "gvs_support_get before gvs_support");
-  CK(cudaSetDevice(ctx->device));
-  const u64 n = ctx->n_runs;
-  if (n == 0) return 0;
-  if (contig) CK(cudaMemcpyAsync(contig, ctx->run_contig.p, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  if (start) CK(cudaMemcpyAsync(start, ctx->run_start.p, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  if (end) CK(cudaMemcpyAsync(end, ctx->run_end.p, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  if (depth) CK(cudaMemcpyAsync(depth, ctx->run_depth.p, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaStreamSynchronize(ctx->stream));
-  return 0;
+  return ctx ? rec_get(ctx, ctx->sup, "gvs_support_get before gvs_support", {contig, start, end, depth}) : GVS_E_ARG;
 }

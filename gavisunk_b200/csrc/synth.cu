@@ -283,16 +283,14 @@ int gvs_synth_plan_scans(gvs_ctx* ctx, DevBuf& segcount, u64 n_reads, u64* read_
   SynthState& S = g_synth;
   const u32* sc = segcount.as<u32>();
   u64* sf = S.seg_first.as<u64>();
-  u64* tot = ctx->counters.as<u64>() + 6;
+  u64 n_segs = 0;
   {
     auto f = [sc] __device__(u64 i) -> u64 { return (u64)sc[i]; };
     auto g = [sf] __device__(u64 i, u64 ex, u64 v) { sf[i] = ex; };
-    CKR((device_scan<u64>(ctx, n_reads, f, g, OpSum(), tot)));
+    CKR(scan_total(ctx, n_reads, f, g, OpSum(), &n_segs));
   }
-  u64 n_segs = 0;
-  CKR(read_dev(ctx, tot, &n_segs));
   S.n_segs = n_segs;
-  CK(cudaMemcpyAsync(sf + n_reads, tot, 8, cudaMemcpyDeviceToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(sf + n_reads, counter<u64>(ctx, CNT_SCAN), 8, cudaMemcpyDeviceToDevice, ctx->stream));
   CKR(gvs_reserve(ctx, S.seg_out, n_segs * 4));
   CKR(gvs_reserve(ctx, S.seg_off, (n_segs + 1) * 8));
   if (n_segs)
@@ -300,14 +298,12 @@ int gvs_synth_plan_scans(gvs_ctx* ctx, DevBuf& segcount, u64 n_reads, u64* read_
            S.seg_out.as<u32>());
   const u32* so = S.seg_out.as<u32>();
   u64* sof = S.seg_off.as<u64>();
-  u64* tot2 = ctx->counters.as<u64>() + 7;
+  u64 total = 0;
   {
     auto f = [so] __device__(u64 i) -> u64 { return (u64)so[i]; };
     auto g = [sof] __device__(u64 i, u64 ex, u64 v) { sof[i] = ex; };
-    CKR((device_scan<u64>(ctx, n_segs, f, g, OpSum(), tot2)));
+    CKR(scan_total(ctx, n_segs, f, g, OpSum(), &total));
   }
-  u64 total = 0;
-  CKR(read_dev(ctx, tot2, &total));
   LAUNCH(k_read_offsets, (unsigned)cdiv(n_reads + 1, 256), 256, 0, sf, sof, n_reads, n_segs, total, read_off_dev);
   if (total_bases) *total_bases = total;
   return 0;

@@ -188,12 +188,10 @@ static int build_group_index_body(gvs_ctx* ctx, const u32* contig, const u32* gr
   LAUNCH(k_grp_rep, grid_for(ctx, n, 256), 256, 0, contig, group, n, gk.as<u64>(), gm.as<u32>(), slots, rep.as<u32>());
   const u32* repp = rep.as<u32>();
   u32* densep = dense.as<u32>();
-  u32* total = (u32*)ctx->counters.as<u64>();
   auto f = [repp] __device__(u64 i) -> u32 { return repp[i] == (u32)i ? 1u : 0u; };
   auto g = [densep] __device__(u64 i, u32 ex, u32 v) { densep[i] = ex; };
-  CKR((device_scan<u32>(ctx, n, f, g, OpSum(), total)));
   u32 ng = 0;
-  CKR(read_dev(ctx, total, &ng));
+  CKR(scan_total(ctx, n, f, g, OpSum(), &ng));
   ctx->n_groups = ng;
   CKR(gvs_reserve(ctx, ctx->grp_contig, (u64)ng * sizeof(u32)));
   CKR(gvs_reserve(ctx, ctx->grp_start, (u64)ng * sizeof(u32)));

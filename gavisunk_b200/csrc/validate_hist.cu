@@ -118,7 +118,7 @@ extern "C" int gvs_hist_mode(gvs_ctx* ctx, int64_t mode[2]) {
   u64 ng = ctx->n_groups;
   mode[0] = mode[1] = 0;
   if (ng == 0) return 0;
-  u32* mx = (u32*)(ctx->counters.as<u64>() + 16);
+  u32* mx = counter(ctx, CNT_HIST_MAX);
   CK(cudaMemsetAsync(mx, 0, 4, ctx->stream));
   u64 grid = cdiv(ng, 256);
   if (grid > (u64)ctx->n_sm * 8) grid = (u64)ctx->n_sm * 8;
@@ -131,7 +131,7 @@ extern "C" int gvs_hist_mode(gvs_ctx* ctx, int64_t mode[2]) {
   CK(cudaMemsetAsync(ctx->cnt_hist.p, 0, 2ull * (M + 1) * 4 + 16, ctx->stream));
   LAUNCH(k_cnt_hist, (unsigned)(cdiv(ng, 256) < (u64)ctx->n_sm * 4 ? cdiv(ng, 256) : (u64)ctx->n_sm * 4), 256, 0, ctx->hist.as<i32>(), ctx->grp_contig.as<u32>(), ctx->contig_hap.as<u8>(), ng,
          M, ctx->cnt_hist.as<u32>());
-  i64* dm = (i64*)(ctx->counters.as<u64>() + 18);
+  i64* dm = counter<i64>(ctx, CNT_MODE);
   LAUNCH(k_mode, 2, 1024, 0, ctx->cnt_hist.as<u32>(), M, dm);
   i64 hm[2];
   CKR(read_dev(ctx, dm, hm, 2));
@@ -154,12 +154,10 @@ extern "C" int gvs_bad_groups(gvs_ctx* ctx, const int64_t limit_floor[2], uint64
            limit_floor[0], limit_floor[1], ctx->bad_flag.as<u8>());
     const u8* bf = ctx->bad_flag.as<u8>();
     u32* bl = ctx->bad_list.as<u32>();
-    u32* tot = (u32*)(ctx->counters.as<u64>() + 20);
     auto f = [bf] __device__(u64 g) -> u32 { return bf[g]; };
     auto g2 = [bl] __device__(u64 g, u32 ex, u32 v) { if (v) bl[ex] = (u32)g; };
-    CKR((device_scan<u32>(ctx, ng, f, g2, OpSum(), tot)));
     u32 nb = 0;
-    CKR(read_dev(ctx, tot, &nb));
+    CKR(scan_total(ctx, ng, f, g2, OpSum(), &nb));
     ctx->n_bad = nb;
   }
   ctx->bad_ready = true;
@@ -213,12 +211,10 @@ extern "C" int gvs_bad_set(gvs_ctx* ctx, const uint32_t* contig, const uint32_t*
       ctx->launches++;
       const u8* bf = ctx->bad_flag.as<u8>();
       u32* bl = ctx->bad_list.as<u32>();
-      u32* tot = (u32*)(ctx->counters.as<u64>() + 20);
       auto f = [bf] __device__(u64 g) -> u32 { return bf[g]; };
       auto g2 = [bl] __device__(u64 g, u32 ex, u32 v) { if (v) bl[ex] = (u32)g; };
-      rc = device_scan<u32>(ctx, ng, f, g2, OpSum(), tot);
       u32 nb = 0;
-      if (!rc) rc = read_dev(ctx, tot, &nb);
+      rc = scan_total(ctx, ng, f, g2, OpSum(), &nb);
       ctx->n_bad = nb;
     }
     cudaStreamSynchronize(ctx->stream);

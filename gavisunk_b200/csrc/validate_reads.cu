@@ -50,13 +50,8 @@ __device__ __forceinline__ bool pair_ok(u32 pi, u32 si, u32 pj, u32 sj) {
   return 9 * ds < 10 * dp && 10 * dp < 11 * ds;
 }
 
-struct ValParams {
-  const u32 *read, *pos, *start, *group, *gidx;  // kept rows
-  const u32* seg_start;
-  u32 n_seg;
-  const u8* bad;             // per group index (null: nothing is bad)
-  const u64* read_off;       // read lengths from offsets ...
-  const u32* read_len;       // ... or explicit
+struct ValParams : SegRows {  // kept rows
+  ReadLens len;
   u32 min_len;
   u32* out_id;               // per kept row slot: validated IDs of the read, from its first row on
   u32* out_gidx;
@@ -96,7 +91,7 @@ __global__ void __launch_bounds__(NT* GROUPS) k_validate(const ValParams V) {
     gsync();
     // read length filter (hard-coded 10000 in the reference, :106-108; Q13)
     const u32 rd = V.read[a];
-    const u32 rlen = V.read_len ? V.read_len[rd] : (u32)(V.read_off[rd + 1] - V.read_off[rd]);
+    const u32 rlen = V.len(rd);
     const bool skip = rlen < V.min_len || mrows < 2;
     // ---- rows minus bad groups (:70-72), input order preserved (a read's rows come in increasing pos) ----
     if (!skip) {
@@ -563,8 +558,8 @@ extern "C" int gvs_validate(gvs_ctx* ctx, uint32_t min_read_len, uint64_t* n_pai
   CK(cudaSetDevice(ctx->device));
   StageTimer tm(ctx, GVS_ST_VALIDATE);
   ctx->val_ready = false;
-  ctx->pl_ready = ctx->sup_ready = false;
-  ctx->dc_ready = ctx->dc_runs_ready = false;
+  ctx->pl.ready = ctx->sup.ready = false;
+  ctx->dc.ready = ctx->dc_runs.ready = false;
   ctx->n_pairs = 0;
   if (n_pairs_out) *n_pairs_out = 0;
   Rows& R = ctx->kept;
@@ -583,24 +578,20 @@ extern "C" int gvs_validate(gvs_ctx* ctx, uint32_t min_read_len, uint64_t* n_pai
   u32* out_gidx = out_id + n;
   u32* seg_cnt = out_gidx + n;
   u32* seg_off = seg_cnt + n_seg;
+  ctx->val_id = out_id; ctx->val_seg_cnt = seg_cnt; ctx->val_seg_off = seg_off;
   CKR(gvs_reserve(ctx, ctx->seg_orient, n_seg));
   // largest read (rows) decides which launches are needed
-  u32* mx_dev = (u32*)(ctx->counters.as<u64>() + 22);
+  u32 max_m = 0;
   {
     auto f2 = [seg_start] __device__(u64 s) -> u32 { return seg_start[s + 1] - seg_start[s]; };
     auto g2 = [] __device__(u64 s, u32 ex, u32 v) {};
-    CKR((device_scan<u32>(ctx, n_seg, f2, g2, OpMax(), mx_dev)));
+    CKR(scan_total(ctx, n_seg, f2, g2, OpMax(), &max_m));
   }
-  u32 max_m = 0;
-  CKR(read_dev(ctx, mx_dev, &max_m));
-  u32* stats = (u32*)(ctx->counters.as<u64>() + 23);
+  u32* stats = counter(ctx, CNT_VAL_STATS);
   CK(cudaMemsetAsync(stats, 0, 8, ctx->stream));
   ValParams V;
-  V.read = R.read.as<u32>(); V.pos = R.pos.as<u32>(); V.start = R.start.as<u32>(); V.group = R.group.as<u32>();
-  V.gidx = R.gidx.as<u32>();
-  V.seg_start = seg_start; V.n_seg = (u32)n_seg;
-  V.bad = ctx->bad_ready ? ctx->bad_flag.as<u8>() : nullptr;
-  V.read_off = ctx->read_off; V.read_len = ctx->have_read_len ? ctx->read_len.as<u32>() : nullptr;
+  (SegRows&)V = seg_rows(ctx, R, ctx->kseg_start, n_seg);
+  V.len = read_lens(ctx);
   V.min_len = min_read_len;
   V.out_id = out_id; V.out_gidx = out_gidx; V.seg_cnt = seg_cnt; V.orient = ctx->seg_orient.as<u8>();
   V.gscratch = nullptr; V.big_cap = 0; V.stats = stats;
@@ -640,14 +631,12 @@ extern "C" int gvs_validate(gvs_ctx* ctx, uint32_t min_read_len, uint64_t* n_pai
   }
   if (tiers) CKR(gvs_join(ctx));
   // compaction of the validated (ID, read) pairs
-  u32* tot = (u32*)(ctx->counters.as<u64>() + 25);
+  u32 np = 0;
   {
     auto f = [seg_cnt] __device__(u64 s) -> u32 { return seg_cnt[s]; };
     auto g = [seg_off] __device__(u64 s, u32 ex, u32 v) { seg_off[s] = ex; };
-    CKR((device_scan<u32>(ctx, n_seg, f, g, OpSum(), tot)));
+    CKR(scan_total(ctx, n_seg, f, g, OpSum(), &np));
   }
-  u32 np = 0;
-  CKR(read_dev(ctx, tot, &np));
   CKR(gvs_reserve(ctx, ctx->pair_read, (u64)np * 4));
   CKR(gvs_reserve(ctx, ctx->pair_contig, (u64)np * 4));
   CKR(gvs_reserve(ctx, ctx->pair_group, (u64)np * 4));
