@@ -43,6 +43,9 @@ PROTOTYPES = {
     "gvs_match": (C.c_int, [vp, u64p]),
     "gvs_rows_get": (C.c_int, [vp, C.c_int, vp, vp, vp, vp, vp]),
     "gvs_diag_filter": (C.c_int, [vp, vp, vp, u64p, u64p]),
+    "gvs_diag_filter_haps": (C.c_int, [vp, vp, vp, C.c_int, u64p, u64p]),
+    "gvs_read_haps": (C.c_int, [vp, u64p]),
+    "gvs_read_haps_get": (C.c_int, [vp] * 9),
     "gvs_best_get": (C.c_int, [vp, vp, vp, vp, vp]),
     "gvs_filter_best": (C.c_int, [vp, vp, u64p]),
     "gvs_contigs_set": (C.c_int, [vp, vp, vp, C.c_uint32]),
@@ -116,7 +119,7 @@ PROTOTYPES["gvs_format_rows"] = (C.c_int64, [C.POINTER(ColStruct), C.c_uint32, C
 GVS_E_KEYERROR = -3
 STAGES = {"probe": 0, "emit": 1, "diag": 2, "hist": 3, "validate": 4, "intervals": 5, "dbbuild": 6, "components": 7, "mode": 8,
           "bad": 9, "merge": 10, "support": 11, "evidence": 12, "screen": 13,
-          "junctions": 14, "discordance": 15}
+          "junctions": 14, "discordance": 15, "readhaps": 16}
 
 _lib = None
 

@@ -12,9 +12,9 @@
   python -m gavisunk_b200.cli split_locs --ont-pos P --kmer-loc L --flag results/S/breaks/hapN_splits_pos.done --hap hapN
   python -m gavisunk_b200.cli split_ont --reads R.. --out temp/S/reads/hapN_1-of-10.fq.gz ..   (seqtk seq -F '#' | rustybam fastq-split)
   python -m gavisunk_b200.cli combine_ont_nofilt <chunk.sunkpos>.. <hapN_detailed.sunkpos>
-  python -m gavisunk_b200.cli fused --sample S --k K --hap1-asm .. --hap2-asm .. --hap1-reads f.. --hap2-reads f.. --outdir D
-                                    [--devices 0,1,..] [--batch-files N] [--detailed] [--support-tracks] [--gap-evidence]
-                                    [--junctions] [--discordance]
+  python -m gavisunk_b200.cli fused --sample S --k K --hap1-asm .. --hap2-asm .. (--hap1-reads f.. --hap2-reads f.. | --reads f..)
+                                    --outdir D [--devices 0,1,..] [--batch-files N] [--detailed] [--support-tracks]
+                                    [--gap-evidence] [--junctions] [--discordance] [--read-haplotypes]
   python -m gavisunk_b200.cli support_tracks <sunkpos> <rlen> <bad_sunks.txt> <fai> <valid.bed> <out.reads.bed> <out.bedgraph> <out.tsv>
   python -m gavisunk_b200.cli gap_evidence <sunkpos> <rlen> <bad_sunks.txt> <fai> <valid.bed> <out.gaps.reads.tsv> <out.gaps.evidence.tsv>
   python -m gavisunk_b200.cli junctions <hapN_detailed.sunkpos> <hapN.rlen> <bad_sunks.txt> <fai1> <fai2> <out.junctions.reads.tsv> <out.junctions.tsv>
@@ -34,6 +34,9 @@ reads that reach both of its sides and the size change their SUNK distances impl
 contig links and breakpoints (no reference counterpart: the diag filter keeps one contig per read).
 `fused --discordance` and `discordance` report collapses and expansions inside validated intervals, from the SUNK spacing
 of the validated reads across them (no reference counterpart).
+`fused --read-haplotypes` reports each read's SUNK vote on both haplotypes and the haplotype it assigns; `fused --reads`
+takes unbinned chunk files and keeps each read's rows on the haplotype its votes assign (no reference counterpart: the
+reference needs the reads binned by haplotype).
 Text parsing / formatting is host
 plumbing; all per-base and per-row work runs in libgavisunk_b200.so.  Errors exit non-zero with a
 message on stderr and never leave a partial output file behind.
@@ -49,7 +52,7 @@ from typing import Dict, List, NamedTuple, Sequence, Tuple
 import numpy as np
 
 from . import io as gio
-from .engine import Engine, encode_kmers
+from .engine import GVS_HAP_ANY, Engine, encode_kmers
 from .parallel import ThreadExchange, shard_chunks
 
 
@@ -651,6 +654,68 @@ def cmd_discordance(argv):
     discordance(*argv)
 
 
+# ------------------------------------------------------------------------------------------------
+# read haplotypes: every read's SUNK vote on both haplotypes (no reference counterpart; DESIGN.md section 5.5e)
+# ------------------------------------------------------------------------------------------------
+READ_HAP_READS_HEADER = "read\tread_len\tbin\tcontig1\tn1\tstrand1\tcontig2\tn2\tstrand2\thap\n"
+_BIN = gio.NameTable(["hap1", "hap2", "unbinned"])
+_ASSIGNED = gio.NameTable(["hap1", "hap2", "tie"])
+_STRAND_OR_NONE = gio.NameTable(["+", "-", "."])
+_NO_VOTE = 0xFFFFFFFF
+
+
+def file_haps(read_bin, rh) -> np.ndarray:
+    """File haplotype (0 / 1) of every run-wide read: its chunk's haplotype (read_bin 0 / 1); for an unbinned read
+    (GVS_HAP_ANY) the one its votes assign (rh = Engine.read_haps() with run-wide read indices), and for a tie or a read
+    without a vote the parity of its index (even: hap1), so that each haplotype's read-length library gets half of the
+    reads SUNKs cannot place."""
+    read_bin = np.asarray(read_bin, np.uint8)
+    fh = read_bin.copy()
+    un = np.flatnonzero(read_bin == GVS_HAP_ANY)
+    fh[un] = (un & 1).astype(np.uint8)
+    if len(rh["read"]):
+        a = (rh["hap"] <= 1) & (read_bin[rh["read"]] == GVS_HAP_ANY)
+        fh[rh["read"][a]] = rh["hap"][a].astype(np.uint8)
+    return fh
+
+
+def read_hap_texts(hap, names, contig_hap, rh, read_bin, read_hap, rtab, read_len, name_rank):
+    """The two read-haplotype files of haplotype `hap`: rh = Engine.read_haps() with run-wide read indices; read_bin /
+    read_hap = chunk haplotype (0, 1, GVS_HAP_ANY) and file haplotype (file_haps) of every run-wide read; rtab / read_len /
+    name_rank = name table, length and bytewise name rank of every run-wide read.  -> (haplotype.reads.tsv: one row per
+    record of a read of file haplotype `hap`, in name order; haplotype.tsv: per contig of `hap` the reads whose vote on
+    `hap` lands on it, by assignment, and a totals row that also counts the reads of file haplotype `hap` without a vote
+    and their bases) bytes"""
+    hn, on = hap + 1, 2 - hap
+    ctab = gio.NameTable(list(names) + ["."])
+    sel = np.flatnonzero(read_hap[rh["read"]] == hap) if len(rh["read"]) else np.zeros(0, np.int64)
+    r = sel[np.lexsort((sel, name_rank[rh["read"][sel]]))]
+    cols = [("name", rh["read"], rtab), ("u32", read_len[rh["read"]]), ("name", read_bin[rh["read"]].astype(np.uint32), _BIN)]
+    for side in "12":
+        c = rh["contig" + side]
+        none = c == _NO_VOTE
+        cols += [("name", np.where(none, len(names), c).astype(np.uint32), ctab), ("u32", rh["n" + side]),
+                 ("name", np.where(none, 2, rh["strand" + side]).astype(np.uint32), _STRAND_OR_NONE)]
+    cols.append(("name", rh["hap"], _ASSIGNED))
+    reads_tsv = READ_HAP_READS_HEADER.encode() + gio.format_rows(cols, sel=r)
+    c = rh[f"contig{hn}"]
+    v = np.flatnonzero(c != _NO_VOTE)
+    nc = len(names)
+    count = lambda m: np.bincount(c[v][m], minlength=nc).astype(np.int64)
+    a = rh["hap"][v]
+    same, other, tie = count(a == hap), count(a == 1 - hap), count(a == 2)
+    out = [f"contig\treads\tassigned_hap{hn}\tassigned_hap{on}\ttie\tno_vote_reads\tno_vote_bases\n"]
+    for ci in np.flatnonzero(np.asarray(contig_hap) == hap).tolist():
+        out.append(f"{names[ci]}\t{same[ci] + other[ci] + tie[ci]}\t{same[ci]}\t{other[ci]}\t{tie[ci]}\t.\t.\n")
+    voted = np.zeros(len(read_hap), bool)
+    voted[rh["read"]] = True
+    nv = np.flatnonzero(~voted & (read_hap == hap))
+    hc = np.asarray(contig_hap) == hap
+    out.append(f"total\t{(same + other + tie)[hc].sum()}\t{same[hc].sum()}\t{other[hc].sum()}\t{tie[hc].sum()}\t{len(nv)}\t"
+               f"{int(read_len[nv].astype(np.int64).sum())}\n")
+    return reads_tsv, "".join(out).encode("latin-1")
+
+
 def cmd_get_gaps(argv):
     """get_gaps.py: paths are string-concatenated, so indir / outdir need their trailing slash (:30,70)"""
     fai1, fai2, sample, indir, outdir = argv
@@ -909,6 +974,9 @@ EVIDENCE_PRODUCTS = {
     "discordance": Evidence("--discordance", "also write final_out/hap{N}.discordance.reads.tsv, .discordance.tsv and "
                             ".discordance.bed (collapses and expansions inside validated intervals)", "spans", Engine.SPAN_COLUMNS,
                             ("discordance.reads.tsv", "discordance.tsv", "discordance.bed")),
+    "read_haplotypes": Evidence("--read-haplotypes", "also write final_out/hap{N}.haplotype.reads.tsv and .haplotype.tsv (each "
+                                "read's SUNK vote on both haplotypes; implied by --reads)", "read_haps", Engine.READ_HAP_COLUMNS,
+                                ("haplotype.reads.tsv", "haplotype.tsv")),
 }
 
 
@@ -960,8 +1028,10 @@ def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int]
     merged across engines) and the gap-evidence records of its own reads; junctions: the junction records of every
     engine's own reads (each batch screened after its diag filter, resolved with the run's bad groups); discordance: the
     discordant spans of every engine's own reads and the discordance runs, with the difference arrays summed like the
-    support's.  -> one result dict per engine (read names / lengths / chunk tables, kept rows, validated pairs,
-    intervals[, placements, support runs][, gap evidence][, junctions][, spans, discordance runs])."""
+    support's; read_haplotypes: every engine's diag filters in haplotype mode and the records of its own reads (file_hap
+    GVS_HAP_ANY: unbinned chunks, always filtered in haplotype mode).  -> one result dict per engine (read names /
+    lengths / chunk tables, kept rows, validated pairs, intervals[, placements, support runs][, gap evidence][,
+    junctions][, spans, discordance runs][, read haplotypes])."""
     import threading
     from concurrent.futures import ThreadPoolExecutor
     for p in files:
@@ -1016,7 +1086,7 @@ def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int]
                         info["rows0"].append(r0)
                 iv, bases = eng.run_batches([bind_for(bi) for bi in range(len(mine))], contig_hap, min_read_len=min_read_len,
                                             allreduce_hist=cx.allreduce_hist, gather_forests=cx.gather_forests, on_batch=on_batch,
-                                            junctions="junctions" in products)
+                                            junctions="junctions" in products, read_haps="read_haplotypes" in products)
                 for old in held:
                     old.close()
             info.update(kept=eng.rows(1, pinned=True), pairs=eng.pairs(pinned=True), iv=iv)
@@ -1029,6 +1099,8 @@ def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int]
                 info.update(junctions=eng.junctions())
             if "discordance" in products:
                 info.update(spans=eng.spans(), discordance=eng.discordance(contig_len, allreduce=cx.allreduce_hist))
+            if "read_haplotypes" in products:
+                info.update(read_haps=eng.read_haps() if mine else {c: np.zeros(0, np.uint32) for c in Engine.READ_HAP_COLUMNS})
             results[di] = info
         except BaseException as ex:  # noqa: BLE001 -- reported by the caller; peers must not wait for this rank
             errors.append(ex)
@@ -1050,11 +1122,12 @@ def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int]
 
 def run_fused(k: int, hap_asm: Sequence[str], hap_reads: Sequence[Sequence[str]], outdir: str, device: int = 0,
               devices: Sequence[int] = None, batch_files: int = 0, batch_gbp: float = 12.0, detailed: bool = False,
-              threads: int = 0, mrsfast_palindromes: bool = False, products: Sequence[str] = ()):
-    """hap_asm: two FASTA paths; hap_reads: two lists of chunk files in scatter order.  Builds the SUNK database on
-    every GPU of `devices`, runs the reads (run_reads) and writes every file of the rules between jellyfish_count and
-    slop_gaps under `outdir`, and the files of the EVIDENCE_PRODUCTS named in `products`.  Returns the first device's
-    engine."""
+              threads: int = 0, mrsfast_palindromes: bool = False, products: Sequence[str] = (), reads: Sequence[str] = ()):
+    """hap_asm: two FASTA paths; hap_reads: two lists of chunk files in scatter order, or None and `reads`: chunk files of
+    unbinned reads, whose haplotypes their SUNK votes assign (implies the read_haplotypes product).  Builds the SUNK
+    database on every GPU of `devices`, runs the reads (run_reads) and writes every file of the rules between
+    jellyfish_count and slop_gaps under `outdir`, and the files of the EVIDENCE_PRODUCTS named in `products`.  Returns the
+    first device's engine."""
     from concurrent.futures import ThreadPoolExecutor
     devices = list(devices) if devices else [device]
     contigs, contig_hap, fai = [], [], [[], []]
@@ -1063,8 +1136,14 @@ def run_fused(k: int, hap_asm: Sequence[str], hap_reads: Sequence[Sequence[str]]
             contigs.append((n, s))
             contig_hap.append(hap)
             fai[hap].append((n, len(s)))
-    files = list(hap_reads[0]) + list(hap_reads[1])
-    file_hap = [0] * len(hap_reads[0]) + [1] * len(hap_reads[1])
+    if (hap_reads is None) == (not reads):
+        raise ValueError("give either the two haplotypes' chunk files or unbinned chunk files")
+    if reads:
+        files, file_hap = list(reads), [GVS_HAP_ANY] * len(reads)
+        products = list(products) + ["read_haplotypes"] * ("read_haplotypes" not in products)
+    else:
+        files = list(hap_reads[0]) + list(hap_reads[1])
+        file_hap = [0] * len(hap_reads[0]) + [1] * len(hap_reads[1])
     for p in files:
         if not os.path.exists(p):
             raise FileNotFoundError(p)
@@ -1114,9 +1193,9 @@ def write_outputs(k, eng, results, contig_len, contig_hap, names, iv, gaps, noda
     lens = np.concatenate([l for r in results for l in r["lens"]] + [np.zeros(0, np.uint32)])
     chunk_first = np.concatenate([cf[:-1] + read_base[i] for i, r in enumerate(results) for cf in r["chunk_first"]] + [np.array([nreads])])
     chunk_hap = np.concatenate([ch for r in results for ch in r["chunk_hap"]] + [np.zeros(0, np.uint8)])
-    read_hap = np.zeros(nreads, np.uint8)
+    read_bin = np.zeros(nreads, np.uint8)
     for c in range(len(chunk_hap)):
-        read_hap[int(chunk_first[c]):int(chunk_first[c + 1])] = chunk_hap[c]
+        read_bin[int(chunk_first[c]):int(chunk_first[c + 1])] = chunk_hap[c]
 
     def cat_rows(key, cols):
         out = {}
@@ -1128,6 +1207,14 @@ def write_outputs(k, eng, results, contig_len, contig_hap, names, iv, gaps, noda
                     parts.append(t[c] + np.uint32(read_base[i]) if (c == "read" and read_base[i]) else t[c])
             out[c] = parts[0] if len(parts) == 1 else (np.concatenate(parts) if parts else np.zeros(0, np.uint32))
         return out
+    # the file haplotype of every read: its chunk's, or for unbinned reads the one its votes assign (file_haps)
+    if "read_haplotypes" in products:
+        rh = cat_rows("read_haps", Engine.READ_HAP_COLUMNS)
+        read_hap = file_haps(read_bin, rh)
+    elif (read_bin == GVS_HAP_ANY).any():
+        raise ValueError("unbinned reads need the read_haplotypes product")
+    else:
+        read_hap = read_bin
     kept = cat_rows("kept", Engine.ROW_COLUMNS)
     pairs = cat_rows("pairs", Engine.PAIR_COLUMNS)
     sunk_cols = lambda t: [("name", t["read"], rtab), ("u32", t["pos"]), ("name", t["contig"], ctab), ("u32", t["start"]), ("u32", t["group"])]
@@ -1226,7 +1313,8 @@ def write_outputs(k, eng, results, contig_len, contig_hap, names, iv, gaps, noda
             support_tracks=lambda r: support_texts(hap_contigs, clen, names, r, results[0]["support"], iv, *reads),
             gap_evidence=lambda r: gap_evidence_texts(gsel, gaps, names, r, *reads),
             junctions=lambda r: junction_texts(r, np.flatnonzero(read_hap[r["read"]] == hap), names, clen, contig_hap, *reads),
-            discordance=lambda r: discordance_texts(hap_contigs, names, r, results[0]["discordance"], *reads))
+            discordance=lambda r: discordance_texts(hap_contigs, names, r, results[0]["discordance"], *reads),
+            read_haplotypes=lambda r: read_hap_texts(hap, names, chap, r, read_bin, read_hap, *reads))
         for p in products:
             _write_all([d("final_out", f"hap{hn}.{ext}") for ext in EVIDENCE_PRODUCTS[p].suffixes], texts[p](rec[p]))
     from concurrent.futures import ThreadPoolExecutor
@@ -1244,8 +1332,10 @@ def cmd_fused(argv):
     ap.add_argument("--k", type=int, default=20)
     ap.add_argument("--hap1-asm", required=True)
     ap.add_argument("--hap2-asm", required=True)
-    ap.add_argument("--hap1-reads", nargs="+", required=True)
-    ap.add_argument("--hap2-reads", nargs="+", required=True)
+    ap.add_argument("--hap1-reads", nargs="+")
+    ap.add_argument("--hap2-reads", nargs="+")
+    ap.add_argument("--reads", nargs="+", help="chunk files of unbinned reads, instead of --hap1-reads / --hap2-reads: each read's "
+                    "haplotype is assigned from its SUNK votes (implies --read-haplotypes)")
     ap.add_argument("--outdir", required=True)
     ap.add_argument("--device", type=int, default=0)
     ap.add_argument("--devices", default=None, help="comma-separated GPU indices: the chunk files are sharded over them")
@@ -1258,10 +1348,14 @@ def cmd_fused(argv):
     for p, e in EVIDENCE_PRODUCTS.items():
         ap.add_argument(e.flag, dest=p, action="store_true", help=e.help)
     a = ap.parse_args(argv)
+    binned = a.hap1_reads is not None or a.hap2_reads is not None
+    if (a.reads is not None) == binned or (binned and (a.hap1_reads is None or a.hap2_reads is None)):
+        ap.error("give either --reads or both --hap1-reads and --hap2-reads")
     devs = [int(x) for x in a.devices.split(",")] if a.devices else [a.device]
-    run_fused(a.k, [a.hap1_asm, a.hap2_asm], [a.hap1_reads, a.hap2_reads], a.outdir, devices=devs, batch_files=a.batch_files,
-              batch_gbp=a.batch_gbp, detailed=a.detailed, threads=a.threads, mrsfast_palindromes=a.mrsfast_palindromes,
-              products=[p for p in EVIDENCE_PRODUCTS if getattr(a, p)])
+    run_fused(a.k, [a.hap1_asm, a.hap2_asm], [a.hap1_reads, a.hap2_reads] if binned else None, a.outdir, devices=devs,
+              batch_files=a.batch_files, batch_gbp=a.batch_gbp, detailed=a.detailed, threads=a.threads,
+              mrsfast_palindromes=a.mrsfast_palindromes, products=[p for p in EVIDENCE_PRODUCTS if getattr(a, p)],
+              reads=a.reads or ())
 
 
 COMMANDS = {"kmerpos_annot3": (cmd_kmerpos_annot3, 4), "rlen": (cmd_rlen, 2), "diag_filter_v3": (cmd_diag_filter_v3, 2),

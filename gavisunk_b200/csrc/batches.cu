@@ -50,6 +50,31 @@ __global__ void __launch_bounds__(256) k_stash_len(u64 n, const ReadLens len, u3
   dst[i] = len((u32)i);
 }
 
+// the batch's read-haplotype records (8 columns, read first) appended to the run's at `have`, read indices made run-wide
+__global__ void __launch_bounds__(256) k_stash_recs(u64 n, u32 base, const u32* __restrict__ src, u64 src_stride, u32* dst,
+                                                    u64 dst_stride, u64 have) {
+  u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  dst[have + i] = src[i] + base;
+#pragma unroll
+  for (u32 c = 1; c < 8; c++) dst[c * dst_stride + have + i] = src[c * src_stride + i];
+}
+
+// grow the run's record table to hold `need` records, keeping the `have` it holds (columns move to the new stride)
+static int grow_recs(gvs_ctx* ctx, RecTable& t, u64 need, u64 have) {
+  if (t.stride >= need) return 0;
+  const u64 stride = need + need / 2 + 64;
+  DevBuf nb;
+  CKR(gvs_reserve(ctx, nb, stride * 8 * 4));
+  for (u32 c = 0; c < 8 && have; c++)
+    CK(cudaMemcpyAsync(nb.as<u32>() + c * stride, t.col(c), have * 4, cudaMemcpyDeviceToDevice, ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  gvs_release(t.buf);
+  t.buf = nb;
+  t.stride = stride;
+  return 0;
+}
+
 extern "C" int gvs_batches_begin(gvs_ctx* ctx) {
   if (!ctx) return GVS_E_ARG;
   CK(cudaSetDevice(ctx->device));
@@ -62,6 +87,8 @@ extern "C" int gvs_batches_begin(gvs_ctx* ctx) {
   ctx->jn_stash.n = 0;  // the junction screens of the run append from here (junctions.cu)
   ctx->jn_reads = 0;
   ctx->jn_in_run = true;
+  ctx->rh_run.n = 0;
+  ctx->rh_run.ready = false;
   return 0;
 }
 
@@ -84,6 +111,13 @@ extern "C" int gvs_batch_stash(gvs_ctx* ctx, uint64_t* read_base) {
            S.contig.as<u32>() + have, S.start.as<u32>() + have, S.group.as<u32>() + have, S.gidx.as<u32>() + have);
   if (nr)
     LAUNCH(k_stash_len, (unsigned)cdiv(nr, 256), 256, 0, nr, read_lens(ctx), ctx->stash_len.as<u32>() + base);
+  if (ctx->rh.ready) {  // the batch's diag filter ran in haplotype mode
+    RecTable &R = ctx->rh_run, &B = ctx->rh;
+    CKR(grow_recs(ctx, R, R.n + B.n + 1, R.n));
+    if (B.n) LAUNCH(k_stash_recs, (unsigned)cdiv(B.n, 256), 256, 0, B.n, (u32)base, B.col(0), B.stride, R.col(0), R.stride, R.n);
+    R.n += B.n;
+    R.ready = true;
+  }
   S.n = have + n;
   ctx->stash_reads = base + nr;
   if (read_base) *read_base = base;
@@ -98,6 +132,9 @@ extern "C" int gvs_batches_bind(gvs_ctx* ctx, uint64_t* n_rows, uint64_t* n_read
   // swap places, so that the next run stashes into this run's (already sized) memory
   std::swap(ctx->kept, ctx->stash);
   std::swap(ctx->read_len, ctx->stash_len);
+  std::swap(ctx->rh, ctx->rh_run);  // the run's read-haplotype records (ready when a batch ran in haplotype mode)
+  ctx->rh_run.n = 0;
+  ctx->rh_run.ready = false;
   if (ctx->kept.read.cap == 0) CKR(gvs_reserve_rows(ctx, ctx->kept, 1));
   if (ctx->read_len.cap == 0) CKR(gvs_reserve(ctx, ctx->read_len, 16));
   ctx->stash.n = 0;

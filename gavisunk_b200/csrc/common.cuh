@@ -149,6 +149,10 @@ struct gvs_ctx {
   Rows stash;
   DevBuf stash_len;
   u64 stash_reads = 0;
+  // haplotype mode of the diag filter (diag.cu): per segment the best contig of both haplotypes, and the records
+  DevBuf rh_scratch;
+  RecTable rh;       // records of the last diag filter in haplotype mode; after gvs_batches_bind those of the run
+  RecTable rh_run;   // records of the run's batches so far (run-wide read indices), appended by gvs_batch_stash
 
   // ---- histogram / bad groups ----
   DevBuf hist, cnt_hist, bad_flag, bad_list;

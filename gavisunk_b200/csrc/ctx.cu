@@ -179,7 +179,8 @@ extern "C" void gvs_destroy(gvs_ctx* c) {
                    &c->seg_orient, &c->rank_of, &c->rank_grp, &c->sup_diff, &c->pl_strand, &c->pl_tmp,
                    &c->sup_depth, &c->sup_gx, &c->sup_cstat, &c->ge_seg_start, &c->ge_cgap, &c->ge_seg, &c->ge_cand, &c->ge_res,
                    &c->jn_seg_start, &c->jn_row_seg, &c->jn_seg_cnt, &c->jn_flags, &c->jn_scr, &c->dc_diff, &c->dc_scr, &c->dc_seg,
-                   &c->pl.buf, &c->sup.buf, &c->ge.buf, &c->jn.buf, &c->dc.buf, &c->dc_runs.buf};
+                   &c->pl.buf, &c->sup.buf, &c->ge.buf, &c->jn.buf, &c->dc.buf, &c->dc_runs.buf, &c->rh_scratch, &c->rh.buf,
+                   &c->rh_run.buf};
   for (DevBuf* b : all) gvs_release(*b);
   release_rows(c->rows);
   release_rows(c->kept);
@@ -417,8 +418,10 @@ static int reads_set_impl(gvs_ctx* ctx, const uint8_t* seq, bool packed, const u
   ctx->match_ready = ctx->diag_ready = ctx->val_ready = false;
   ctx->have_read_len = false;  // lengths come from this batch's offsets, not from an earlier gvs_reads_meta / gvs_batches_bind
   if (chunk_first[0] != 0 || chunk_first[n_chunks] != n_reads) return gvs_fail(ctx, GVS_E_ARG, "chunk_first must span [0, n_reads]");
-  for (u32 c = 0; c < n_chunks; c++)
+  for (u32 c = 0; c < n_chunks; c++) {
     if (chunk_first[c] > chunk_first[c + 1]) return gvs_fail(ctx, GVS_E_ARG, "chunk_first not monotone");
+    if (chunk_hap[c] > GVS_HAP_ANY) return gvs_fail(ctx, GVS_E_ARG, "chunk haplotype %u (0, 1 or GVS_HAP_ANY)", chunk_hap[c]);
+  }
   ctx->h_chunk_first.assign(chunk_first, chunk_first + n_chunks + 1);
   ctx->h_chunk_hap.assign(chunk_hap, chunk_hap + n_chunks);
   ctx->n_chunks = n_chunks;

@@ -14,6 +14,9 @@
 //   k_seg_tie     ... and resolved by replaying Nim's Table[string, _] slot order (murmur3 & mask,
 //                 linear probing, growth at count*3 > cap*2, capacity sticky within a chunk)
 //   k_keep_rows   rows on the best contig survive (all of them, Q11)
+// Haplotype mode (gvs_diag_filter_haps): candidates on the contigs of both haplotypes, k_seg_best_haps keeps the best
+// of each, k_seg_tie<true> replays the ties per (read, haplotype), k_seg_pick keeps the chunk's or the assigned
+// haplotype's choice, and the records of the reads with a vote on either are written by one scan.
 #include "common.cuh"
 
 #define NOBEST 0xFFFFFFFFu
@@ -443,16 +446,21 @@ __global__ void __launch_bounds__(256) k_seg_best(u32 n_seg, const u32* __restri
   seg_tie[s] = (ok && ties > 1) ? 1 : 0;
 }
 
-// replay Nim's Table for the reads whose optimum is shared by several contigs
+// replay Nim's Table for the reads whose optimum is shared by several contigs.  HAPS: a tie entry is 2 * segment +
+// haplotype, only that haplotype's candidates compete, and best / dir are written per entry
+template <bool HAPS>
 __global__ void __launch_bounds__(64) k_seg_tie(const u32* __restrict__ tie_seg, u32 n_tie, const u32* __restrict__ seg_start,
                                                 const u32* __restrict__ seg_cap, const u32* __restrict__ cidx_excl,
                                                 const u32* __restrict__ cand_row, const u32* __restrict__ row_cnt,
                                                 const u32* __restrict__ contig, const u32* __restrict__ contig_hash,
                                                 const u32* __restrict__ cand_good, const u8* __restrict__ cand_dir,
-                                                u32* scratch, u32 maxcap, u32* seg_best, u8* seg_dir) {
+                                                const u8* __restrict__ contig_hap, u32* scratch, u32 maxcap, u32* seg_best,
+                                                u8* seg_dir) {
   u32 t = blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= n_tie) return;
-  u32 s = tie_seg[t];
+  const u32 e = tie_seg[t];
+  const u32 s = HAPS ? e >> 1 : e;
+  auto mine = [&](u32 ci) { return !HAPS || contig_hap[contig[cand_row[ci]]] == (e & 1); };
   u32 a = seg_start[s], b = seg_start[s + 1];
   u32* A = scratch + (u64)t * 2 * maxcap;
   u32* B = A + maxcap;
@@ -465,11 +473,11 @@ __global__ void __launch_bounds__(64) k_seg_tie(const u32* __restrict__ tie_seg,
       u32 ncap = cap * 2;
       for (u32 i = 0; i < ncap; i++) B[i] = NOBEST;
       for (u32 i = 0; i < cap; i++) {
-        u32 e = A[i];
-        if (e == NOBEST) continue;
-        u32 h = contig_hash[e] & (ncap - 1);
+        u32 x = A[i];
+        if (x == NOBEST) continue;
+        u32 h = contig_hash[x] & (ncap - 1);
         while (B[h] != NOBEST) h = (h + 1) & (ncap - 1);
-        B[h] = e;
+        B[h] = x;
       }
       u32* tmp = A; A = B; B = tmp;
       cap = ncap;
@@ -483,20 +491,73 @@ __global__ void __launch_bounds__(64) k_seg_tie(const u32* __restrict__ tie_seg,
   u32 c0 = cidx_excl[a], c1 = cidx_excl[b];
   u32 maxgood = 0, maxhit = 0;
   for (u32 ci = c0; ci < c1; ci++) {
+    if (!mine(ci)) continue;
     u32 g = cand_good[ci], h = row_cnt[cand_row[ci]];
     if (g > maxgood || (g == maxgood && h < maxhit)) { maxgood = g; maxhit = h; }
   }
   for (u32 i = 0; i < cap; i++) {  // `for k,v in posStarts.pairs()`: slot order
-    u32 e = A[i];
-    if (e == NOBEST) continue;
+    u32 x = A[i];
+    if (x == NOBEST) continue;
     for (u32 ci = c0; ci < c1; ci++) {
-      if (contig[cand_row[ci]] == e && cand_good[ci] == maxgood && row_cnt[cand_row[ci]] == maxhit) {
-        seg_best[s] = e;
-        seg_dir[s] = cand_dir[ci];
+      if (contig[cand_row[ci]] == x && cand_good[ci] == maxgood && row_cnt[cand_row[ci]] == maxhit && mine(ci)) {
+        seg_best[e] = x;
+        seg_dir[e] = cand_dir[ci];
         return;
       }
     }
   }
+}
+
+// haplotype mode: k_seg_best with one accumulator per haplotype, results at 2 * segment + haplotype
+__global__ void __launch_bounds__(256) k_seg_best_haps(u32 n_seg, const u32* __restrict__ seg_start,
+                                                       const u32* __restrict__ cidx_excl, const u32* __restrict__ cand_row,
+                                                       const u32* __restrict__ row_cnt, const u32* __restrict__ contig,
+                                                       const u8* __restrict__ contig_hap, const u32* __restrict__ cand_good,
+                                                       const u8* __restrict__ cand_dir, u32* hap_best, u32* hap_good,
+                                                       u8* hap_dir, u8* hap_tie) {
+  u32 s = blockIdx.x * blockDim.x + threadIdx.x;
+  if (s >= n_seg) return;
+  struct Acc {
+    u32 maxgood = 0, maxhit = 0, best = NOBEST, ties = 0;
+    u8 dir = 0;
+  } acc[2];
+  auto upd = [](Acc& a, u32 g, u32 h, u32 c, u8 d) {
+    if (g > a.maxgood || (g == a.maxgood && g > 0 && h < a.maxhit)) {
+      a.maxgood = g; a.maxhit = h; a.best = c; a.dir = d; a.ties = 1;
+    } else if (g == a.maxgood && g > 0 && h == a.maxhit) {
+      a.ties++;
+    }
+  };
+  u32 c0 = cidx_excl[seg_start[s]], c1 = cidx_excl[seg_start[s + 1]];
+  for (u32 ci = c0; ci < c1; ci++) {
+    const u32 c = contig[cand_row[ci]], g = cand_good[ci], h = row_cnt[cand_row[ci]];
+    if (contig_hap[c]) upd(acc[1], g, h, c, cand_dir[ci]);
+    else upd(acc[0], g, h, c, cand_dir[ci]);
+  }
+#pragma unroll
+  for (int k = 0; k < 2; k++) {
+    const bool ok = acc[k].maxgood > 1;
+    hap_best[2 * s + k] = ok ? acc[k].best : NOBEST;
+    hap_good[2 * s + k] = ok ? acc[k].maxgood : 0;
+    hap_dir[2 * s + k] = acc[k].dir;
+    hap_tie[2 * s + k] = (ok && acc[k].ties > 1) ? 1 : 0;
+  }
+}
+
+// assignment of a read from its two votes (n = 0 without a vote): 0 / 1, 2 = tie, 3 = none
+__device__ __forceinline__ u32 hap_assign(u32 n0, u32 n1) { return n0 > n1 ? 0u : n1 > n0 ? 1u : n0 ? 2u : 3u; }
+
+// the kept haplotype's choice becomes the segment's: the chunk's haplotype, or the assigned one of an unbinned read
+__global__ void __launch_bounds__(256) k_seg_pick(u32 n_seg, const u8* __restrict__ seg_hap, const u32* __restrict__ hap_best,
+                                                  const u32* __restrict__ hap_good, const u8* __restrict__ hap_dir,
+                                                  u32* seg_best, u32* seg_good, u8* seg_dir) {
+  u32 s = blockIdx.x * blockDim.x + threadIdx.x;
+  if (s >= n_seg) return;
+  const u32 sh = seg_hap[s];
+  const u32 k = sh < GVS_HAP_ANY ? sh : hap_assign(hap_good[2 * s], hap_good[2 * s + 1]);
+  seg_best[s] = k < 2 ? hap_best[2 * s + k] : NOBEST;
+  seg_good[s] = k < 2 ? hap_good[2 * s + k] : 0;
+  seg_dir[s] = k < 2 ? hap_dir[2 * s + k] : 0;
 }
 
 __global__ void __launch_bounds__(256) k_keep_rows(u64 n, const u32* __restrict__ keep_excl, const u32* __restrict__ row_seg,
@@ -540,12 +601,14 @@ struct DiagScratch {
   u8 *seg_hap, *seg_dir, *seg_tie, *cand_dir;
 };
 
-static int diag_impl(gvs_ctx* ctx, u64* n_best_out, u64* n_kept_out) {
+static int diag_impl(gvs_ctx* ctx, bool haps, u64* n_best_out, u64* n_kept_out) {
   Rows& R = ctx->rows;
   u64 n = R.n;
   ctx->kept.n = 0;
   ctx->n_best = 0;
   ctx->n_seg = 0;
+  ctx->rh.n = 0;
+  ctx->rh.ready = haps;
   if (n == 0) return 0;
   StageTimer tm(ctx, GVS_ST_DIAG);
   const u32 *read = R.read.as<u32>(), *pos = R.pos.as<u32>(), *contig = R.contig.as<u32>(), *start = R.start.as<u32>(),
@@ -592,10 +655,6 @@ static int diag_impl(gvs_ctx* ctx, u64* n_best_out, u64* n_kept_out) {
     const u32* rc = D.row_cnt;
     const u8* sh = D.seg_hap;
     u32 *cidx = D.cidx, *crow = D.cand_row, *cvoff = D.cand_voff;
-    auto f = [rc, contig, contig_hap, sh, row_seg] __device__(u64 j) -> u64 {
-      u32 c = rc[j];
-      return (c >= 2 && contig_hap[contig[j]] == sh[row_seg[j]]) ? ((1ull << 32) | c) : 0ull;
-    };
     auto g = [cidx, crow, cvoff] __device__(u64 j, u64 ex, u64 v) {
       cidx[j] = (u32)(ex >> 32);
       if (v) {
@@ -603,7 +662,19 @@ static int diag_impl(gvs_ctx* ctx, u64* n_best_out, u64* n_kept_out) {
         cvoff[ex >> 32] = (u32)ex;
       }
     };
-    CKR(scan_total(ctx, n, f, g, OpSum(), &packed));
+    if (haps) {  // the contigs of either haplotype
+      auto f = [rc, contig, contig_hap] __device__(u64 j) -> u64 {
+        u32 c = rc[j];
+        return (c >= 2 && contig_hap[contig[j]] <= 1) ? ((1ull << 32) | c) : 0ull;
+      };
+      CKR(scan_total(ctx, n, f, g, OpSum(), &packed));
+    } else {
+      auto f = [rc, contig, contig_hap, sh, row_seg] __device__(u64 j) -> u64 {
+        u32 c = rc[j];
+        return (c >= 2 && contig_hap[contig[j]] == sh[row_seg[j]]) ? ((1ull << 32) | c) : 0ull;
+      };
+      CKR(scan_total(ctx, n, f, g, OpSum(), &packed));
+    }
   }
   u32 n_cand = (u32)(packed >> 32);
   CK(cudaMemcpyAsync(D.cidx + n, &n_cand, 4, cudaMemcpyHostToDevice, ctx->stream));
@@ -618,16 +689,31 @@ static int diag_impl(gvs_ctx* ctx, u64* n_best_out, u64* n_kept_out) {
     LAUNCH(k_cand_vote<1024>, (unsigned)ctx->n_sm * 2, 1024, 0, D.cand_row, D.cand_voff, big_list, n_big, D.row_cnt, D.v_pos,
            D.v_start, D.v_group, D.cand_good, D.cand_dir);
   }
-  LAUNCH(k_seg_best, (unsigned)cdiv(n_seg, 256), 256, 0, (u32)n_seg, seg_start, D.cidx, D.cand_row, D.row_cnt, contig,
-         D.cand_good, D.cand_dir, D.seg_best, D.seg_good, D.seg_dir, D.seg_tie);
+  // haplotype mode: per segment and haplotype best, good, dir, tie at 2 * s + h, and the tie list over those entries
+  u32 *hap_best = nullptr, *hap_good = nullptr, *hap_tie_seg = nullptr;
+  u8 *hap_dir = nullptr, *hap_tie = nullptr;
+  if (haps) {
+    CKR(gvs_reserve(ctx, ctx->rh_scratch, (n_seg + 1) * 2 * (4 * 3 + 2)));
+    hap_best = ctx->rh_scratch.as<u32>();
+    hap_good = hap_best + 2 * n_seg;
+    hap_tie_seg = hap_good + 2 * n_seg;
+    hap_dir = (u8*)(hap_tie_seg + 2 * n_seg);
+    hap_tie = hap_dir + 2 * n_seg;
+    StageTimer th(ctx, GVS_ST_READHAPS);
+    LAUNCH(k_seg_best_haps, (unsigned)cdiv(n_seg, 256), 256, 0, (u32)n_seg, seg_start, D.cidx, D.cand_row, D.row_cnt, contig,
+           contig_hap, D.cand_good, D.cand_dir, hap_best, hap_good, hap_dir, hap_tie);
+  } else {
+    LAUNCH(k_seg_best, (unsigned)cdiv(n_seg, 256), 256, 0, (u32)n_seg, seg_start, D.cidx, D.cand_row, D.row_cnt, contig,
+           D.cand_good, D.cand_dir, D.seg_best, D.seg_good, D.seg_dir, D.seg_tie);
+  }
   // ---- ties: Table capacity at the start of each read (sticky within a chunk) ----
   u32 n_tie = 0;
   {
-    const u8* st = D.seg_tie;
-    u32* ts = D.tie_seg;
+    const u8* st = haps ? hap_tie : D.seg_tie;
+    u32* ts = haps ? hap_tie_seg : D.tie_seg;
     auto f = [st] __device__(u64 s) -> u32 { return st[s]; };
     auto g = [ts] __device__(u64 s, u32 ex, u32 v) { if (v) ts[ex] = (u32)s; };
-    CKR(scan_total(ctx, n_seg, f, g, OpSum(), &n_tie));
+    CKR(scan_total(ctx, haps ? 2 * n_seg : n_seg, f, g, OpSum(), &n_tie));
   }
   if (n_tie) {
     const u32 *sc = D.seg_chunk, *nd = D.seg_ndist;
@@ -651,8 +737,43 @@ static int diag_impl(gvs_ctx* ctx, u64* n_best_out, u64* n_kept_out) {
     }
     DevBuf& sb = ctx->scan_tmp2;
     CKR(gvs_reserve(ctx, sb, (u64)n_tie * 2 * maxcap * 4));
-    LAUNCH(k_seg_tie, (unsigned)cdiv(n_tie, 64), 64, 0, D.tie_seg, n_tie, seg_start, D.seg_cap, D.cidx, D.cand_row, D.row_cnt,
-           contig, ctx->contig_hash.as<u32>(), D.cand_good, D.cand_dir, sb.as<u32>(), maxcap, D.seg_best, D.seg_dir);
+    if (haps)
+      LAUNCH(k_seg_tie<true>, (unsigned)cdiv(n_tie, 64), 64, 0, hap_tie_seg, n_tie, seg_start, D.seg_cap, D.cidx, D.cand_row,
+             D.row_cnt, contig, ctx->contig_hash.as<u32>(), D.cand_good, D.cand_dir, contig_hap, sb.as<u32>(), maxcap, hap_best,
+             hap_dir);
+    else
+      LAUNCH(k_seg_tie<false>, (unsigned)cdiv(n_tie, 64), 64, 0, D.tie_seg, n_tie, seg_start, D.seg_cap, D.cidx, D.cand_row,
+             D.row_cnt, contig, ctx->contig_hash.as<u32>(), D.cand_good, D.cand_dir, contig_hap, sb.as<u32>(), maxcap, D.seg_best,
+             D.seg_dir);
+  }
+  if (haps) {
+    StageTimer th(ctx, GVS_ST_READHAPS);
+    LAUNCH(k_seg_pick, (unsigned)cdiv(n_seg, 256), 256, 0, (u32)n_seg, D.seg_hap, hap_best, hap_good, hap_dir, D.seg_best,
+           D.seg_good, D.seg_dir);
+    // records: one per segment with a vote on either haplotype, in segment (read) order
+    CKR(rec_reserve(ctx, ctx->rh, 8, n_seg));
+    RecTable& T = ctx->rh;
+    u32* cols[8];
+    for (u32 c = 0; c < 8; c++) cols[c] = T.col(c);
+    u32 *r_read = cols[0], *r_c1 = cols[1], *r_n1 = cols[2], *r_s1 = cols[3], *r_c2 = cols[4], *r_n2 = cols[5], *r_s2 = cols[6],
+        *r_hap = cols[7];
+    const u32 *hb = hap_best, *hg = hap_good;
+    const u8* hd = hap_dir;
+    auto f = [hb] __device__(u64 s) -> u32 { return (hb[2 * s] != NOBEST || hb[2 * s + 1] != NOBEST) ? 1u : 0u; };
+    auto g = [=] __device__(u64 s, u32 ex, u32 v) {
+      if (!v) return;
+      r_read[ex] = read[seg_start[s]];
+      r_c1[ex] = hb[2 * s];
+      r_n1[ex] = hg[2 * s];
+      r_s1[ex] = hb[2 * s] != NOBEST ? hd[2 * s] ^ 1u : 0u;  // dir 1 = '+' -> strand 0
+      r_c2[ex] = hb[2 * s + 1];
+      r_n2[ex] = hg[2 * s + 1];
+      r_s2[ex] = hb[2 * s + 1] != NOBEST ? hd[2 * s + 1] ^ 1u : 0u;
+      r_hap[ex] = hap_assign(hg[2 * s], hg[2 * s + 1]);
+    };
+    u32 n_rec = 0;
+    CKR(scan_total(ctx, n_seg, f, g, OpSum(), &n_rec));
+    T.n = n_rec;
   }
   // ---- kept rows + best list ----
   u32* kt = counter(ctx, CNT_KEPT);
@@ -693,6 +814,11 @@ static int diag_impl(gvs_ctx* ctx, u64* n_best_out, u64* n_kept_out) {
 
 extern "C" int gvs_diag_filter(gvs_ctx* ctx, const uint8_t* contig_hap, const uint32_t* contig_hash, uint64_t* n_best,
                                uint64_t* n_kept) {
+  return gvs_diag_filter_haps(ctx, contig_hap, contig_hash, 0, n_best, n_kept);
+}
+
+extern "C" int gvs_diag_filter_haps(gvs_ctx* ctx, const uint8_t* contig_hap, const uint32_t* contig_hash, int read_haps,
+                                    uint64_t* n_best, uint64_t* n_kept) {
   if (!ctx) return GVS_E_ARG;
   if (!ctx->match_ready) return gvs_fail(ctx, GVS_E_STATE, "gvs_diag_filter before gvs_match");
   if (!contig_hap || !contig_hash) return gvs_fail(ctx, GVS_E_ARG, "null contig tables");
@@ -701,12 +827,28 @@ extern "C" int gvs_diag_filter(gvs_ctx* ctx, const uint8_t* contig_hap, const ui
   ctx->val_ready = false;
   CKR(to_dev(ctx, ctx->contig_hap, contig_hap, ctx->n_contigs));
   CKR(to_dev(ctx, ctx->contig_hash, contig_hash, ctx->n_contigs));
+  bool haps = read_haps != 0;
+  for (u8 h : ctx->h_chunk_hap) haps |= h == GVS_HAP_ANY;
   u64 nb = 0, nk = 0;
-  CKR(diag_impl(ctx, &nb, &nk));
+  CKR(diag_impl(ctx, haps, &nb, &nk));
   if (n_best) *n_best = nb;
   if (n_kept) *n_kept = nk;
   ctx->diag_ready = true;
   return 0;
+}
+
+extern "C" int gvs_read_haps(gvs_ctx* ctx, uint64_t* n_records) {
+  if (!ctx) return GVS_E_ARG;
+  if (!ctx->rh.ready) return gvs_fail(ctx, GVS_E_STATE, "gvs_read_haps without a diag filter in haplotype mode");
+  if (n_records) *n_records = ctx->rh.n;
+  return 0;
+}
+
+extern "C" int gvs_read_haps_get(gvs_ctx* ctx, uint32_t* read, uint32_t* contig1, uint32_t* n1, uint32_t* strand1,
+                                 uint32_t* contig2, uint32_t* n2, uint32_t* strand2, uint32_t* hap) {
+  return ctx ? rec_get(ctx, ctx->rh, "gvs_read_haps_get without a diag filter in haplotype mode",
+                       {read, contig1, n1, strand1, contig2, n2, strand2, hap})
+             : GVS_E_ARG;
 }
 
 extern "C" int gvs_best_get(gvs_ctx* ctx, uint32_t* read_idx, uint32_t* contig, uint32_t* ngood, uint8_t* dir) {

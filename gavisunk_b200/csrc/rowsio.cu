@@ -62,6 +62,8 @@ extern "C" int gvs_reads_meta(gvs_ctx* ctx, const uint32_t* read_len, uint64_t n
   CK(cudaSetDevice(ctx->device));
   if (!chunk_first || !chunk_hap || n_chunks == 0) return gvs_fail(ctx, GVS_E_ARG, "null chunk arrays");
   if (chunk_first[0] != 0 || chunk_first[n_chunks] != n_reads) return gvs_fail(ctx, GVS_E_ARG, "chunk_first must span [0, n_reads]");
+  for (u32 c = 0; c < n_chunks; c++)
+    if (chunk_hap[c] > GVS_HAP_ANY) return gvs_fail(ctx, GVS_E_ARG, "chunk haplotype %u (0, 1 or GVS_HAP_ANY)", chunk_hap[c]);
   CKR(gvs_pipe_join(ctx));
   ctx->seg_tile_end.clear();
   ctx->seg_packed.clear();

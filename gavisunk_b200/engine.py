@@ -16,6 +16,8 @@ import numpy as np
 from . import _lib
 from ._lib import GavisunkError, GavisunkKeyError
 
+GVS_HAP_ANY = 2  # chunk haplotype of unbinned reads: the diag filter assigns each read from its SUNK votes
+
 _LUT = np.zeros(256, dtype=np.uint64)
 for _ch, _v in (("A", 0), ("C", 1), ("G", 2), ("T", 3), ("U", 3)):
     _LUT[ord(_ch)] = _v
@@ -371,17 +373,30 @@ class Engine:
             n = self.n_rows if which == 0 else self.n_kept
         return self._table(f"rows{which}", self.lib.gvs_rows_get, n, self.ROW_COLUMNS, lead=(which,), pinned=pinned)
 
-    def diag_filter(self, contig_hap: Sequence[int]) -> Tuple[int, int]:
+    def diag_filter(self, contig_hap: Sequence[int], read_haps: bool = False) -> Tuple[int, int]:
         """diag_filter_v3 + diag_filter_step2 (workflow/src/diag_filter_v3.nim:18-229,
         workflow/src/diag_filter_step2.nim:13-66).  contig_hap[c] = haplotype whose .fai lists
-        contig c (255 = neither)."""
+        contig c (255 = neither).  read_haps: also vote on the other haplotype and keep the records for
+        read_haps() (include/gavisunk_b200.h gvs_diag_filter_haps); always on for a batch with GVS_HAP_ANY chunks,
+        whose reads keep their rows on the haplotype their votes assign."""
         ch = _c(contig_hap, np.uint8)
         hh = np.array([nim_hash(n) for n in self.contig_names], dtype=np.uint32)
         assert len(ch) == len(self.contig_names)
         a, b = C.c_uint64(), C.c_uint64()
-        self._ck(self.lib.gvs_diag_filter(self.ctx, _ptr(ch), _ptr(hh), C.byref(a), C.byref(b)))
+        self._ck(self.lib.gvs_diag_filter_haps(self.ctx, _ptr(ch), _ptr(hh), 1 if read_haps else 0, C.byref(a), C.byref(b)))
         self.n_best, self.n_kept = int(a.value), int(b.value)
         return self.n_best, self.n_kept
+
+    READ_HAP_COLUMNS = ("read", "contig1", "n1", "strand1", "contig2", "n2", "strand2", "hap")
+
+    def read_haps(self, pinned: bool = False) -> Dict[str, np.ndarray]:
+        """Read haplotypes (no reference counterpart; include/gavisunk_b200.h gvs_diag_filter_haps): one record per read
+        with a vote on either haplotype, of the last diag filter in haplotype mode, or of the run after run_batches --
+        read (run-wide index), per haplotype the voted contig (0xFFFFFFFF: none), its votes n (0: none) and strand
+        (0 '+', 1 '-'), and the assignment hap (0, 1, 2 = tie)."""
+        n = C.c_uint64()
+        self._ck(self.lib.gvs_read_haps(self.ctx, C.byref(n)))
+        return self._table("read_haps", self.lib.gvs_read_haps_get, int(n.value), self.READ_HAP_COLUMNS, pinned=pinned)
 
     def best(self) -> Dict[str, np.ndarray]:
         return self._table("best", self.lib.gvs_best_get, self.n_best, ("read", "contig", "ngood", "dir"),
@@ -442,7 +457,7 @@ class Engine:
         return self.n_kept, self.n_reads
 
     def run_batches(self, binds, contig_hap: Sequence[int], min_read_len: int = 10000, allreduce_hist=None,
-                    gather_forests=None, on_batch=None, junctions: bool = False):
+                    gather_forests=None, on_batch=None, junctions: bool = False, read_haps: bool = False):
         """The hot path over a run whose reads come in several batches (a sample's chunk files, or the shard of
         them this GPU owns).  The reference gathers all chunks of a haplotype before the global stages
         (workflow/Snakefile:23-24, workflow/rules/tagONT.smk:112-131; badsunks_AR.py:20-27 counts over every
@@ -454,14 +469,16 @@ class Engine:
              forest, ONE forest all-gather (`gather_forests`), intervals.
         Results equal run_all() on the concatenation of the batches; read indices of rows(1) / pairs() count
         through the batches in order.  junctions: also screen every batch after its diag filter (junction_screen),
-        so that junctions() reports the run's records afterwards.  Returns (intervals, [read_base of every batch])."""
+        so that junctions() reports the run's records afterwards.  read_haps: run every diag filter in haplotype mode,
+        so that read_haps() reports the run's records afterwards (batches with GVS_HAP_ANY chunks always are).
+        Returns (intervals, [read_base of every batch])."""
         self.batches_begin()
         bases, hp = [], 0
         rows = best = 0
         for b, bind in enumerate(binds):
             bind(self)
             rows += self.match()
-            best += self.diag_filter(contig_hap)[0]
+            best += self.diag_filter(contig_hap, read_haps)[0]
             if junctions:
                 self.junction_screen(min_read_len)
             hp = self.group_hist(accumulate=True)

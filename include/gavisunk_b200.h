@@ -61,7 +61,8 @@ enum {
   GVS_ST_SCREEN = 13,   /* junction screen of one batch (gvs_junction_screen)                     */
   GVS_ST_JUNCTIONS = 14, /* junction records (gvs_junctions): no reference counterpart            */
   GVS_ST_DISCORDANCE = 15, /* distance discordance (gvs_spans, gvs_discordance): no reference counterpart */
-  GVS_ST_COUNT = 16
+  GVS_ST_READHAPS = 16, /* haplotype mode of the diag filter (gvs_diag_filter_haps): votes per haplotype, records */
+  GVS_ST_COUNT = 17
 };
 
 /* ------------------------------------------------------------------------------------------ */
@@ -189,10 +190,12 @@ int64_t gvs_format_rows(const gvs_col* cols, uint32_t n_cols, uint64_t n_rows, c
  *   chunk_first    n_chunks+1 read indices: chunk c = reads [chunk_first[c], chunk_first[c+1]);
  *                  the kmerpos_annot3 `prevLoc` carry (nim:82-84, SURVEY Q4) restarts per chunk
  *   chunk_hap      n_chunks entries, the haplotype (0/1) whose .fai the chunk's reads are
- *                  filtered against (workflow/rules/tagONT.smk:79,92)
+ *                  filtered against (workflow/rules/tagONT.smk:79,92), or GVS_HAP_ANY: unbinned reads,
+ *                  whose haplotype the diag filter assigns from their SUNK votes (gvs_diag_filter_haps)
  * on_device != 0: seq and read_off are device pointers that stay valid until the next
  * gvs_reads_* call (no copy is made); chunk arrays are always host memory.
  * With on_device == 0 the arrays are copied host->device on the context's stream. */
+enum { GVS_HAP_ANY = 2 };
 int gvs_reads_set(gvs_ctx* ctx, const uint8_t* seq, const uint64_t* read_off, uint64_t n_reads,
                   const uint64_t* chunk_first, const uint8_t* chunk_hap, uint32_t n_chunks,
                   int on_device);
@@ -266,6 +269,27 @@ int gvs_rows_get(gvs_ctx* ctx, int which, uint32_t* read_idx, uint32_t* pos, uin
  * n_best = reads that got a best contig, n_kept = rows that survive. */
 int gvs_diag_filter(gvs_ctx* ctx, const uint8_t* contig_hap, const uint32_t* contig_hash,
                     uint64_t* n_best, uint64_t* n_kept);
+/* Read haplotypes: the diag filter's vote taken once per haplotype.  No reference counterpart.  For a read r and a
+ * haplotype h:
+ *   vote_h(r)    the (contig, n, dir) diag_filter_v3 prints for r when it runs over r's chunk with haplotype h's .fai
+ *                (candidates limited to the contigs of h; the Table replay of ties still holds every contig of the
+ *                read, so slot order and the capacity carried through the chunk do not depend on h); no vote when
+ *                maxgood <= 1.  n_h = n, or 0 without a vote;
+ *   assigned(r)  h when n_h > n_(1-h), tie when n_0 == n_1 >= 2, none when both are 0.
+ * Reads of a binned chunk (haplotype 0/1) keep their rows exactly as gvs_diag_filter keeps them, from the vote of
+ * the chunk's haplotype; the other vote is only reported.  Reads of a GVS_HAP_ANY chunk keep their rows on
+ * vote_assigned(r)'s contig; a tie or none read keeps no rows and has no best row.
+ * Haplotype mode is on when read_haps != 0 or a chunk of the batch is GVS_HAP_ANY; with it off gvs_diag_filter_haps
+ * is gvs_diag_filter.  With it on, the filter also writes one record per read with n_0 >= 2 or n_1 >= 2, in read
+ * order: read, contig1, n1, strand1, contig2, n2, strand2, hap (contig 0xFFFFFFFF and n 0 without a vote; strand 0
+ * '+', 1 '-'; hap 0 / 1 / 2 = tie).  gvs_batch_stash appends them to the run's records with run-wide read indices,
+ * which gvs_batches_bind makes current.  gvs_read_haps: *n_records of the last filter in haplotype mode (or of the
+ * run after gvs_batches_bind); gvs_read_haps_get: host buffers of *n_records entries, any pointer may be NULL. */
+int gvs_diag_filter_haps(gvs_ctx* ctx, const uint8_t* contig_hap, const uint32_t* contig_hash, int read_haps,
+                         uint64_t* n_best, uint64_t* n_kept);
+int gvs_read_haps(gvs_ctx* ctx, uint64_t* n_records);
+int gvs_read_haps_get(gvs_ctx* ctx, uint32_t* read, uint32_t* contig1, uint32_t* n1, uint32_t* strand1, uint32_t* contig2,
+                      uint32_t* n2, uint32_t* strand2, uint32_t* hap);
 /* rows of {hap}_{i}_diag.sunkpos: read, contig, n, dir (0 = '-', 1 = '+') */
 int gvs_best_get(gvs_ctx* ctx, uint32_t* read_idx, uint32_t* contig, uint32_t* ngood,
                  uint8_t* dir);
