@@ -14,11 +14,12 @@
   python -m gavisunk_b200.cli combine_ont_nofilt <chunk.sunkpos>.. <hapN_detailed.sunkpos>
   python -m gavisunk_b200.cli fused --sample S --k K --hap1-asm .. --hap2-asm .. (--hap1-reads f.. --hap2-reads f.. | --reads f..)
                                     --outdir D [--devices 0,1,..] [--batch-files N] [--detailed] [--support-tracks]
-                                    [--gap-evidence] [--junctions] [--discordance] [--read-haplotypes]
+                                    [--gap-evidence] [--junctions] [--discordance] [--read-haplotypes] [--inversions]
   python -m gavisunk_b200.cli support_tracks <sunkpos> <rlen> <bad_sunks.txt> <fai> <valid.bed> <out.reads.bed> <out.bedgraph> <out.tsv>
   python -m gavisunk_b200.cli gap_evidence <sunkpos> <rlen> <bad_sunks.txt> <fai> <valid.bed> <out.gaps.reads.tsv> <out.gaps.evidence.tsv>
   python -m gavisunk_b200.cli junctions <hapN_detailed.sunkpos> <hapN.rlen> <bad_sunks.txt> <fai1> <fai2> <out.junctions.reads.tsv> <out.junctions.tsv>
   python -m gavisunk_b200.cli discordance <sunkpos> <rlen> <bad_sunks.txt> <fai> <out.discordance.reads.tsv> <out.discordance.tsv> <out.discordance.bed>
+  python -m gavisunk_b200.cli inversions <sunkpos> <rlen> <bad_sunks.txt> <fai> <out.inversions.reads.tsv> <out.inversions.bed>
 
 The first four replace workflow/scripts/{kmerpos_annot3,rlen,diag_filter_v3,diag_filter_step2}
 (workflow/rules/tagONT.smk:36,73,92,110) one to one; the next six replace badsunks_AR.py,
@@ -37,6 +38,8 @@ of the validated reads across them (no reference counterpart).
 `fused --read-haplotypes` reports each read's SUNK vote on both haplotypes and the haplotype it assigns; `fused --reads`
 takes unbinned chunk files and keeps each read's rows on the haplotype its votes assign (no reference counterpart: the
 reference needs the reads binned by haplotype).
+`fused --inversions` and `inversions` report the reads whose SUNKs switch strand inside a contig, and cluster them into
+inversion calls (no reference counterpart: the validation takes each read's orientation majority).
 Text parsing / formatting is host
 plumbing; all per-base and per-row work runs in libgavisunk_b200.so.  Errors exit non-zero with a
 message on stderr and never leave a partial output file behind.
@@ -470,6 +473,19 @@ _CLASS = gio.NameTable(["link", "breakpoint"])
 JUNCTION_CHAIN = 10000  # start distance that still chains two records into one cluster
 
 
+def chains(items, at):
+    """items sorted by item[at] (stable) and cut into maximal chains whose consecutive values are at most JUNCTION_CHAIN
+    apart"""
+    items = sorted(items, key=lambda t: t[at])
+    out = [[items[0]]]
+    for t in items[1:]:
+        if t[at] - out[-1][-1][at] <= JUNCTION_CHAIN:
+            out[-1].append(t)
+        else:
+            out.append([t])
+    return out
+
+
 def junction_columns(jn, contig_len):
     """Host columns of junction records (Engine.junctions()): read_gap = pos2 - pos1; leave1 = distance from flank 1 to
     the end of contig1 the read leaves through (len1 - start1 on '+', start1 on '-'); enter2 = distance from the end of
@@ -510,16 +526,6 @@ def junction_texts(jn, sel, names, contig_len, contig_hap, rtab, read_len, name_
         if (b[0], b[2]) < (a[0], a[2]):
             a, b = (b[0], 1 - b[1], b[2]), (a[0], 1 - a[1], a[2])
         keyed[(a[0], a[1], b[0], b[1])].append((a[2], b[2], int(implied[i]), int(cls[i]) == 0))
-
-    def chains(items, at):
-        items = sorted(items, key=lambda t: t[at])
-        out = [[items[0]]]
-        for t in items[1:]:
-            if t[at] - out[-1][-1][at] <= JUNCTION_CHAIN:
-                out[-1].append(t)
-            else:
-                out.append([t])
-        return out
     lower_median = lambda v: sorted(v)[(len(v) - 1) // 2]
     clusters = []
     for (c1, d1, c2, d2), items in keyed.items():
@@ -652,6 +658,79 @@ def discordance(sunkpos_p, rlen_p, badsunks_p, fai_p, out_reads_tsv, out_runs_ts
 
 def cmd_discordance(argv):
     discordance(*argv)
+
+
+# ------------------------------------------------------------------------------------------------
+# inversions: reads whose SUNKs switch strand inside a contig (no reference counterpart; DESIGN.md section 5.5f)
+# ------------------------------------------------------------------------------------------------
+INVERSION_READS_HEADER = ("contig\tread\tread_len\tstrand1\tids1\tlo1\thi1\tid1\tstart1\tpos1\tstrand2\tids2\tlo2\thi2\tid2\t"
+                          "start2\tpos2\tread_gap\tkind\n")
+INVERSION_MIN_READS = 3  # distinct reads of a called cluster
+_SWITCH_KIND = gio.NameTable(["inversion", "foldback"])
+
+
+def switch_kinds(sw) -> np.ndarray:
+    """1 (foldback) for a record of Engine.strand_switches() whose two blocks overlap on the assembly (max(lo1, lo2) <=
+    min(hi1, hi2)), else 0 (inversion)"""
+    return (np.maximum(sw["lo1"], sw["lo2"]) <= np.minimum(sw["hi1"], sw["hi2"])).astype(np.uint32)
+
+
+def inversion_calls(sw, sel, min_reads=INVERSION_MIN_READS):
+    """Calls from the records sel of Engine.strand_switches(): the `inversion` records of each contig, keyed by (a, b) =
+    (min(start1, start2), max(start1, start2)), chained by a and then by b (chains); a cluster of >= min_reads distinct
+    reads is a call.  -> sorted list of (contig, start, end, reads, switches, spanning): start / end = lower medians of a /
+    b, switches = its records, spanning = its reads with 2 or more records (one at each breakpoint)"""
+    kind = switch_kinds(sw)
+    keyed = defaultdict(list)
+    for i in np.asarray(sel, np.int64).tolist():
+        if kind[i] == 0:
+            s1, s2 = int(sw["start1"][i]), int(sw["start2"][i])
+            keyed[int(sw["contig"][i])].append((min(s1, s2), max(s1, s2), int(sw["read"][i])))
+    lower_median = lambda v: sorted(v)[(len(v) - 1) // 2]
+    out = []
+    for c, items in keyed.items():
+        for ch in chains(items, 0):
+            for cl in chains(ch, 1):
+                per_read = defaultdict(int)
+                for t in cl:
+                    per_read[t[2]] += 1
+                if len(per_read) >= min_reads:
+                    out.append((c, lower_median([t[0] for t in cl]), lower_median([t[1] for t in cl]), len(per_read), len(cl),
+                                sum(1 for v in per_read.values() if v >= 2)))
+    return sorted(out)
+
+
+def inversion_texts(hap_contigs, names, sw, rtab, read_len, name_rank):
+    """The two inversion files of one haplotype: hap_contigs = its contig ids; sw = Engine.strand_switches() with run-wide
+    read indices; rtab / read_len / name_rank = name table, length and bytewise name rank of every run-wide read.  The
+    records of the haplotype's contigs go to inversions.reads.tsv in (read name, record) order, with read_gap = pos2 -
+    pos1 and kind (switch_kinds); the calls (inversion_calls) to inversions.bed.  -> (inversions.reads.tsv,
+    inversions.bed) bytes"""
+    ctab = gio.NameTable(names)
+    inhap = np.zeros(len(names), bool)
+    inhap[np.asarray(hap_contigs, np.int64)] = True
+    sel = np.flatnonzero(inhap[sw["contig"]])
+    r = sel[np.lexsort((sel, name_rank[sw["read"][sel]]))]
+    cols = [("name", sw["contig"], ctab), ("name", sw["read"], rtab), ("u32", read_len[sw["read"]])]
+    for side in "12":
+        cols += [("name", sw["strand" + side], _STRAND)] + [("u32", sw[c + side]) for c in ("ids", "lo", "hi", "id", "start", "pos")]
+    cols += [("i64", sw["pos2"].astype(np.int64) - sw["pos1"].astype(np.int64)), ("name", switch_kinds(sw), _SWITCH_KIND)]
+    reads_tsv = INVERSION_READS_HEADER.encode() + gio.format_rows(cols, sel=r)
+    bed = "".join(f"{names[c]}\t{a}\t{b}\tinversion\t{n}\t{k}\t{sp}\n" for c, a, b, n, k, sp in inversion_calls(sw, sel))
+    return reads_tsv, bed.encode("latin-1")
+
+
+def inversions(sunkpos_p, rlen_p, badsunks_p, fai_p, out_reads_tsv, out_bed):
+    """Inversions of one haplotype from the files of the per-rule path ({hap}.sunkpos, {hap}.rlen, bad_sunks.txt, the
+    .fai): reads grouped by (contig, read name) as process_by_contig groups them per contig, the reference's fixed minimum
+    read length."""
+    eng, names, _, _, reads = _keyed_hap(sunkpos_p, rlen_p, badsunks_p, fai_p)
+    sw = eng.strand_switches(10000)  # the reference's fixed minimum read length (process-by-contig_lowmem_AR.py:106, SURVEY Q13)
+    _write_all((out_reads_tsv, out_bed), inversion_texts(list(range(len(names))), names, sw, *reads))
+
+
+def cmd_inversions(argv):
+    inversions(*argv)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -977,6 +1056,9 @@ EVIDENCE_PRODUCTS = {
     "read_haplotypes": Evidence("--read-haplotypes", "also write final_out/hap{N}.haplotype.reads.tsv and .haplotype.tsv (each "
                                 "read's SUNK vote on both haplotypes; implied by --reads)", "read_haps", Engine.READ_HAP_COLUMNS,
                                 ("haplotype.reads.tsv", "haplotype.tsv")),
+    "inversions": Evidence("--inversions", "also write final_out/hap{N}.inversions.reads.tsv and .inversions.bed (reads whose SUNKs "
+                           "switch strand inside a contig, and inversion calls)", "switches", Engine.SWITCH_COLUMNS,
+                           ("inversions.reads.tsv", "inversions.bed")),
 }
 
 
@@ -1029,9 +1111,10 @@ def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int]
     engine's own reads (each batch screened after its diag filter, resolved with the run's bad groups); discordance: the
     discordant spans of every engine's own reads and the discordance runs, with the difference arrays summed like the
     support's; read_haplotypes: every engine's diag filters in haplotype mode and the records of its own reads (file_hap
-    GVS_HAP_ANY: unbinned chunks, always filtered in haplotype mode).  -> one result dict per engine (read names /
+    GVS_HAP_ANY: unbinned chunks, always filtered in haplotype mode); inversions: the strand-switch records of every
+    engine's own reads, from its kept rows and the run's bad groups.  -> one result dict per engine (read names /
     lengths / chunk tables, kept rows, validated pairs, intervals[, placements, support runs][, gap evidence][,
-    junctions][, spans, discordance runs][, read haplotypes])."""
+    junctions][, spans, discordance runs][, read haplotypes][, strand switches])."""
     import threading
     from concurrent.futures import ThreadPoolExecutor
     for p in files:
@@ -1101,6 +1184,8 @@ def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int]
                 info.update(spans=eng.spans(), discordance=eng.discordance(contig_len, allreduce=cx.allreduce_hist))
             if "read_haplotypes" in products:
                 info.update(read_haps=eng.read_haps() if mine else {c: np.zeros(0, np.uint32) for c in Engine.READ_HAP_COLUMNS})
+            if "inversions" in products:
+                info.update(switches=eng.strand_switches(min_read_len))
             results[di] = info
         except BaseException as ex:  # noqa: BLE001 -- reported by the caller; peers must not wait for this rank
             errors.append(ex)
@@ -1314,7 +1399,8 @@ def write_outputs(k, eng, results, contig_len, contig_hap, names, iv, gaps, noda
             gap_evidence=lambda r: gap_evidence_texts(gsel, gaps, names, r, *reads),
             junctions=lambda r: junction_texts(r, np.flatnonzero(read_hap[r["read"]] == hap), names, clen, contig_hap, *reads),
             discordance=lambda r: discordance_texts(hap_contigs, names, r, results[0]["discordance"], *reads),
-            read_haplotypes=lambda r: read_hap_texts(hap, names, chap, r, read_bin, read_hap, *reads))
+            read_haplotypes=lambda r: read_hap_texts(hap, names, chap, r, read_bin, read_hap, *reads),
+            inversions=lambda r: inversion_texts(hap_contigs, names, r, *reads))
         for p in products:
             _write_all([d("final_out", f"hap{hn}.{ext}") for ext in EVIDENCE_PRODUCTS[p].suffixes], texts[p](rec[p]))
     from concurrent.futures import ThreadPoolExecutor
@@ -1364,7 +1450,7 @@ COMMANDS = {"kmerpos_annot3": (cmd_kmerpos_annot3, 4), "rlen": (cmd_rlen, 2), "d
             "covprob": (cmd_covprob, None), "split_locs": (cmd_split_locs, None), "fused": (cmd_fused, None),
             "split_ont": (cmd_split_ont, None), "combine_ont_nofilt": (cmd_combine_ont_nofilt, None),
             "support_tracks": (cmd_support_tracks, 8), "gap_evidence": (cmd_gap_evidence, 7),
-            "junctions": (cmd_junctions, 7), "discordance": (cmd_discordance, 7)}
+            "junctions": (cmd_junctions, 7), "discordance": (cmd_discordance, 7), "inversions": (cmd_inversions, 6)}
 
 
 def main(argv=None):

@@ -201,6 +201,11 @@ struct gvs_ctx {
   RecTable dc;                      // span records of gvs_spans: 8 columns
   RecTable dc_runs;                 // runs of gvs_discordance: contig, start, end, spans, longer, shorter
 
+  // ---- strand switches (inversions.cu) ----
+  DevBuf sw_seg_start, sw_scr, sw_seg;  // segments of the kept rows when gvs_validate's are not current; per kept row
+                                        // scratch (7 u32 arrays + 1 byte); per segment records
+  RecTable sw;                      // records: 16 columns
+
   // ---- components / intervals / gaps ----
   DevBuf parent, present, comp_min, comp_max, comp_cnt;
   DevBuf comp_rank;  // unsorted group tables only: [smallest member rank per root | root per interval rank]
@@ -593,6 +598,57 @@ struct SegRows {
 static inline SegRows seg_rows(const gvs_ctx* ctx, const Rows& r, const DevBuf& seg_start, u64 n_seg) {
   return {r.read.as<u32>(), r.pos.as<u32>(), r.contig.as<u32>(), r.start.as<u32>(), r.group.as<u32>(), r.gidx.as<u32>(),
           seg_start.as<u32>(), (u32)n_seg, ctx->bad_ready ? ctx->bad_flag.as<u8>() : nullptr};
+}
+
+// Cut the elements i of [a, b) with in(i), in order, into maximal runs of one key(i) (one warp): idx[i] = run of i,
+// *first / *last (may be null) = per run its first / last element at a + run.  Returns the number of runs.  Junctions
+// cut rows by contig, strand switches cut ordered rows by strand.
+template <typename In, typename Key>
+__device__ u32 warp_runs(u32 a, u32 b, In in, Key key, u32* idx, u32* first, u32* last, int lane) {
+  u32 nrun = 0, carry_c = 0xFFFFFFFFu, carry_i = 0;
+  const u32 lt = (1u << lane) - 1;
+  for (u32 c0 = a; c0 < b; c0 += 32) {
+    const u32 i = c0 + lane;
+    const bool q = i < b && in(i);
+    const u32 c = q ? key(i) : 0xFFFFFFFFu;
+    const u32 m = __ballot_sync(0xFFFFFFFFu, q);
+    const u32 pm = m & lt;
+    const int src = pm ? 31 - __clz(pm) : lane;
+    const u32 pc = __shfl_sync(0xFFFFFFFFu, c, src), pi = __shfl_sync(0xFFFFFFFFu, i, src);
+    const u32 prev_c = pm ? pc : carry_c, prev_i = pm ? pi : carry_i;
+    const bool nw = q && prev_c != c;
+    const u32 nm = __ballot_sync(0xFFFFFFFFu, nw);
+    if (q) {
+      const u32 r = nrun + __popc(nm & (lt | (1u << lane))) - 1;
+      idx[i] = r;
+      if (nw) {
+        if (first) first[a + r] = i;
+        if (last && r > 0) last[a + r - 1] = prev_i;
+      }
+    }
+    if (m) {
+      const int hi = 31 - __clz(m);
+      carry_c = __shfl_sync(0xFFFFFFFFu, c, hi);
+      carry_i = __shfl_sync(0xFFFFFFFFu, i, hi);
+    }
+    nrun += __popc(nm);
+  }
+  if (last && nrun && lane == 0) last[a + nrun - 1] = carry_i;
+  return nrun;
+}
+
+// element i is the first of its ID id(i) within its run / block of warp_runs: no earlier element j with in(j) and the
+// same idx has the ID (the elements of one idx are contiguous among those with in(), so the look-back stops at the
+// first one of another idx)
+template <typename In, typename Id>
+__device__ __forceinline__ bool warp_first_in(const u32* idx, u32 a, u32 i, In in, Id id) {
+  const u32 r = idx[i], g = id(i);
+  for (u32 j = i; j-- > a;) {
+    if (!in(j)) continue;
+    if (idx[j] != r) return true;
+    if (id(j) == g) return false;
+  }
+  return true;
 }
 
 // read lengths: explicit (gvs_reads_meta, a batches run) or from the offsets of the batch, clamped to 32 bits

@@ -136,51 +136,15 @@ struct JnScratch {
   u32 *first, *last, *up, *down;  // per block: first / last row, ratio-passing pairs rising / falling
 };
 
-// Cut the flagged rows (fa & flag) of [a, b) into maximal runs on one contig, in row order: idx[i] = run of row i,
-// *first_row / *last_row (may be null) = per run its first / last row at a + run.  Returns the number of runs.
-__device__ u32 jn_runs(const JnRows& R, u32 a, u32 b, u8 flag, u32* idx, u32* first_row, u32* last_row, int lane) {
-  u32 nrun = 0, carry_c = 0xFFFFFFFFu, carry_i = 0;
-  const u32 lt = (1u << lane) - 1;
-  for (u32 c0 = a; c0 < b; c0 += 32) {
-    const u32 i = c0 + lane;
-    const bool q = i < b && (R.fa[i] & flag);
-    const u32 c = q ? R.contig[i] : 0xFFFFFFFFu;
-    const u32 m = __ballot_sync(0xFFFFFFFFu, q);
-    const u32 pm = m & lt;
-    const int src = pm ? 31 - __clz(pm) : lane;
-    const u32 pc = __shfl_sync(0xFFFFFFFFu, c, src), pi = __shfl_sync(0xFFFFFFFFu, i, src);
-    const u32 prev_c = pm ? pc : carry_c, prev_i = pm ? pi : carry_i;
-    const bool nw = q && prev_c != c;
-    const u32 nm = __ballot_sync(0xFFFFFFFFu, nw);
-    if (q) {
-      const u32 r = nrun + __popc(nm & (lt | (1u << lane))) - 1;
-      idx[i] = r;
-      if (nw) {
-        if (first_row) first_row[a + r] = i;
-        if (last_row && r > 0) last_row[a + r - 1] = prev_i;
-      }
-    }
-    if (m) {
-      const int hi = 31 - __clz(m);
-      carry_c = __shfl_sync(0xFFFFFFFFu, c, hi);
-      carry_i = __shfl_sync(0xFFFFFFFFu, i, hi);
-    }
-    nrun += __popc(nm);
-  }
-  if (last_row && nrun && lane == 0) last_row[a + nrun - 1] = carry_i;
-  return nrun;
+// runs of the flagged rows (fa & flag) on one contig, in row order (warp_runs)
+__device__ __forceinline__ u32 jn_runs(const JnRows& R, u32 a, u32 b, u8 flag, u32* idx, u32* first_row, u32* last_row, int lane) {
+  return warp_runs(a, b, [&](u32 i) { return (R.fa[i] & flag) != 0; }, [&](u32 i) { return R.contig[i]; }, idx, first_row,
+                   last_row, lane);
 }
 
-// first row of its ID within its run / block: no earlier flagged row of the same idx has the ID (the rows of one idx
-// are contiguous among the flagged rows, so the look-back stops at the first flagged row of another idx)
+// first flagged row of its ID within its run / block (warp_first_in)
 __device__ __forceinline__ bool jn_first_in(const JnRows& R, const u32* idx, u32 a, u32 i, u8 flag) {
-  const u32 r = idx[i], id = R.group[i];
-  for (u32 j = i; j-- > a;) {
-    if (!(R.fa[j] & flag)) continue;
-    if (idx[j] != r) return true;
-    if (R.group[j] == id) return false;
-  }
-  return true;
+  return warp_first_in(idx, a, i, [&](u32 j) { return (R.fa[j] & flag) != 0; }, [&](u32 j) { return R.group[j]; });
 }
 
 // per stashed read: blocks, and the number of records (consecutive block pairs)

@@ -656,6 +656,18 @@ class Engine:
         self._ck(self.lib.gvs_junctions(self.ctx, C.byref(n)))
         return self._table("junctions", self.lib.gvs_junctions_get, int(n.value), self.JUNCTION_COLUMNS)
 
+    SWITCH_COLUMNS = ("read", "contig", "strand1", "ids1", "lo1", "hi1", "id1", "start1", "pos1", "strand2", "ids2", "lo2", "hi2",
+                      "id2", "start2", "pos2")
+
+    def strand_switches(self, min_read_len: int = 10000, pinned: bool = False) -> Dict[str, np.ndarray]:
+        """Reads whose SUNKs switch strand inside one contig (no reference counterpart; include/gavisunk_b200.h
+        gvs_strand_switches), from the kept rows minus the bad groups, reads of length >= min_read_len: one record per pair
+        of consecutive blocks of one strand -- read (run-wide index), contig, then per block its strand (0 '+', 1 '-'),
+        distinct IDs, smallest / largest start and the (ID, start, pos) of its row next to the switch."""
+        n = C.c_uint64()
+        self._ck(self.lib.gvs_strand_switches(self.ctx, int(min_read_len), C.byref(n)))
+        return self._table("switches", self.lib.gvs_strand_switches_get, int(n.value), self.SWITCH_COLUMNS, pinned=pinned)
+
     def covprob_table(self, kbp, cnt, genome_kbp: float, pn: float) -> np.ndarray:
         """covprob.py:56-100."""
         kbp = _c(kbp, np.int64)

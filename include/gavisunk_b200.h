@@ -62,7 +62,8 @@ enum {
   GVS_ST_JUNCTIONS = 14, /* junction records (gvs_junctions): no reference counterpart            */
   GVS_ST_DISCORDANCE = 15, /* distance discordance (gvs_spans, gvs_discordance): no reference counterpart */
   GVS_ST_READHAPS = 16, /* haplotype mode of the diag filter (gvs_diag_filter_haps): votes per haplotype, records */
-  GVS_ST_COUNT = 17
+  GVS_ST_SWITCHES = 17, /* strand switches inside a contig (gvs_strand_switches): no reference counterpart       */
+  GVS_ST_COUNT = 18
 };
 
 /* ------------------------------------------------------------------------------------------ */
@@ -471,6 +472,31 @@ int gvs_junctions(gvs_ctx* ctx, uint64_t* n_records);
 int gvs_junctions_get(gvs_ctx* ctx, uint32_t* read, uint32_t* contig1, uint32_t* strand1, uint32_t* ids1, uint32_t* id1,
                       uint32_t* start1, uint32_t* pos1, uint32_t* contig2, uint32_t* strand2, uint32_t* ids2, uint32_t* id2,
                       uint32_t* start2, uint32_t* pos2);
+
+/* Strand switches: reads whose SUNKs switch strand inside one contig (inversions, fold-back chimeras).  No reference
+ * counterpart: the validation takes each read's orientation majority (process-by-contig_lowmem_AR.py:151-152) and an
+ * inversion keeps its length, so a read validates straight across it.
+ * Inputs: the kept rows (read, pos, contig, start, ID = group) of gvs_diag_filter / gvs_batches_bind / gvs_rows_set(1)
+ * minus the rows of bad groups (when set), reads of length >= min_read_len; a read's rows are those of its segment on
+ * the contig of its first row (as gvs_gap_evidence takes them).  Per read:
+ *   order    rows by ascending pos, ties in row order (gvs_match rows already are: positions rise within a read);
+ *   strand   of row i: over the read's rows j with a different ID that pass 9*|dstart| < 10*|dpos| < 11*|dstart| with
+ *            it, up_i = pairs with (pos_j > pos_i) == (start_j > start_i), down_i = the others; 0 ('+') when up_i >
+ *            down_i, 1 ('-') when down_i > up_i, else unoriented (also a row without a partner);
+ *   blocks   the oriented rows, in order, cut into maximal runs of one strand; runs of fewer than 3 distinct IDs are
+ *            dropped, then runs left adjacent with one strand are merged (one pass: the junction rule with strand in
+ *            place of contig);
+ *   records  one per consecutive block pair (B_i, B_i+1), whose strands differ: read (run-wide, as in gvs_pairs_get),
+ *            contig, strand1, ids1 (distinct IDs of B_i), lo1 / hi1 (smallest / largest start of B_i), (id1, start1,
+ *            pos1) of B_i's last row, strand2, ids2, lo2, hi2, (id2, start2, pos2) of B_i+1's first row; in (read,
+ *            block) order.
+ * An inversion [x, y) makes every read across a breakpoint give a record with {start1, start2} near {x, y}; a fold-back
+ * chimera (a read followed by its reverse complement) gives one whose blocks overlap on the assembly.
+ * gvs_strand_switches_get: host buffers of *n_records entries, any pointer may be NULL. */
+int gvs_strand_switches(gvs_ctx* ctx, uint32_t min_read_len, uint64_t* n_records);
+int gvs_strand_switches_get(gvs_ctx* ctx, uint32_t* read, uint32_t* contig, uint32_t* strand1, uint32_t* ids1, uint32_t* lo1,
+                            uint32_t* hi1, uint32_t* id1, uint32_t* start1, uint32_t* pos1, uint32_t* strand2, uint32_t* ids2,
+                            uint32_t* lo2, uint32_t* hi2, uint32_t* id2, uint32_t* start2, uint32_t* pos2);
 
 /* covprob.py:56-100: table[0..3499] of gap-spanning probabilities from the read-length
  * histogram.  kbp[n_bins], cnt[n_bins] = distinct int(len/1000) values and their multiplicities
