@@ -61,6 +61,7 @@ PROTOTYPES = {
     "gvs_batches_bind": (C.c_int, [vp, u64p, u64p]),
     "gvs_validate": (C.c_int, [vp, C.c_uint32, u64p]),
     "gvs_pairs_get": (C.c_int, [vp, vp, vp, vp, vp]),
+    "gvs_validate_stats": (C.c_int, [vp, u64p]),
     "gvs_components_local": (C.c_int, [vp, C.POINTER(vp)]),
     "gvs_components_merge_all": (C.c_int, [vp, vp, C.c_uint32, C.c_uint32]),
     "gvs_placements": (C.c_int, [vp, u64p, C.POINTER(vp)]),

@@ -3,11 +3,16 @@
 //
 // One thread group per read: a warp for reads with <= 64 rows (8 reads per 256-thread block, no block
 // barriers), a 256-thread block with shared memory up to 512 rows, a 1024-thread block with global
-// scratch beyond.  Rows minus bad groups -> rank-sort by (assembly start, read position) -> every
-// pair (i<j) tested with the integer form of the reference's float64 ratio test (0.9 < dpos/dstart <
-// 1.1  <=>  9*ds < 10*dp < 11*ds, exact for 32-bit inputs) -> orientation majority -> "multipos"
-// clean-up -> connected components of the graph on group IDs -> largest component (ties: the
-// component holding the earliest vertex in graph-tool's insertion order) -> output in vertex order.
+// scratch beyond.  Rows minus bad groups -> stable rank-sort by assembly start (equal starts keep input
+// order) -> every pair (i<j) tested with the integer form of the reference's float64 ratio test (0.9 <
+// dpos/dstart < 1.1  <=>  9*ds < 10*dp < 11*ds, exact for 32-bit inputs) -> orientation majority (ties:
+// 0) -> "multipos" clean-up, which works on (ID, read position) pairs as the reference's value_counts
+// does: an ID is multi-positioned when its oriented edges put it at more than one read position, its
+// good position is the one with the most edge ends (ties: first appearance in the edge list), and an
+// edge whose left end is such an ID off its good position survives only if its right end sits at that
+// good position, whatever the right end's ID -> connected components of the graph on group IDs ->
+// largest component (ties: the component holding the earliest vertex in graph-tool's insertion order)
+// -> output in vertex order.
 //
 // Every pass is row-centric and branch-free: the thread that owns row r walks all rows q with
 // shared-memory broadcast reads and predicated arithmetic; the pair predicate is recomputed instead
@@ -22,11 +27,11 @@
 #define NOT64 0xFFFFFFFFFFFFFFFFull
 
 #define F_MULTI 1u   // the row's ID occurs at more than one read position among the oriented edges
-#define F_GOOD 2u    // ... and this row is the ID's most frequent position
+#define F_GOOD 2u    // the row's read position is its ID's good position (most edge ends over all rows at it)
 #define F_PRES 4u    // the row has at least one surviving edge
 
 struct VWork {
-  u32 *P, *S, *ID, *G;        // rows sorted by (assembly start, read position)
+  u32 *P, *S, *ID, *G;        // rows sorted by assembly start (stable)
   u32 *uP, *uS, *uID, *uG;    // rows after bad-group removal (any order)
   u32 *deg, *rep, *label, *csize, *flags;
   u64 *key, *tv, *ct;
@@ -63,9 +68,10 @@ struct ValParams : SegRows {  // kept rows
   u32* stats;                // [0] reads whose clean-up removed every edge (reference would raise)
 };
 
-// NT threads per read, GROUPS reads per block; GLOBAL: working arrays in global scratch
+// NT threads per read, GROUPS reads per block; GLOBAL: working arrays in global scratch.  The block tier keeps 5
+// blocks per SM resident (its 40 KB of shared memory allow 5, and its grid has 5 per SM): at most 51 registers.
 template <int NT, int GROUPS, bool GLOBAL>
-__global__ void __launch_bounds__(NT* GROUPS) k_validate(const ValParams V) {
+__global__ void __launch_bounds__(NT* GROUPS, NT == 256 ? 5 : 0) k_validate(const ValParams V) {
   extern __shared__ __align__(16) u8 smem[];
   __shared__ u32 s_n0[GROUPS], s_n1[GROUPS], s_m[GROUPS], s_kept[GROUPS], s_bestroot[GROUPS], s_flag[GROUPS], s_dup[GROUPS];
   __shared__ u32 s_pmin[GROUPS], s_pmax[GROUPS];  // span of the read's positions (all threads of the group)
@@ -93,7 +99,7 @@ __global__ void __launch_bounds__(NT* GROUPS) k_validate(const ValParams V) {
     const u32 rd = V.read[a];
     const u32 rlen = V.len(rd);
     const bool skip = rlen < V.min_len || mrows < 2;
-    // ---- rows minus bad groups (:70-72), input order preserved (a read's rows come in increasing pos) ----
+    // ---- rows minus bad groups (:70-72), input order preserved ----
     if (!skip) {
       u32 kept_so_far = 0;
       for (u32 base = 0; base < mrows; base += NT) {
@@ -136,9 +142,9 @@ __global__ void __launch_bounds__(NT* GROUPS) k_validate(const ValParams V) {
       if (tid == 0) V.seg_cnt[s] = 0;
       continue;
     }
-    // ---- sort by (start, pos): sort_values(['rname','start']) is stable and rows of a read come in
-    //      increasing pos (:100).  Reads follow one strand: their starts are usually already strictly
-    //      ascending or strictly descending, which makes the sort a copy; otherwise rank sort. ----
+    // ---- sort by start, equal starts in input order: sort_values(['rname','start']) is stable (:100).
+    //      Reads follow one strand: their starts are usually already strictly ascending or strictly
+    //      descending, which makes the sort a copy; otherwise rank sort. ----
     {
       u32 not_asc = 0, not_desc = 0;
       for (u32 i = tid; i + 1 < m; i += NT) {
@@ -158,8 +164,8 @@ __global__ void __launch_bounds__(NT* GROUPS) k_validate(const ValParams V) {
         if (mono == 0) {
           rank = 0;
           for (u32 j = 0; j < m; j++) {
-            u32 sj = w.uS[j], pj = w.uP[j];
-            rank += (sj < si) | ((sj == si) & (pj < pi));
+            u32 sj = w.uS[j];
+            rank += (sj < si) | ((sj == si) & (j < i));
           }
         }
         w.P[rank] = pi;
@@ -312,7 +318,8 @@ __global__ void __launch_bounds__(NT* GROUPS) k_validate(const ValParams V) {
     }
     const u32 orient = s_n1[grp] > s_n0[grp];  // np.unique sorted + argmax: a tie keeps 0 (:151-152)
     if (!s_dup[grp]) {
-      // Every ID sits on exactly one row: the multipos clean-up (:161-181) cannot drop anything, a vertex is
+      // Every ID sits on exactly one row, so at one read position (rows of different IDs may share one): the
+      // multipos clean-up (:161-181) cannot drop anything, a vertex is
       // a row, and what pass C would derive follows from the first partners found in pass AB -- presence
       // = degree > 0, first appearance in the edge list = the earlier of (r, first right partner) as a
       // source and (first left partner, r) as a target, first label = smallest neighbour or itself.
@@ -339,43 +346,66 @@ __global__ void __launch_bounds__(NT* GROUPS) k_validate(const ValParams V) {
           w.deg[r] = w.label[r];
           w.key[r] = w.ct[r];
         }
-        w.ct[r] = NOT64;
       }
       gsync();
-      // ---- multipos (:161-181): IDs seen at more than one read position keep their most frequent one ----
+      // ---- multipos (:161-181) counts (ID, read position) pairs, not rows: rows that share both (a read name
+      //      merged from two chunk files) are one entry whose count sums their edge ends and whose first
+      //      appearance is the earliest of theirs.  label / ct hold these per row until pass C. ----
       for (u32 r = tid; r < m; r += NT) {
-        const u32 id = w.ID[r], dr = w.deg[r];
-        const u64 kr = w.key[r];
-        u32 first = r, multi = 0, good = dr > 0;
+        const u32 id = w.ID[r], pr = w.P[r];
+        u32 c = 0;
+        u64 k = NOT64;
         for (u32 q = 0; q < m; q++) {
-          u32 same = (w.ID[q] == id);
-          u32 dq = w.deg[q];
+          const u32 same = (w.ID[q] == id) & (w.P[q] == pr), dq = w.deg[q];
+          const u64 kq = w.key[q];
+          c += same ? dq : 0u;
+          k = (same && dq && kq < k) ? kq : k;
+        }
+        w.label[r] = c;
+        w.ct[r] = k;
+      }
+      gsync();
+      // ---- multipos: an ID seen at more than one read position keeps the one with the most edge ends (ties:
+      //      first appearance); uP (dead in this path) holds that good position for every row of the ID ----
+      for (u32 r = tid; r < m; r += NT) {
+        const u32 id = w.ID[r];
+        u32 first = r, tot = 0, bc = 0, bp = 0;
+        u64 bk = NOT64;
+        for (u32 q = 0; q < m; q++) {
+          const u32 same = (w.ID[q] == id);
+          const u32 cq = w.label[q];
+          const u64 kq = w.ct[q];
           first = (same & (q < first)) ? q : first;
-          u32 other = same & (q != r) & (dq > 0);
-          multi |= other;
-          u32 beats = other & ((dq > dr) | ((dq == dr) & (w.key[q] < kr)));
-          good &= beats ^ 1u;
+          tot += same ? w.deg[q] : 0u;  // edge ends of the ID over all its rows
+          const u32 beats = same & (cq > 0) & ((cq > bc) | ((cq == bc) & (kq < bk)));
+          bc = beats ? cq : bc;
+          bk = beats ? kq : bk;
+          bp = beats ? w.P[q] : bp;
         }
         w.rep[r] = first;
-        w.flags[r] = ((multi & (dr > 0)) ? F_MULTI : 0u) | (good ? F_GOOD : 0u);
+        w.uP[r] = bp;
+        // more edge ends than its good position holds: the ID sits at another position too
+        w.flags[r] = (tot > bc ? F_MULTI : 0u) | ((bc > 0 && w.P[r] == bp) ? F_GOOD : 0u);
       }
       gsync();
       // ---- pass C: surviving edges (:189-192): presence, first appearance, first label ----
-      // edge (lo, hi) is dropped iff the LEFT row's ID is multi-positioned, lo is not that ID's good row and
-      // hi is not that ID's good row either (left end only: Q14)
+      // edge (lo, hi) is dropped iff the LEFT row's ID is multi-positioned, lo is off that ID's good position and
+      // hi is at another read position too, whatever hi's ID (left end only: Q14)
       {
         u32 nk = 0;
         for (u32 r = tid; r < m; r += NT) {
-          const u32 pr = w.P[r], sr = w.S[r], idr = w.ID[r], fr = w.flags[r];
+          const u32 pr = w.P[r], sr = w.S[r], fr = w.flags[r], gr = w.uP[r];
+          w.ct[r] = NOT64;  // (no longer read: the component pass below takes minima into it)
           u64 tmin = NOT64;
           u32 lab = NOV;
           for (u32 q = 0; q < m; q++) {
-            u32 pq = w.P[q], sq = w.S[q], idq = w.ID[q], fq = w.flags[q];
+            u32 pq = w.P[q], sq = w.S[q], fq = w.flags[q];
             u32 hi = q > r;
             u32 sg = hi ? (pr > pq) : (pq > pr);
             u32 e = pair_ok(pr, sr, pq, sq) & (q != r) & (sg == orient);
-            u32 fl = hi ? fr : fq, fh = hi ? fq : fr;  // flags of the left / right row of the pair
-            u32 drop = ((fl & F_MULTI) != 0) & ((fl & F_GOOD) == 0) & (((fh & F_GOOD) == 0) | (idq != idr));
+            u32 fl = hi ? fr : fq;                                // flags of the left row of the pair
+            u32 gl = hi ? gr : w.uP[q], ph = hi ? pq : pr;        // its ID's good position, right row's position
+            u32 drop = ((fl & F_MULTI) != 0) & ((fl & F_GOOD) == 0) & (ph != gl);
             u32 kept = e & (drop ^ 1u);
             u32 lo_row = hi ? r : q, hi_row = hi ? q : r;
             u64 et = 2 * ((u64)lo_row * m + hi_row) + (hi ^ 1u);  // source before target
@@ -427,7 +457,7 @@ __global__ void __launch_bounds__(NT* GROUPS) k_validate(const ValParams V) {
       for (u32 r = tid; r < m; r += NT) {
         const u32 fr = w.flags[r];
         if (!(fr & F_PRES)) continue;
-        const u32 pr = w.P[r], sr = w.S[r], idr = w.ID[r];
+        const u32 pr = w.P[r], sr = w.S[r], idr = w.ID[r], gr = w.uP[r];
         u32 lab = w.label[r];
         const u32 lab0 = lab;
         for (u32 q = 0; q < m; q++) {
@@ -435,8 +465,8 @@ __global__ void __launch_bounds__(NT* GROUPS) k_validate(const ValParams V) {
           u32 hi = q > r;
           u32 sg = hi ? (pr > pq) : (pq > pr);
           u32 e = pair_ok(pr, sr, pq, sq) & (q != r) & (sg == orient);
-          u32 fl = hi ? fr : fq, fh = hi ? fq : fr;
-          u32 drop = ((fl & F_MULTI) != 0) & ((fl & F_GOOD) == 0) & (((fh & F_GOOD) == 0) | (idq != idr));
+          u32 fl = hi ? fr : fq;
+          u32 drop = ((fl & F_MULTI) != 0) && ((fl & F_GOOD) == 0) && ((hi ? pq : pr) != (hi ? gr : w.uP[q]));  // as in pass C
           u32 link = (e & (drop ^ 1u)) | ((idq == idr) & ((fq & F_PRES) != 0));  // edge, or same vertex
           u32 lq = w.label[q];  // may already be this round's value: only speeds convergence up
           lab = (link && lq < lab) ? lq : lab;
@@ -662,5 +692,15 @@ extern "C" int gvs_pairs_get(gvs_ctx* ctx, uint32_t* read_idx, uint32_t* contig,
   if (group) CK(cudaMemcpyAsync(group, ctx->pair_group.p, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
   if (group_index) CK(cudaMemcpyAsync(group_index, ctx->pair_gidx.p, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
+  return 0;
+}
+
+extern "C" int gvs_validate_stats(gvs_ctx* ctx, uint64_t* n_empty) {
+  if (!ctx || !n_empty) return GVS_E_ARG;
+  if (!ctx->val_ready) return gvs_fail(ctx, GVS_E_STATE, "gvs_validate_stats before gvs_validate");
+  CK(cudaSetDevice(ctx->device));
+  u32 v = 0;
+  if (ctx->kept.n) CKR(read_dev(ctx, counter(ctx, CNT_VAL_STATS), &v));  // (no rows: gvs_validate left the counter alone)
+  *n_empty = v;
   return 0;
 }

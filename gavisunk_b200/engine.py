@@ -547,6 +547,12 @@ class Engine:
         self.n_pairs = int(n.value)
         return self.n_pairs
 
+    def validate_empty_reads(self) -> int:
+        """reads of the last validate() whose multipos clean-up dropped every oriented edge (they validate nothing)"""
+        n = C.c_uint64()
+        self._ck(self.lib.gvs_validate_stats(self.ctx, C.byref(n)))
+        return int(n.value)
+
     PAIR_COLUMNS = ("read", "contig", "group", "gidx")
 
     def pairs(self, pinned: bool = False) -> Dict[str, np.ndarray]:

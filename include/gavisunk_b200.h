@@ -350,6 +350,9 @@ int gvs_batches_bind(gvs_ctx* ctx, uint64_t* n_rows, uint64_t* n_reads);
 int gvs_validate(gvs_ctx* ctx, uint32_t min_read_len, uint64_t* n_pairs);
 int gvs_pairs_get(gvs_ctx* ctx, uint32_t* read_idx, uint32_t* contig, uint32_t* group,
                   uint32_t* group_index);
+/* after gvs_validate: *n_empty = reads of the last validation whose multipos clean-up dropped every oriented edge
+ * (the reference would build an empty graph and raise there; such a read validates nothing). */
+int gvs_validate_stats(gvs_ctx* ctx, uint64_t* n_empty);
 
 /* process-by-contig_lowmem_AR.py:215-260 contig-wide components.  The union-find parent array
  * (n_groups uint32, index = group_index) is exposed so that several GPUs can merge their
