@@ -15,11 +15,14 @@
   python -m gavisunk_b200.cli fused --sample S --k K --hap1-asm .. --hap2-asm .. (--hap1-reads f.. --hap2-reads f.. | --reads f..)
                                     --outdir D [--devices 0,1,..] [--batch-files N] [--detailed] [--support-tracks]
                                     [--gap-evidence] [--junctions] [--discordance] [--read-haplotypes] [--inversions]
+                                    [--sunk-depth]
   python -m gavisunk_b200.cli support_tracks <sunkpos> <rlen> <bad_sunks.txt> <fai> <valid.bed> <out.reads.bed> <out.bedgraph> <out.tsv>
   python -m gavisunk_b200.cli gap_evidence <sunkpos> <rlen> <bad_sunks.txt> <fai> <valid.bed> <out.gaps.reads.tsv> <out.gaps.evidence.tsv>
   python -m gavisunk_b200.cli junctions <hapN_detailed.sunkpos> <hapN.rlen> <bad_sunks.txt> <fai1> <fai2> <out.junctions.reads.tsv> <out.junctions.tsv>
   python -m gavisunk_b200.cli discordance <sunkpos> <rlen> <bad_sunks.txt> <fai> <out.discordance.reads.tsv> <out.discordance.tsv> <out.discordance.bed>
   python -m gavisunk_b200.cli inversions <sunkpos> <rlen> <bad_sunks.txt> <fai> <out.inversions.reads.tsv> <out.inversions.bed>
+  python -m gavisunk_b200.cli sunk_depth <kmer.loc> <fai1> <fai2> <bad_sunks.txt> <hap1_detailed.sunkpos> <hap2_detailed.sunkpos>
+                                         <hap1.sunkpos> <hap2.sunkpos> <hapN> <out.depth.bedgraph> <out.depth.bed> <out.depth.tsv>
 
 The first four replace workflow/scripts/{kmerpos_annot3,rlen,diag_filter_v3,diag_filter_step2}
 (workflow/rules/tagONT.smk:36,73,92,110) one to one; the next six replace badsunks_AR.py,
@@ -40,6 +43,8 @@ takes unbinned chunk files and keeps each read's rows on the haplotype its votes
 reference needs the reads binned by haplotype).
 `fused --inversions` and `inversions` report the reads whose SUNKs switch strand inside a contig, and cluster them into
 inversion calls (no reference counterpart: the validation takes each read's orientation majority).
+`fused --sunk-depth` and `sunk_depth` report the SUNK hits and reads of every group over all match rows, and call them into
+collapsed and depleted stretches (no reference counterpart: the bad-SUNK filter removes collapsed groups).
 Text parsing / formatting is host
 plumbing; all per-base and per-row work runs in libgavisunk_b200.so.  Errors exit non-zero with a
 message on stderr and never leave a partial output file behind.
@@ -50,7 +55,7 @@ import argparse
 import os
 import sys
 from collections import defaultdict
-from typing import Dict, List, NamedTuple, Sequence, Tuple
+from typing import Dict, List, NamedTuple, Optional, Sequence, Tuple
 
 import numpy as np
 
@@ -734,6 +739,159 @@ def cmd_inversions(argv):
 
 
 # ------------------------------------------------------------------------------------------------
+# SUNK hit depth: how many copies the reads say each group has (no reference counterpart; DESIGN.md section 5.5g)
+# ------------------------------------------------------------------------------------------------
+DEPTH_TSV_HEADER = "class\tmin_sunks\tmax_sunks\tgroups\thit_groups\tbaseline\tfallback\n"
+DEPTH_CLASSES = 6              # size classes min(5, floor(log2(sunks)))
+DEPTH_MIN_CLASS_GROUPS = 100   # groups with a hit that a class needs for a baseline of its own
+
+
+def depth_classes(sunks) -> np.ndarray:
+    """size class min(5, floor(log2(sunks))) of every group (class 0 for a group without .loc rows)"""
+    return np.searchsorted(np.array([2, 4, 8, 16, 32], np.int64), np.asarray(sunks, np.int64), side="right")
+
+
+def depth_baselines(hits, cls, sel, min_class_groups=DEPTH_MIN_CLASS_GROUPS):
+    """Per size class of the groups `sel` of one haplotype: (groups, hit groups, baseline, fallback).  The baseline is the
+    lower median of hits over the class's groups with hits >= 1, or over those of all classes (fallback) when the class has
+    fewer than min_class_groups; None for every class when no group of sel has a hit."""
+    h, c = np.asarray(hits, np.int64)[sel], np.asarray(cls)[sel]
+    hit = h >= 1
+    lower_median = lambda v: int(np.sort(v)[(len(v) - 1) // 2])
+    every = lower_median(h[hit]) if hit.any() else None
+    out = []
+    for q in range(DEPTH_CLASSES):
+        m = c == q
+        hq = h[m & hit]
+        fallback = len(hq) < min_class_groups
+        out.append((int(m.sum()), len(hq), every if (fallback or every is None) else lower_median(hq), fallback))
+    return out
+
+
+def depth_calls(g_contig, g_start, hits, reads, sunks, bad, hap_contigs, contig_len, high_permille=1750, low_permille=250,
+                max_gap_groups=2, min_groups=5, min_class_groups=DEPTH_MIN_CLASS_GROUPS):
+    """Collapsed and depleted stretches of one haplotype from the per-group SUNK hit depth (Engine.depth(): g_contig /
+    g_start = the group table, hits, reads, sunks; bad = group indices of the bad list), exact integer arithmetic.
+    hap_contigs = the haplotype's contig ids in .fai order.  With B = the baseline of the group's size class
+    (depth_baselines), a group is high when 1000*hits >= high_permille*B and low when 1000*hits <= low_permille*B.  Per
+    contig and state, the groups of that state in start order chain when at most max_gap_groups groups lie between
+    consecutive ones; a chain of >= min_groups marked groups is a call (`collapse` for high, `depleted` for low): start =
+    its first marked group's start, end = the start of the group after its last marked one (the contig length when there
+    is none), groups = groups from the first to the last marked one, ratio = lower median of floor(1000*hits/B) over the
+    marked groups, copies = (ratio + 500) // 1000, tandem = 2*sum(hits) >= 3*sum(reads) over them (collapses only),
+    bad = marked groups in the bad list.  -> (calls sorted by (contig in .fai order, start, end, kind): tuples (contig,
+    start, end, kind, groups, marked, ratio, copies, tandem or None, bad), depth_baselines of the haplotype)"""
+    g_contig = np.asarray(g_contig, np.int64)
+    g_start = np.asarray(g_start, np.int64)
+    hap_contigs = np.asarray(hap_contigs, np.int64)
+    fai_pos = np.full(int(max(g_contig.max(initial=-1), hap_contigs.max(initial=-1))) + 1, -1, np.int64)
+    fai_pos[hap_contigs] = np.arange(len(hap_contigs))
+    sel = np.flatnonzero(fai_pos[g_contig] >= 0)
+    cls = depth_classes(sunks)
+    base = depth_baselines(hits, cls, sel, min_class_groups)
+    if base[0][2] is None:
+        return [], base
+    order = sel[np.lexsort((g_start[sel], fai_pos[g_contig[sel]]))]
+    B = np.asarray([b[2] for b in base], np.int64)[cls[order]]
+    h = np.asarray(hits, np.int64)[order]
+    rd = np.asarray(reads, np.int64)[order]
+    c = g_contig[order]
+    is_bad = np.zeros(len(g_contig), bool)
+    is_bad[np.asarray(bad, np.int64)] = True
+    calls = []
+    for kind, marked in (("collapse", 1000 * h >= high_permille * B), ("depleted", 1000 * h <= low_permille * B)):
+        p = np.flatnonzero(marked)
+        head = np.ones(len(p), bool)
+        head[1:] = (c[p[1:]] != c[p[:-1]]) | (p[1:] - p[:-1] - 1 > max_gap_groups)
+        heads = np.flatnonzero(head)
+        for a, b in zip(heads.tolist(), np.append(heads[1:], len(p)).tolist()):
+            m = p[a:b]
+            if len(m) < min_groups:
+                continue
+            first, last = int(m[0]), int(m[-1])
+            ci = int(c[first])
+            end = int(g_start[order[last + 1]]) if last + 1 < len(order) and c[last + 1] == ci else int(contig_len[ci])
+            ratio = int(np.sort(1000 * h[m] // B[m])[(len(m) - 1) // 2])
+            tandem = int(2 * h[m].sum() >= 3 * rd[m].sum()) if kind == "collapse" else None
+            calls.append((ci, int(g_start[order[first]]), end, kind, last - first + 1, len(m), ratio, (ratio + 500) // 1000, tandem,
+                          int(is_bad[order[m]].sum())))
+    calls.sort(key=lambda t: (int(fai_pos[t[0]]), t[1], t[2], t[3]))
+    return calls, base
+
+
+def depth_texts(hap_contigs, names, contig_len, groups, dp, runs, bad):
+    """The three SUNK-depth files of one haplotype: hap_contigs = its contig ids in .fai order; groups = Engine.groups(),
+    dp = Engine.depth(), runs = Engine.depth_runs(), bad = group indices of the bad list.  -> (depth.bedgraph: the runs of
+    its contigs; depth.bed: depth_calls; depth.tsv: the baseline of every size class) bytes"""
+    ctab = gio.NameTable(names)
+    inhap = np.zeros(len(names), bool)
+    inhap[np.asarray(hap_contigs, np.int64)] = True
+    bedgraph = gio.format_rows([("name", runs["contig"], ctab)] + [("u32", runs[c]) for c in ("start", "end", "hits", "reads", "kept")],
+                               sel=np.flatnonzero(inhap[runs["contig"]]))
+    calls, base = depth_calls(groups["contig"], groups["group"], dp["hits"], dp["reads"], dp["sunks"], bad, hap_contigs, contig_len)
+    bed = "".join(f"{names[c]}\t{a}\t{b}\t{kind}\t{ng}\t{nm}\t{ratio}\t{copies}\t{'.' if tandem is None else tandem}\t{nb}\n"
+                  for c, a, b, kind, ng, nm, ratio, copies, tandem, nb in calls)
+    out = [DEPTH_TSV_HEADER]
+    for q, (n, nh, b, fb) in enumerate(base):
+        out.append(f"{q}\t{1 << q}\t{(2 << q) - 1 if q + 1 < DEPTH_CLASSES else '.'}\t{n}\t{nh}\t{'.' if b is None else b}\t"
+                   f"{'.' if b is None else int(fb)}\n")
+    return bedgraph, bed.encode("latin-1"), "".join(out).encode("latin-1")
+
+
+def sunk_depth(loc_p, fai1_p, fai2_p, badsunks_p, detailed1_p, detailed2_p, sunkpos1_p, sunkpos2_p, hap, out_bedgraph, out_bed,
+               out_tsv):
+    """SUNK hit depth of haplotype `hap` (hap1 / hap2) from the files of the per-rule path: the group table and the SUNKs of
+    each group from mrsfast/kmer.loc (identical rows, as mrsfast writes a palindromic SUNK, taken once); hits and reads from
+    both {hap}_detailed.sunkpos (combine_ont_nofilt: every match row; a read is a run of consecutive rows with one name,
+    diag_filter_v3.nim:64); kept from both {hap}.sunkpos, as badsunks_AR.py counts them; bad groups from bad_sunks.txt;
+    contigs in fai1-then-fai2 order."""
+    h = {"hap1": 0, "hap2": 1, "1": 0, "2": 1}.get(str(hap))
+    if h is None:
+        raise ValueError(f"haplotype {hap!r} is not hap1 or hap2")
+    fai = [gio.read_fai(fai1_p), gio.read_fai(fai2_p)]
+    names = [n for f in fai for n, _ in f]
+    clen = [l for f in fai for _, l in f]
+    cidx = {}
+    for i, n in enumerate(names):
+        cidx.setdefault(n, i)
+    badset = _read_badsunks(badsunks_p)
+    loc = list(dict.fromkeys(zip(*gio.read_loc(loc_p))))
+    for c, _, _, _ in loc:
+        if c not in cidx:
+            raise KeyError(f"contig {c} of {loc_p} is in neither {fai1_p} nor {fai2_p}")
+    parts = {}
+    for key, paths in (("detailed", (detailed1_p, detailed2_p)), ("kept", (sunkpos1_p, sunkpos2_p))):
+        cols, r0 = [], 0
+        for path in paths:
+            _, cnames, rnames, c = _rows_from_sunkpos(path)
+            for n in cnames:
+                if n not in cidx:
+                    raise KeyError(f"contig {n} of {path} is in neither {fai1_p} nor {fai2_p}")
+            remap = np.asarray([cidx[n] for n in cnames] + [0], np.uint32)
+            cols.append((c[0] + np.uint32(r0), c[1], remap[c[2]], c[3], c[4]))
+            r0 += len(rnames)
+        parts[key] = ([np.concatenate([t[j] for t in cols]) for j in range(5)], r0)
+    kmers = [km.encode() for _, _, km, _ in loc]
+    eng = Engine(len(kmers[0]) if kmers and 1 <= len(kmers[0]) <= 32 else 20)
+    km = encode_kmers(kmers)
+    eng.load_loc(km, km, [cidx[c] for c, _, _, _ in loc], [s for _, s, _, _ in loc], [g for _, _, _, g in loc], names)
+    eng.set_reads_meta(np.zeros(max(1, parts["detailed"][1], parts["kept"][1]), np.uint32))
+    eng.set_rows(0, *parts["detailed"][0])
+    eng.sunk_depth()
+    eng.set_rows(1, *parts["kept"][0])
+    eng.group_hist()
+    _set_bad(eng, badset, names)
+    chap = np.asarray([0] * len(fai[0]) + [1] * len(fai[1]))
+    texts = depth_texts(np.flatnonzero(chap == h).tolist(), names, clen, eng.groups(), eng.depth(), eng.depth_runs(clen),
+                        eng.bad_list())
+    _write_all((out_bedgraph, out_bed, out_tsv), texts)
+
+
+def cmd_sunk_depth(argv):
+    sunk_depth(*argv)
+
+
+# ------------------------------------------------------------------------------------------------
 # read haplotypes: every read's SUNK vote on both haplotypes (no reference counterpart; DESIGN.md section 5.5e)
 # ------------------------------------------------------------------------------------------------
 READ_HAP_READS_HEADER = "read\tread_len\tbin\tcontig1\tn1\tstrand1\tcontig2\tn2\tstrand2\thap\n"
@@ -1036,7 +1194,7 @@ class Evidence(NamedTuple):
     """An optional output of `fused` that the reference does not produce"""
     flag: str
     help: str
-    records: str                  # run_reads' result key of its per-engine records, concatenated run-wide
+    records: Optional[str]        # run_reads' result key of its per-engine records, concatenated run-wide (None: no records)
     columns: Tuple[str, ...]      # their columns
     suffixes: Tuple[str, ...]     # final_out/hap{N}.{suffix}, in the order its *_texts returns them
 
@@ -1059,6 +1217,9 @@ EVIDENCE_PRODUCTS = {
     "inversions": Evidence("--inversions", "also write final_out/hap{N}.inversions.reads.tsv and .inversions.bed (reads whose SUNKs "
                            "switch strand inside a contig, and inversion calls)", "switches", Engine.SWITCH_COLUMNS,
                            ("inversions.reads.tsv", "inversions.bed")),
+    "sunk_depth": Evidence("--sunk-depth", "also write final_out/hap{N}.depth.bedgraph, .depth.bed and .depth.tsv (SUNK hits and "
+                           "reads of every group over all match rows, and collapsed and depleted stretches)", None, (),
+                           ("depth.bedgraph", "depth.bed", "depth.tsv")),
 }
 
 
@@ -1112,9 +1273,10 @@ def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int]
     discordant spans of every engine's own reads and the discordance runs, with the difference arrays summed like the
     support's; read_haplotypes: every engine's diag filters in haplotype mode and the records of its own reads (file_hap
     GVS_HAP_ANY: unbinned chunks, always filtered in haplotype mode); inversions: the strand-switch records of every
-    engine's own reads, from its kept rows and the run's bad groups.  -> one result dict per engine (read names /
-    lengths / chunk tables, kept rows, validated pairs, intervals[, placements, support runs][, gap evidence][,
-    junctions][, spans, discordance runs][, read haplotypes][, strand switches])."""
+    engine's own reads, from its kept rows and the run's bad groups; sunk_depth: every batch's match rows counted per group
+    and the per-group counts and runs, with the counts summed across engines like the support's.  -> one result dict per
+    engine (read names / lengths / chunk tables, kept rows, validated pairs, intervals[, placements, support runs][, gap
+    evidence][, junctions][, spans, discordance runs][, read haplotypes][, strand switches][, depth, depth runs])."""
     import threading
     from concurrent.futures import ThreadPoolExecutor
     for p in files:
@@ -1169,7 +1331,8 @@ def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int]
                         info["rows0"].append(r0)
                 iv, bases = eng.run_batches([bind_for(bi) for bi in range(len(mine))], contig_hap, min_read_len=min_read_len,
                                             allreduce_hist=cx.allreduce_hist, gather_forests=cx.gather_forests, on_batch=on_batch,
-                                            junctions="junctions" in products, read_haps="read_haplotypes" in products)
+                                            junctions="junctions" in products, read_haps="read_haplotypes" in products,
+                                            sunk_depth="sunk_depth" in products)
                 for old in held:
                     old.close()
             info.update(kept=eng.rows(1, pinned=True), pairs=eng.pairs(pinned=True), iv=iv)
@@ -1186,6 +1349,8 @@ def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int]
                 info.update(read_haps=eng.read_haps() if mine else {c: np.zeros(0, np.uint32) for c in Engine.READ_HAP_COLUMNS})
             if "inversions" in products:
                 info.update(switches=eng.strand_switches(min_read_len))
+            if "sunk_depth" in products:
+                info.update(depth=eng.depth(allreduce=cx.allreduce_hist), depth_runs=eng.depth_runs(contig_len))
             results[di] = info
         except BaseException as ex:  # noqa: BLE001 -- reported by the caller; peers must not wait for this rank
             errors.append(ex)
@@ -1358,7 +1523,8 @@ def write_outputs(k, eng, results, contig_len, contig_hap, names, iv, gaps, noda
     kept_c = by_contig(kept["contig"], kept["read"])
     # a read lives on one engine: the evidence records of all engines, read indices made run-wide (runs are the same on
     # every engine)
-    rec = {p: cat_rows(EVIDENCE_PRODUCTS[p].records, EVIDENCE_PRODUCTS[p].columns) for p in products}
+    rec = {p: cat_rows(EVIDENCE_PRODUCTS[p].records, EVIDENCE_PRODUCTS[p].columns) if EVIDENCE_PRODUCTS[p].records else None
+           for p in products}
     pair_c = by_contig(pairs["contig"], pairs["read"], name_rank)  # reads in name order, pairs of a read in vertex order
     if db_files:
         loc_c = by_contig(db["contig"])
@@ -1400,7 +1566,8 @@ def write_outputs(k, eng, results, contig_len, contig_hap, names, iv, gaps, noda
             junctions=lambda r: junction_texts(r, np.flatnonzero(read_hap[r["read"]] == hap), names, clen, contig_hap, *reads),
             discordance=lambda r: discordance_texts(hap_contigs, names, r, results[0]["discordance"], *reads),
             read_haplotypes=lambda r: read_hap_texts(hap, names, chap, r, read_bin, read_hap, *reads),
-            inversions=lambda r: inversion_texts(hap_contigs, names, r, *reads))
+            inversions=lambda r: inversion_texts(hap_contigs, names, r, *reads),
+            sunk_depth=lambda r: depth_texts(hap_contigs, names, clen, gtab, results[0]["depth"], results[0]["depth_runs"], bad))
         for p in products:
             _write_all([d("final_out", f"hap{hn}.{ext}") for ext in EVIDENCE_PRODUCTS[p].suffixes], texts[p](rec[p]))
     from concurrent.futures import ThreadPoolExecutor
@@ -1450,7 +1617,8 @@ COMMANDS = {"kmerpos_annot3": (cmd_kmerpos_annot3, 4), "rlen": (cmd_rlen, 2), "d
             "covprob": (cmd_covprob, None), "split_locs": (cmd_split_locs, None), "fused": (cmd_fused, None),
             "split_ont": (cmd_split_ont, None), "combine_ont_nofilt": (cmd_combine_ont_nofilt, None),
             "support_tracks": (cmd_support_tracks, 8), "gap_evidence": (cmd_gap_evidence, 7),
-            "junctions": (cmd_junctions, 7), "discordance": (cmd_discordance, 7), "inversions": (cmd_inversions, 6)}
+            "junctions": (cmd_junctions, 7), "discordance": (cmd_discordance, 7), "inversions": (cmd_inversions, 6),
+            "sunk_depth": (cmd_sunk_depth, 12)}
 
 
 def main(argv=None):

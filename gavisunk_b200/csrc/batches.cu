@@ -89,6 +89,7 @@ extern "C" int gvs_batches_begin(gvs_ctx* ctx) {
   ctx->jn_in_run = true;
   ctx->rh_run.n = 0;
   ctx->rh_run.ready = false;
+  ctx->dp_ready = false;  // the next gvs_sunk_depth(accumulate = 1) starts from zero (depth.cu)
   return 0;
 }
 

@@ -206,6 +206,15 @@ struct gvs_ctx {
                                         // scratch (7 u32 arrays + 1 byte); per segment records
   RecTable sw;                      // records: 16 columns
 
+  // ---- SUNK hit depth (depth.cu) ----
+  DevBuf dp_cnt;                    // int32[2][n_groups] by group index: hits, reads (summed over the batches of a run)
+  DevBuf dp_seg_start, dp_row_seg, dp_scr;  // segments of the match rows; per match row scratch of the non-monotone reads
+  DevBuf dp_sunks;                  // u32[n_groups]: .loc rows per group
+  DevBuf dp_diff;                   // int32[3][n_groups] by rank: differences of hits, reads, kept
+  u64 dp_gen = 0, dp_sunks_gen = ~0ull;  // grp_gen dp_cnt / dp_sunks were counted for
+  bool dp_ready = false;
+  RecTable dp_runs;                 // runs of gvs_depth_runs: contig, start, end, hits, reads, kept
+
   // ---- components / intervals / gaps ----
   DevBuf parent, present, comp_min, comp_max, comp_cnt;
   DevBuf comp_rank;  // unsorted group tables only: [smallest member rank per root | root per interval rank]
@@ -649,6 +658,32 @@ __device__ __forceinline__ bool warp_first_in(const u32* idx, u32 a, u32 i, In i
     if (id(j) == g) return false;
   }
   return true;
+}
+
+// Order the n keys key(x[k]) ascending into y: a copy or a reversal when they are strictly monotone (a one-strand read),
+// else a rank sort.  One warp.  Distinct keys fill y; equal keys all land on the slot of their rank, leaving the slots
+// after it unwritten (the SUNK hit depth counts distinct groups that way).  Discordance orders validated IDs and usable
+// rows with it.
+template <typename K>
+__device__ __forceinline__ void warp_order(const u32* x, u32* y, u32 n, K key, int lane) {
+  bool up = true, down = true;
+  for (u32 k = lane; k + 1 < n; k += 32) {
+    const u64 k0 = key(x[k]), k1 = key(x[k + 1]);
+    up &= k0 < k1;
+    down &= k0 > k1;
+  }
+  up = __all_sync(0xFFFFFFFFu, up);
+  down = __all_sync(0xFFFFFFFFu, down);
+  for (u32 k = lane; k < n; k += 32) {
+    u32 r = up ? k : n - 1 - k;
+    if (!up && !down) {
+      const u64 kk = key(x[k]);
+      r = 0;
+      for (u32 j = 0; j < n; j++) r += key(x[j]) < kk;
+    }
+    y[r] = x[k];
+  }
+  __syncwarp();
 }
 
 // read lengths: explicit (gvs_reads_meta, a batches run) or from the offsets of the batch, clamped to 32 bits

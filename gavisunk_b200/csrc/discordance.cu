@@ -40,30 +40,6 @@ __device__ __forceinline__ u32 dc_find(const DcParams& P, const u32* vid, u32 c,
   return l < c && vid[l] == id ? l : DC_NONE;
 }
 
-// Order the n distinct keys key(x[k]) ascending into y: a copy or a reversal when they are monotone (a one-strand read),
-// else a rank sort.  One warp.
-template <typename K>
-__device__ __forceinline__ void dc_order(const u32* x, u32* y, u32 n, K key, int lane) {
-  bool up = true, down = true;
-  for (u32 k = lane; k + 1 < n; k += 32) {
-    const u64 k0 = key(x[k]), k1 = key(x[k + 1]);
-    up &= k0 < k1;
-    down &= k0 > k1;
-  }
-  up = __all_sync(0xFFFFFFFFu, up);
-  down = __all_sync(0xFFFFFFFFu, down);
-  for (u32 k = lane; k < n; k += 32) {
-    u32 r = up ? k : n - 1 - k;
-    if (!up && !down) {
-      const u64 kk = key(x[k]);
-      r = 0;
-      for (u32 j = 0; j < n; j++) r += key(x[j]) < kk;
-    }
-    y[r] = x[k];
-  }
-  __syncwarp();
-}
-
 __global__ void __launch_bounds__(256) k_dc_spans(const DcParams P) {
   const u32 s = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
@@ -74,7 +50,7 @@ __global__ void __launch_bounds__(256) k_dc_spans(const DcParams P) {
   if (c >= 2) {
     u32 *vid = P.vid + a, *cnt = P.cnt + a;
     // validated IDs in ascending order (gvs_validate lists them in vertex order: usually row order, so monotone)
-    dc_order(P.val_id + a, vid, c, [](u32 id) -> u64 { return id; }, lane);
+    warp_order(P.val_id + a, vid, c, [](u32 id) -> u64 { return id; }, lane);
     for (u32 j = lane; j < c; j += 32) cnt[j] = 0;
     __syncwarp();
     const u32 c0 = P.contig[a];
@@ -100,7 +76,7 @@ __global__ void __launch_bounds__(256) k_dc_spans(const DcParams P) {
     if (nu >= 2) {
       u32* srt = P.sidx + a;
       const u32 *st = P.start, *gr = P.group;
-      dc_order(u, srt, nu, [st, gr](u32 i) -> u64 { return ((u64)st[i] << 32) | gr[i]; }, lane);
+      warp_order(u, srt, nu, [st, gr](u32 i) -> u64 { return ((u64)st[i] << 32) | gr[i]; }, lane);
       // spans (srt[k], srt[k+1]); their classes go to u[k] (the row-order copy is dead)
       for (u32 k = lane; k + 1 < nu; k += 32) {
         const u32 i = srt[k], j = srt[k + 1];

@@ -457,7 +457,8 @@ class Engine:
         return self.n_kept, self.n_reads
 
     def run_batches(self, binds, contig_hap: Sequence[int], min_read_len: int = 10000, allreduce_hist=None,
-                    gather_forests=None, on_batch=None, junctions: bool = False, read_haps: bool = False):
+                    gather_forests=None, on_batch=None, junctions: bool = False, read_haps: bool = False,
+                    sunk_depth: bool = False):
         """The hot path over a run whose reads come in several batches (a sample's chunk files, or the shard of
         them this GPU owns).  The reference gathers all chunks of a haplotype before the global stages
         (workflow/Snakefile:23-24, workflow/rules/tagONT.smk:112-131; badsunks_AR.py:20-27 counts over every
@@ -470,7 +471,8 @@ class Engine:
         Results equal run_all() on the concatenation of the batches; read indices of rows(1) / pairs() count
         through the batches in order.  junctions: also screen every batch after its diag filter (junction_screen),
         so that junctions() reports the run's records afterwards.  read_haps: run every diag filter in haplotype mode,
-        so that read_haps() reports the run's records afterwards (batches with GVS_HAP_ANY chunks always are).
+        so that read_haps() reports the run's records afterwards (batches with GVS_HAP_ANY chunks always are).  sunk_depth:
+        also count every batch's match rows (sunk_depth, accumulated), so that depth() reports the run's SUNK hit depth.
         Returns (intervals, [read_base of every batch])."""
         self.batches_begin()
         bases, hp = [], 0
@@ -478,6 +480,8 @@ class Engine:
         for b, bind in enumerate(binds):
             bind(self)
             rows += self.match()
+            if sunk_depth:
+                self.sunk_depth(accumulate=True)
             best += self.diag_filter(contig_hap, read_haps)[0]
             if junctions:
                 self.junction_screen(min_read_len)
@@ -488,9 +492,11 @@ class Engine:
             bases.append(base)
         self.batches_bind()
         self.n_rows, self.n_best = rows, best
-        if not bases:  # a rank without a batch still takes part in both exchanges
+        if not bases:  # a rank without a batch still takes part in both exchanges (and in depth()'s)
             self.set_contigs(contig_hap)
             hp = self.group_hist(accumulate=True)
+            if sunk_depth:
+                self.sunk_depth(accumulate=True)
         return self._global_stages(hp, min_read_len, allreduce_hist, gather_forests), bases
 
     def db_groups(self) -> int:
@@ -599,6 +605,43 @@ class Engine:
         callable that sums the bad-SUNK histogram)."""
         return self._runs("discordance", self.lib.gvs_discordance, self.lib.gvs_discordance_get, self.DISCORDANCE_COLUMNS,
                           "_dc_diff_ptr", contig_len, allreduce)
+
+    def sunk_depth(self, accumulate: bool = False) -> int:
+        """SUNK hit depth of the current match rows (after match() or set_rows(0); no reference counterpart;
+        include/gavisunk_b200.h gvs_sunk_depth): adds every row to hits[g] and every distinct (read, group) to reads[g].
+        accumulate: add to the previous counts (run_batches starts from zero at its batches_begin).  Returns the device
+        pointer of the int32[2][n_groups] array."""
+        p = C.c_void_p()
+        self._ck(self.lib.gvs_sunk_depth(self.ctx, 1 if accumulate else 0, C.byref(p)))
+        self._dp_ptr = int(p.value or 0)
+        self._dp_summed = False
+        return self._dp_ptr
+
+    def _n_groups(self) -> int:
+        n = C.c_uint64()
+        self._ck(self.lib.gvs_groups_count(self.ctx, C.byref(n)))
+        return int(n.value)
+
+    def depth(self, allreduce=None) -> Dict[str, np.ndarray]:
+        """Per group index (the table of groups()): hits, reads (int32, of sunk_depth), sunks (.loc rows) and kept (the
+        int32 histogram of group_hist).  With several GPUs `allreduce(ptr, n)` sums the hits and reads (n = 2 * n_groups)
+        across ranks in place first (the callable that sums the bad-SUNK histogram), once per sunk_depth(): a later call
+        reads the counts summed already."""
+        ng = self._n_groups()
+        if allreduce is not None and not getattr(self, "_dp_summed", False):
+            allreduce(self._dp_ptr, 2 * ng)
+            self._dp_summed = True
+        out = self._table("depth", self.lib.gvs_sunk_depth_get, ng, ("hits", "reads", "sunks"), dtypes=dict(hits=np.int32, reads=np.int32))
+        out["kept"] = self.groups(with_hist=True)["count"]
+        return out
+
+    DEPTH_COLUMNS = ("contig", "start", "end", "hits", "reads", "kept")
+
+    def depth_runs(self, contig_len: Sequence[int]) -> Dict[str, np.ndarray]:
+        """SUNK hit depth runs after sunk_depth() (and depth()'s all-reduce) and group_hist(): (contig, start, end, hits,
+        reads, kept) tiling every contig in segment space."""
+        return self._runs("depth_runs", self.lib.gvs_depth_runs, self.lib.gvs_depth_runs_get, self.DEPTH_COLUMNS, "_dp_ptr",
+                          contig_len, None)
 
     def components_local(self) -> int:
         """this GPU's forest of the validated pairs; returns the device pointer of its uint32[n_groups] parent array"""

@@ -63,7 +63,8 @@ enum {
   GVS_ST_DISCORDANCE = 15, /* distance discordance (gvs_spans, gvs_discordance): no reference counterpart */
   GVS_ST_READHAPS = 16, /* haplotype mode of the diag filter (gvs_diag_filter_haps): votes per haplotype, records */
   GVS_ST_SWITCHES = 17, /* strand switches inside a contig (gvs_strand_switches): no reference counterpart       */
-  GVS_ST_COUNT = 18
+  GVS_ST_DEPTH = 18,    /* SUNK hit depth (gvs_sunk_depth, gvs_depth_runs): no reference counterpart                */
+  GVS_ST_COUNT = 19
 };
 
 /* ------------------------------------------------------------------------------------------ */
@@ -500,6 +501,33 @@ int gvs_strand_switches(gvs_ctx* ctx, uint32_t min_read_len, uint64_t* n_records
 int gvs_strand_switches_get(gvs_ctx* ctx, uint32_t* read, uint32_t* contig, uint32_t* strand1, uint32_t* ids1, uint32_t* lo1,
                             uint32_t* hi1, uint32_t* id1, uint32_t* start1, uint32_t* pos1, uint32_t* strand2, uint32_t* ids2,
                             uint32_t* lo2, uint32_t* hi2, uint32_t* id2, uint32_t* start2, uint32_t* pos2);
+
+/* SUNK hit depth: how many copies the reads say each SUNK group has.  No reference counterpart: badsunks_AR.py removes the
+ * groups with too many kept rows (a collapse of c genomic copies gives its SUNKs about c times the hits) and validation
+ * then reports a gap there.  Per group index g (the group table of gvs_db_export / gvs_groups_get):
+ *   hits[g]   the match rows of gvs_match / gvs_rows_set(0) with group g: every contig of both haplotypes, every read, no
+ *             read-length minimum, no bad-group filter (the rows of combine_ont_nofilt, before the diag filter keeps one
+ *             contig per read: reads from a collapsed copy elsewhere often have their best contig elsewhere);
+ *   reads[g]  the distinct read records among those rows: a read counts once per group however often it re-enters it;
+ *   kept[g]   the histogram of gvs_group_hist (kept rows per group, summed over ranks);
+ *   sunks[g]  the .loc rows of group g.
+ * An interspersed collapse (copies at other loci) raises hits and reads; a tandem collapse raises hits only (each read
+ * crosses the one assembled copy several times).
+ * gvs_sunk_depth adds the current match rows (none after gvs_batches_bind or before any gvs_match) to an int32[2][n_groups]
+ * array -- hits at [g], reads at [n_groups + g] -- whose device pointer *depth_dev receives.  Inside a batches run it
+ * accumulates from gvs_batches_begin on (accumulate != 0); accumulate = 0 replaces.  It writes no buffer of the other
+ * stages.  Several GPUs sum the 2*n_groups entries (as the histogram of gvs_group_hist; a read lives on one GPU, so the
+ * sums are exact) before gvs_sunk_depth_get / gvs_depth_runs.
+ * gvs_sunk_depth_get: host buffers of n_groups entries, any pointer may be NULL.
+ * gvs_depth_runs: per base x, the (hits, reads, kept) of x's segment [ID_r, ID_r+1) as runs (contig, start, end, hits, reads,
+ * kept) that tile [0, contig_len[c]) of every contig in (contig, start) order, maximal, with a zero head run before a
+ * contig's first group (as gvs_discordance tiles its counts).  GVS_E_STATE before gvs_group_hist or gvs_sunk_depth.
+ * The calls (collapsed and depleted stretches) are the caller's: DESIGN.md section 5.5g. */
+int gvs_sunk_depth(gvs_ctx* ctx, int accumulate, int32_t** depth_dev);
+int gvs_sunk_depth_get(gvs_ctx* ctx, int32_t* hits, int32_t* reads, uint32_t* sunks);
+int gvs_depth_runs(gvs_ctx* ctx, const uint32_t* contig_len, uint64_t* n_runs);
+int gvs_depth_runs_get(gvs_ctx* ctx, uint32_t* contig, uint32_t* start, uint32_t* end, uint32_t* hits, uint32_t* reads,
+                       uint32_t* kept);
 
 /* covprob.py:56-100: table[0..3499] of gap-spanning probabilities from the read-length
  * histogram.  kbp[n_bins], cnt[n_bins] = distinct int(len/1000) values and their multiplicities
