@@ -31,6 +31,7 @@ PROTOTYPES = {
     "gvs_db_load_loc": (C.c_int, [vp, vp, C.c_uint64, vp, vp, vp, vp, C.c_uint64, C.c_uint32]),
     "gvs_db_build": (C.c_int, [vp, vp, vp, C.c_uint32, C.c_int]),
     "gvs_set_probe_variant": (C.c_int, [vp, C.c_int]),
+    "gvs_set_db_passes": (C.c_int, [vp, C.c_int]),
     "gvs_db_size": (C.c_int, [vp, u64p, u64p]),
     "gvs_db_export": (C.c_int, [vp, vp, vp, vp, vp, vp]),
     "gvs_reads_set": (C.c_int, [vp, vp, vp, C.c_uint64, vp, vp, C.c_uint32, C.c_int]),

@@ -81,6 +81,7 @@ struct gvs_ctx {
   u64 filt_words = 0;                                            // number of 16-byte blocks, power of two
   bool filt_fp = false;                                          // block layout: word 3 = sub-mer fingerprints (gvs_fp_bit), keys in words 0..2
   int probe_variant = 0;                                         // gvs_set_probe_variant: 0 by size, 1 small-database, 2 large-database
+  int db_passes = 0;                                             // gvs_set_db_passes: 0 by free memory, else the count passes of gvs_db_build
   DevBuf filt1;                                                  // presence filter of the sub-mers (large databases)
   u64 filt1_words = 0;                                           // 0 = single-level filter
   DevBuf contig_hap, contig_hash, contig_len;

@@ -259,6 +259,13 @@ extern "C" int gvs_set_probe_variant(gvs_ctx* ctx, int variant) {
   return 0;
 }
 
+extern "C" int gvs_set_db_passes(gvs_ctx* ctx, int n) {
+  if (!ctx) return GVS_E_ARG;
+  if (n < 0 || n > 64) return gvs_fail(ctx, GVS_E_ARG, "database passes must be 0 (by free memory) or 1..64");
+  ctx->db_passes = n;
+  return 0;
+}
+
 extern "C" int gvs_set_host_pack(gvs_ctx* ctx, int mode, int threads) {
   if (!ctx) return GVS_E_ARG;
   if (mode < GVS_PACK_OFF || mode > GVS_PACK_ALTERNATE) return gvs_fail(ctx, GVS_E_ARG, "unknown host pack mode %d", mode);

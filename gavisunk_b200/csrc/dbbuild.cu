@@ -176,7 +176,7 @@ __global__ void __launch_bounds__(DT, DB_BLOCKS) k_db_count(const DbCountParams 
       f = ((f << 2) | b) & kmask;
       r = (r >> 2) | ((3 - b) << topsh);
       bool ok = (p0 + i < P.total) && (((B >> (i + 1)) & vmask) == 0) && (((I >> i) & imask) == 0);
-      if (ok && k < 32) {
+      if (ok) {
         u64 c = f < r ? f : r;
         u64 h = gvs_mix(c);
         if (P.n_parts == 1 || (u32)h % P.n_parts == P.part) {  // low hash bits pick the pass, high bits the bucket
@@ -245,7 +245,7 @@ __global__ void __launch_bounds__(256) k_db_rows(const u32* __restrict__ bitmap,
     loc_kmer[row] = f < r ? f : r;
     loc_contig[row] = c;
     loc_start[row] = (u32)(p - cstart);
-    // SUNKs in [max(p-k, cstart), p-1]?  (k <= 31 positions back: inside `hist`)
+    // SUNKs in [max(p-k, cstart), p-1]?  (k <= 32 positions back: inside `hist`)
     u64 lowp = (p >= (u64)k && p - k > cstart) ? p - k : cstart;
     int span = (int)(p - lowp);  // 0..k
     u64 m = span ? (((1ull << span) - 1) << (32 + b - span)) : 0ull;
@@ -283,19 +283,20 @@ static int db_build_device(gvs_ctx* ctx, const u8* seq, const u64* contig_off, u
                            DevBuf& keys, DevBuf& vals, DevBuf& bitmap, DevBuf& wrank, DevBuf& head, DevBuf& hrow,
                            DevBuf& gex) {
   const int k = ctx->k;
-  u64 n_tiles = cdiv(total, DTILE);
+  u64 n_tiles = cdiv(total, DTILE);  // 0 when every contig is empty: no window, an empty database
   CKR(gvs_reserve(ctx, ctx->tile_first, n_tiles * 4));
-  LAUNCH(k_db_tile_index, (unsigned)cdiv(n_tiles, 256), 256, 0, contig_off, (u64)n_contigs, n_tiles, ctx->tile_first.as<u32>());
-  // count-table sizing: <= `total` distinct k-mers; load <= 2/3; P passes so that it fits
+  if (n_tiles)
+    LAUNCH(k_db_tile_index, (unsigned)cdiv(n_tiles, 256), 256, 0, contig_off, (u64)n_contigs, n_tiles, ctx->tile_first.as<u32>());
+  // count-table sizing: <= `total` distinct k-mers; load <= 2/3; P passes so that it fits (or as gvs_set_db_passes says)
   size_t free_b = 0, tot_b = 0;
   CK(cudaMemGetInfo(&free_b, &tot_b));
   u64 n_words = cdiv(total, 32) + 2;
   u64 budget = (u64)(free_b * 0.70) - n_words * 4;
-  u32 n_parts = 1;
+  u32 n_parts = ctx->db_passes ? (u32)ctx->db_passes : 1;
   u64 slots;
   for (;;) {
     slots = (((total / n_parts) * 3 / 2 + 1024) + 3) & ~3ull;  // load <= 2/3, whole buckets of 4
-    if (slots * 16 <= budget || n_parts >= 64) break;
+    if (ctx->db_passes || slots * 16 <= budget || n_parts >= 64) break;
     n_parts += 1;
   }
   if ((slots >> 2) >= (1ull << 32)) return gvs_fail(ctx, GVS_E_OVERFLOW, "SUNK count table has too many buckets");
@@ -313,7 +314,7 @@ static int db_build_device(gvs_ctx* ctx, const u8* seq, const u64* contig_off, u
     P.kv = keys.as<u64>(); P.slots = slots; P.n_parts = n_parts; P.part = part;
     u64 grid = (u64)ctx->n_sm * DB_BLOCKS;
     if (grid > n_tiles) grid = n_tiles;
-    LAUNCH(k_db_count, (unsigned)grid, DT, 0, P);
+    if (grid) LAUNCH(k_db_count, (unsigned)grid, DT, 0, P);
     LAUNCH(k_db_mark, grid_cap(ctx, slots, 256, 16), 256, 0, keys.as<u64>(), slots, bitmap.as<u32>());
   }
   // rank of every SUNK

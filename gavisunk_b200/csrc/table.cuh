@@ -4,7 +4,8 @@
 //   filt      u32[filt_words]   word-blocked Bloom filter, 2 bits per key inside ONE 32-bit word;
 //                               sized to stay L2-resident (<= 64 MiB), probed once per read base
 //   tab_kv    u64[2 tab_slots]  open-addressed canonical k-mers, buckets of 4 slots, load factor <= 0.5, EMPTY =
-//                               all ones (k <= 31 => < 2^62); a bucket is 64 bytes: 4 keys, then their 4 value
+//                               all ones (k <= 31 => < 2^62; at k = 32 the all-T k-mer's
+//                               canonical form is all-A); a bucket is 64 bytes: 4 keys, then their 4 value
 //                               words (low: .loc row or GVS_ROW_MISSING / GVS_ROW_NOTINDB, high: the row's dense
 //                               group index) -- one HBM access per lookup
 //                               (tab_keys u64[tab_slots] / tab_rows u32[tab_slots] only exist while the table is built)

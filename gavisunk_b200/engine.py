@@ -309,6 +309,11 @@ class Engine:
         database is loaded / built; results are identical)."""
         self._ck(self.lib.gvs_set_probe_variant(self.ctx, int(variant)))
 
+    def set_db_passes(self, n: int = 0):
+        """Count passes of build_db / build_db_device: 0 (default) as few as the free device memory allows, 1..64
+        exactly n (the database is the same; call before the build)."""
+        self._ck(self.lib.gvs_set_db_passes(self.ctx, int(n)))
+
     def set_host_pack(self, mode: int = 1, threads: int = 0):
         """How the segments of a pipelined ASCII host batch travel: as they are (PACK_OFF), 2-bit packed by
         `threads` host threads (PACK_ALL), or whichever keeps both the PCIe link and the cores busy

@@ -109,7 +109,8 @@ int gvs_db_load_loc(gvs_ctx* ctx, const uint64_t* db_kmer, uint64_t n_db,
  * assembly that occur exactly once, their location and the start of their merged
  * (overlapping-or-book-ended) run.  seq = concatenated contig sequences (ASCII, any case, non-ACGT
  * breaks windows), contig_off[n_contigs+1] = offsets into seq.  `seq_on_device` != 0: both
- * pointers are device memory. */
+ * pointers are device memory.  Any k from 1 to 32; contigs that are empty or shorter than k contribute no
+ * window, and an assembly without a SUNK gives an empty database (gvs_db_size 0, 0). */
 int gvs_db_build(gvs_ctx* ctx, const uint8_t* seq, const uint64_t* contig_off, uint32_t n_contigs,
                  int seq_on_device);
 
@@ -119,6 +120,13 @@ int gvs_db_build(gvs_ctx* ctx, const uint8_t* seq, const uint64_t* contig_off, u
  * -- results are identical; tests force either one on the golden cases.  Takes effect at the next
  * gvs_db_load_loc / gvs_db_build (the filter layout is part of the database). */
 int gvs_set_probe_variant(gvs_ctx* ctx, int variant);
+
+/* gvs_db_build hash-partitions the canonical k-mers into n passes over the assembly, each with its own count table
+ * of (total / n) * 3/2 + 1024 slots.  n = 0 (default): the fewest passes whose table fits 70 % of the free device
+ * memory (by that formula two for a 2 x 3.1 Gbp diploid assembly on a 180 GB GPU); n = 1..64: exactly n passes,
+ * whatever the memory (GVS_E_NOMEM if the table does not fit).  The database does not depend on n; tests force it
+ * to reach the multi-pass build on small assemblies.  Takes effect at the next gvs_db_build. */
+int gvs_set_db_passes(gvs_ctx* ctx, int n);
 
 int gvs_db_size(gvs_ctx* ctx, uint64_t* n_sunks, uint64_t* n_groups);
 /* kmer.loc rows in file order ((contig, start) order for a built database): host buffers of
