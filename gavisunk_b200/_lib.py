@@ -89,6 +89,10 @@ PROTOTYPES = {
     "gvs_sunk_depth_get": (C.c_int, [vp] * 4),
     "gvs_depth_runs": (C.c_int, [vp, vp, u64p]),
     "gvs_depth_runs_get": (C.c_int, [vp] * 7),
+    "gvs_allele_support": (C.c_int, [vp, C.c_int, C.POINTER(vp)]),
+    "gvs_allele_support_get": (C.c_int, [vp] * 5),
+    "gvs_allele_runs": (C.c_int, [vp, vp, u64p]),
+    "gvs_allele_runs_get": (C.c_int, [vp] * 6),
     "gvs_covprob_table": (C.c_int, [vp, vp, vp, C.c_uint32, C.c_double, C.c_double, vp]),
     "gvs_covprob_gaps": (C.c_int, [vp, vp, vp, C.c_uint64, vp, vp, vp, C.c_uint64, vp, vp, vp]),
     "gvs_slop": (C.c_int, [vp, vp, vp, vp, C.c_uint64, vp, C.c_uint32, C.c_int64]),
@@ -127,7 +131,8 @@ PROTOTYPES["gvs_format_rows"] = (C.c_int64, [C.POINTER(ColStruct), C.c_uint32, C
 GVS_E_KEYERROR = -3
 STAGES = {"probe": 0, "emit": 1, "diag": 2, "hist": 3, "validate": 4, "intervals": 5, "dbbuild": 6, "components": 7, "mode": 8,
           "bad": 9, "merge": 10, "support": 11, "evidence": 12, "screen": 13,
-          "junctions": 14, "discordance": 15, "readhaps": 16, "switches": 17, "depth": 18}
+          "junctions": 14, "discordance": 15, "readhaps": 16, "switches": 17, "depth": 18,
+          "alleles": 19}
 
 _lib = None
 

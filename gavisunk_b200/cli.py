@@ -15,7 +15,7 @@
   python -m gavisunk_b200.cli fused --sample S --k K --hap1-asm .. --hap2-asm .. (--hap1-reads f.. --hap2-reads f.. | --reads f..)
                                     --outdir D [--devices 0,1,..] [--batch-files N] [--detailed] [--support-tracks]
                                     [--gap-evidence] [--junctions] [--discordance] [--read-haplotypes] [--inversions]
-                                    [--sunk-depth]
+                                    [--sunk-depth] [--allele-support]
   python -m gavisunk_b200.cli support_tracks <sunkpos> <rlen> <bad_sunks.txt> <fai> <valid.bed> <out.reads.bed> <out.bedgraph> <out.tsv>
   python -m gavisunk_b200.cli gap_evidence <sunkpos> <rlen> <bad_sunks.txt> <fai> <valid.bed> <out.gaps.reads.tsv> <out.gaps.evidence.tsv>
   python -m gavisunk_b200.cli junctions <hapN_detailed.sunkpos> <hapN.rlen> <bad_sunks.txt> <fai1> <fai2> <out.junctions.reads.tsv> <out.junctions.tsv>
@@ -23,6 +23,8 @@
   python -m gavisunk_b200.cli inversions <sunkpos> <rlen> <bad_sunks.txt> <fai> <out.inversions.reads.tsv> <out.inversions.bed>
   python -m gavisunk_b200.cli sunk_depth <kmer.loc> <fai1> <fai2> <bad_sunks.txt> <hap1_detailed.sunkpos> <hap2_detailed.sunkpos>
                                          <hap1.sunkpos> <hap2.sunkpos> <hapN> <out.depth.bedgraph> <out.depth.bed> <out.depth.tsv>
+  python -m gavisunk_b200.cli allele_support <kmer.loc> <fai1> <fai2> <hap1_detailed.sunkpos> <hap2_detailed.sunkpos> <hapN>
+                                             <out.alleles.bedgraph> <out.alleles.bed> <out.alleles.tsv> <out.alleles.classes.tsv>
 
 The first four replace workflow/scripts/{kmerpos_annot3,rlen,diag_filter_v3,diag_filter_step2}
 (workflow/rules/tagONT.smk:36,73,92,110) one to one; the next six replace badsunks_AR.py,
@@ -45,6 +47,8 @@ reference needs the reads binned by haplotype).
 inversion calls (no reference counterpart: the validation takes each read's orientation majority).
 `fused --sunk-depth` and `sunk_depth` report the SUNK hits and reads of every group over all match rows, and call them into
 collapsed and depleted stretches (no reference counterpart: the bad-SUNK filter removes collapsed groups).
+`fused --allele-support` and `allele_support` report, per SUNK group, the reads of its own and of the other haplotype that
+carry it, and call them into phase flips, switched blocks and consensus errors (no reference counterpart).
 Text parsing / formatting is host
 plumbing; all per-base and per-row work runs in libgavisunk_b200.so.  Errors exit non-zero with a
 message on stderr and never leave a partial output file behind.
@@ -892,6 +896,154 @@ def cmd_sunk_depth(argv):
 
 
 # ------------------------------------------------------------------------------------------------
+# allele support: the reads of each group's own and other haplotype (no reference counterpart; DESIGN.md section 5.5h)
+# ------------------------------------------------------------------------------------------------
+ALLELE_TSV_HEADER = ("contig\tgroups\tassessed\tflipped\tflips\tswitches\terrors\terror_eligible\tshared\thamming_ppm\t"
+                     "switch_ppm\n")
+ALLELE_CLASSES_HEADER = "class\tmin_sunks\tmax_sunks\tgroups\town_groups\tbaseline\tfallback\n"
+
+
+def allele_calls(g_contig, g_start, g_end, own, other, sunks, hap_contigs, min_reads=3, flip_permille=200, min_baseline=10,
+                 max_gap_groups=2, min_switch_groups=3, min_class_groups=DEPTH_MIN_CLASS_GROUPS):
+    """Phase flips, switched blocks and consensus errors of one haplotype from the per-group allele support
+    (Engine.alleles(): g_contig / g_start = the group table, g_end, own, other, sunks), exact integer arithmetic.
+    hap_contigs = the haplotype's contig ids in .fai order.  Per group, with t = own + other:
+      assessed     t >= min_reads;
+      flipped      other >= min_reads and 1000*own <= flip_permille*t;
+      shared       own >= min_reads, other >= min_reads, not flipped;
+      eligible     the baseline B of its size class (depth_baselines over own: the lower median of own over the class's
+                   groups with an own read, with the same fallback) is >= min_baseline;
+      unsupported  t == 0, eligible, and the nearest group on each side on the contig (start order) assessed.
+    Per contig, flipped groups in start order chain when at most max_gap_groups assessed, non-flipped groups lie between
+    them; a chain of >= min_switch_groups is one `switch` call, each group of a shorter one a `flip` call.  Each unsupported
+    group is an `error` call.  A call spans its first marked group's start to its last marked group's end; groups = the
+    groups from the first to the last marked one, marked = its flipped / unsupported groups, own / other summed over them.
+    -> (calls sorted by (contig in .fai order, start, end, kind): tuples (contig, start, end, kind, groups, marked, own,
+    other); per contig of hap_contigs (groups, assessed, flipped, flips, switches, errors, error_eligible, shared);
+    depth_baselines of own)"""
+    g_contig = np.asarray(g_contig, np.int64)
+    g_start = np.asarray(g_start, np.int64)
+    g_end = np.asarray(g_end, np.int64)
+    hap_contigs = np.asarray(hap_contigs, np.int64)
+    fai_pos = np.full(int(max(g_contig.max(initial=-1), hap_contigs.max(initial=-1))) + 1, -1, np.int64)
+    fai_pos[hap_contigs] = np.arange(len(hap_contigs))
+    sel = np.flatnonzero(fai_pos[g_contig] >= 0)
+    cls = depth_classes(sunks)
+    base = depth_baselines(own, cls, sel, min_class_groups)
+    order = sel[np.lexsort((g_start[sel], fai_pos[g_contig[sel]]))]
+    B = np.asarray([-1 if b[2] is None else b[2] for b in base], np.int64)[cls[order]]
+    o = np.asarray(own, np.int64)[order]
+    t = o + np.asarray(other, np.int64)[order]
+    ot = t - o
+    c = g_contig[order]
+    assessed = t >= min_reads
+    flipped = (ot >= min_reads) & (1000 * o <= flip_permille * t)
+    shared = (o >= min_reads) & (ot >= min_reads) & ~flipped
+    eligible = B >= min_baseline
+    first = np.ones(len(order), bool)
+    first[1:] = c[1:] != c[:-1]
+    last = np.ones(len(order), bool)
+    last[:-1] = c[1:] != c[:-1]
+    left = np.zeros(len(order), bool)
+    left[1:] = assessed[:-1]
+    right = np.zeros(len(order), bool)
+    right[:-1] = assessed[1:]
+    unsupported = (t == 0) & eligible & left & ~first & right & ~last
+    calls = []
+    span = lambda a, b, kind, m: (int(c[a]), int(g_start[order[a]]), int(g_end[order[b]]), kind, b - a + 1, len(m), int(o[m].sum()),
+                                  int(ot[m].sum()))
+    f = np.flatnonzero(flipped)
+    between = np.cumsum(assessed & ~flipped)  # assessed, non-flipped groups up to each position
+    head = np.ones(len(f), bool)
+    head[1:] = (c[f[1:]] != c[f[:-1]]) | (between[f[1:]] - between[f[:-1]] > max_gap_groups)
+    heads = np.flatnonzero(head)
+    for a, b in zip(heads.tolist(), np.append(heads[1:], len(f)).tolist()):
+        m = f[a:b]
+        if len(m) >= min_switch_groups:
+            calls.append(span(int(m[0]), int(m[-1]), "switch", m))
+        else:
+            calls += [span(int(i), int(i), "flip", m[k:k + 1]) for k, i in enumerate(m.tolist())]
+    calls += [span(i, i, "error", np.array([i])) for i in np.flatnonzero(unsupported).tolist()]
+    calls.sort(key=lambda x: (int(fai_pos[x[0]]), x[1], x[2], x[3]))
+    per = {int(ci): [0] * 8 for ci in hap_contigs}
+    for ci in np.unique(c).tolist():
+        m = c == ci
+        per[ci][:3] = [int(m.sum()), int(assessed[m].sum()), int(flipped[m].sum())]
+        per[ci][6:] = [int(eligible[m].sum()), int(shared[m].sum())]
+    for x in calls:
+        per[x[0]][3 + ("flip", "switch", "error").index(x[3])] += 1
+    return calls, [tuple(per[int(ci)]) for ci in hap_contigs], base
+
+
+def allele_texts(hap_contigs, names, contig_len, groups, al, runs, **kw):
+    """The four allele-support files of one haplotype: hap_contigs = its contig ids in .fai order; groups = Engine.groups(),
+    al = Engine.alleles(), runs = Engine.allele_runs(); kw: the thresholds of allele_calls.  -> (alleles.bedgraph: the runs
+    of its contigs; alleles.bed: the calls; alleles.tsv: the per-contig summary and a `*` total line; alleles.classes.tsv:
+    the baseline of own of every size class) bytes"""
+    ctab = gio.NameTable(names)
+    inhap = np.zeros(len(names), bool)
+    inhap[np.asarray(hap_contigs, np.int64)] = True
+    bedgraph = gio.format_rows([("name", runs["contig"], ctab)] + [("u32", runs[c]) for c in ("start", "end", "own", "other")],
+                               sel=np.flatnonzero(inhap[runs["contig"]]))
+    calls, per, base = allele_calls(groups["contig"], groups["group"], al["end"], al["own"], al["other"], al["sunks"], hap_contigs, **kw)
+    bed = "".join(f"{names[c]}\t{a}\t{b}\t{kind}\t{ng}\t{nm}\t{o}\t{t}\n" for c, a, b, kind, ng, nm, o, t in calls)
+    ppm = lambda x, n: str(10 ** 6 * x // n) if n else "."
+    tsv = [ALLELE_TSV_HEADER]
+    for name, v in [(names[c], v) for c, v in zip(hap_contigs, per)] + [("*", tuple(map(sum, zip((0,) * 8, *per))))]:
+        tsv.append("\t".join([name] + [str(x) for x in v] + [ppm(v[2], v[1]), ppm(2 * v[4], v[1])]) + "\n")
+    classes = [ALLELE_CLASSES_HEADER]
+    for q, (n, nh, b, fb) in enumerate(base):
+        classes.append(f"{q}\t{1 << q}\t{(2 << q) - 1 if q + 1 < DEPTH_CLASSES else '.'}\t{n}\t{nh}\t{'.' if b is None else b}\t"
+                       f"{'.' if b is None else int(fb)}\n")
+    return bedgraph, bed.encode("latin-1"), "".join(tsv).encode("latin-1"), "".join(classes).encode("latin-1")
+
+
+def allele_support(loc_p, fai1_p, fai2_p, detailed1_p, detailed2_p, hap, out_bedgraph, out_bed, out_tsv, out_classes):
+    """Allele support of haplotype `hap` (hap1 / hap2) from the files of the per-rule path: the group table, the SUNKs and
+    ends of each group from mrsfast/kmer.loc (identical rows, as mrsfast writes a palindromic SUNK, taken once); own and
+    other from both {hap}_detailed.sunkpos (combine_ont_nofilt: every match row; a read is a run of consecutive rows with
+    one name, diag_filter_v3.nim:64), the file that holds a read giving its haplotype; contigs in fai1-then-fai2 order."""
+    h = {"hap1": 0, "hap2": 1, "1": 0, "2": 1}.get(str(hap))
+    if h is None:
+        raise ValueError(f"haplotype {hap!r} is not hap1 or hap2")
+    fai = [gio.read_fai(fai1_p), gio.read_fai(fai2_p)]
+    names = [n for f in fai for n, _ in f]
+    clen = [l for f in fai for _, l in f]
+    cidx = {}
+    for i, n in enumerate(names):
+        cidx.setdefault(n, i)
+    loc = list(dict.fromkeys(zip(*gio.read_loc(loc_p))))
+    for c, _, _, _ in loc:
+        if c not in cidx:
+            raise KeyError(f"contig {c} of {loc_p} is in neither {fai1_p} nor {fai2_p}")
+    cols, first = [], [0]
+    for path in (detailed1_p, detailed2_p):
+        _, cnames, rnames, c = _rows_from_sunkpos(path)
+        for n in cnames:
+            if n not in cidx:
+                raise KeyError(f"contig {n} of {path} is in neither {fai1_p} nor {fai2_p}")
+        remap = np.asarray([cidx[n] for n in cnames] + [0], np.uint32)
+        cols.append((c[0] + np.uint32(first[-1]), c[1], remap[c[2]], c[3], c[4]))
+        first.append(first[-1] + len(rnames))
+    kmers = [km.encode() for _, _, km, _ in loc]
+    eng = Engine(len(kmers[0]) if kmers and 1 <= len(kmers[0]) <= 32 else 20)
+    km = encode_kmers(kmers)
+    eng.load_loc(km, km, [cidx[c] for c, _, _, _ in loc], [s for _, s, _, _ in loc], [g for _, _, _, g in loc], names)
+    n_reads = max(1, first[-1])  # the reads of file 1 form chunk 0 (haplotype 0), those of file 2 chunk 1 (haplotype 1)
+    eng.set_reads_meta(np.zeros(n_reads, np.uint32), [0, first[1], n_reads], [0, 1])
+    eng.set_rows(0, *[np.concatenate([t[j] for t in cols]) for j in range(5)])
+    chap = np.asarray([0] * len(fai[0]) + [1] * len(fai[1]))
+    eng.set_contigs(chap)
+    eng.allele_support()
+    texts = allele_texts(np.flatnonzero(chap == h).tolist(), names, clen, eng.groups(), eng.alleles(), eng.allele_runs(clen))
+    _write_all((out_bedgraph, out_bed, out_tsv, out_classes), texts)
+
+
+def cmd_allele_support(argv):
+    allele_support(*argv)
+
+
+# ------------------------------------------------------------------------------------------------
 # read haplotypes: every read's SUNK vote on both haplotypes (no reference counterpart; DESIGN.md section 5.5e)
 # ------------------------------------------------------------------------------------------------
 READ_HAP_READS_HEADER = "read\tread_len\tbin\tcontig1\tn1\tstrand1\tcontig2\tn2\tstrand2\thap\n"
@@ -1220,6 +1372,10 @@ EVIDENCE_PRODUCTS = {
     "sunk_depth": Evidence("--sunk-depth", "also write final_out/hap{N}.depth.bedgraph, .depth.bed and .depth.tsv (SUNK hits and "
                            "reads of every group over all match rows, and collapsed and depleted stretches)", None, (),
                            ("depth.bedgraph", "depth.bed", "depth.tsv")),
+    "allele_support": Evidence("--allele-support", "also write final_out/hap{N}.alleles.bedgraph, .alleles.bed, .alleles.tsv and "
+                               ".alleles.classes.tsv (the reads of each SUNK group's own and other haplotype, and phase flips, "
+                               "switched blocks and consensus errors)", None, (),
+                               ("alleles.bedgraph", "alleles.bed", "alleles.tsv", "alleles.classes.tsv")),
 }
 
 
@@ -1274,9 +1430,11 @@ def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int]
     support's; read_haplotypes: every engine's diag filters in haplotype mode and the records of its own reads (file_hap
     GVS_HAP_ANY: unbinned chunks, always filtered in haplotype mode); inversions: the strand-switch records of every
     engine's own reads, from its kept rows and the run's bad groups; sunk_depth: every batch's match rows counted per group
-    and the per-group counts and runs, with the counts summed across engines like the support's.  -> one result dict per
-    engine (read names / lengths / chunk tables, kept rows, validated pairs, intervals[, placements, support runs][, gap
-    evidence][, junctions][, spans, discordance runs][, read haplotypes][, strand switches][, depth, depth runs])."""
+    and the per-group counts and runs, with the counts summed across engines like the support's; allele_support: every
+    batch's match rows counted per group by read haplotype after its diag filter, and the per-group counts and runs,
+    summed likewise.  -> one result dict per engine (read names / lengths / chunk tables, kept rows, validated pairs,
+    intervals[, placements, support runs][, gap evidence][, junctions][, spans, discordance runs][, read haplotypes][,
+    strand switches][, depth, depth runs][, alleles, allele runs])."""
     import threading
     from concurrent.futures import ThreadPoolExecutor
     for p in files:
@@ -1332,7 +1490,8 @@ def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int]
                 iv, bases = eng.run_batches([bind_for(bi) for bi in range(len(mine))], contig_hap, min_read_len=min_read_len,
                                             allreduce_hist=cx.allreduce_hist, gather_forests=cx.gather_forests, on_batch=on_batch,
                                             junctions="junctions" in products, read_haps="read_haplotypes" in products,
-                                            sunk_depth="sunk_depth" in products)
+                                            sunk_depth="sunk_depth" in products,
+                                            allele_support="allele_support" in products)
                 for old in held:
                     old.close()
             info.update(kept=eng.rows(1, pinned=True), pairs=eng.pairs(pinned=True), iv=iv)
@@ -1351,6 +1510,8 @@ def run_reads(engines, contig_hap, files: Sequence[str], file_hap: Sequence[int]
                 info.update(switches=eng.strand_switches(min_read_len))
             if "sunk_depth" in products:
                 info.update(depth=eng.depth(allreduce=cx.allreduce_hist), depth_runs=eng.depth_runs(contig_len))
+            if "allele_support" in products:
+                info.update(alleles=eng.alleles(allreduce=cx.allreduce_hist), allele_runs=eng.allele_runs(contig_len))
             results[di] = info
         except BaseException as ex:  # noqa: BLE001 -- reported by the caller; peers must not wait for this rank
             errors.append(ex)
@@ -1567,7 +1728,8 @@ def write_outputs(k, eng, results, contig_len, contig_hap, names, iv, gaps, noda
             discordance=lambda r: discordance_texts(hap_contigs, names, r, results[0]["discordance"], *reads),
             read_haplotypes=lambda r: read_hap_texts(hap, names, chap, r, read_bin, read_hap, *reads),
             inversions=lambda r: inversion_texts(hap_contigs, names, r, *reads),
-            sunk_depth=lambda r: depth_texts(hap_contigs, names, clen, gtab, results[0]["depth"], results[0]["depth_runs"], bad))
+            sunk_depth=lambda r: depth_texts(hap_contigs, names, clen, gtab, results[0]["depth"], results[0]["depth_runs"], bad),
+            allele_support=lambda r: allele_texts(hap_contigs, names, clen, gtab, results[0]["alleles"], results[0]["allele_runs"]))
         for p in products:
             _write_all([d("final_out", f"hap{hn}.{ext}") for ext in EVIDENCE_PRODUCTS[p].suffixes], texts[p](rec[p]))
     from concurrent.futures import ThreadPoolExecutor
@@ -1618,7 +1780,7 @@ COMMANDS = {"kmerpos_annot3": (cmd_kmerpos_annot3, 4), "rlen": (cmd_rlen, 2), "d
             "split_ont": (cmd_split_ont, None), "combine_ont_nofilt": (cmd_combine_ont_nofilt, None),
             "support_tracks": (cmd_support_tracks, 8), "gap_evidence": (cmd_gap_evidence, 7),
             "junctions": (cmd_junctions, 7), "discordance": (cmd_discordance, 7), "inversions": (cmd_inversions, 6),
-            "sunk_depth": (cmd_sunk_depth, 12)}
+            "sunk_depth": (cmd_sunk_depth, 12), "allele_support": (cmd_allele_support, 10)}
 
 
 def main(argv=None):

@@ -90,6 +90,7 @@ extern "C" int gvs_batches_begin(gvs_ctx* ctx) {
   ctx->rh_run.n = 0;
   ctx->rh_run.ready = false;
   ctx->dp_ready = false;  // the next gvs_sunk_depth(accumulate = 1) starts from zero (depth.cu)
+  ctx->al_ready = false;  // ... and gvs_allele_support(accumulate = 1) (alleles.cu)
   return 0;
 }
 

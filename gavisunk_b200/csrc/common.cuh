@@ -216,6 +216,16 @@ struct gvs_ctx {
   bool dp_ready = false;
   RecTable dp_runs;                 // runs of gvs_depth_runs: contig, start, end, hits, reads, kept
 
+  // ---- allele support (alleles.cu) ----
+  DevBuf al_cnt;                    // int32[2][n_groups] by group index: own, other (summed over the batches of a run)
+  DevBuf al_hap;                    // u8 per read of the batch: its file haplotype
+  DevBuf al_seg_start, al_row_seg, al_scr;  // segments of the match rows; per match row scratch of the non-monotone reads
+  DevBuf al_sunks, al_end;          // u32[n_groups]: .loc rows per group, last SUNK start + k
+  DevBuf al_diff;                   // int32[2][n_groups] by rank: differences of own, other
+  u64 al_gen = 0, al_loc_gen = ~0ull;  // grp_gen al_cnt / al_sunks and al_end were counted for
+  bool al_ready = false;
+  RecTable al_runs;                 // runs of gvs_allele_runs: contig, start, end, own, other
+
   // ---- components / intervals / gaps ----
   DevBuf parent, present, comp_min, comp_max, comp_cnt;
   DevBuf comp_rank;  // unsorted group tables only: [smallest member rank per root | root per interval rank]
@@ -659,6 +669,16 @@ __device__ __forceinline__ bool warp_first_in(const u32* idx, u32 a, u32 i, In i
     if (id(j) == g) return false;
   }
   return true;
+}
+
+// the chunk of a read: the last chunk whose first read is at or below it (the diag filter, the allele support)
+__device__ __forceinline__ u32 chunk_of_read(const u64* __restrict__ chunk_first, u32 n_chunks, u32 read) {
+  u32 lo = 0, hi = n_chunks;
+  while (hi - lo > 1) {
+    u32 mid = (lo + hi) >> 1;
+    if (chunk_first[mid] <= read) lo = mid; else hi = mid;
+  }
+  return lo;
 }
 
 // Order the n keys key(x[k]) ascending into y: a copy or a reversal when they are strictly monotone (a one-strand read),

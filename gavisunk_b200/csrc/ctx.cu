@@ -181,7 +181,9 @@ extern "C" void gvs_destroy(gvs_ctx* c) {
                    &c->jn_seg_start, &c->jn_row_seg, &c->jn_seg_cnt, &c->jn_flags, &c->jn_scr, &c->dc_diff, &c->dc_scr, &c->dc_seg,
                    &c->pl.buf, &c->sup.buf, &c->ge.buf, &c->jn.buf, &c->dc.buf, &c->dc_runs.buf, &c->rh_scratch, &c->rh.buf,
                    &c->rh_run.buf, &c->sw_seg_start, &c->sw_scr, &c->sw_seg, &c->sw.buf, &c->dp_cnt, &c->dp_seg_start, &c->dp_row_seg,
-                   &c->dp_scr, &c->dp_sunks, &c->dp_diff, &c->dp_runs.buf};
+                   &c->dp_scr, &c->dp_sunks, &c->dp_diff, &c->dp_runs.buf, &c->al_cnt,
+                   &c->al_hap, &c->al_seg_start, &c->al_row_seg, &c->al_scr, &c->al_sunks, &c->al_end, &c->al_diff,
+                   &c->al_runs.buf};
   for (DevBuf* b : all) gvs_release(*b);
   release_rows(c->rows);
   release_rows(c->kept);

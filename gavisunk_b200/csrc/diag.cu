@@ -45,15 +45,6 @@ int gvs_build_segments(gvs_ctx* ctx, const u32* read, u64 n, DevBuf& seg_start, 
   return 0;
 }
 
-__device__ __forceinline__ u32 chunk_of_read(const u64* __restrict__ chunk_first, u32 n_chunks, u32 read) {
-  u32 lo = 0, hi = n_chunks;
-  while (hi - lo > 1) {
-    u32 mid = (lo + hi) >> 1;
-    if (chunk_first[mid] <= read) lo = mid; else hi = mid;
-  }
-  return lo;
-}
-
 __global__ void __launch_bounds__(256) k_seg_info(const u32* __restrict__ read, const u32* __restrict__ seg_start, u32 n_seg,
                                                   const u64* __restrict__ chunk_first, const u8* __restrict__ chunk_hap,
                                                   u32 n_chunks, u32* seg_chunk, u8* seg_hap, u32* seg_ndist) {

@@ -463,7 +463,7 @@ class Engine:
 
     def run_batches(self, binds, contig_hap: Sequence[int], min_read_len: int = 10000, allreduce_hist=None,
                     gather_forests=None, on_batch=None, junctions: bool = False, read_haps: bool = False,
-                    sunk_depth: bool = False):
+                    sunk_depth: bool = False, allele_support: bool = False):
         """The hot path over a run whose reads come in several batches (a sample's chunk files, or the shard of
         them this GPU owns).  The reference gathers all chunks of a haplotype before the global stages
         (workflow/Snakefile:23-24, workflow/rules/tagONT.smk:112-131; badsunks_AR.py:20-27 counts over every
@@ -478,6 +478,8 @@ class Engine:
         so that junctions() reports the run's records afterwards.  read_haps: run every diag filter in haplotype mode,
         so that read_haps() reports the run's records afterwards (batches with GVS_HAP_ANY chunks always are).  sunk_depth:
         also count every batch's match rows (sunk_depth, accumulated), so that depth() reports the run's SUNK hit depth.
+        allele_support: also count every batch's match rows by read haplotype after its diag filter (allele_support,
+        accumulated; unbinned reads take the haplotype that filter assigns), so that alleles() reports the run's counts.
         Returns (intervals, [read_base of every batch])."""
         self.batches_begin()
         bases, hp = [], 0
@@ -488,6 +490,8 @@ class Engine:
             if sunk_depth:
                 self.sunk_depth(accumulate=True)
             best += self.diag_filter(contig_hap, read_haps)[0]
+            if allele_support:
+                self.allele_support(accumulate=True)
             if junctions:
                 self.junction_screen(min_read_len)
             hp = self.group_hist(accumulate=True)
@@ -497,11 +501,13 @@ class Engine:
             bases.append(base)
         self.batches_bind()
         self.n_rows, self.n_best = rows, best
-        if not bases:  # a rank without a batch still takes part in both exchanges (and in depth()'s)
+        if not bases:  # a rank without a batch still takes part in both exchanges (and in depth()'s and alleles()')
             self.set_contigs(contig_hap)
             hp = self.group_hist(accumulate=True)
             if sunk_depth:
                 self.sunk_depth(accumulate=True)
+            if allele_support:
+                self.allele_support(accumulate=True)
         return self._global_stages(hp, min_read_len, allreduce_hist, gather_forests), bases
 
     def db_groups(self) -> int:
@@ -646,6 +652,38 @@ class Engine:
         """SUNK hit depth runs after sunk_depth() (and depth()'s all-reduce) and group_hist(): (contig, start, end, hits,
         reads, kept) tiling every contig in segment space."""
         return self._runs("depth_runs", self.lib.gvs_depth_runs, self.lib.gvs_depth_runs_get, self.DEPTH_COLUMNS, "_dp_ptr",
+                          contig_len, None)
+
+    def allele_support(self, accumulate: bool = False) -> int:
+        """Allele support of the current match rows (after match() or set_rows(0), and after the diag filter of a batch
+        with unbinned chunks; no reference counterpart; include/gavisunk_b200.h gvs_allele_support): adds every distinct
+        (read, group) to own[g] when the read's file haplotype is the group's, else to other[g].  accumulate: add to the
+        previous counts (run_batches starts from zero at its batches_begin).  Returns the device pointer of the
+        int32[2][n_groups] array."""
+        p = C.c_void_p()
+        self._ck(self.lib.gvs_allele_support(self.ctx, 1 if accumulate else 0, C.byref(p)))
+        self._al_ptr = int(p.value or 0)
+        self._al_summed = False
+        return self._al_ptr
+
+    def alleles(self, allreduce=None) -> Dict[str, np.ndarray]:
+        """Per group index (the table of groups()): own, other (int32, of allele_support), sunks (.loc rows) and end (last
+        SUNK start + k).  With several GPUs `allreduce(ptr, n)` sums own and other (n = 2 * n_groups) across ranks in place
+        first (the callable that sums the bad-SUNK histogram), once per allele_support(): a later call reads the counts
+        summed already."""
+        ng = self._n_groups()
+        if allreduce is not None and not getattr(self, "_al_summed", False):
+            allreduce(self._al_ptr, 2 * ng)
+            self._al_summed = True
+        return self._table("alleles", self.lib.gvs_allele_support_get, ng, ("own", "other", "sunks", "end"),
+                           dtypes=dict(own=np.int32, other=np.int32))
+
+    ALLELE_COLUMNS = ("contig", "start", "end", "own", "other")
+
+    def allele_runs(self, contig_len: Sequence[int]) -> Dict[str, np.ndarray]:
+        """Allele support runs after allele_support() (and alleles()' all-reduce): (contig, start, end, own, other) tiling
+        every contig in segment space."""
+        return self._runs("allele_runs", self.lib.gvs_allele_runs, self.lib.gvs_allele_runs_get, self.ALLELE_COLUMNS, "_al_ptr",
                           contig_len, None)
 
     def components_local(self) -> int:

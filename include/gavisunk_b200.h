@@ -64,7 +64,8 @@ enum {
   GVS_ST_READHAPS = 16, /* haplotype mode of the diag filter (gvs_diag_filter_haps): votes per haplotype, records */
   GVS_ST_SWITCHES = 17, /* strand switches inside a contig (gvs_strand_switches): no reference counterpart       */
   GVS_ST_DEPTH = 18,    /* SUNK hit depth (gvs_sunk_depth, gvs_depth_runs): no reference counterpart                */
-  GVS_ST_COUNT = 19
+  GVS_ST_ALLELES = 19,  /* allele support (gvs_allele_support, gvs_allele_runs): no reference counterpart          */
+  GVS_ST_COUNT = 20
 };
 
 /* ------------------------------------------------------------------------------------------ */
@@ -536,6 +537,37 @@ int gvs_sunk_depth_get(gvs_ctx* ctx, int32_t* hits, int32_t* reads, uint32_t* su
 int gvs_depth_runs(gvs_ctx* ctx, const uint32_t* contig_len, uint64_t* n_runs);
 int gvs_depth_runs_get(gvs_ctx* ctx, uint32_t* contig, uint32_t* start, uint32_t* end, uint32_t* hits, uint32_t* reads,
                        uint32_t* kept);
+
+/* Allele support: whether the reads of each SUNK group's own haplotype carry it, the other haplotype's reads carry it,
+ * or no read does.  No reference counterpart.  At a heterozygous site the haplotypes' k-mers differ, so each haplotype
+ * has a group of its own there that only its reads should carry.
+ * Read haplotype hap(r): the file haplotype of read r (the haplotype whose sunkpos/ files hold it, cli.file_haps): the
+ * chunk's haplotype for a binned chunk; for a GVS_HAP_ANY chunk the haplotype its votes assign (the records of the
+ * batch's diag filter in haplotype mode), and for a tie or a read without a vote the parity of its run-wide read index
+ * (even: haplotype 0), as gvs_batch_stash numbers the batch's reads.
+ * Per group index g (the group table of gvs_db_export / gvs_groups_get), with H = contig_hap[grp_contig[g]]:
+ *   own[g]    the distinct reads r with a match row of group g and hap(r) == H;
+ *   other[g]  the same with hap(r) == 1 - H;
+ * over the match rows of gvs_match / gvs_rows_set(0): every contig of both haplotypes, before the diag filter, no
+ * read-length minimum, no bad-group filter (the rows gvs_sunk_depth counts).  A group on a contig of neither haplotype
+ * counts nothing; for the others own + other equals reads of gvs_sunk_depth.
+ *   sunks[g]  the .loc rows of group g;  end[g]  its last SUNK's start + k (group start + k without .loc rows).
+ * gvs_allele_support adds the current match rows (none after gvs_batches_bind or before any gvs_match) to an
+ * int32[2][n_groups] array -- own at [g], other at [n_groups + g] -- whose device pointer *support_dev receives.  Inside
+ * a batches run it accumulates from gvs_batches_begin on (accumulate != 0); accumulate = 0 replaces.  Call it between a
+ * batch's diag filter and its gvs_batch_stash (the parity uses the index the stash will give).  GVS_E_STATE before a
+ * group table or contig haplotypes, and on match rows of a batch with GVS_HAP_ANY chunks whose diag filter has not run.
+ * Several GPUs sum the 2*n_groups entries (as the histogram of gvs_group_hist; a read lives on one GPU, so the sums are
+ * exact) before gvs_allele_support_get / gvs_allele_runs.
+ * gvs_allele_support_get: host buffers of n_groups entries, any pointer may be NULL.
+ * gvs_allele_runs: per base x, the (own, other) of x's segment [ID_r, ID_r+1) as runs (contig, start, end, own, other)
+ * that tile [0, contig_len[c]) of every contig in (contig, start) order, maximal, with a zero head run before a contig's
+ * first group.  GVS_E_STATE before gvs_allele_support or after the group table changed.
+ * The calls (phase flips, switched blocks, consensus errors) are the caller's: DESIGN.md section 5.5h. */
+int gvs_allele_support(gvs_ctx* ctx, int accumulate, int32_t** support_dev);
+int gvs_allele_support_get(gvs_ctx* ctx, int32_t* own, int32_t* other, uint32_t* sunks, uint32_t* end);
+int gvs_allele_runs(gvs_ctx* ctx, const uint32_t* contig_len, uint64_t* n_runs);
+int gvs_allele_runs_get(gvs_ctx* ctx, uint32_t* contig, uint32_t* start, uint32_t* end, uint32_t* own, uint32_t* other);
 
 /* covprob.py:56-100: table[0..3499] of gap-spanning probabilities from the read-length
  * histogram.  kbp[n_bins], cnt[n_bins] = distinct int(len/1000) values and their multiplicities
